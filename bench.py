@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the CTC hot path (BASELINE.json metric: CTC fwd+bwd utterances/s & HBM GB/s % peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c2] [--dump-outputs DIR]
 
 One "step" = one forward+backward pass of CTCLoss(reduce=True, size_average=True,
 after_logsoftmax=False) over one synthetic batch of the named workload (default BASELINE
@@ -382,8 +382,10 @@ def timed_replays(steps_fn, n_steps, bk, dev, barrier, flush_buf, after=None):
     return sum(a.elapsed_time(b) for a, b in pairs)
 
 
-def measure_bucket(bk, dev, world, steps, warmup, barrier, flush_buf, with_autograd=True, profile_steps=20):
-    """value / per-kernel times of one workload on this rank's bucket (max over ranks is taken by the caller)."""
+def measure_bucket(bk, dev, world, steps, warmup, barrier, flush_buf, with_autograd=True, profile_steps=20,
+                   keep_outputs=False):
+    """value / per-kernel times of one workload on this rank's bucket (max over ranks is taken by the caller).
+    keep_outputs: also return, copied to the host, the (loss, grad) the last timed replay produced."""
     import torch
     from end2end_b200 import CTCLoss, _lib
     from end2end_b200.distributed import ShardedCTCLoss
@@ -414,6 +416,9 @@ def measure_bucket(bk, dev, world, steps, warmup, barrier, flush_buf, with_autog
     res["launches"] = _lib.launch_count() - l0
     res["ms"] = ms
     res["loss"] = float(graphs[(steps - 1) % n].loss if hasattr(graphs[0], "loss") else graphs[(steps - 1) % n].total)
+    if keep_outputs:
+        last = graphs[(steps - 1) % n]
+        res["outputs"] = ((last.loss if hasattr(last, "loss") else last.total).cpu(), last.grad.cpu())
     if with_autograd:
         leaves = [x.detach().requires_grad_() for x in bk.x]
 
@@ -441,6 +446,32 @@ def measure_bucket(bk, dev, world, steps, warmup, barrier, flush_buf, with_autog
     res["crit"] = crit
     del graphs
     return res
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(dirname, loss, grad, rank, world):
+    """Write what the last timed step returned to its caller -- the reduced loss and d loss / d logits -- as
+    <dirname>/loss.npy and grad.npy (float32; float64 for float64 logits), so that two builds can be compared on the
+    same seeded inputs.  A gradient larger than the budget (64 MB over all ranks) is cut to a seeded sample of whole
+    utterances, whose batch indices go to grad_utterances.npy.  Under torchrun every rank writes its bucket's
+    outputs with a _rank<r> suffix."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    out_dtype = torch.float64 if grad.dtype == torch.float64 else torch.float32
+    row_bytes = grad[0].numel() * (8 if out_dtype == torch.float64 else 4)
+    keep = max(1, (DUMP_BYTES // world - 4096) // (row_bytes + 8))     # 4 kB: .npy headers and the loss
+    arrays = {"loss": loss.to(out_dtype)}
+    if grad.size(0) > keep:
+        idx = torch.randperm(grad.size(0), generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        grad = grad[idx]
+        arrays["grad_utterances"] = idx.to(torch.float64)
+    arrays["grad"] = grad.to(out_dtype)
+    suffix = "_rank%d" % rank if world > 1 else ""
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + suffix + ".npy"), t.numpy())
 
 
 def roofline_block(bk, res, steps, peak, peak_src, wl):
@@ -512,9 +543,12 @@ def run_ours(args, wl):
     if sampler:
         sampler.wait_first()
     w0 = time.perf_counter()
-    res = measure_bucket(bk, dev, world, args.steps, args.warmup, barrier, flush_buf, with_autograd=False, profile_steps=0)
+    res = measure_bucket(bk, dev, world, args.steps, args.warmup, barrier, flush_buf, with_autograd=False, profile_steps=0,
+                         keep_outputs=bool(args.dump_outputs))
     w1 = time.perf_counter()
     clocks = sampler.summary(w0, w1) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res.pop("outputs"), rank, world)
     ms = max_over_ranks(res["ms"])
     assert res["loss"] == res["loss"] and abs(res["loss"]) != float("inf"), "non-finite loss in the timed region"
     launches = res["launches"]
@@ -753,6 +787,8 @@ def main():
     ap.add_argument("--check", type=int, default=-1, help="utterances per rank compared with the oracle before timing (0: skip)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the per_workload / greedy / strong blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the loss and gradient of the last timed step to DIR/<name>.npy (at most 64 MB)")
     ap.add_argument("--greedy", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--_child", action="store_true", help=argparse.SUPPRESS)
     args = ap.parse_args()

@@ -58,15 +58,6 @@ def build(which=("loss", "decoder"), verbose=False):
              extra_cflags=["-O3", "-DKENLM_MAX_ORDER=6", "-DHAVE_ZLIB", "-DNDEBUG", "-w"],
              extra_ldflags=["-lz"], build_directory=d, verbose=verbose, is_python_module=False)
         built.append(d)
-    # the reference's own unittest files, staged (not committed: oracle/_ref is git-ignored) so that the GPU box
-    # can run them UNMODIFIED against the drop-in pytorch_end2end package (tests/test_reference_suite.py)
-    tdir = os.path.join(OUT, "tests")
-    os.makedirs(tdir, exist_ok=True)
-    import shutil
-    for name in ("test_ctc.py", "test_ctc_decoder.py"):
-        src = os.path.join(REF, "tests", name)
-        if os.path.exists(src):
-            shutil.copyfile(src, os.path.join(tdir, name))
     # keep only what must travel to the GPU box
     for d in built:
         for f in os.listdir(d):

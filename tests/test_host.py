@@ -158,8 +158,9 @@ def test_module_api_surface():
     dec = e.CTCDecoder(beam_width=20, lm_path="/no/such/model.arpa")   # KenLM decoding stays the reference's CPU code
     with pytest.raises(NotImplementedError):
         dec.decode(torch.zeros(1, 2, 3))
-    with pytest.raises(RuntimeError, match="no CPU fallback"):            # beam search without a device fails loudly
-        e.CTCDecoder(beam_width=20).decode(torch.zeros(1, 2, 3))
+    if not torch.cuda.is_available():                                     # beam search without a device fails loudly
+        with pytest.raises(RuntimeError, match="no CPU fallback"):
+            e.CTCDecoder(beam_width=20).decode(torch.zeros(1, 2, 3))
     assert list(inspect.signature(e.CTCLossEngine.compute).parameters)[1:5] == [
         "logits", "targets", "logits_lengths", "targets_lengths"]
     assert list(inspect.signature(e.CTCGreedyEngine.decode_greedy).parameters)[1:] == ["logits_", "logits_lengths_"]
