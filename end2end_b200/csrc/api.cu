@@ -673,15 +673,23 @@ int e2e_ctc_host_free(void* p) {
 }
 
 // ---- Viterbi forced alignment (SURVEY 8(f2)) -------------------------------------------------------
+// The alignment has its own width limit (viterbi_supported), not the loss kernels' kMaxTargets.
+static int check_viterbi(const e2e_ctc_desc* desc, int32_t is_ctc) {
+  int rc = check_desc(desc, false);
+  if (rc != E2E_OK) return rc;
+  if (desc->max_targets < 0) { set_error("bad max_targets %d", desc->max_targets); return E2E_ERR_INVALID_ARGUMENT; }
+  return viterbi_supported(*desc, is_ctc ? 1 : 0) ? E2E_OK : E2E_ERR_UNSUPPORTED;
+}
+
 size_t e2e_ctc_viterbi_workspace_bytes(const e2e_ctc_desc* desc, int32_t is_ctc) {
-  if (check_desc(desc, true) != E2E_OK) return 0;
+  if (check_viterbi(desc, is_ctc) != E2E_OK) return 0;
   return align256(viterbi_workspace_bytes(*desc, is_ctc ? 1 : 0));
 }
 
 int e2e_ctc_viterbi_align_device(const e2e_ctc_desc* desc, int32_t is_ctc, const void* log_probs, const void* targets,
                                  const void* logits_lengths, const void* targets_lengths, int64_t* aligned,
                                  void* workspace, size_t workspace_bytes, void* cuda_stream) {
-  int rc = check_desc(desc, true);
+  int rc = check_viterbi(desc, is_ctc);
   if (rc != E2E_OK) return rc;
   if (!log_probs || !logits_lengths || !targets_lengths || !aligned || (!targets && desc->max_targets > 0)) {
     set_error("null pointer argument");
@@ -699,6 +707,7 @@ size_t e2e_ctc_noblank_workspace_bytes(const e2e_ctc_desc* desc) {
     set_error("bad descriptor");
     return 0;
   }
+  if (!noblank_supported(*desc)) return 0;
   return align256(noblank_workspace_bytes(*desc));
 }
 
@@ -706,7 +715,7 @@ int e2e_ctc_noblank_fwd_bwd_device(const e2e_ctc_desc* desc, int32_t space_idx, 
                                    const void* logits_lengths, const void* targets_lengths, void* losses, void* grads,
                                    void* workspace, size_t workspace_bytes, void* cuda_stream) {
   const size_t need = e2e_ctc_noblank_workspace_bytes(desc);
-  if (!need) return E2E_ERR_INVALID_ARGUMENT;
+  if (!need) return desc && desc->max_targets >= 0 && !noblank_supported(*desc) ? E2E_ERR_UNSUPPORTED : E2E_ERR_INVALID_ARGUMENT;
   if (!log_probs || !logits_lengths || !targets_lengths || !losses || !grads || (!targets && desc->max_targets > 0)) {
     set_error("null pointer argument");
     return E2E_ERR_INVALID_ARGUMENT;

@@ -251,9 +251,11 @@ bool beam_supported(const e2e_ctc_desc& d, int beam_width);
 int launch_beam(const e2e_ctc_desc& d, int beam_width, int space_idx, double wip, const void* logits, const void* in_len,
                 int64_t* decoded, int64_t* decoded_len, int64_t* ties, char* ws, cudaStream_t s);
 size_t noblank_workspace_bytes(const e2e_ctc_desc& d);
+bool noblank_supported(const e2e_ctc_desc& d);
 int launch_noblank(const e2e_ctc_desc& d, int space_idx, const void* lp, const void* targets, const void* in_len,
                    const void* tgt_len, void* losses, void* grads, char* ws, cudaStream_t s);
 size_t viterbi_workspace_bytes(const e2e_ctc_desc& d, int is_ctc);
+bool viterbi_supported(const e2e_ctc_desc& d, int is_ctc);
 int launch_viterbi(const e2e_ctc_desc& d, int is_ctc, const void* lp, const void* targets, const void* in_len,
                    const void* tgt_len, int64_t* aligned, char* ws, cudaStream_t s);
 

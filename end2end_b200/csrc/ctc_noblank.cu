@@ -186,6 +186,25 @@ __global__ void ctc_noblank_kernel(const NbParams p) {
 }  // namespace
 
 static int noblank_cells(const e2e_ctc_desc& d) { return d.max_targets + 2; }
+static int noblank_cells_thr(const e2e_ctc_desc& d) { return (noblank_cells(d) + 31) & ~31; }
+static size_t noblank_smem(const e2e_ctc_desc& d) {
+  return ((((size_t)(2 * noblank_cells(d) + 2 + d.alphabet + 2)) * 4 + 15) & ~(size_t)15) +
+         (size_t)4 * (noblank_cells_thr(d) + 2) * sizeof(double);
+}
+
+// One thread per lattice cell and sweep in one CTA: Lmax + 2 <= 1024 cells (Lmax <= 1022); the labels, the symbol
+// lists and the sweep rows share one CTA's shared memory (200 KB).
+bool noblank_supported(const e2e_ctc_desc& d) {
+  if (d.max_targets > 1022) {
+    set_error("ctc_without_blank: target length %d exceeds this build's limit 1022", d.max_targets);
+    return false;
+  }
+  if (noblank_smem(d) > 200 * 1024) {
+    set_error("ctc_without_blank: alphabet %d too large for one CTA's shared memory", d.alphabet);
+    return false;
+  }
+  return true;
+}
 
 size_t noblank_workspace_bytes(const e2e_ctc_desc& d) {
   return 256 + (size_t)2 * d.batch * d.max_frames * noblank_cells(d) * sizeof(double);
@@ -203,12 +222,11 @@ int launch_noblank(const e2e_ctc_desc& d, int space_idx, const void* lp, const v
   p.status = reinterpret_cast<int*>(ws);
   p.alpha = reinterpret_cast<double*>(ws + 256);
   p.beta = p.alpha + (size_t)d.batch * d.max_frames * p.Smax;
-  int ct = (p.Smax + 31) & ~31;
-  if (ct > 1024) { set_error("ctc_without_blank: target length %d too long for one CTA", d.max_targets); return E2E_ERR_UNSUPPORTED; }
+  if (!noblank_supported(d)) return E2E_ERR_UNSUPPORTED;
+  const int ct = noblank_cells_thr(d);
   p.cells_thr = ct;
   const int threads = 2 * ct <= 1024 ? 2 * ct : ct;
-  const size_t smem = ((((size_t)(2 * p.Smax + 2 + p.V + 2)) * 4 + 15) & ~(size_t)15) + (size_t)4 * (ct + 2) * sizeof(double);
-  if (smem > 200 * 1024) { set_error("ctc_without_blank: alphabet %d too large", d.alphabet); return E2E_ERR_UNSUPPORTED; }
+  const size_t smem = noblank_smem(d);
   static int attr_smem[64];
   int dev = 0;
   E2E_CUDA_TRY(cudaGetDevice(&dev));

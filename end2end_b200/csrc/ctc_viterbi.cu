@@ -17,6 +17,10 @@
 // registers, the two neighbour cells come from a double-buffered shared-memory row (one __syncthreads per frame),
 // emissions are fetched a block of frames ahead (off the dependent chain).  Backpointers are one byte per thread
 // per frame (2 bits per cell): in shared memory when the utterance fits, else in the caller's workspace.
+//
+// Width limit: at most kVitMaxThreads threads of kVitMaxCpt cells, i.e. lattices of <= 2048 cells (CTC: 2 L + 1, so
+// L <= 1023; ASG: L <= 2048).  The 4-cells-per-thread instantiations use 105-110 registers a thread, so a CTA of more
+// than 576 threads could not launch at all; __launch_bounds__ holds the compiler to what 512 threads allow.
 #include "common.cuh"
 
 namespace e2e {
@@ -35,12 +39,14 @@ struct VitParams {
 };
 
 constexpr long long kIgnore = -100;   // torch.full(..., fill_value=-100) in get_alignment_3d
+constexpr int kVitMaxThreads = 512;
+constexpr int kVitMaxCpt = 4;
 
 // ET: the type emissions are staged in -- float for 32/16-bit inputs (exact), double for f64 inputs
 // CPT: lattice cells per thread (1, 2 or 4).  Few cells per thread = more warps per scheduler to hide the latency of the
 // dependent compare/select chain (with 4 cells per thread BASELINE config 2 ran one warp per scheduler at ~1200 cycles per frame).
 template <typename ET, int CPT>
-__global__ void ctc_viterbi_kernel(const VitParams p) {
+__global__ void __launch_bounds__(kVitMaxThreads) ctc_viterbi_kernel(const VitParams p) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int b = blockIdx.x, tid = threadIdx.x, nthr = blockDim.x;
   long long* out = p.aligned + (long long)b * p.T;
@@ -179,7 +185,7 @@ __global__ void ctc_viterbi_kernel(const VitParams p) {
 
 static int viterbi_cpt(const e2e_ctc_desc& d, int is_ctc) {
   const int Smax = is_ctc ? 2 * d.max_targets + 1 : d.max_targets;
-  return Smax <= 512 ? 1 : (Smax <= 1024 ? 2 : 4);          // up to 16 / 16 / 10 warps per CTA
+  return Smax <= 512 ? 1 : (Smax <= 1024 ? 2 : 4);          // up to 16 warps per CTA
 }
 static int viterbi_threads(const e2e_ctc_desc& d, int is_ctc) {
   const int Smax = is_ctc ? 2 * d.max_targets + 1 : d.max_targets;
@@ -187,6 +193,15 @@ static int viterbi_threads(const e2e_ctc_desc& d, int is_ctc) {
   int thr = (Smax + cpt - 1) / cpt;
   thr = (thr + 31) & ~31;
   return thr < 32 ? 32 : thr;
+}
+
+bool viterbi_supported(const e2e_ctc_desc& d, int is_ctc) {
+  const long long cells = is_ctc ? 2LL * d.max_targets + 1 : d.max_targets;
+  if (cells <= kVitMaxThreads * kVitMaxCpt) return true;
+  set_error("viterbi: target length %d exceeds this build's limit %d (%s lattice of at most %d cells)", d.max_targets,
+            is_ctc ? (kVitMaxThreads * kVitMaxCpt - 1) / 2 : kVitMaxThreads * kVitMaxCpt, is_ctc ? "CTC" : "ASG",
+            kVitMaxThreads * kVitMaxCpt);
+  return false;
 }
 
 size_t viterbi_workspace_bytes(const e2e_ctc_desc& d, int is_ctc) {
@@ -219,7 +234,7 @@ int launch_viterbi(const e2e_ctc_desc& d, int is_ctc, const void* lp, const void
   p.bp_global = reinterpret_cast<unsigned char*>(ws) + 256;
   p.B = d.batch; p.T = d.max_frames; p.V = d.alphabet; p.Lmax = d.max_targets; p.blank = d.blank_idx; p.is_ctc = is_ctc;
   const int cpt = viterbi_cpt(d, is_ctc), thr = viterbi_threads(d, is_ctc);
-  if (thr > 1024) { set_error("viterbi: target length %d too long for one CTA", d.max_targets); return E2E_ERR_UNSUPPORTED; }
+  if (!viterbi_supported(d, is_ctc)) return E2E_ERR_UNSUPPORTED;
   p.bp_stride = thr;
   const int Smax = is_ctc ? 2 * d.max_targets + 1 : d.max_targets;
   const size_t fixed = (((size_t)(Smax + 4) * 4 + 15) & ~(size_t)15) + (size_t)2 * (cpt * thr + 2) * 8;

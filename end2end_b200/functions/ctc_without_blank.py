@@ -30,6 +30,8 @@ def ctc_without_blank_3d_loss(log_probs, targets, logits_lengths, targets_length
     if not _dense3(lp):
         lp = lp.contiguous()
     B, T, V = lp.shape
+    if B < 1 or T < 1 or V < 1:
+        raise ValueError("empty logits %s" % (tuple(lp.shape),))
     if targets.dim() != 2 or targets.size(0) != B:
         raise ValueError("targets must be [batch, max_target_length]")
     if not -1 <= space_idx < V:
@@ -49,8 +51,8 @@ def ctc_without_blank_3d_loss(log_probs, targets, logits_lengths, targets_length
     d.targets_stride_b = targets.stride(0) if targets.size(1) > 0 else 0
     with _on_device(dev):
         n = L.e2e_ctc_noblank_workspace_bytes(ctypes.byref(d))
-        if n == 0:
-            raise _lib.E2EError(1, L.e2e_last_error_string().decode("utf-8", "replace"))
+        if n == 0:   # the shape is valid (checked above): the lattice or the alphabet is beyond the build's limits
+            raise NotImplementedError(L.e2e_last_error_string().decode("utf-8", "replace"))
         ws = torch.empty(n, dtype=torch.uint8, device=dev)
         losses = torch.empty(B, dtype=lp.dtype, device=dev)
         grads = torch.empty_strided(lp.size(), lp.stride(), dtype=lp.dtype, device=dev)

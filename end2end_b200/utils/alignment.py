@@ -30,6 +30,8 @@ def get_alignment_3d_device(log_probs, targets, logits_lengths, targets_lengths,
     if not _dense3(lp):
         lp = lp.contiguous()
     B, T, V = lp.shape
+    if B < 1 or T < 1 or V < 1:
+        raise ValueError("empty log_probs %s" % (tuple(lp.shape),))
     if targets.dim() != 2 or targets.size(0) != B:
         raise ValueError("targets must be [batch, max_target_length]")
     if not 0 <= blank_idx < V:
@@ -49,8 +51,8 @@ def get_alignment_3d_device(log_probs, targets, logits_lengths, targets_lengths,
     d.targets_stride_b = targets.stride(0) if targets.size(1) > 0 else 0
     with _on_device(dev):
         n = L.e2e_ctc_viterbi_workspace_bytes(ctypes.byref(d), 1 if is_ctc else 0)
-        if n == 0:
-            raise _lib.E2EError(2, L.e2e_last_error_string().decode("utf-8", "replace"))
+        if n == 0:   # the shape is valid (checked above): the lattice or the alphabet is beyond the build's limits
+            raise NotImplementedError(L.e2e_last_error_string().decode("utf-8", "replace"))
         ws = torch.empty(n, dtype=torch.uint8, device=dev)
         out = torch.empty(B, T, dtype=torch.int64, device=dev)
         _lib.check(L.e2e_ctc_viterbi_align_device(ctypes.byref(d), 1 if is_ctc else 0, _ptr(lp), _ptr(targets), _ptr(ll),

@@ -195,7 +195,9 @@ void e2e_ctc_graph_destroy(e2e_ctc_graph* graph);
  * utterance's frames (the reference's fill value).  Bit-exact with the reference: fp64 max-plus recursion with its
  * comparison order and window.  desc->blank_idx is the blank (the reference hard-codes 0).  A logits length of 0
  * leaves the row at -100; out-of-range lengths / labels set status bits (e2e_ctc_loss_check_device on the
- * workspace) and leave -100. */
+ * workspace) and leave -100.  Limit: lattices of at most 2048 cells, i.e. desc->max_targets <= 1023 for CTC
+ * (2 L + 1 cells) and <= 2048 for ASG (L cells), independent of the loss's limit (e2e_ctc_get_limits); beyond it
+ * the workspace query returns 0 and the alignment E2E_ERR_UNSUPPORTED, with the reason in e2e_last_error_string. */
 size_t e2e_ctc_viterbi_workspace_bytes(const e2e_ctc_desc* desc, int32_t is_ctc);
 int e2e_ctc_viterbi_align_device(const e2e_ctc_desc* desc, int32_t is_ctc, const void* log_probs,
                                  const void* targets, const void* logits_lengths, const void* targets_lengths,
@@ -207,7 +209,10 @@ int e2e_ctc_viterbi_align_device(const e2e_ctc_desc* desc, int32_t is_ctc, const
  * _ctc_without_blank_loss (:13-88) under _ctc_without_blank_3d_loss (:91-117).  `log_probs` are log-probabilities
  * [B,T,V]; space_idx = -1: the lattice is the target sequence itself; otherwise one optional `space_idx` cell is
  * added at either end.  losses[b] = -log Z; grads[b,t,v] = exp(lp) - posterior for t < T_b and 0 past the
- * utterance's frames; an utterance with no alignment gives +inf / NaN as in the reference.  fp64 log-space. */
+ * utterance's frames; an utterance with no alignment gives +inf / NaN as in the reference.  fp64 log-space.
+ * Limit: desc->max_targets <= 1022, and the labels plus one int per symbol in 200 KB of shared memory (any alphabet up
+ * to 40,000 symbols); beyond it the workspace query returns 0 and the loss E2E_ERR_UNSUPPORTED, with the reason in
+ * e2e_last_error_string. */
 size_t e2e_ctc_noblank_workspace_bytes(const e2e_ctc_desc* desc);
 int e2e_ctc_noblank_fwd_bwd_device(const e2e_ctc_desc* desc, int32_t space_idx, const void* log_probs,
                                    const void* targets, const void* logits_lengths, const void* targets_lengths,

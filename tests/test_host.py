@@ -272,3 +272,55 @@ def test_beam_workspace_query_and_limits(lib_built):
     assert L.e2e_ctc_beam_workspace_bytes(ctypes.byref(d), 100) > 0
     d.alphabet = 32768                                     # rows of this size do not fit shared memory
     assert L.e2e_ctc_beam_workspace_bytes(ctypes.byref(d), 100) == 0
+
+
+def _neighbour_desc(B, T, V, Lmax):
+    from end2end_b200 import _lib
+    d = _lib.Desc()
+    d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, Lmax
+    d.blank_idx, d.dtype = 0, _lib.E2E_F32
+    d.targets_itype = d.lengths_itype = _lib.E2E_I64
+    d.logits_stride_b, d.logits_stride_t = T * V, V
+    d.targets_stride_b = Lmax
+    return d
+
+
+def test_viterbi_workspace_query_and_limits(lib_built):
+    """The alignment has its own width limit, lattices of at most 2048 cells, not the loss's 639 labels: CTC (2 L + 1
+    cells) up to L = 1023, ASG (L cells) up to L = 2048.  One label more is refused by the size query, without a device."""
+    import ctypes
+    from end2end_b200 import _lib
+    L = _lib.load()
+    for is_ctc, widest in ((1, 1023), (0, 2048)):
+        d = _neighbour_desc(4, 2 * widest, 29, widest)
+        n = L.e2e_ctc_viterbi_workspace_bytes(ctypes.byref(d), is_ctc)
+        assert 256 + 4 * 2 * widest * 512 <= n < 256 + 4 * 2 * widest * 512 + 256   # one backpointer byte per thread and frame
+        for lmax in (640, widest // 2):                                # beyond the loss's limit, below the alignment's
+            d.max_targets = lmax
+            assert L.e2e_ctc_viterbi_workspace_bytes(ctypes.byref(d), is_ctc) > 0
+        d.max_targets = widest + 1
+        assert L.e2e_ctc_viterbi_workspace_bytes(ctypes.byref(d), is_ctc) == 0
+        assert "limit" in L.e2e_last_error_string().decode()
+    d = _neighbour_desc(4, 50, 29, 0)
+    assert L.e2e_ctc_viterbi_workspace_bytes(ctypes.byref(d), 1) > 0
+    d.max_targets = -1
+    assert L.e2e_ctc_viterbi_workspace_bytes(ctypes.byref(d), 1) == 0
+
+
+def test_noblank_workspace_query_and_limits(lib_built):
+    """CTC without blank runs one thread per lattice cell in one CTA: Lmax + 2 <= 1024 cells.  The size query applies
+    that limit (and the shared-memory bound on the alphabet) so that nothing is allocated for a shape that cannot run."""
+    import ctypes
+    from end2end_b200 import _lib
+    L = _lib.load()
+    d = _neighbour_desc(4, 1100, 29, 1022)
+    n = L.e2e_ctc_noblank_workspace_bytes(ctypes.byref(d))
+    assert n == 256 + 2 * 4 * 1100 * 1024 * 8                    # alpha and beta rows in fp64
+    d.max_targets = 1023
+    assert L.e2e_ctc_noblank_workspace_bytes(ctypes.byref(d)) == 0
+    assert "1022" in L.e2e_last_error_string().decode()
+    d.max_targets, d.alphabet, d.logits_stride_t = 30, 40000, 40000
+    assert L.e2e_ctc_noblank_workspace_bytes(ctypes.byref(d)) > 0
+    d.alphabet = d.logits_stride_t = 60000                          # the per-symbol lists no longer fit shared memory
+    assert L.e2e_ctc_noblank_workspace_bytes(ctypes.byref(d)) == 0
+    assert "alphabet" in L.e2e_last_error_string().decode()
