@@ -3,13 +3,13 @@
 Hot path only: CTC loss forward+backward and greedy CTC decoding, as hand-written CUDA kernels in
 ``libe2e_ctc.so`` (C ABI in ``include/e2e_ctc.h``).  See DESIGN.md / INTEGRATION.md.
 """
-from .decoders.ctc_decoder import CTCDecoder, CTCDecoderError, DecoderResults
+from .decoders.ctc_decoder import CTCDecoder, CTCDecoderError, DecoderResults, NBestResults
 from .encoders.text_encoders import CTCEncoder
 from .engine import CTCGreedyEngine, CTCLossEngine, GraphedStep
 from .functions.forward_backward import ForwardBackwardLossFunction
 from .modules.ctc_loss import CTCLoss, ForwardBackwardLossBase, GraphedCTCStep
 
 __all__ = ["CTCLoss", "CTCDecoder", "CTCEncoder", "CTCLossEngine", "CTCGreedyEngine",
-           "ForwardBackwardLossFunction", "ForwardBackwardLossBase", "CTCDecoderError", "DecoderResults",
+           "ForwardBackwardLossFunction", "ForwardBackwardLossBase", "CTCDecoderError", "DecoderResults", "NBestResults",
            "GraphedStep", "GraphedCTCStep"]
 __version__ = "0.1.0"

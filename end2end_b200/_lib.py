@@ -31,6 +31,7 @@ EXPORTS = (
     "e2e_ctc_noblank_workspace_bytes", "e2e_ctc_noblank_fwd_bwd_device",
     "e2e_ctc_host_alloc", "e2e_ctc_host_free",
     "e2e_ctc_beam_workspace_bytes", "e2e_ctc_beam_decode_device", "e2e_ctc_engine_beam_host",
+    "e2e_ctc_beam_nbest_workspace_bytes", "e2e_ctc_beam_nbest_device", "e2e_ctc_engine_beam_nbest_host",
 )
 KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order")
 
@@ -119,6 +120,12 @@ def load():
     L.e2e_ctc_beam_decode_device.restype = ctypes.c_int
     L.e2e_ctc_engine_beam_host.argtypes = [vp, dp, i32, i32, dbl, vp, vp, vp, vp, vp]
     L.e2e_ctc_engine_beam_host.restype = ctypes.c_int
+    L.e2e_ctc_beam_nbest_workspace_bytes.argtypes = [dp, i32, i32]
+    L.e2e_ctc_beam_nbest_workspace_bytes.restype = sz
+    L.e2e_ctc_beam_nbest_device.argtypes = [dp, i32, i32, i32, dbl, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    L.e2e_ctc_beam_nbest_device.restype = ctypes.c_int
+    L.e2e_ctc_engine_beam_nbest_host.argtypes = [vp, dp, i32, i32, i32, dbl, vp, vp, vp, vp, vp, vp, vp]
+    L.e2e_ctc_engine_beam_nbest_host.restype = ctypes.c_int
     L.e2e_ctc_host_alloc.argtypes = [sz, ctypes.POINTER(vp)]
     L.e2e_ctc_host_alloc.restype = ctypes.c_int
     L.e2e_ctc_host_free.argtypes = [vp]

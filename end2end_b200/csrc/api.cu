@@ -625,10 +625,14 @@ int e2e_ctc_greedy_decode_device(const e2e_ctc_desc* desc, const void* logits, c
 }
 
 // ---- LM-free prefix beam search (SURVEY 8(f3)) -----------------------------------------------------------
-static int check_beam(const e2e_ctc_desc* desc, int32_t beam_width, int32_t space_idx, double wip) {
+static int check_beam(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx, double wip) {
   int rc = check_desc(desc, false);
   if (rc != E2E_OK) return rc;
   if (beam_width < 1) { set_error("beam_width %d < 1", beam_width); return E2E_ERR_INVALID_ARGUMENT; }
+  if (n_best < 1 || n_best > beam_width) {
+    set_error("n_best %d outside [1, beam_width = %d]", n_best, beam_width);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
   if (space_idx < -1 || space_idx >= desc->alphabet) { set_error("space_idx %d outside [-1,%d)", space_idx, desc->alphabet); return E2E_ERR_INVALID_ARGUMENT; }
   if (!(wip == wip) || wip == INFINITY || wip == -INFINITY) { set_error("wip must be finite"); return E2E_ERR_INVALID_ARGUMENT; }
   if (!beam_supported(*desc, beam_width)) {
@@ -639,21 +643,38 @@ static int check_beam(const e2e_ctc_desc* desc, int32_t beam_width, int32_t spac
   return E2E_OK;
 }
 
+size_t e2e_ctc_beam_nbest_workspace_bytes(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best) {
+  if (check_beam(desc, beam_width, n_best, -1, 0.0) != E2E_OK) return 0;
+  return align256(beam_workspace_bytes(*desc, beam_width));   // the trie; the n_best backtraces need nothing more
+}
+
 size_t e2e_ctc_beam_workspace_bytes(const e2e_ctc_desc* desc, int32_t beam_width) {
-  if (check_beam(desc, beam_width, -1, 0.0) != E2E_OK) return 0;
-  return align256(beam_workspace_bytes(*desc, beam_width));
+  return e2e_ctc_beam_nbest_workspace_bytes(desc, beam_width, 1);
+}
+
+int e2e_ctc_beam_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx, double wip,
+                              const void* logits, const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths,
+                              double* scores, double* log_probs, int64_t* ties, void* workspace, size_t workspace_bytes,
+                              void* cuda_stream) {
+  int rc = check_beam(desc, beam_width, n_best, space_idx, wip);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !decoded || !decoded_lengths || !scores) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  rc = check_ws(workspace, workspace_bytes, e2e_ctc_beam_nbest_workspace_bytes(desc, beam_width, n_best));
+  if (rc != E2E_OK) return rc;
+  return launch_beam(*desc, beam_width, n_best, space_idx, wip, logits, logits_lengths, decoded, decoded_lengths, scores,
+                     log_probs, ties, reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 int e2e_ctc_beam_decode_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t space_idx, double wip,
                                const void* logits, const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths,
                                int64_t* ties, void* workspace, size_t workspace_bytes, void* cuda_stream) {
-  int rc = check_beam(desc, beam_width, space_idx, wip);
+  int rc = check_beam(desc, beam_width, 1, space_idx, wip);
   if (rc != E2E_OK) return rc;
   if (!logits || !decoded || !decoded_lengths) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
   rc = check_ws(workspace, workspace_bytes, e2e_ctc_beam_workspace_bytes(desc, beam_width));
   if (rc != E2E_OK) return rc;
-  return launch_beam(*desc, beam_width, space_idx, wip, logits, logits_lengths, decoded, decoded_lengths, ties,
-                     reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
+  return launch_beam(*desc, beam_width, 1, space_idx, wip, logits, logits_lengths, decoded, decoded_lengths, nullptr, nullptr,
+                     ties, reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 // ---- pinned host memory for result buffers -------------------------------------------------------
@@ -1072,11 +1093,13 @@ int e2e_ctc_engine_greedy_host(e2e_ctc_engine* e, const e2e_ctc_desc* desc, cons
   return E2E_OK;
 }
 
-int e2e_ctc_engine_beam_host(e2e_ctc_engine* e, const e2e_ctc_desc* desc, int32_t beam_width, int32_t space_idx, double wip,
-                             const void* logits, const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths,
-                             int64_t* ties) {
+// decode (n_best == 1, scores == NULL) and the N-best list share one path; results land in the engine's decoded /
+// decoded_len buffers (decoded_len: lengths [B,N], ties [B], scores [B,N], log_probs [B,N])
+static int engine_beam_host(e2e_ctc_engine* e, const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx,
+                            double wip, const void* logits, const void* logits_lengths, int64_t* decoded,
+                            int64_t* decoded_lengths, double* scores, double* log_probs, int64_t* ties) {
   if (!e) { set_error("null engine"); return E2E_ERR_INVALID_ARGUMENT; }
-  int rc = check_beam(desc, beam_width, space_idx, wip);
+  int rc = check_beam(desc, beam_width, n_best, space_idx, wip);
   if (rc != E2E_OK) return rc;
   if (!logits || !decoded || !decoded_lengths) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
   const e2e_ctc_desc& d = *desc;
@@ -1087,25 +1110,47 @@ int e2e_ctc_engine_beam_host(e2e_ctc_engine* e, const e2e_ctc_desc* desc, int32_
   E2E_CUDA_TRY(cudaSetDevice(e->device));
   const size_t n_log = (size_t)d.batch * d.max_frames * d.alphabet * elem_size(d.dtype);
   const size_t n_len = (size_t)d.batch * (d.lengths_itype == E2E_I64 ? 8 : 4);
-  const size_t n_dec = (size_t)d.batch * d.max_frames * 8, n_dl = (size_t)d.batch * 8;
-  const size_t n_ws = e2e_ctc_beam_workspace_bytes(desc, beam_width);
+  const size_t n_hyp = (size_t)d.batch * n_best;
+  const size_t n_dec = n_hyp * d.max_frames * 8, n_dl = n_hyp * 8, n_ties = (size_t)d.batch * 8;
+  const size_t n_ws = e2e_ctc_beam_nbest_workspace_bytes(desc, beam_width, n_best);
   if ((rc = e->logits.ensure(n_log)) || (rc = e->in_len.ensure(n_len)) || (rc = e->decoded.ensure(n_dec)) ||
-      (rc = e->decoded_len.ensure(2 * n_dl)) || (rc = e->ws.ensure(n_ws)))
+      (rc = e->decoded_len.ensure(n_dl + n_ties + (scores ? 2 * n_dl : 0))) || (rc = e->ws.ensure(n_ws)))
     return rc;
   cudaStream_t s = e->stream;
   E2E_CUDA_TRY(cudaMemcpyAsync(e->logits.p, logits, n_log, cudaMemcpyHostToDevice, s));
   if (logits_lengths) E2E_CUDA_TRY(cudaMemcpyAsync(e->in_len.p, logits_lengths, n_len, cudaMemcpyHostToDevice, s));
   int64_t* d_len = reinterpret_cast<int64_t*>(e->decoded_len.p);
-  rc = launch_beam(d, beam_width, space_idx, wip, e->logits.p, logits_lengths ? e->in_len.p : nullptr,
-                   reinterpret_cast<int64_t*>(e->decoded.p), d_len, d_len + d.batch, reinterpret_cast<char*>(e->ws.p), s);
+  int64_t* d_ties = d_len + n_hyp;
+  double* d_scores = scores ? reinterpret_cast<double*>(d_ties + d.batch) : nullptr;
+  double* d_lp = scores && log_probs ? d_scores + n_hyp : nullptr;
+  rc = launch_beam(d, beam_width, n_best, space_idx, wip, e->logits.p, logits_lengths ? e->in_len.p : nullptr,
+                   reinterpret_cast<int64_t*>(e->decoded.p), d_len, d_scores, d_lp, d_ties, reinterpret_cast<char*>(e->ws.p), s);
   if (rc != E2E_OK) return rc;
   E2E_CUDA_TRY(cudaMemcpyAsync(decoded, e->decoded.p, n_dec, cudaMemcpyDeviceToHost, s));
   E2E_CUDA_TRY(cudaMemcpyAsync(decoded_lengths, d_len, n_dl, cudaMemcpyDeviceToHost, s));
-  if (ties) E2E_CUDA_TRY(cudaMemcpyAsync(ties, d_len + d.batch, n_dl, cudaMemcpyDeviceToHost, s));
+  if (ties) E2E_CUDA_TRY(cudaMemcpyAsync(ties, d_ties, n_ties, cudaMemcpyDeviceToHost, s));
+  if (d_scores) E2E_CUDA_TRY(cudaMemcpyAsync(scores, d_scores, n_dl, cudaMemcpyDeviceToHost, s));
+  if (d_lp) E2E_CUDA_TRY(cudaMemcpyAsync(log_probs, d_lp, n_dl, cudaMemcpyDeviceToHost, s));
   E2E_CUDA_TRY(cudaStreamSynchronize(s));
   e->h2d = n_log + (logits_lengths ? n_len : 0);
-  e->d2h = n_dec + n_dl + (ties ? n_dl : 0);
+  e->d2h = n_dec + n_dl + (ties ? n_ties : 0) + (d_scores ? n_dl : 0) + (d_lp ? n_dl : 0);
   return E2E_OK;
+}
+
+int e2e_ctc_engine_beam_host(e2e_ctc_engine* e, const e2e_ctc_desc* desc, int32_t beam_width, int32_t space_idx, double wip,
+                             const void* logits, const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths,
+                             int64_t* ties) {
+  return engine_beam_host(e, desc, beam_width, 1, space_idx, wip, logits, logits_lengths, decoded, decoded_lengths, nullptr,
+                          nullptr, ties);
+}
+
+int e2e_ctc_engine_beam_nbest_host(e2e_ctc_engine* e, const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best,
+                                   int32_t space_idx, double wip, const void* logits, const void* logits_lengths,
+                                   int64_t* decoded, int64_t* decoded_lengths, double* scores, double* log_probs,
+                                   int64_t* ties) {
+  if (!scores) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  return engine_beam_host(e, desc, beam_width, n_best, space_idx, wip, logits, logits_lengths, decoded, decoded_lengths,
+                          scores, log_probs, ties);
 }
 
 int e2e_ctc_engine_last_traffic(const e2e_ctc_engine* e, uint64_t* h2d_bytes, uint64_t* d2h_bytes) {

@@ -248,8 +248,10 @@ int launch_greedy(const e2e_ctc_desc& d, const void* logits, const void* in_len,
                   int64_t* decoded_len, char* ws, cudaStream_t s);
 size_t beam_workspace_bytes(const e2e_ctc_desc& d, int beam_width);
 bool beam_supported(const e2e_ctc_desc& d, int beam_width);
-int launch_beam(const e2e_ctc_desc& d, int beam_width, int space_idx, double wip, const void* logits, const void* in_len,
-                int64_t* decoded, int64_t* decoded_len, int64_t* ties, char* ws, cudaStream_t s);
+// decoded [B, n_best, T], decoded_len [B, n_best]; scores / log_probs [B, n_best] or null (log_probs is ignored without scores)
+int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
+                const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
+                char* ws, cudaStream_t s);
 size_t noblank_workspace_bytes(const e2e_ctc_desc& d);
 bool noblank_supported(const e2e_ctc_desc& d);
 int launch_noblank(const e2e_ctc_desc& d, int space_idx, const void* lp, const void* targets, const void* in_len,

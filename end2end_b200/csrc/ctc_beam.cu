@@ -54,12 +54,14 @@ struct __align__(16) BeamNode {   // 16 bytes
 struct BeamParams {
   const void* logits; int dtype; long long sb, st;
   const void* in_len; int len_is64;
-  long long* decoded;        // [B, T] zero padded
-  long long* decoded_len;    // [B]
+  long long* decoded;        // [B, n_best, T] zero padded
+  long long* decoded_len;    // [B, n_best]
+  double* scores;            // [B, n_best] or null: the ranking score
+  double* log_probs;         // [B, n_best] or null: log p of the prefix, without the word penalty
   long long* ties;           // [B] or null
   BeamNode* nodes;           // [B][node_cap]
   long long node_cap;
-  int B, T, V, blank, beam, space, from_logits;
+  int B, T, V, blank, beam, space, from_logits, n_best;
   int prefilter;             // large alphabets: only the beam+2 most probable symbols of a frame (and the space) are extended
   int kc_cap;                // keys the shared-memory cache holds (0: none)
   double wip;
@@ -716,39 +718,51 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
     { const BeamBuf tmp = C; C = N; N = tmp; }
   }
 
-  // ---- the best prefix (:413-419) and its symbols (get_sentence, :225-239) -----------------------------------------
+  // ---- the n_best best prefixes (:413-419: the reference sorts the final list) and their symbols (get_sentence, :225-239).
+  //      Every member ranks itself by counting over the keys: rank = keys above + equal keys at lower positions, so rank 0
+  //      is the member the reference's prefixes[0] is when no two scores are equal. ----------------------------------------
   __syncthreads();   // the last frame's tail still reads the member keys
   if (tid < W) S.mkey[tid] = beam_key(beam_score(beam_lse(C.pnb[tid], C.pb[tid]), C.nw[tid], p.wip));
+  if (tid == 0) s_tie_now = 0;
   __syncthreads();
-  long long* out = p.decoded + (long long)b * p.T;
-  if (warp == 0) {
-    unsigned long long bk = 0ull; int bi = 0x7fffffff;
-    for (int s = lane; s < W; s += 32) { const unsigned long long k = S.mkey[s]; if (bi == 0x7fffffff || k > bk) { bk = k; bi = s; } }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) {
-      const unsigned long long ok = __shfl_xor_sync(0xffffffffu, bk, o); const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (oi != 0x7fffffff && (bi == 0x7fffffff || ok > bk || (ok == bk && oi < bi))) { bk = ok; bi = oi; }
-    }
-    int same = 0;
-    for (int s = lane; s < W; s += 32) same += (S.mkey[s] == bk);
-    same = warp_sum(same);
-    if (lane == 0) {
-      if (same > 1) s_ties++;
-      const int depth = C.dep[bi];
-      int n = C.node[bi];
+  const int NB = p.n_best;
+  long long* out = p.decoded + (long long)b * NB * p.T;
+  if (tid < W) {
+    const unsigned long long k = S.mkey[tid];
+    int rank = 0, same = 0;
+    for (int j = 0; j < W; j++) { const unsigned long long o = S.mkey[j]; rank += o > k || (o == k && j < tid); same += o == k; }
+    if (rank < NB) {
+      if (same > 1) s_tie_now = 1;                       // the returned list depends on equal final scores
+      const int depth = C.dep[tid];
+      long long* row = out + (long long)rank * p.T;
       int len;
-      if (depth == 0) { out[0] = -1; len = 1; }          // the empty prefix: get_sentence pushes the root's last_char = -1
+      if (depth == 0) { row[0] = -1; len = 1; }          // the empty prefix: get_sentence pushes the root's last_char = -1
       else {
         len = depth;
-        for (int i = depth - 1; i >= 0; i--) { const BeamNode q = nodes[n]; out[i] = q.chr; n = q.parent; }
+        int n = C.node[tid];
+        for (int i = depth - 1; i >= 0; i--) { const BeamNode q = nodes[n]; row[i] = q.chr; n = q.parent; }
       }
-      p.decoded_len[b] = len;
-      if (p.ties) p.ties[b] = s_ovf ? -1 : s_ties;
-      s_need = len;
+      const long long o = (long long)b * NB + rank;
+      p.decoded_len[o] = len;
+      if (p.scores) {
+        const double lp = beam_lse(C.pnb[tid], C.pb[tid]);
+        p.scores[o] = beam_score(lp, C.nw[tid], p.wip);
+        if (p.log_probs) p.log_probs[o] = lp;
+      }
+      S.cgt[rank] = len;
     }
+  } else if (tid < NB) {                                 // fewer members than asked for: empty slots
+    const long long o = (long long)b * NB + tid;
+    p.decoded_len[o] = 0;
+    if (p.scores) { p.scores[o] = -INFINITY; if (p.log_probs) p.log_probs[o] = -INFINITY; }
+    S.cgt[tid] = 0;
   }
   __syncthreads();
-  for (int k = s_need + tid; k < p.T; k += kBeamThreads) out[k] = 0;
+  if (tid == 0 && p.ties) p.ties[b] = s_ovf ? -1 : s_ties + s_tie_now;
+  for (int i = tid; i < NB * p.T; i += kBeamThreads) {
+    const int r = i / p.T;
+    if (i - r * p.T >= S.cgt[r]) out[i] = 0;
+  }
 }
 
 size_t beam_smem_bytes(int V, int WB, size_t kc_cap) {
@@ -793,12 +807,14 @@ bool beam_supported(const e2e_ctc_desc& d, int beam_width) {
   return beam_width >= 1 && beam_width <= kBeamMaxWidth && beam_mode(d.alphabet, beam_width).ok;
 }
 
-int launch_beam(const e2e_ctc_desc& d, int beam_width, int space_idx, double wip, const void* logits, const void* in_len,
-                int64_t* decoded, int64_t* decoded_len, int64_t* ties, char* ws, cudaStream_t s) {
+int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
+                const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
+                char* ws, cudaStream_t s) {
   BeamParams p;
   p.logits = logits; p.dtype = d.dtype; p.sb = d.logits_stride_b; p.st = d.logits_stride_t;
   p.in_len = in_len; p.len_is64 = d.lengths_itype == E2E_I64;
   p.decoded = reinterpret_cast<long long*>(decoded); p.decoded_len = reinterpret_cast<long long*>(decoded_len);
+  p.scores = scores; p.log_probs = scores ? log_probs : nullptr; p.n_best = n_best;
   p.ties = reinterpret_cast<long long*>(ties);
   p.nodes = reinterpret_cast<BeamNode*>(ws);
   p.node_cap = (long long)d.max_frames * beam_width + 1;

@@ -4,9 +4,11 @@
 * greedy: ``decode`` with ``beam_width == 1`` and ``decode_greedy`` (decoders/ctc_decoder.py:92-93, 117-149;
   src/decoders/ctc_decoder.cpp:443-490);
 * prefix beam search WITHOUT a language model: ``decode`` with ``beam_width > 1`` and no ``lm_path``
-  (decoders/ctc_decoder.py:76-115; src/decoders/ctc_decoder.cpp:153-198, 353-441) -- SURVEY.md 8(f3).
+  (decoders/ctc_decoder.py:76-115; src/decoders/ctc_decoder.cpp:153-198, 353-441) -- SURVEY.md 8(f3);
+* the N best prefixes of that search with their scores: ``decode_nbest``, for rescoring with any language model on the
+  host (N-best rescoring).
 
-KenLM rescoring (``lm_path``) stays the reference's CPU code and is out of scope; asking for it here raises
+KenLM decoding (``lm_path``) stays the reference's CPU code and is out of scope; asking for it here raises
 ``NotImplementedError`` instead of silently decoding without the model.
 """
 from collections import namedtuple
@@ -23,6 +25,12 @@ class CTCDecoderError(Exception):
 DecoderResults = namedtuple("DecoderResults", ["decoded_targets",
                                                "decoded_targets_lengths",
                                                "decoded_sentences"])
+
+NBestResults = namedtuple("NBestResults", ["decoded_targets",
+                                           "decoded_targets_lengths",
+                                           "decoded_sentences",
+                                           "scores",
+                                           "log_probs"])
 
 
 class CTCDecoder:
@@ -77,6 +85,37 @@ class CTCDecoder:
             logits_=logits, logits_lengths_=logits_lengths, from_logits=not self._after_logsoftmax)
         decoded_sentences = self._sentences(decoded_targets, decoded_targets_lengths)
         return DecoderResults(decoded_targets, decoded_targets_lengths, decoded_sentences)
+
+    def decode_nbest(self, logits, logits_lengths=None, *, n_best):
+        """The ``n_best`` best prefixes of the LM-free prefix beam search and their scores, for rescoring with a
+        language model of the caller's choice.  Always the prefix beam search: with ``beam_width == 1`` that is a
+        beam of width 1, not the greedy path ``decode`` takes.
+
+        :param logits: as for ``decode``
+        :param logits_lengths: ``(B,)`` or ``None`` (decode all frames)
+        :param n_best: ``1 <= n_best <= beam_width``
+        :return: ``NBestResults(decoded_targets [B, N, longest hypothesis] int64 zero padded, decoded_targets_lengths
+            [B, N] int64, decoded_sentences list[B] of list[N] str, scores [B, N] float64, log_probs [B, N] float64)``
+            -- CPU tensors.  Hypotheses are ranked by ``scores = log_probs - number of words * wip``, highest first
+            (equal scores in beam order), so hypothesis 0 is what ``decode`` returns for ``beam_width > 1``;
+            ``log_probs`` is the prefix's acoustic log-probability without the word penalty.  The empty prefix is the
+            single symbol ``-1`` with length 1, as in ``decode``; slots past the number of prefixes the final beam
+            holds (short utterances, tiny alphabets) have length 0, sentence ``""`` and ``-inf`` scores
+        """
+        if self._lm_path:
+            raise NotImplementedError(
+                "decoding with a KenLM language model stays the reference's CPU code and is outside this engine's "
+                "scope; construct CTCDecoder without lm_path and rescore the decode_nbest list with the model")
+        if not 1 <= int(n_best) <= self._decoder.beam_width:
+            raise ValueError("n_best %d outside [1, beam_width = %d]" % (int(n_best), self._decoder.beam_width))
+        if self._time_major:
+            logits = logits.transpose(1, 0)
+        decoded_targets, decoded_targets_lengths, scores, log_probs = self._decoder.decode_nbest(
+            logits, logits_lengths, n_best=int(n_best), from_logits=not self._after_logsoftmax)
+        B, N = decoded_targets_lengths.shape
+        flat = self._sentences(decoded_targets.reshape(B * N, -1), decoded_targets_lengths.reshape(-1))
+        decoded_sentences = [flat[b * N:(b + 1) * N] for b in range(B)]
+        return NBestResults(decoded_targets, decoded_targets_lengths, decoded_sentences, scores, log_probs)
 
     def decode_greedy(self, logits, logits_lengths=None):
         """

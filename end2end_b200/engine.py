@@ -658,3 +658,75 @@ class CTCBeamEngine(CTCGreedyEngine):
         # ctc_decoder.cpp:186-196: the result matrix is as wide as the longest decoded sequence
         width = int(lengths.max()) if lengths.numel() else 0
         return decoded[:, :width].contiguous(), lengths
+
+    def _n_best(self, n_best):
+        n_best = self.beam_width if n_best is None else int(n_best)
+        if not 1 <= n_best <= self.beam_width:
+            raise ValueError("n_best %d outside [1, beam_width = %d]" % (n_best, self.beam_width))
+        return n_best
+
+    def decode_nbest_device(self, logits, logits_lengths=None, n_best=None, from_logits=False):
+        """The ``n_best`` best prefixes of the same search (default: the whole final beam), device tensors in, device
+        tensors out (no synchronisation): ``(decoded [B,N,T] int64 zero padded, lengths [B,N], scores [B,N] float64,
+        log_probs [B,N] float64, ties [B])``.  Ranked by ``scores = log_probs - words * wip``, highest first, equal
+        scores in beam order; hypothesis 0 is what ``decode_device`` returns.  Slots past the number of prefixes in
+        the final beam have length 0 and ``-inf`` scores (see include/e2e_ctc.h)."""
+        _require_cuda()
+        n_best = self._n_best(n_best)
+        logits = logits.detach()
+        dev = logits.device
+        if not _dense3(logits):
+            logits = logits.contiguous()
+        if logits_lengths is not None:
+            logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
+        d = self._beam_desc(logits, logits_lengths, from_logits)
+        B, T = logits.size(0), logits.size(1)
+        with _on_device(dev):
+            need = self._L.e2e_ctc_beam_nbest_workspace_bytes(ctypes.byref(d), self.beam_width, n_best)
+            if need == 0:
+                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            decoded = torch.empty(B, n_best, T, dtype=torch.int64, device=dev)
+            lengths = torch.empty(B, n_best, dtype=torch.int64, device=dev)
+            scores = torch.empty(B, n_best, dtype=torch.float64, device=dev)
+            log_probs = torch.empty(B, n_best, dtype=torch.float64, device=dev)
+            ties = torch.empty(B, dtype=torch.int64, device=dev)
+            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            _lib.check(self._L.e2e_ctc_beam_nbest_device(
+                ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip, _ptr(logits), _ptr(logits_lengths),
+                _ptr(decoded), _ptr(lengths), _ptr(scores), _ptr(log_probs), _ptr(ties), _ptr(ws), ws.numel(),
+                _stream(dev)))
+        return decoded, lengths, scores, log_probs, ties
+
+    def decode_nbest(self, logits_, logits_lengths_=None, n_best=None, from_logits=False):
+        """``decode_nbest_device`` for CPU or CUDA input, CPU results (CPU input goes through the host engine, as in
+        ``decode``): ``(decoded [B,N,longest hypothesis], lengths [B,N], scores [B,N], log_probs [B,N])``;
+        ``last_ties`` holds the tie counters."""
+        _require_cuda()
+        n_best = self._n_best(n_best)
+        logits = logits_.detach()
+        if logits.is_cuda:
+            out = self.decode_nbest_device(logits, logits_lengths_, n_best, from_logits)
+            decoded, lengths, scores, log_probs, ties = (t.cpu() for t in out)
+        else:
+            if not (logits.is_contiguous() or logits.permute(1, 0, 2).is_contiguous()):
+                logits = logits.contiguous()
+            lengths_in = None
+            if logits_lengths_ is not None:
+                lengths_in = _as_index(logits_lengths_, torch.device("cpu"), "logits_lengths").contiguous()
+            d = self._beam_desc(logits, lengths_in, from_logits)
+            B, T = logits.size(0), logits.size(1)
+            decoded = torch.empty(B, n_best, T, dtype=torch.int64, pin_memory=True)
+            lengths = torch.empty(B, n_best, dtype=torch.int64, pin_memory=True)
+            scores = torch.empty(B, n_best, dtype=torch.float64, pin_memory=True)
+            log_probs = torch.empty(B, n_best, dtype=torch.float64, pin_memory=True)
+            ties = torch.empty(B, dtype=torch.int64, pin_memory=True)
+            dev = torch.cuda.current_device()
+            h = self._host.get(dev)
+            if h is None:
+                h = self._host[dev] = _HostEngine(dev)
+            _lib.check(self._L.e2e_ctc_engine_beam_nbest_host(
+                h.handle, ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip, _ptr(logits),
+                _ptr(lengths_in), _ptr(decoded), _ptr(lengths), _ptr(scores), _ptr(log_probs), _ptr(ties)))
+        self.last_ties = ties
+        width = int(lengths.max()) if lengths.numel() else 0
+        return decoded[:, :, :width].contiguous(), lengths, scores, log_probs

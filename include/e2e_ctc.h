@@ -259,6 +259,30 @@ int e2e_ctc_beam_decode_device(const e2e_ctc_desc* desc, int32_t beam_width, int
                                int64_t* decoded_lengths, int64_t* ties, void* workspace, size_t workspace_bytes,
                                void* cuda_stream);
 
+/* The N best prefixes of the same search and their scores: what a caller needs to rescore the list with a language model
+ * of its own (N-best rescoring).  Nothing in the search changes: after the last frame the beam_width final prefixes are
+ * ranked, and the first n_best are returned.  e2e_ctc_beam_decode_device is the n_best == 1 call.
+ *   ranking: by score = log p(prefix) - num_words * wip, highest first; among EQUAL scores the lower position in the
+ *       final beam goes first (the rule of the best-1 pick above).  Hypothesis 0 is what e2e_ctc_beam_decode_device
+ *       returns;
+ *   n_best: 1 <= n_best <= beam_width (E2E_ERR_INVALID_ARGUMENT otherwise; the workspace query then returns 0);
+ *   decoded: [B,N,T] int64 zero padded; decoded_lengths: [B,N] int64.  The empty prefix is the single symbol -1 with
+ *       length 1, as above;
+ *   scores: [B,N] float64, the ranking score log p - num_words * wip;
+ *   log_probs (optional, [B,N] float64): log p(prefix) = log(p_blank + p_not_blank), without the word penalty;
+ *   slots past the number of prefixes in the final beam (short utterances, tiny alphabets): length 0, all-zero
+ *       symbols, scores = log_probs = -inf;
+ *   ties (optional, [B] int64): the prune ties counted as above, plus 1 when the returned list depends on equal final
+ *       scores (a prefix of rank < N has the same score as another prefix of the final beam; for N = 1 that is the
+ *       final-pick tie above); -1, as for e2e_ctc_beam_decode_device, when the list of pruned prefixes that still
+ *       block an extension overflowed.
+ * The workspace is the same as e2e_ctc_beam_workspace_bytes(desc, beam_width). */
+size_t e2e_ctc_beam_nbest_workspace_bytes(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best);
+int e2e_ctc_beam_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx, double wip,
+                              const void* logits, const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths,
+                              double* scores, double* log_probs, int64_t* ties, void* workspace, size_t workspace_bytes,
+                              void* cuda_stream);
+
 /* -------------------------------------------------------------- engine, host pointers ------ */
 
 typedef struct e2e_ctc_engine e2e_ctc_engine;
@@ -285,6 +309,12 @@ int e2e_ctc_engine_greedy_host(e2e_ctc_engine* engine, const e2e_ctc_desc* desc,
 int e2e_ctc_engine_beam_host(e2e_ctc_engine* engine, const e2e_ctc_desc* desc, int32_t beam_width, int32_t space_idx,
                              double wip, const void* logits, const void* logits_lengths, int64_t* decoded,
                              int64_t* decoded_lengths, int64_t* ties);
+
+/* Host-buffer form of the N-best list (see e2e_ctc_beam_nbest_device); log_probs and ties may be NULL. */
+int e2e_ctc_engine_beam_nbest_host(e2e_ctc_engine* engine, const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best,
+                                   int32_t space_idx, double wip, const void* logits, const void* logits_lengths,
+                                   int64_t* decoded, int64_t* decoded_lengths, double* scores, double* log_probs,
+                                   int64_t* ties);
 
 /* Pinned (page-locked, device-addressable) host memory for result buffers: when `losses` / `grads` of
  * e2e_ctc_engine_loss_host live in such memory the kernels store into them directly and no copy-out stage runs. */
