@@ -677,6 +677,47 @@ int e2e_ctc_beam_decode_device(const e2e_ctc_desc* desc, int32_t beam_width, int
                      ties, reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
+// ---- CTC log-likelihood of N hypotheses per utterance (K9) -------------------------------------------
+static int check_score(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  int rc = check_desc(desc, true);
+  if (rc != E2E_OK) return rc;
+  if (n_hyp < 1) { set_error("n_hyp %d < 1", n_hyp); return E2E_ERR_INVALID_ARGUMENT; }
+  if (desc->max_targets > 0 && desc->targets_stride_b < desc->max_targets) {
+    set_error("hypothesis row stride %lld < max_targets %d", (long long)desc->targets_stride_b, desc->max_targets);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  if (desc->logits_stride_b < 0 || desc->logits_stride_t < 0) { set_error("negative logits stride"); return E2E_ERR_INVALID_ARGUMENT; }
+  if ((long long)desc->batch * n_hyp > 0x7fffffffLL) {
+    set_error("batch %d x n_hyp %d hypotheses exceed this build's limit", desc->batch, n_hyp);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  if (!score_supported(*desc)) {
+    set_error("score: max_targets %d with alphabet %d does not fit shared memory", desc->max_targets, desc->alphabet);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  return E2E_OK;
+}
+
+size_t e2e_ctc_score_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  if (check_score(desc, n_hyp) != E2E_OK) return 0;
+  return 256;   // nothing is stashed; 0 stays the "unsupported" answer
+}
+
+int e2e_ctc_score_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                         const void* logits_lengths, const void* hyp_lengths, double* scores, void* workspace,
+                         size_t workspace_bytes, void* cuda_stream) {
+  int rc = check_score(desc, n_hyp);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !hyp_lengths || !scores || (!hyps && desc->max_targets > 0)) {
+    set_error("null pointer argument");
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  rc = check_ws(workspace, workspace_bytes, e2e_ctc_score_workspace_bytes(desc, n_hyp));
+  if (rc != E2E_OK) return rc;
+  return launch_score(*desc, n_hyp, logits, hyps, logits_lengths, hyp_lengths, scores,
+                      reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
 // ---- pinned host memory for result buffers -------------------------------------------------------
 // The host-buffer entry points write their results straight into PINNED caller buffers (see e2e_ctc_engine_loss_host);
 // a binding that has no pinned allocator of its own takes its result buffers from here.

@@ -112,7 +112,7 @@ constexpr int kFlagInfeasible = 1, kFlagInvalid = 2;
 void set_error(const char* fmt, ...);
 
 // Launch accounting + optional per-kernel device timing (CUDA events on the launching stream).
-enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kNumKernels };
+enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kNumKernels };
 void launch_begin(int kind, cudaStream_t s);
 void launch_end(int kind, cudaStream_t s);
 struct KernelTimer {   // brackets exactly one kernel launch
@@ -252,6 +252,10 @@ bool beam_supported(const e2e_ctc_desc& d, int beam_width);
 int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
                 const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
                 char* ws, cudaStream_t s);
+// N hypotheses per utterance: hyps [B * n_hyp, max_targets], hyp_len [B * n_hyp], scores [B * n_hyp] = -(CTC loss)
+bool score_supported(const e2e_ctc_desc& d);
+int launch_score(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
+                 const void* hyp_len, double* scores, cudaStream_t s);
 size_t noblank_workspace_bytes(const e2e_ctc_desc& d);
 bool noblank_supported(const e2e_ctc_desc& d);
 int launch_noblank(const e2e_ctc_desc& d, int space_idx, const void* lp, const void* targets, const void* in_len,

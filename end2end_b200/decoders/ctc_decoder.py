@@ -6,7 +6,8 @@
 * prefix beam search WITHOUT a language model: ``decode`` with ``beam_width > 1`` and no ``lm_path``
   (decoders/ctc_decoder.py:76-115; src/decoders/ctc_decoder.cpp:153-198, 353-441) -- SURVEY.md 8(f3);
 * the N best prefixes of that search with their scores: ``decode_nbest``, for rescoring with any language model on the
-  host (N-best rescoring).
+  host (N-best rescoring);
+* the exact CTC log-likelihood of given transcripts, N per utterance: ``score`` (``decode_nbest``'s list or any other).
 
 KenLM decoding (``lm_path``) stays the reference's CPU code and is out of scope; asking for it here raises
 ``NotImplementedError`` instead of silently decoding without the model.
@@ -116,6 +117,32 @@ class CTCDecoder:
         flat = self._sentences(decoded_targets.reshape(B * N, -1), decoded_targets_lengths.reshape(-1))
         decoded_sentences = [flat[b * N:(b + 1) * N] for b in range(B)]
         return NBestResults(decoded_targets, decoded_targets_lengths, decoded_sentences, scores, log_probs)
+
+    def score(self, logits, hypotheses, hypotheses_lengths, logits_lengths=None):
+        """The CTC log-likelihood ``log p(hypothesis | logits)`` of N transcripts per utterance: minus the CTC loss of each
+        (utterance, hypothesis) pair, summed over every alignment -- where ``decode_nbest``'s ``log_probs`` sums only the
+        alignments that survived the beam.  Forward only, on the GPU; the utterance's frames are read and normalised once
+        for several hypotheses, not once per hypothesis.
+
+        :param logits: as for ``decode`` (``time_major``, ``after_logsoftmax`` and ``blank_idx`` apply)
+        :param hypotheses: ``(B, N, max length)`` int32 / int64 labels, zero padded; ``decode_nbest``'s
+            ``decoded_targets`` as they come
+        :param hypotheses_lengths: ``(B, N)``; the single symbol ``-1`` with length 1 (``decode``'s empty result) is the
+            empty hypothesis
+        :param logits_lengths: ``(B,)`` or ``None`` (all frames)
+        :return: ``(B, N)`` float64 CPU tensor.  An infeasible hypothesis (more labels and repeats than frames) scores
+            ``-inf``; the empty hypothesis scores ``sum_t log p(blank | t)``.  Slots ``decode_nbest`` left unused
+            (length 0) score as the empty transcript: mask them with ``nbest.scores == -inf``
+        """
+        if self._time_major:
+            logits = logits.transpose(1, 0)
+        if hypotheses.dim() == 3 and hypotheses.size(2) > 0 and hypotheses_lengths.shape == hypotheses.shape[:2]:
+            # decode's empty result, [-1] with length 1, is the empty hypothesis (no sync: an element-wise select)
+            dev = hypotheses_lengths.device
+            empty = (hypotheses[:, :, 0].to(dev) == -1) & (hypotheses_lengths == 1)
+            hypotheses_lengths = torch.where(empty, torch.zeros_like(hypotheses_lengths), hypotheses_lengths)
+        return self._decoder.score_device(logits, hypotheses, hypotheses_lengths, logits_lengths,
+                                          from_logits=not self._after_logsoftmax).cpu()
 
     def decode_greedy(self, logits, logits_lengths=None):
         """

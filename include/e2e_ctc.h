@@ -283,6 +283,29 @@ int e2e_ctc_beam_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int3
                               double* scores, double* log_probs, int64_t* ties, void* workspace, size_t workspace_bytes,
                               void* cuda_stream);
 
+/* ------------------------------------------------------- N hypotheses per utterance: score ---- */
+
+/* The CTC log-likelihood log p(y | x) of n_hyp hypotheses per utterance, forward only (no gradient, nothing kept for a
+ * backward): scores[b * n_hyp + n] = minus the loss of e2e_ctc_loss_forward_device for utterance b with hypothesis n as
+ * its target.  For rescoring N-best lists (this library's or another system's), confidence and verification scores.
+ *   hyps: [B * n_hyp, max_targets] of targets_itype, row stride desc->targets_stride_b; row b * n_hyp + n is hypothesis
+ *       n of utterance b (NULL allowed when max_targets == 0);
+ *   hyp_lengths: [B * n_hyp] of lengths_itype, 0 <= length <= max_targets (0: the empty hypothesis, which scores
+ *       sum_t log p(blank | t));
+ *   logits_lengths: [B] of lengths_itype, or NULL for max_frames;
+ *   scores: [B * n_hyp] float64 whatever desc->dtype.  An infeasible hypothesis (T_b < L + repeats) scores -inf.
+ *       A hypothesis length outside [0, max_targets] or a label outside [0, alphabet) gives that hypothesis NaN; a
+ *       logits length outside [1, max_frames] gives every hypothesis of the utterance NaN.  Nothing out of range is read.
+ *   desc->from_logits: the row log-softmax of the loss and the beam search, (x - max) - log sum exp in the input's
+ *       precision, rounded to the input dtype for 16-bit inputs; the lattice is fp64.
+ * Limits: max_targets <= e2e_ctc_limits.max_targets (639) and alphabet <= e2e_ctc_limits.max_alphabet; beyond them, or
+ * with n_hyp < 1, the workspace query returns 0 and sets the error message.  The kernel needs no scratch memory: the
+ * query returns 256 bytes within the limits, and the workspace pointer is checked like every other one. */
+size_t e2e_ctc_score_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp);
+int e2e_ctc_score_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                         const void* logits_lengths, const void* hyp_lengths, double* scores, void* workspace,
+                         size_t workspace_bytes, void* cuda_stream);
+
 /* -------------------------------------------------------------- engine, host pointers ------ */
 
 typedef struct e2e_ctc_engine e2e_ctc_engine;
@@ -334,7 +357,7 @@ uint64_t e2e_ctc_launch_count(void);
  * bracketed by CUDA events on its launching stream.  e2e_ctc_profile_read() waits for the pending
  * events, then fills ms[k] (summed device milliseconds) and launches[k] per kernel kind
  * k = 0 row_stats, 1 lattice, 2 gradient, 3 loss_reduce, 4 argmax, 5 collapse, 6 scale_rows, 7 viterbi,
- * 8 ctc_without_blank, 9 beam_search, 10 order (n_kinds >= 11),
+ * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score (n_kinds >= 12),
  * and clears the record.  All launches since the previous read must have been made on ONE device. */
 int e2e_ctc_profile_enable(int32_t on);
 int e2e_ctc_profile_read(double* ms, uint64_t* launches, int32_t n_kinds);

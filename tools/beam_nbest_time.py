@@ -53,15 +53,16 @@ def child(lib_path, launches, with_nbest):
         for _ in range(2):
             launch()
         torch.cuda.synchronize()
-        ms = (ctypes.c_double * 11)()
-        cnt = (ctypes.c_uint64 * 11)()
+        n_kinds = len(_lib.KERNEL_KINDS)
+        ms = (ctypes.c_double * n_kinds)()
+        cnt = (ctypes.c_uint64 * n_kinds)()
         ok(L.e2e_ctc_profile_enable(1))
-        ok(L.e2e_ctc_profile_read(ms, cnt, 11))
+        ok(L.e2e_ctc_profile_read(ms, cnt, n_kinds))
         for _ in range(launches):
             flush.add_(1)
             launch()
         torch.cuda.synchronize()
-        ok(L.e2e_ctc_profile_read(ms, cnt, 11))
+        ok(L.e2e_ctc_profile_read(ms, cnt, n_kinds))
         ok(L.e2e_ctc_profile_enable(0))
         assert cnt[KIND_BEAM] == launches, cnt[KIND_BEAM]
         return ms[KIND_BEAM] / launches
