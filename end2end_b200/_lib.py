@@ -33,6 +33,7 @@ EXPORTS = (
     "e2e_ctc_beam_workspace_bytes", "e2e_ctc_beam_decode_device", "e2e_ctc_engine_beam_host",
     "e2e_ctc_beam_nbest_workspace_bytes", "e2e_ctc_beam_nbest_device", "e2e_ctc_engine_beam_nbest_host",
     "e2e_ctc_score_workspace_bytes", "e2e_ctc_score_device",
+    "e2e_ctc_align_nbest_workspace_bytes", "e2e_ctc_align_nbest_device",
 )
 KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score")
 
@@ -131,6 +132,10 @@ def load():
     L.e2e_ctc_score_workspace_bytes.restype = sz
     L.e2e_ctc_score_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, sz, vp]
     L.e2e_ctc_score_device.restype = ctypes.c_int
+    L.e2e_ctc_align_nbest_workspace_bytes.argtypes = [dp, i32]
+    L.e2e_ctc_align_nbest_workspace_bytes.restype = sz
+    L.e2e_ctc_align_nbest_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    L.e2e_ctc_align_nbest_device.restype = ctypes.c_int
     L.e2e_ctc_host_alloc.argtypes = [sz, ctypes.POINTER(vp)]
     L.e2e_ctc_host_alloc.restype = ctypes.c_int
     L.e2e_ctc_host_free.argtypes = [vp]

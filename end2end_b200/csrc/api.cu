@@ -745,7 +745,7 @@ static int check_viterbi(const e2e_ctc_desc* desc, int32_t is_ctc) {
 
 size_t e2e_ctc_viterbi_workspace_bytes(const e2e_ctc_desc* desc, int32_t is_ctc) {
   if (check_viterbi(desc, is_ctc) != E2E_OK) return 0;
-  return align256(viterbi_workspace_bytes(*desc, is_ctc ? 1 : 0));
+  return align256(viterbi_workspace_bytes(*desc, is_ctc ? 1 : 0, 1, 0));
 }
 
 int e2e_ctc_viterbi_align_device(const e2e_ctc_desc* desc, int32_t is_ctc, const void* log_probs, const void* targets,
@@ -759,8 +759,49 @@ int e2e_ctc_viterbi_align_device(const e2e_ctc_desc* desc, int32_t is_ctc, const
   }
   rc = check_ws(workspace, workspace_bytes, e2e_ctc_viterbi_workspace_bytes(desc, is_ctc));
   if (rc != E2E_OK) return rc;
-  return launch_viterbi(*desc, is_ctc ? 1 : 0, log_probs, targets, logits_lengths, targets_lengths, aligned,
-                        reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
+  return launch_viterbi(*desc, is_ctc ? 1 : 0, 1, 0, log_probs, targets, logits_lengths, targets_lengths, aligned, nullptr,
+                        nullptr, nullptr, reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+// ---- Viterbi alignment of N hypotheses per utterance (K1 + K6) ---------------------------------------------------------
+static int check_align_nbest(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  int rc = check_viterbi(desc, 1);
+  if (rc != E2E_OK) return rc;
+  if (n_hyp < 1) { set_error("n_hyp %d < 1", n_hyp); return E2E_ERR_INVALID_ARGUMENT; }
+  if (desc->max_targets > 0 && desc->targets_stride_b < desc->max_targets) {
+    set_error("hypothesis row stride %lld < max_targets %d", (long long)desc->targets_stride_b, desc->max_targets);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  if (desc->logits_stride_b < 0 || desc->logits_stride_t < 0) { set_error("negative logits stride"); return E2E_ERR_INVALID_ARGUMENT; }
+  if ((long long)desc->batch * n_hyp > 0x7fffffffLL) {
+    set_error("batch %d x n_hyp %d lattices exceed the grid (2^31 - 1 CTAs)", desc->batch, n_hyp);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  return E2E_OK;
+}
+
+size_t e2e_ctc_align_nbest_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  if (check_align_nbest(desc, n_hyp) != E2E_OK) return 0;
+  return align256(viterbi_workspace_bytes(*desc, 1, n_hyp, desc->from_logits ? 1 : 0));   // 0 (message set) on overflow
+}
+
+int e2e_ctc_align_nbest_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                               const void* logits_lengths, const void* hyp_lengths, int64_t* aligned, int64_t* token_starts,
+                               int64_t* token_ends, double* path_scores, void* workspace, size_t workspace_bytes,
+                               void* cuda_stream) {
+  int rc = check_align_nbest(desc, n_hyp);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !hyp_lengths || !aligned || !path_scores || (desc->max_targets > 0 && (!hyps || !token_starts || !token_ends))) {
+    set_error("null pointer argument");
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  const size_t need = e2e_ctc_align_nbest_workspace_bytes(desc, n_hyp);
+  if (need == 0) return E2E_ERR_UNSUPPORTED;
+  rc = check_ws(workspace, workspace_bytes, need);
+  if (rc != E2E_OK) return rc;
+  return launch_viterbi(*desc, 1, n_hyp, desc->from_logits ? 1 : 0, logits, hyps, logits_lengths, hyp_lengths, aligned,
+                        desc->max_targets > 0 ? token_starts : nullptr, desc->max_targets > 0 ? token_ends : nullptr,
+                        path_scores, reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 // ---- CTC without blank (SURVEY 8(f4)) ---------------------------------------------------------------

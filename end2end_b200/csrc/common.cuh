@@ -192,6 +192,16 @@ __device__ __forceinline__ void store_from_double(void* base, int dtype, long lo
   }
 }
 
+// torch's row log-softmax, (x - max) - log sum exp(x - max), in the input's accumulation type; rounded to the input dtype
+// for 16-bit inputs, as F.log_softmax returns it (the rule of the beam search, the scorer and the aligner)
+template <typename T>
+__device__ __forceinline__ double normalise(typename Elem<T>::acc_t x, typename Elem<T>::acc_t m, typename Elem<T>::acc_t ls) {
+  using raw_t = typename Elem<T>::acc_t;
+  raw_t v = (x - m) - ls;
+  if (sizeof(T) == 2) { T r; Elem<T>::store(&r, (float)v); v = (raw_t)Elem<T>::get(r); }
+  return (double)v;
+}
+
 // 2^d as a double; 0 below the normal range, clamped above.
 __device__ __forceinline__ double pow2i(int d) {
   d = min(d, 1023);
@@ -260,9 +270,13 @@ size_t noblank_workspace_bytes(const e2e_ctc_desc& d);
 bool noblank_supported(const e2e_ctc_desc& d);
 int launch_noblank(const e2e_ctc_desc& d, int space_idx, const void* lp, const void* targets, const void* in_len,
                    const void* tgt_len, void* losses, void* grads, char* ws, cudaStream_t s);
-size_t viterbi_workspace_bytes(const e2e_ctc_desc& d, int is_ctc);
+// n_hyp lattices per utterance: targets [B * n_hyp, max_targets], tgt_len [B * n_hyp], aligned [B * n_hyp, T];
+// from_logits: raw-logit input (K1 statistics in the workspace); token spans [B * n_hyp, max_targets] and path scores
+// [B * n_hyp] are optional (CTC only).  Workspace: 0 when the size overflows size_t (message set).
+size_t viterbi_workspace_bytes(const e2e_ctc_desc& d, int is_ctc, int n_hyp, int from_logits);
 bool viterbi_supported(const e2e_ctc_desc& d, int is_ctc);
-int launch_viterbi(const e2e_ctc_desc& d, int is_ctc, const void* lp, const void* targets, const void* in_len,
-                   const void* tgt_len, int64_t* aligned, char* ws, cudaStream_t s);
+int launch_viterbi(const e2e_ctc_desc& d, int is_ctc, int n_hyp, int from_logits, const void* lp, const void* targets,
+                   const void* in_len, const void* tgt_len, int64_t* aligned, int64_t* token_starts, int64_t* token_ends,
+                   double* path_scores, char* ws, cudaStream_t s);
 
 }  // namespace e2e

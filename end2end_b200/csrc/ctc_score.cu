@@ -63,16 +63,6 @@ __device__ __forceinline__ double lse2(double a, double b) {
   return a > b ? a + log(1.0 + exp(b - a)) : b + log(1.0 + exp(a - b));
 }
 
-// torch's row log-softmax, (x - max) - log sum exp(x - max), in the input's accumulation type; rounded to the input dtype
-// for 16-bit inputs, as F.log_softmax returns it (the beam kernel's rule, ctc_beam.cu)
-template <typename T>
-__device__ __forceinline__ double normalise(typename Elem<T>::acc_t x, typename Elem<T>::acc_t m, typename Elem<T>::acc_t ls) {
-  using raw_t = typename Elem<T>::acc_t;
-  raw_t v = (x - m) - ls;
-  if (sizeof(T) == 2) { T r; Elem<T>::store(&r, (float)v); v = (raw_t)Elem<T>::get(r); }
-  return (double)v;
-}
-
 // max and log sum exp of one row, reduced by one warp
 template <typename T>
 __device__ __forceinline__ void row_stats(const T* r, int V, int lane, typename Elem<T>::acc_t* m_out,

@@ -7,7 +7,9 @@
   (decoders/ctc_decoder.py:76-115; src/decoders/ctc_decoder.cpp:153-198, 353-441) -- SURVEY.md 8(f3);
 * the N best prefixes of that search with their scores: ``decode_nbest``, for rescoring with any language model on the
   host (N-best rescoring);
-* the exact CTC log-likelihood of given transcripts, N per utterance: ``score`` (``decode_nbest``'s list or any other).
+* the exact CTC log-likelihood of given transcripts, N per utterance: ``score`` (``decode_nbest``'s list or any other);
+* timestamps of given transcripts, N per utterance: ``align`` -- the best path, each token's frame span, word spans and
+  the best path's log-probability.
 
 KenLM decoding (``lm_path``) stays the reference's CPU code and is out of scope; asking for it here raises
 ``NotImplementedError`` instead of silently decoding without the model.
@@ -16,7 +18,7 @@ from collections import namedtuple
 
 import torch
 
-from ..engine import CTCBeamEngine
+from ..engine import ALIGN_MAX_TARGETS, CTCBeamEngine
 
 
 class CTCDecoderError(Exception):
@@ -32,6 +34,30 @@ NBestResults = namedtuple("NBestResults", ["decoded_targets",
                                            "decoded_sentences",
                                            "scores",
                                            "log_probs"])
+
+AlignmentResults = namedtuple("AlignmentResults", ["alignments",
+                                                   "token_starts",
+                                                   "token_ends",
+                                                   "path_scores",
+                                                   "word_spans"])
+
+
+def word_spans(tokens, starts, ends, labels):
+    """``[(word, start_frame, end_frame)]`` of one aligned hypothesis: a word is a maximal run of tokens other than the
+    label ``" "``; it spans from its first token's start to its last token's end (``-1`` where the path had no finite
+    score).  ``tokens``, ``starts`` and ``ends`` are lists over the hypothesis's tokens."""
+    out, word = [], None
+    for tok, t0, t1 in zip(tokens, starts, ends):
+        sym = labels[tok]
+        if sym == " ":
+            word = None
+        elif word is None:
+            word = [sym, t0, t1]
+            out.append(word)
+        else:
+            word[0] += sym
+            word[2] = t1
+    return [tuple(w) for w in out]
 
 
 class CTCDecoder:
@@ -143,6 +169,52 @@ class CTCDecoder:
             hypotheses_lengths = torch.where(empty, torch.zeros_like(hypotheses_lengths), hypotheses_lengths)
         return self._decoder.score_device(logits, hypotheses, hypotheses_lengths, logits_lengths,
                                           from_logits=not self._after_logsoftmax).cpu()
+
+    def align(self, logits, hypotheses, hypotheses_lengths, logits_lengths=None):
+        """Timestamps of N transcripts per utterance: the best-path (Viterbi) alignment of each (utterance, hypothesis) pair,
+        each token's frame span, word spans and the best path's log-probability, on the GPU.  The utterance's frames are
+        read once for all of its hypotheses.  Times are frames: converting them to seconds takes the model's frame shift,
+        which the decoder does not know.
+
+        :param logits: as for ``decode`` (``time_major``, ``after_logsoftmax`` and ``blank_idx`` apply)
+        :param hypotheses: ``(B, N, max length)`` int32 / int64 labels, zero padded (``decode_nbest``'s
+            ``decoded_targets`` as they come), or ``(B, max length)`` for one hypothesis per utterance (``decode`` /
+            ``decode_greedy``'s ``decoded_targets``)
+        :param hypotheses_lengths: ``(B, N)`` or ``(B,)`` to match; the single symbol ``-1`` with length 1 (``decode``'s
+            empty result) is the empty hypothesis, and so are the slots ``decode_nbest`` left unused (length 0): mask
+            them with ``nbest.scores == -inf``
+        :param logits_lengths: ``(B,)`` or ``None`` (all frames)
+        :return: ``AlignmentResults(alignments [B, N, T] int64, token_starts [B, N, Lmax] int64, token_ends [B, N, Lmax]
+            int64, path_scores [B, N] float64, word_spans)`` -- CPU tensors.  ``alignments`` holds the label id of every
+            frame on the best path (``-100`` past the utterance's frames), as ``get_alignment_3d`` does; token ``k`` of a
+            hypothesis covers the frames ``[token_starts, token_ends)`` (``-1`` past its length); ``path_scores`` is the
+            best path's log-probability, ``<= score`` (the sum over all paths).  An infeasible hypothesis (more labels
+            and repeats than frames) has ``-inf`` and spans of ``-1``.  ``word_spans[b][n]`` is a list of ``(word,
+            start_frame, end_frame)``, words being runs of tokens between ``" "`` labels; ``None`` without ``labels``.
+            ``Lmax`` is the width of ``hypotheses``; a width past the aligner's limit (1023) is cut to the longest
+            hypothesis
+        """
+        if self._time_major:
+            logits = logits.transpose(1, 0)
+        if hypotheses.dim() == 2:                       # one hypothesis per utterance: decode's / decode_greedy's result
+            hypotheses, hypotheses_lengths = hypotheses[:, None], hypotheses_lengths.reshape(-1, 1)
+        if hypotheses.dim() == 3 and hypotheses.size(2) > 0 and hypotheses_lengths.shape == hypotheses.shape[:2]:
+            # decode's empty result, [-1] with length 1, is the empty hypothesis (no sync: an element-wise select)
+            dev = hypotheses_lengths.device
+            empty = (hypotheses[:, :, 0].to(dev) == -1) & (hypotheses_lengths == 1)
+            hypotheses_lengths = torch.where(empty, torch.zeros_like(hypotheses_lengths), hypotheses_lengths)
+            if hypotheses.size(2) > ALIGN_MAX_TARGETS and hypotheses_lengths.numel():
+                hypotheses = hypotheses[:, :, :max(int(hypotheses_lengths.max()), 0)]
+        aligned, starts, ends, path_scores = (t.cpu() for t in self._decoder.align_device(
+            logits, hypotheses, hypotheses_lengths, logits_lengths, from_logits=not self._after_logsoftmax))
+        spans = None
+        if self._labels:
+            B, N = path_scores.shape
+            hyps, lens = hypotheses.cpu().tolist(), hypotheses_lengths.cpu().tolist()
+            s0, s1 = starts.tolist(), ends.tolist()
+            spans = [[word_spans(hyps[b][n][:lens[b][n]], s0[b][n], s1[b][n], self._labels) for n in range(N)]
+                     for b in range(B)]
+        return AlignmentResults(aligned, starts, ends, path_scores, spans)
 
     def decode_greedy(self, logits, logits_lengths=None):
         """

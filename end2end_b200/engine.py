@@ -72,6 +72,8 @@ def _as_index(t, device, name):
 
 
 _LIMITS = None
+#: longest hypothesis the Viterbi aligner takes (csrc/ctc_viterbi.cu: lattices of at most 2048 cells, 2 L + 1 for CTC)
+ALIGN_MAX_TARGETS = 1023
 
 
 def _limits():
@@ -806,3 +808,85 @@ class CTCBeamEngine(CTCGreedyEngine):
                 ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(scores),
                 _ptr(ws), ws.numel(), _stream(dev)))
         return scores
+
+    def align_device(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):
+        """Best-path (Viterbi) alignment of N hypotheses per utterance over the CTC lattice, on the logits' device and without
+        synchronising: ``(alignments [B, N, T] int64, token_starts [B, N, Lmax] int64, token_ends [B, N, Lmax] int64,
+        path_scores [B, N] float64)``.  ``hyps`` ``[B, N, Lmax]`` and ``hyp_lengths`` ``[B, N]``, int32 or int64, any device;
+        ``logits_lengths`` ``[B]`` or ``None`` (all frames).  ``alignments[b, n]`` is the label id of every frame on the best
+        path (``get_alignment_3d``'s row for that hypothesis, ``-100`` past the utterance's frames); token ``k`` covers the
+        frames ``[token_starts, token_ends)``; ``path_scores`` is the best path's log-probability (``<= score_device``).  An
+        infeasible hypothesis gives ``-inf`` and spans of ``-1``; out-of-range lengths / labels raise ``ValueError`` when
+        they live on the host and give NaN scores and ``-1`` spans when they live on the device.  Input on the CPU is
+        copied to the current CUDA device."""
+        _require_cuda()
+        logits = logits.detach()
+        if logits.dim() != 3:
+            raise ValueError("logits must be [batch, frames, alphabet], got %s" % (tuple(logits.shape),))
+        if logits.dtype not in _DTYPES:
+            raise TypeError("unsupported logits dtype %s" % logits.dtype)
+        B, T, V = logits.shape
+        if B < 1 or T < 1 or V < 1:
+            raise ValueError("empty logits %s" % (tuple(logits.shape),))
+        if not 0 <= self.blank_idx < V:
+            raise ValueError("blank_idx %d outside the alphabet [0,%d)" % (self.blank_idx, V))
+        if hyps.dim() != 3 or hyps.size(0) != B:
+            raise ValueError("hyps must be [batch, n_hyp, max_length], got %s" % (tuple(hyps.shape),))
+        N, Lmax = hyps.size(1), hyps.size(2)
+        if N < 1:
+            raise ValueError("hyps holds no hypothesis")
+        if tuple(hyp_lengths.shape) != (B, N):
+            raise ValueError("hyp_lengths must have shape [batch, n_hyp] = %s, got %s" % ((B, N), tuple(hyp_lengths.shape)))
+        if logits_lengths is not None and (logits_lengths.dim() != 1 or logits_lengths.numel() != B):
+            raise ValueError("logits_lengths must have shape [batch]")
+        lim = _limits()
+        if Lmax > ALIGN_MAX_TARGETS or V > lim.max_alphabet:
+            raise NotImplementedError("the aligner supports hypothesis length <= %d and alphabet <= %d"
+                                      % (ALIGN_MAX_TARGETS, lim.max_alphabet))
+        # the loss's rule (_Problem): host-resident lengths / labels are checked here, device-resident ones on the device
+        if logits_lengths is not None and not logits_lengths.is_cuda:
+            ll = logits_lengths.to(torch.int64)
+            if bool((ll < 1).any()) or bool((ll > T).any()):
+                raise ValueError("logits_lengths must be in [1, %d]" % T)
+        if not hyp_lengths.is_cuda:
+            hl = hyp_lengths.to(torch.int64)
+            if bool((hl < 0).any()) or bool((hl > Lmax).any()):
+                raise ValueError("hyp_lengths must be in [0, %d]" % Lmax)
+            if not hyps.is_cuda and Lmax > 0:
+                valid = torch.arange(Lmax) < hl.unsqueeze(-1)
+                hg = hyps.to(torch.int64)
+                if bool(((hg < 0) | (hg >= V))[valid].any()):
+                    raise ValueError("hypothesis labels must be in [0, %d)" % V)
+        dev = logits.device if logits.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        with _on_device(dev):
+            if not logits.is_cuda:
+                logits = logits.to(dev)
+            if not _dense3(logits):
+                logits = logits.contiguous()
+            hyps = _as_index(hyps, dev, "hyps").reshape(B * N, Lmax)
+            if Lmax > 0 and hyps.stride(1) != 1:
+                hyps = hyps.contiguous()
+            hyp_lengths = _as_index(hyp_lengths, dev, "hyp_lengths").reshape(B * N).contiguous()
+            if logits_lengths is not None:
+                logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
+                if logits_lengths.dtype != hyp_lengths.dtype:
+                    logits_lengths, hyp_lengths = logits_lengths.to(torch.int64), hyp_lengths.to(torch.int64)
+            d = _lib.Desc()
+            d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, Lmax
+            d.blank_idx, d.dtype = self.blank_idx, _DTYPES[logits.dtype]
+            d.targets_itype, d.lengths_itype = _ITYPES[hyps.dtype], _ITYPES[hyp_lengths.dtype]
+            d.from_logits = 1 if from_logits else 0
+            d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
+            d.targets_stride_b = hyps.stride(0) if Lmax > 0 else 0
+            need = self._L.e2e_ctc_align_nbest_workspace_bytes(ctypes.byref(d), N)
+            if need == 0:
+                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            aligned = torch.empty(B, N, T, dtype=torch.int64, device=dev)
+            starts = torch.empty(B, N, Lmax, dtype=torch.int64, device=dev)
+            ends = torch.empty(B, N, Lmax, dtype=torch.int64, device=dev)
+            path_scores = torch.empty(B, N, dtype=torch.float64, device=dev)
+            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            _lib.check(self._L.e2e_ctc_align_nbest_device(
+                ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(aligned),
+                _ptr(starts), _ptr(ends), _ptr(path_scores), _ptr(ws), ws.numel(), _stream(dev)))
+        return aligned, starts, ends, path_scores

@@ -203,6 +203,38 @@ int e2e_ctc_viterbi_align_device(const e2e_ctc_desc* desc, int32_t is_ctc, const
                                  const void* targets, const void* logits_lengths, const void* targets_lengths,
                                  int64_t* aligned, void* workspace, size_t workspace_bytes, void* cuda_stream);
 
+/* ------------------------------------------- N hypotheses per utterance: alignment and timestamps ---- */
+
+/* The best-path (Viterbi) alignment of n_hyp hypotheses per utterance over the CTC lattice, with each token's frame span
+ * and the best path's log-probability: timestamps for transcripts (this library's N-best lists or any other).  Lattice
+ * r = b * n_hyp + n aligns hypothesis n of utterance b against utterance b's frames, read once from `logits` (no
+ * replicated input).  e2e_ctc_viterbi_align_device is the n_hyp == 1, log-prob, no-span call of the same kernel.
+ *   logits: log-probabilities [B,T,V] (desc strides) when desc->from_logits == 0, raw logits when it is 1 (the row
+ *       log-softmax of the scorer and the beam search: (x - max) - log sum exp in the input's precision, rounded to the
+ *       input dtype for 16-bit inputs);
+ *   hyps: [B * n_hyp, max_targets] of targets_itype, row stride desc->targets_stride_b (NULL allowed when max_targets
+ *       == 0); hyp_lengths: [B * n_hyp]; logits_lengths: [B] or NULL for max_frames;
+ *   aligned: [B * n_hyp, T] int64, row r exactly what e2e_ctc_viterbi_align_device (is_ctc = 1) writes for utterance b's
+ *       frames with hypothesis r as its target: the label id of every frame, -100 past the utterance's frames;
+ *   path_scores: [B * n_hyp] float64, the best path's log-probability (the final cell the backtrace starts from; the
+ *       final blank wins unless the final label is strictly better): a sum of fp64-widened log-probabilities in frame
+ *       order.  The empty hypothesis gives sum_t log p(blank | t); an infeasible one (T_b < L + repeats) -inf; a
+ *       hypothesis length outside [0, max_targets] or a label outside [0, alphabet) NaN, and a logits length outside
+ *       [1, max_frames] NaN for every hypothesis of the utterance (with -100 rows and status bits as
+ *       e2e_ctc_viterbi_align_device sets them).  path_scores <= the e2e_ctc_score_device score wherever both are finite;
+ *   token_starts, token_ends: [B * n_hyp, max_targets] int64 (may be NULL when max_targets == 0): token k < L covers the
+ *       frames [start, end) whose path cell is label cell 2 k + 1 -- non-empty, disjoint and increasing; -1 in slots
+ *       k >= L and wherever the path score is not > -inf.
+ * Workspace: 256 status bytes, the row statistics of raw-logit input (8 bytes a frame, 16 for F64) and one backpointer
+ * byte per thread per frame of every lattice.  Limits: those of the Viterbi alignment (max_targets <= 1023) and alphabet <=
+ * e2e_ctc_limits.max_alphabet; beyond them, with n_hyp < 1, or when B * n_hyp exceeds 2^31 - 1 or the workspace size
+ * overflows, the workspace query returns 0 and sets the error message. */
+size_t e2e_ctc_align_nbest_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp);
+int e2e_ctc_align_nbest_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                               const void* logits_lengths, const void* hyp_lengths, int64_t* aligned, int64_t* token_starts,
+                               int64_t* token_ends, double* path_scores, void* workspace, size_t workspace_bytes,
+                               void* cuda_stream);
+
 /* ------------------------------------------------------------------- CTC without blank ----- */
 
 /* Loss and gradient of the blank-free CTC variant -- the reference's pytorch_end2end/functions/ctc_without_blank.py:
