@@ -8,8 +8,9 @@ from .encoders.text_encoders import CTCEncoder
 from .engine import CTCGreedyEngine, CTCLossEngine, GraphedStep
 from .functions.forward_backward import ForwardBackwardLossFunction
 from .modules.ctc_loss import CTCLoss, ForwardBackwardLossBase, GraphedCTCStep
+from .modules.ctc_score import CTCScore
 
-__all__ = ["CTCLoss", "CTCDecoder", "CTCEncoder", "CTCLossEngine", "CTCGreedyEngine",
+__all__ = ["CTCLoss", "CTCScore", "CTCDecoder", "CTCEncoder", "CTCLossEngine", "CTCGreedyEngine",
            "ForwardBackwardLossFunction", "ForwardBackwardLossBase", "CTCDecoderError", "DecoderResults", "NBestResults", "AlignmentResults",
            "GraphedStep", "GraphedCTCStep"]
 __version__ = "0.1.0"

@@ -33,9 +33,11 @@ EXPORTS = (
     "e2e_ctc_beam_workspace_bytes", "e2e_ctc_beam_decode_device", "e2e_ctc_engine_beam_host",
     "e2e_ctc_beam_nbest_workspace_bytes", "e2e_ctc_beam_nbest_device", "e2e_ctc_engine_beam_nbest_host",
     "e2e_ctc_score_workspace_bytes", "e2e_ctc_score_device",
+    "e2e_ctc_score_backward_workspace_bytes", "e2e_ctc_score_backward_device",
     "e2e_ctc_align_nbest_workspace_bytes", "e2e_ctc_align_nbest_device",
 )
-KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score")
+KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score",
+                "score_backward", "score_backward_rows")
 
 
 class Desc(ctypes.Structure):
@@ -132,6 +134,10 @@ def load():
     L.e2e_ctc_score_workspace_bytes.restype = sz
     L.e2e_ctc_score_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, sz, vp]
     L.e2e_ctc_score_device.restype = ctypes.c_int
+    L.e2e_ctc_score_backward_workspace_bytes.argtypes = [dp, i32]
+    L.e2e_ctc_score_backward_workspace_bytes.restype = sz
+    L.e2e_ctc_score_backward_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    L.e2e_ctc_score_backward_device.restype = ctypes.c_int
     L.e2e_ctc_align_nbest_workspace_bytes.argtypes = [dp, i32]
     L.e2e_ctc_align_nbest_workspace_bytes.restype = sz
     L.e2e_ctc_align_nbest_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]

@@ -468,15 +468,17 @@ int e2e_ctc_profile_enable(int32_t on) {
 }
 
 int e2e_ctc_profile_read(double* ms, uint64_t* launches, int32_t n_kinds) {
-  if (!ms || !launches || n_kinds < kNumKernels) { set_error("profile_read needs %d slots", (int)kNumKernels); return E2E_ERR_INVALID_ARGUMENT; }
+  if (!ms || !launches || n_kinds < kMinProfileKinds) { set_error("profile_read needs %d slots", (int)kMinProfileKinds); return E2E_ERR_INVALID_ARGUMENT; }
   for (int i = 0; i < n_kinds; i++) { ms[i] = 0.0; launches[i] = 0; }
   std::lock_guard<std::mutex> lk(g_prof_mu);
   for (EventPair& ev : g_prof_pending) {
     E2E_CUDA_TRY(cudaEventSynchronize(ev.b));
     float t = 0.f;
     E2E_CUDA_TRY(cudaEventElapsedTime(&t, ev.a, ev.b));
-    ms[ev.kind] += (double)t;
-    launches[ev.kind] += 1;
+    if (ev.kind < n_kinds) {
+      ms[ev.kind] += (double)t;
+      launches[ev.kind] += 1;
+    }
     g_prof_free.emplace_back(ev.a, ev.b);
   }
   g_prof_pending.clear();
@@ -716,6 +718,40 @@ int e2e_ctc_score_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* lo
   if (rc != E2E_OK) return rc;
   return launch_score(*desc, n_hyp, logits, hyps, logits_lengths, hyp_lengths, scores,
                       reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+// ---- the scorer's backward (K10 + row kernel) ------------------------------------------------------------
+static int check_score_backward(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  int rc = check_score(desc, n_hyp);
+  if (rc != E2E_OK) return rc;
+  if (desc->grads_stride_b < 0 || desc->grads_stride_t < 0) { set_error("negative gradient stride"); return E2E_ERR_INVALID_ARGUMENT; }
+  if (!score_backward_supported(*desc)) {
+    set_error("score backward: max_targets %d with alphabet %d does not fit shared memory", desc->max_targets, desc->alphabet);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  return E2E_OK;
+}
+
+size_t e2e_ctc_score_backward_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  if (check_score_backward(desc, n_hyp) != E2E_OK) return 0;
+  return score_backward_workspace_bytes(*desc, n_hyp);   // 0 (message set) on overflow
+}
+
+int e2e_ctc_score_backward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                                  const void* logits_lengths, const void* hyp_lengths, const double* grad_scores,
+                                  void* grads, void* workspace, size_t workspace_bytes, void* cuda_stream) {
+  int rc = check_score_backward(desc, n_hyp);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !hyp_lengths || !grad_scores || !grads || (!hyps && desc->max_targets > 0)) {
+    set_error("null pointer argument");
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  const size_t need = e2e_ctc_score_backward_workspace_bytes(desc, n_hyp);
+  if (need == 0) return E2E_ERR_UNSUPPORTED;
+  rc = check_ws(workspace, workspace_bytes, need);
+  if (rc != E2E_OK) return rc;
+  return launch_score_backward(*desc, n_hyp, logits, hyps, logits_lengths, hyp_lengths, grad_scores, grads,
+                               reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 // ---- pinned host memory for result buffers -------------------------------------------------------

@@ -112,7 +112,9 @@ constexpr int kFlagInfeasible = 1, kFlagInvalid = 2;
 void set_error(const char* fmt, ...);
 
 // Launch accounting + optional per-kernel device timing (CUDA events on the launching stream).
-enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kNumKernels };
+enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kKernelScoreGrad, kKernelScoreRows, kNumKernels };
+// e2e_ctc_profile_read's smallest n_kinds: the kinds up to kKernelScore (kinds added later are dropped for such callers)
+constexpr int kMinProfileKinds = kKernelScore + 1;
 void launch_begin(int kind, cudaStream_t s);
 void launch_end(int kind, cudaStream_t s);
 struct KernelTimer {   // brackets exactly one kernel launch
@@ -266,6 +268,12 @@ int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx
 bool score_supported(const e2e_ctc_desc& d);
 int launch_score(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
                  const void* hyp_len, double* scores, cudaStream_t s);
+// the scorer's backward (K10 + its row kernel): grad_scores [B * n_hyp] float64, grads of desc->dtype (grads strides);
+// workspace: 0 with the message set when a size overflows or a grid exceeds 2^31 - 1 CTAs
+bool score_backward_supported(const e2e_ctc_desc& d);
+size_t score_backward_workspace_bytes(const e2e_ctc_desc& d, int n_hyp);
+int launch_score_backward(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
+                          const void* hyp_len, const double* grad_scores, void* grads, char* ws, cudaStream_t s);
 size_t noblank_workspace_bytes(const e2e_ctc_desc& d);
 bool noblank_supported(const e2e_ctc_desc& d);
 int launch_noblank(const e2e_ctc_desc& d, int space_idx, const void* lp, const void* targets, const void* in_len,

@@ -16,9 +16,8 @@ KenLM decoding (``lm_path``) stays the reference's CPU code and is out of scope;
 """
 from collections import namedtuple
 
-import torch
-
 from ..engine import ALIGN_MAX_TARGETS, CTCBeamEngine
+from ..utils.hypotheses import empty_marker_as_empty
 
 
 class CTCDecoderError(Exception):
@@ -162,11 +161,7 @@ class CTCDecoder:
         """
         if self._time_major:
             logits = logits.transpose(1, 0)
-        if hypotheses.dim() == 3 and hypotheses.size(2) > 0 and hypotheses_lengths.shape == hypotheses.shape[:2]:
-            # decode's empty result, [-1] with length 1, is the empty hypothesis (no sync: an element-wise select)
-            dev = hypotheses_lengths.device
-            empty = (hypotheses[:, :, 0].to(dev) == -1) & (hypotheses_lengths == 1)
-            hypotheses_lengths = torch.where(empty, torch.zeros_like(hypotheses_lengths), hypotheses_lengths)
+        hypotheses_lengths = empty_marker_as_empty(hypotheses, hypotheses_lengths)
         return self._decoder.score_device(logits, hypotheses, hypotheses_lengths, logits_lengths,
                                           from_logits=not self._after_logsoftmax).cpu()
 
@@ -198,11 +193,8 @@ class CTCDecoder:
             logits = logits.transpose(1, 0)
         if hypotheses.dim() == 2:                       # one hypothesis per utterance: decode's / decode_greedy's result
             hypotheses, hypotheses_lengths = hypotheses[:, None], hypotheses_lengths.reshape(-1, 1)
+        hypotheses_lengths = empty_marker_as_empty(hypotheses, hypotheses_lengths)
         if hypotheses.dim() == 3 and hypotheses.size(2) > 0 and hypotheses_lengths.shape == hypotheses.shape[:2]:
-            # decode's empty result, [-1] with length 1, is the empty hypothesis (no sync: an element-wise select)
-            dev = hypotheses_lengths.device
-            empty = (hypotheses[:, :, 0].to(dev) == -1) & (hypotheses_lengths == 1)
-            hypotheses_lengths = torch.where(empty, torch.zeros_like(hypotheses_lengths), hypotheses_lengths)
             if hypotheses.size(2) > ALIGN_MAX_TARGETS and hypotheses_lengths.numel():
                 hypotheses = hypotheses[:, :, :max(int(hypotheses_lengths.max()), 0)]
         aligned, starts, ends, path_scores = (t.cpu() for t in self._decoder.align_device(

@@ -733,14 +733,12 @@ class CTCBeamEngine(CTCGreedyEngine):
         width = int(lengths.max()) if lengths.numel() else 0
         return decoded[:, :, :width].contiguous(), lengths, scores, log_probs
 
-    def score_device(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):
-        """CTC log-likelihood log p(hypothesis | x) of N hypotheses per utterance: ``[B, N]`` float64 on the logits' device,
-        minus the CTC loss of each (utterance, hypothesis) pair, without synchronising.  ``hyps`` ``[B, N, Lmax]`` and
-        ``hyp_lengths`` ``[B, N]``, int32 or int64, any device; ``logits_lengths`` ``[B]`` or ``None`` (all frames).
-        Forward only: no gradient and nothing kept for one.  An infeasible hypothesis scores ``-inf``; out-of-range
-        lengths / labels raise ``ValueError`` when they live on the host and give NaN scores when they live on the
-        device.  Input on the CPU is copied to the current CUDA device."""
-        _require_cuda()
+    def _score_args(self, logits, hyps, hyp_lengths, logits_lengths, from_logits):
+        """The checks and the C descriptor shared by ``score_device`` and ``score_backward_device``: returns ``(logits,
+        hyps [B*N, Lmax], hyp_lengths [B*N], logits_lengths, desc, device, N)`` with every tensor on the device.  It
+        enters ``_on_device(device)`` itself for the copies and returns outside it: callers enter it again for their
+        allocations and the launch.  Host-resident lengths / labels are checked here, device-resident ones on the device
+        (the loss's rule, ``_Problem``)."""
         logits = logits.detach()
         if logits.dim() != 3:
             raise ValueError("logits must be [batch, frames, alphabet], got %s" % (tuple(logits.shape),))
@@ -764,7 +762,6 @@ class CTCBeamEngine(CTCGreedyEngine):
         if Lmax > lim.max_targets or V > lim.max_alphabet:
             raise NotImplementedError("the scorer supports hypothesis length <= %d and alphabet <= %d"
                                       % (lim.max_targets, lim.max_alphabet))
-        # the loss's rule (_Problem): host-resident lengths / labels are checked here, device-resident ones on the device
         if logits_lengths is not None and not logits_lengths.is_cuda:
             ll = logits_lengths.to(torch.int64)
             if bool((ll < 1).any()) or bool((ll > T).any()):
@@ -792,22 +789,70 @@ class CTCBeamEngine(CTCGreedyEngine):
                 logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
                 if logits_lengths.dtype != hyp_lengths.dtype:
                     logits_lengths, hyp_lengths = logits_lengths.to(torch.int64), hyp_lengths.to(torch.int64)
-            d = _lib.Desc()
-            d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, Lmax
-            d.blank_idx, d.dtype = self.blank_idx, _DTYPES[logits.dtype]
-            d.targets_itype, d.lengths_itype = _ITYPES[hyps.dtype], _ITYPES[hyp_lengths.dtype]
-            d.from_logits = 1 if from_logits else 0
-            d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
-            d.targets_stride_b = hyps.stride(0) if Lmax > 0 else 0
+        d = _lib.Desc()
+        d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, Lmax
+        d.blank_idx, d.dtype = self.blank_idx, _DTYPES[logits.dtype]
+        d.targets_itype, d.lengths_itype = _ITYPES[hyps.dtype], _ITYPES[hyp_lengths.dtype]
+        d.from_logits = 1 if from_logits else 0
+        d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
+        d.targets_stride_b = hyps.stride(0) if Lmax > 0 else 0
+        return logits, hyps, hyp_lengths, logits_lengths, d, dev, N
+
+    def score_device(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):
+        """CTC log-likelihood log p(hypothesis | x) of N hypotheses per utterance: ``[B, N]`` float64 on the logits' device,
+        minus the CTC loss of each (utterance, hypothesis) pair, without synchronising.  ``hyps`` ``[B, N, Lmax]`` and
+        ``hyp_lengths`` ``[B, N]``, int32 or int64, any device; ``logits_lengths`` ``[B]`` or ``None`` (all frames).
+        Forward only: no gradient and nothing kept for one (``score_backward_device`` computes it).  An infeasible
+        hypothesis scores ``-inf``; out-of-range lengths / labels raise ``ValueError`` when they live on the host and give
+        NaN scores when they live on the device.  Input on the CPU is copied to the current CUDA device."""
+        _require_cuda()
+        logits, hyps, hyp_lengths, logits_lengths, d, dev, N = self._score_args(logits, hyps, hyp_lengths, logits_lengths,
+                                                                               from_logits)
+        with _on_device(dev):
             need = self._L.e2e_ctc_score_workspace_bytes(ctypes.byref(d), N)
             if need == 0:
                 raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
-            scores = torch.empty(B, N, dtype=torch.float64, device=dev)
+            scores = torch.empty(d.batch, N, dtype=torch.float64, device=dev)
             ws = torch.empty(need, dtype=torch.uint8, device=dev)
             _lib.check(self._L.e2e_ctc_score_device(
                 ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(scores),
                 _ptr(ws), ws.numel(), _stream(dev)))
         return scores
+
+    def score_backward_workspace_bytes(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):
+        """Workspace bytes ``score_backward_device`` allocates for these arguments."""
+        _require_cuda()
+        _, _, _, _, d, dev, N = self._score_args(logits, hyps, hyp_lengths, logits_lengths, from_logits)
+        with _on_device(dev):
+            return int(self._L.e2e_ctc_score_backward_workspace_bytes(ctypes.byref(d), N))
+
+    def score_backward_device(self, logits, hyps, hyp_lengths, grad_scores, logits_lengths=None, from_logits=False):
+        """The gradient of ``sum(grad_scores * score_device(...))`` with respect to ``logits``, on the logits' device (CPU
+        input: the current CUDA device) without synchronising: a tensor of the logits' shape and dtype, in their layout
+        when it is dense.  With ``gamma_bn(t, v)`` the occupancy of symbol ``v`` at frame ``t`` under hypothesis ``n``:
+        ``sum_n g[b,n] gamma_bn(t,v)`` for log-probabilities, ``sum_n g[b,n] (gamma_bn(t,v) - softmax(x_bt)_v)`` for raw
+        logits, 0 past the utterance's frames.  This is the derivative of the score; it is not ``CTCLoss``'s convention
+        (``exp(lp) - gamma`` on log-probabilities, ``exp(lp)`` in padding rows).  ``grad_scores`` ``[B, N]`` (float64
+        on the device): a hypothesis with ``g == 0`` costs no sweep; an infeasible one contributes 0; a device-resident
+        bad length or label gives NaN rows for its utterance only."""
+        _require_cuda()
+        logits, hyps, hyp_lengths, logits_lengths, d, dev, N = self._score_args(logits, hyps, hyp_lengths, logits_lengths,
+                                                                               from_logits)
+        B = d.batch
+        if tuple(grad_scores.shape) != (B, N):
+            raise ValueError("grad_scores must have shape [batch, n_hyp] = %s, got %s" % ((B, N), tuple(grad_scores.shape)))
+        with _on_device(dev):
+            need = self._L.e2e_ctc_score_backward_workspace_bytes(ctypes.byref(d), N)
+            if need == 0:
+                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            g = grad_scores.detach().to(dev, torch.float64).contiguous()
+            grads = torch.empty_like(logits)
+            d.grads_stride_b, d.grads_stride_t = grads.stride(0), grads.stride(1)
+            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            _lib.check(self._L.e2e_ctc_score_backward_device(
+                ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(g),
+                _ptr(grads), _ptr(ws), ws.numel(), _stream(dev)))
+        return grads
 
     def align_device(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):
         """Best-path (Viterbi) alignment of N hypotheses per utterance over the CTC lattice, on the logits' device and without

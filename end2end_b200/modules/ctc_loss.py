@@ -89,6 +89,9 @@ class CTCLoss(ForwardBackwardLossBase):
     :param after_logsoftmax: the input already went through log-softmax (else: raw network outputs)
     :param time_major: logits are ``(T, B, V)`` instead of ``(B, T, V)``
     :param blank_idx: id of the blank label, default ``0``
+
+    With ``after_logsoftmax=True`` the gradient keeps the reference engine's convention, ``exp(lp) - posterior`` on every
+    frame (``exp(lp)`` in padding rows); ``CTCScore``'s gradient is the plain derivative of the score instead.
     """
 
     def __init__(self, size_average=None, reduce=None, after_logsoftmax=False, time_major=False, blank_idx=0):

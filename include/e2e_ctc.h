@@ -338,6 +338,33 @@ int e2e_ctc_score_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* lo
                          const void* logits_lengths, const void* hyp_lengths, double* scores, void* workspace,
                          size_t workspace_bytes, void* cuda_stream);
 
+/* The gradient of those scores for N-best sequence training (minimum word error rate and other objectives over the
+ * list): given g[b * n_hyp + n] = d objective / d scores[b * n_hyp + n], the true derivative of the objective with respect
+ * to the input, where gamma_bn(t, v) = sum_{s: ext[s] = v} alpha_t(s) beta_t(s) / p is hypothesis n's occupancy of symbol
+ * v at frame t (it sums to 1 over v):
+ *   log-probability input (desc->from_logits == 0): grads[b,t,v] = sum_n g[b,n] gamma_bn(t,v) for t < T_b;
+ *   raw logits (desc->from_logits == 1): grads[b,t,v] = sum_n g[b,n] (gamma_bn(t,v) - softmax(x_bt)_v) for t < T_b, the
+ *       softmax being exp of the row log-softmax of e2e_ctc_score_device (16-bit rounding included);
+ *   padding frames t >= T_b: 0.
+ * Unlike e2e_ctc_loss_backward_device on log-probability input, there is no exp(lp) term and padding rows are 0: this is
+ * the derivative of the score, not the reference engine's gradient convention.  The lattice is the one the score sums
+ * over; for a label equal to the blank next to a different label the reference's beta differs from it, and this gradient
+ * follows the score.
+ *   grad_scores: [B * n_hyp] float64 on the device.  A hypothesis with g == 0 costs no sweep and contributes nothing; an
+ *       infeasible one (score -inf) contributes exactly 0 whatever its g;
+ *   grads: [B,T,V] of desc->dtype with strides desc->grads_stride_b / grads_stride_t (unit alphabet stride), every element
+ *       written once.  A hypothesis length or label out of range (a NaN score) makes the utterance's rows t < T_b NaN --
+ *       the rows are shared by all its hypotheses -- and a logits length out of range all of its rows; other utterances
+ *       are untouched.
+ * fp64 lattice and accumulation in a fixed order, no floating-point atomics: bitwise reproducible.  Limits as for the
+ * score.  Workspace: per hypothesis an alpha checkpoint per staged block of frames and one block of alpha, per group of
+ * eight hypotheses a partial [T,V] float64 block; the query returns 0 and sets the message past the limits, with
+ * n_hyp < 1, when the size overflows size_t or when a grid exceeds 2^31 - 1 CTAs.  Enqueues only; never allocates. */
+size_t e2e_ctc_score_backward_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp);
+int e2e_ctc_score_backward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                                  const void* logits_lengths, const void* hyp_lengths, const double* grad_scores,
+                                  void* grads, void* workspace, size_t workspace_bytes, void* cuda_stream);
+
 /* -------------------------------------------------------------- engine, host pointers ------ */
 
 typedef struct e2e_ctc_engine e2e_ctc_engine;
@@ -389,8 +416,8 @@ uint64_t e2e_ctc_launch_count(void);
  * bracketed by CUDA events on its launching stream.  e2e_ctc_profile_read() waits for the pending
  * events, then fills ms[k] (summed device milliseconds) and launches[k] per kernel kind
  * k = 0 row_stats, 1 lattice, 2 gradient, 3 loss_reduce, 4 argmax, 5 collapse, 6 scale_rows, 7 viterbi,
- * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score (n_kinds >= 12),
- * and clears the record.  All launches since the previous read must have been made on ONE device. */
+ * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score, 12 score_backward, 13 score_backward_rows (n_kinds >= 12;
+ * the kinds past n_kinds are not reported), and clears the record.  All launches since the previous read must have been made on ONE device. */
 int e2e_ctc_profile_enable(int32_t on);
 int e2e_ctc_profile_read(double* ms, uint64_t* launches, int32_t n_kinds);
 
