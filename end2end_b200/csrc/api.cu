@@ -190,13 +190,11 @@ static bool make_wave_plan(const e2e_ctc_desc& d, bool fused, LossPlan* p) {
   if (!K) return false;
   WaveLayout L;
   L.K = K; L.NW = NW;
-  L.NC = NW >= 4 ? 6 : 2;
+  L.NC = wave_combiners(NW);
   L.NP = NW >= 4 ? 2 : 1;
-  if (L.NC < 1 || L.NC > 8 || (L.NP != 1 && L.NP != 2 && L.NP != 4)) return false;
   // experiment knobs (read once per process; a production process never sets them)
-  static const int wv_nc = env_int("E2E_CTC_WAVE_NC", 0), wv_np = env_int("E2E_CTC_WAVE_NP", 0), wv_nap = env_int("E2E_CTC_WAVE_NAP", -1),
+  static const int wv_np = env_int("E2E_CTC_WAVE_NP", 0), wv_nap = env_int("E2E_CTC_WAVE_NAP", -1),
                    wv_smsp = env_int("E2E_CTC_WAVE_BY_SMSP", 0), wv_r = env_int("E2E_CTC_WAVE_R", 0), wv_rv = env_int("E2E_CTC_WAVE_RV", 0);
-  if (wv_nc >= 1 && wv_nc <= 8) L.NC = wv_nc;
   if (wv_np == 1 || wv_np == 2 || wv_np == 4) L.NP = wv_np;
   L.nap = wv_nap >= 0 ? wv_nap : 32;
   L.by_smsp = wv_smsp ? 1 : 0;
@@ -209,20 +207,21 @@ static bool make_wave_plan(const e2e_ctc_desc& d, bool fused, LossPlan* p) {
   }
   if (L.nwarps > (NW <= 4 ? 16 : 32)) return false;
   const int lanes = 32 * NW, roww = lanes * (K + 1);
-  L.es = (d.alphabet + 2) | 1;   // odd: the producer's lane-per-frame stores are bank-conflict free
+  const int ecols = d.alphabet + 2;   // V symbols, the zero column padding cells read, the row normaliser
   L.vpad = (d.alphabet + 3) & ~3;
   L.RV = lanes * K >= 1024 ? 16 : 32;
   if (wv_rv == 8 || wv_rv == 16 || wv_rv == 32 || wv_rv == 64) L.RV = wv_rv;
   L.R = 128;   // producer blocks are 32 frames: two per producer in flight
   if (wv_r == 64 || wv_r == 128 || wv_r == 256) L.R = wv_r;
   if (L.R < 64 || (L.R & (L.R - 1))) return false;
-  while (L.R > 64 && (size_t)L.R * L.es * 8 > (size_t)(NW >= 4 ? 64 : 40) * 1024) L.R >>= 1;
+  while (L.R > 64 && (size_t)(L.R + 1) * ecols * 8 > (size_t)(NW >= 4 ? 64 : 40) * 1024) L.R >>= 1;
+  L.ecs = L.R + 1;
   if (L.RV > L.R / 2) L.RV = L.R / 2;
   if (L.RV < kWaveCF || (L.RV & (L.RV - 1))) return false;
   size_t off = 0;
   L.off_lab = 0; off = (size_t)align16i((size_t)(lanes * K / 2 + 1) * 4);
   L.off_occ = (int)off; off = (size_t)align16i(off + (size_t)(lanes * K / 2 + d.alphabet + 2) * 4);   // label indices by symbol + offsets
-  L.off_E = (int)off; off = (size_t)align16i(off + (size_t)L.R * L.es * 8);
+  L.off_E = (int)off; off = (size_t)align16i(off + (size_t)ecols * L.ecs * 8);
   L.off_valw = (int)off; off += (size_t)L.RV * lanes * K * 4;
   L.off_vale = (int)off; off += (size_t)L.RV * lanes * 4;
   L.off_stage = (int)off; off += (size_t)L.NC * kWavePF * (roww + 4) * 4;

@@ -45,15 +45,18 @@ constexpr int kSweepPFWide = E2E_SWEEP_PF_WIDE;
 constexpr int kWaveCF = 8;       // wave kernel: frames per hand-off chunk
 constexpr int kWaveRB = 32;      // boundary-slot ring depth (frames)
 constexpr int kWavePF = 4;       // stashed rows each combiner warp keeps in flight
+// combiner warps of the wave kernel: a compile-time count, so that the lattice warps' ring check is straight-line code
+__host__ __device__ constexpr int wave_combiners(int NW) { return NW >= 4 ? 6 : 2; }
 // shared-memory layout and role counts of the wave kernel (ctc_wave_impl.cuh)
 struct WaveLayout {
   int K, NW;        // cells per lane, lattice warps per sweep
-  int NP, NC;       // producer (row log-softmax) warps, combiner warps
+  int NP, NC;       // producer (row log-softmax) warps, combiner warps (wave_combiners(NW))
   int by_smsp;      // lay the roles out by SM sub-partition (warp id % 4): latency configurations
   int nwarps;       // warps per CTA
   int nap;          // nanoseconds a waiting producer / combiner warp sleeps between polls (0: spin)
   int R, RV;        // frames in the emission ring / in the val ring (powers of two)
-  int es;           // doubles per emission-ring frame: V symbols, a zero column, the row normaliser
+  int ecs;          // the emission ring is column-major (V symbols, a zero column, the row normaliser): doubles per
+                    // column, R + 1 (odd: the combiners' symbol-per-lane reads spread over the banks)
   int vpad;         // u32 posterior accumulators per combiner warp
   int off_lab, off_occ, off_E, off_valw, off_vale, off_stage, off_acc, off_bnd, off_ctl, total;
 };

@@ -35,7 +35,8 @@
 //    the exponent of the nearest lane with mass below it (ballot + indexed shuffle).
 //  * The kernel image must stay small: with three roles resident on every SM the instruction cache is a
 //    first-order constraint (DESIGN.md), hence runtime `BWD` outside the lattice loop and rolled loops in
-//    the producer / prologue paths.
+//    the producer / prologue paths.  One lattice loop serves every wavefront position: a copy per position
+//    (first / middle / last warp) made the loop branch-free too, but measured 137 us instead of 101 on c2.
 #pragma once
 #include <cstdlib>
 #include <type_traits>
@@ -181,8 +182,8 @@ __device__ __noinline__ double wave_produce_block(const WaveParams& p, const Wav
   const int i = i0 + lane;
   if (i >= Ti) return 0.0;
   const long long ro = xbase + (long long)(BWD ? (Ti - 1 - i) : i) * p.st;
-  double* Erow = sv.E + (size_t)(i & (L.R - 1)) * L.es;
-  const int V = p.V;
+  double* Ef = sv.E + (i & (L.R - 1));   // this frame's slot of the column-major ring: symbol v at Ef[v * ecs]
+  const int V = p.V, ecs = L.ecs;
   float m = -INFINITY, s = 0.f;
   bool nan = false;
   if (REG) {
@@ -196,20 +197,20 @@ __device__ __noinline__ double wave_produce_block(const WaveParams& p, const Wav
     float ls = logf(s);
     if (nan) { m = NAN; ls = NAN; }
 #pragma unroll
-    for (int v = 0; v < 32; v++) if (v < V) Erow[v] = wv_emission(xv[v], m, ls, p.from_logits);
+    for (int v = 0; v < 32; v++) if (v < V) Ef[v * ecs] = wv_emission(xv[v], m, ls, p.from_logits);
     const double mls = (double)m + (double)ls;
-    Erow[V] = 0.0;                                       // the column padding cells read
-    Erow[V + 1] = p.from_logits ? 1.0 : exp(mls);        // turns the emission back into exp(x)
+    Ef[V * ecs] = 0.0;                                   // the column padding cells read
+    Ef[(V + 1) * ecs] = p.from_logits ? 1.0 : exp(mls);  // turns the emission back into exp(x)
     return mls;
   } else {
     for (int v = 0; v < V; v++) { const float x = wv_load_logit(p.logits, p.dtype, ro + v); nan |= x != x; m = fmaxf(m, x); }
     for (int v = 0; v < V; v++) s += expf(wv_load_logit(p.logits, p.dtype, ro + v) - m);
     float ls = logf(s);
     if (nan) { m = NAN; ls = NAN; }
-    for (int v = 0; v < V; v++) Erow[v] = wv_emission(wv_load_logit(p.logits, p.dtype, ro + v), m, ls, p.from_logits);
+    for (int v = 0; v < V; v++) Ef[v * ecs] = wv_emission(wv_load_logit(p.logits, p.dtype, ro + v), m, ls, p.from_logits);
     const double mls = (double)m + (double)ls;
-    Erow[V] = 0.0;
-    Erow[V + 1] = p.from_logits ? 1.0 : exp(mls);
+    Ef[V * ecs] = 0.0;
+    Ef[(V + 1) * ecs] = p.from_logits ? 1.0 : exp(mls);
     return mls;
   }
 }
@@ -245,28 +246,33 @@ __device__ void wave_producer(const WaveParams& p, const WaveView& sv, int b, in
 // multipliers of the next group's first frame), so a frame is the recurrence, one shuffle, one boundary
 // slot and two shared-memory stores.  Four frames shrink a cell by at most 2^-600 (fp32 emissions are
 // >= 2^-149), well inside the fp64 range below the re-centred block maximum.
+// The frames of a full group are straight-line code (no branch or reconvergence point between them, one
+// divergence check per group): whether the warp takes its boundary cell from warp w-1 (HIN) or hands one to
+// warp w+1 (HOUT) enters the frame body only through selects and a predicated store, and the first group (no
+// boundary into frame 0, no re-centring to apply) is peeled off the loop.
 template <int K, int NW, bool BWD>
 __device__ void wave_lattice(const WaveParams& p, const WaveView& sv, int b, int Ti, int Li, int w, int lane, long long* dbgp) {
+  const bool HIN = NW > 1 && w > 0, HOUT = NW > 1 && w + 1 < NW;
   const long long tstart = WV_CLK();
   constexpr unsigned FULL = 0xffffffffu;
-  constexpr int H = K / 2, LANES = 32 * NW, CF = kWaveCF, RB = kWaveRB, G = 4;
+  constexpr int H = K / 2, LANES = 32 * NW, CF = kWaveCF, RB = kWaveRB, G = 4, NC = wave_combiners(NW);
   const WaveLayout& L = p.L;
   const int S = 2 * Li + 1;
   const int g = w * 32 + lane;
   const int m0 = g * K;
 
-  int ecol[H];
-  double skipd[H];   // 1.0 where the label cell may also gather from s-2 (a different, non-blank label), else 0.0
+  const double* ecol[H];   // emission-ring column of each label cell (the zero column past L_i)
+  double skipd[H];         // 1.0 where the label cell may also gather from s-2 (a different, non-blank label), else 0.0
 #pragma unroll
   for (int h = 0; h < H; h++) {
     const int li = g * H + h;
     const bool lv = li < Li;
     const int lab = sv.lab[li];        // padded with blank past L_i
-    ecol[h] = lv ? lab : p.V;          // the zero column
+    ecol[h] = sv.E + (size_t)(lv ? lab : p.V) * L.ecs;
     const bool sk = lv && li >= 1 && lab != p.blank && lab != sv.lab[li - 1];
     skipd[h] = sk ? 1.0 : 0.0;
   }
-  const int bcol = p.blank;
+  const double* const bcol = sv.E + (size_t)p.blank * L.ecs;
 
   double x[K];
 #pragma unroll
@@ -275,9 +281,7 @@ __device__ void wave_lattice(const WaveParams& p, const WaveView& sv, int b, int
   double fb = lane == 0 ? 0.0 : 1.0;
   int en_next = 0;
   double f_next = 1.0, fb_next = fb;
-  bool pending = false;
   int src_e = 0;                       // exponent of the last boundary value received from the previous warp
-  const bool has_in = NW > 1 && w > 0, has_out = NW > 1 && w + 1 < NW;
   const uint4* const bnd_in = sv.bnd + (size_t)(w > 0 ? w - 1 : 0) * RB;
   uint4* const bnd_out = sv.bnd + (size_t)w * RB;
 
@@ -288,15 +292,15 @@ __device__ void wave_lattice(const WaveParams& p, const WaveView& sv, int b, int
     const int needv = i0 + CF - L.RV;        // frames below this have left the val ring
     const int needb = i0 + CF - RB + 1;      // the boundary slots this chunk overwrites have been read
     const int ev = wv_ld_acquire(er);
-    const int cm = wv_min_prog<8>(sv.ctl->comb_done, L.NC);
-    const int lp = has_out ? wv_ld_acquire(&sv.ctl->lat_prog[w + 1]) : 0x7fffffff;
+    const int cm = wv_min_prog<NC>(sv.ctl->comb_done, NC);
+    const int lp = HOUT ? wv_ld_acquire(&sv.ctl->lat_prog[w + 1]) : 0x7fffffff;
     if (ev <= bi || cm < needv || lp < needb) {
       const long long t0 = WV_CLK();
       while (wv_ld_acquire(er) <= bi) {}
       const long long t1 = WV_CLK();
-      while (wv_min_prog<8>(sv.ctl->comb_done, L.NC) < needv) {}
+      while (wv_min_prog<NC>(sv.ctl->comb_done, NC) < needv) {}
       const long long t2 = WV_CLK();
-      if (has_out) { while (wv_ld_acquire(&sv.ctl->lat_prog[w + 1]) < needb) {} }
+      if (HOUT) { while (wv_ld_acquire(&sv.ctl->lat_prog[w + 1]) < needb) {} }
       WV_DBG_ADD(1, t1 - t0); WV_DBG_ADD(2, t2 - t1); WV_DBG_ADD(3, WV_CLK() - t2);
     }
   };
@@ -304,28 +308,32 @@ __device__ void wave_lattice(const WaveParams& p, const WaveView& sv, int b, int
   // One group of G frames.  FULLG (all G frames exist): the boundary slots of the whole group are fetched up
   // front -- the warp waits for the previous warp to finish the group's third frame, so it runs one group
   // behind it -- and the body is straight-line code the compiler can schedule across frames.  Otherwise (the
-  // last, partial group) every frame polls its own slot.
-  auto group = [&](auto full_c, int i0) {
-    constexpr bool FULLG = decltype(full_c)::value;
-    // emissions of the whole group up front (rows past T_i are stale ring memory: loaded, never used)
-    const double* Erow0 = sv.E + (size_t)(i0 & (L.R - 1)) * L.es;
+  // last, partial group) every frame polls its own slot.  FIRST: the group of frame 0.
+  auto group = [&](auto full_c, auto first_c, int i0) {
+    constexpr bool FULLG = decltype(full_c)::value, FIRST = decltype(first_c)::value;
+    // emissions of the whole group up front (rows past T_i are stale ring memory: loaded, never used); R is a
+    // multiple of G, so the group's frames are adjacent in every column
+    const int f0 = i0 & (L.R - 1);
     double mb[G], ml[G][H];
 #pragma unroll
     for (int k = 0; k < G; k++) {
-      mb[k] = Erow0[(size_t)k * L.es + bcol];
+      mb[k] = bcol[f0 + k];
 #pragma unroll
-      for (int h = 0; h < H; h++) ml[k][h] = Erow0[(size_t)k * L.es + ecol[h]];
+      for (int h = 0; h < H; h++) ml[k][h] = ecol[h][f0 + k];
     }
+    // boundary slots: RB is a multiple of G, so frames i0 .. i0+G-1 sit in slots r0 .. r0+G-1 (no wrap)
+    const int r0 = i0 & (RB - 1);
     uint4 qg[G];
 #pragma unroll
     for (int k = 0; k < G; k++) qg[k] = make_uint4(0u, 0u, 0u, 0u);
-    if (FULLG && has_in) {
+    if (FULLG && HIN) {
       const int last = i0 + G - 2;   // frame i needs the boundary of frame i-1
       const long long t0 = WV_CLK();
-      do { qg[G - 1] = wv_ld_volatile_v4(bnd_in + (last & (RB - 1))); } while ((int)qg[G - 1].w != last + 1);
+      do { qg[G - 1] = wv_ld_volatile_v4(bnd_in + r0 + G - 2); } while ((int)qg[G - 1].w != last + 1);
       WV_DBG_ADD(4, WV_CLK() - t0);
+      if (!FIRST) qg[0] = wv_ld_volatile_v4(bnd_in + ((i0 - 1) & (RB - 1)));
 #pragma unroll
-      for (int k = 0; k < G - 1; k++) qg[k] = wv_ld_volatile_v4(bnd_in + ((i0 + k - 1) & (RB - 1)));
+      for (int k = 1; k < G - 1; k++) qg[k] = wv_ld_volatile_v4(bnd_in + r0 + k - 1);
     }
     uint32_t* const valw0 = sv.valw + ((size_t)(i0 & (L.RV - 1)) * LANES + g) * K;
     int* const vale0 = sv.vale + (size_t)(i0 & (L.RV - 1)) * LANES + g;
@@ -333,16 +341,19 @@ __device__ void wave_lattice(const WaveParams& p, const WaveView& sv, int b, int
     for (int k = 0; k < G; k++) {
       const int i = i0 + k;
       if (FULLG || i < Ti) {
-        const bool apply = k == 0 && pending;
+        const bool apply = !FIRST && k == 0;            // the re-centring of the previous group
+        const bool bnd_on = HIN && (!FIRST || k > 0);   // a boundary value arrives from the previous warp
         // boundary cell from the previous lane; from the previous warp through its slot
-        double bxs = __shfl_up_sync(FULL, x[K - 1], 1) * fb;
+        // explicit roundings in the recurrence: with the group in straight-line code the compiler would otherwise
+        // contract a product with the next frame's sum into an FMA, and the cells would change in the last bit
+        double bxs = __dmul_rn(__shfl_up_sync(FULL, x[K - 1], 1), fb);
         const uint4* slot = bnd_in + ((i - 1) & (RB - 1));
         uint4 q = qg[k];
-        if (!FULLG && has_in && i > 0) q = wv_ld_volatile_v4(slot);
-        if (FULLG && has_in && i > 0) {
-          src_e = (int)q.z;
-          const double bin = __hiloint2double((int)q.y, (int)q.x) * pow2i(min(src_e - e, 600));   // bounded: a few more lane hops (2^192 each) before the next re-centring cannot overflow
-          if (lane == 0) bxs = bin;
+        if (!FULLG && bnd_on) q = wv_ld_volatile_v4(slot);
+        if (FULLG && (!FIRST || k > 0)) {   // selects, no branch: q is all zero in the first warp
+          src_e = HIN ? (int)q.z : src_e;
+          const double bin = __dmul_rn(__hiloint2double((int)q.y, (int)q.x), pow2i(min(src_e - e, 600)));   // bounded: a few more lane hops (2^192 each) before the next re-centring cannot overflow
+          bxs = (HIN && lane == 0) ? bin : bxs;
         }
         if (k == 2) {
           // where the lane's scale should move (applied at the next group's first frame): block maximum into [1,2)
@@ -361,49 +372,48 @@ __device__ void wave_lattice(const WaveParams& p, const WaveView& sv, int b, int
           const unsigned live = __ballot_sync(FULL, alive);
           const int D = kExpSlack * __popc(live & ((2u << lane) - 1u));
           int v = alive ? e + ((mhi >> 20) - 1023) + D : 2 * kNegExp;
-          if (has_in) v = max(v, src_e);              // the previous warp's boundary lane, as lane -1 (D = 0)
+          v = HIN ? max(v, src_e) : v;                // the previous warp's boundary lane, as lane -1 (D = 0)
 #pragma unroll
           for (int d = 1; d < 32; d <<= 1) {
             const int t = __shfl_up_sync(FULL, v, d);
-            if (lane >= d) v = max(v, t);
+            v = lane >= d ? max(v, t) : v;
           }
           const int en = v < kNegExp ? e : v - D;     // nothing with mass up to here: keep the scale
           const int nb_en = __shfl_up_sync(FULL, en, 1);
           en_next = en;
           f_next = pow2i(e - en);
           fb_next = lane == 0 ? 0.0 : pow2i(nb_en - en);
-          pending = true;
         }
         double mulb = mb[k], mull[H];
 #pragma unroll
         for (int h = 0; h < H; h++) mull[h] = ml[k][h];
         if (apply) {
-          mulb *= f_next;
+          mulb = __dmul_rn(mulb, f_next);
 #pragma unroll
-          for (int h = 0; h < H; h++) mull[h] *= f_next;
+          for (int h = 0; h < H; h++) mull[h] = __dmul_rn(mull[h], f_next);
         }
         // cell j gathers j, j-1 and (label cells, when allowed) j-2 of the previous frame; in place, top down
         double so[K];
 #pragma unroll
         for (int j = K - 1; j >= 2; j--) {
-          double a = x[j] + x[j - 1];
+          double a = __dadd_rn(x[j], x[j - 1]);
           if (j & 1) a = fma(skipd[j >> 1], x[j - 2], a);
           so[j] = a;
-          x[j] = a * ((j & 1) ? mull[j >> 1] : mulb);
+          x[j] = __dmul_rn(a, (j & 1) ? mull[j >> 1] : mulb);
         }
-        if (!FULLG && has_in && i > 0) {
+        if (!FULLG && bnd_on) {
           const long long t0 = WV_CLK();
           while ((int)q.w != i) q = wv_ld_volatile_v4(slot);
           WV_DBG_ADD(4, WV_CLK() - t0);
           src_e = (int)q.z;
-          const double bin = __hiloint2double((int)q.y, (int)q.x) * pow2i(min(src_e - e, 600));   // bounded: a few more lane hops (2^192 each) before the next re-centring cannot overflow
+          const double bin = __dmul_rn(__hiloint2double((int)q.y, (int)q.x), pow2i(min(src_e - e, 600)));
           if (lane == 0) bxs = bin;
         }
         {
-          so[1] = fma(skipd[0], bxs, x[1] + x[0]);
-          x[1] = so[1] * mull[0];
-          so[0] = x[0] + bxs;
-          x[0] = so[0] * mulb;
+          so[1] = fma(skipd[0], bxs, __dadd_rn(x[1], x[0]));
+          x[1] = __dmul_rn(so[1], mull[0]);
+          so[0] = __dadd_rn(x[0], bxs);
+          x[0] = __dmul_rn(so[0], mulb);
         }
         // drop the frame into the val ring: alpha with its emission (forward), beta before its emission (backward)
         {
@@ -416,26 +426,38 @@ __device__ void wave_lattice(const WaveParams& p, const WaveView& sv, int b, int
           vale0[(size_t)k * LANES] = BWD ? e : (apply ? en_next : e);
         }
         if (apply) { e = en_next; fb = fb_next; }
-        if (has_out)
-          wv_st_volatile_v4_if(bnd_out + (i & (RB - 1)),
-                               make_uint4((uint32_t)__double2loint(x[K - 1]), (uint32_t)__double2hiint(x[K - 1]), (uint32_t)e, (uint32_t)(i + 1)),
-                               lane == 31);
+        wv_st_volatile_v4_if(bnd_out + r0 + k,
+                             make_uint4((uint32_t)__double2loint(x[K - 1]), (uint32_t)__double2hiint(x[K - 1]), (uint32_t)e, (uint32_t)(i + 1)),
+                             HOUT && lane == 31);
       }
     }
-    // publish the group (combiners and the ring owners poll these)
-    __syncwarp();
-    if (lane == 0) wv_st_release(&sv.ctl->lat_prog[w], min(i0 + G, Ti));
   };
 
-  int i0 = 0;
-  for (; i0 + G <= Ti; i0 += G) {
-    if ((i0 & (CF - 1)) == 0) chunk_wait(i0);
-    group(std::true_type{}, i0);
+  // frames [0, n) swept and in the val ring (combiners and the ring owners poll this): after every group.  Once per
+  // 8-frame chunk measured slower on c2 (137 -> 146 us, in the build with a lattice loop per wavefront position,
+  // DESIGN.md K2w): the combiners then take frames in bursts of eight and the lattice warps wait for the val ring
+  auto publish = [&](int n) {
+    __syncwarp();
+    if (lane == 0) wv_st_release(&sv.ctl->lat_prog[w], n);
+  };
+  chunk_wait(0);
+  if (Ti < G) {
+    group(std::false_type{}, std::true_type{}, 0);
+  } else {
+    group(std::true_type{}, std::true_type{}, 0);
+    publish(G);
+    int i0 = G;
+    for (; i0 + G <= Ti; i0 += G) {
+      if ((i0 & (CF - 1)) == 0) chunk_wait(i0);
+      group(std::true_type{}, std::false_type{}, i0);
+      publish(i0 + G);
+    }
+    if (i0 < Ti) {
+      if ((i0 & (CF - 1)) == 0) chunk_wait(i0);
+      group(std::false_type{}, std::false_type{}, i0);
+    }
   }
-  if (i0 < Ti) {
-    if ((i0 & (CF - 1)) == 0) chunk_wait(i0);
-    group(std::false_type{}, i0);
-  }
+  publish(Ti);
   WV_DBG_ADD(0, WV_CLK() - tstart);
   // exit cells S-1 and S-2 of the last frame: Z = their sum (ctc_loss.cpp:63-70)
 #pragma unroll
@@ -636,8 +658,9 @@ __device__ void wave_combiner(const WaveParams& p, const WaveView& sv, int b, in
     // A lane sums the posteriors of its symbol's label cells in list order.
     {
       const int t = frame_t(i);
-      const double* Erow = sv.E + (size_t)(i & (L.R - 1)) * L.es;
-      const float rs = (float)Erow[p.V + 1];
+      const double* Ef = sv.E + (i & (L.R - 1));
+      const int ecs = L.ecs;
+      const float rs = (float)Ef[(p.V + 1) * ecs];
       const long long gbase = (long long)b * p.gsb + (long long)t * p.gst;
       for (int v = lane; v < p.V; v += 32) {
         // the symbol's label cells are contiguous in the row: four independent partial sums, fixed order
@@ -650,7 +673,7 @@ __device__ void wave_combiner(const WaveParams& p, const WaveView& sv, int b, in
           a3 += kk + 3 < k1 ? post[kk + 3] : 0.f;
         }
         const float a = (a0 + a1) + (a2 + a3);
-        const float gv = sc * ((float)Erow[v] * rs - a * (1.f / 2147483648.f));
+        const float gv = sc * ((float)Ef[v * ecs] * rs - a * (1.f / 2147483648.f));
         if (p.dtype == E2E_F32) reinterpret_cast<float*>(p.grads)[gbase + v] = gv;
         else if (p.dtype == E2E_BF16) reinterpret_cast<__nv_bfloat16*>(p.grads)[gbase + v] = __float2bfloat16_rn(gv);
         else reinterpret_cast<__half*>(p.grads)[gbase + v] = __float2half_rn(gv);
