@@ -3,7 +3,7 @@
 Hot path only: CTC loss forward+backward and greedy CTC decoding, as hand-written CUDA kernels in
 ``libe2e_ctc.so`` (C ABI in ``include/e2e_ctc.h``).  See DESIGN.md / INTEGRATION.md.
 """
-from .decoders.ctc_decoder import AlignmentResults, CTCDecoder, CTCDecoderError, DecoderResults, NBestResults
+from .decoders.ctc_decoder import AlignmentResults, CTCDecoder, CTCDecoderError, DecoderResults, ErrorCounts, NBestResults
 from .encoders.text_encoders import CTCEncoder
 from .engine import CTCGreedyEngine, CTCLossEngine, GraphedStep
 from .functions.forward_backward import ForwardBackwardLossFunction
@@ -12,5 +12,6 @@ from .modules.ctc_score import CTCScore
 
 __all__ = ["CTCLoss", "CTCScore", "CTCDecoder", "CTCEncoder", "CTCLossEngine", "CTCGreedyEngine",
            "ForwardBackwardLossFunction", "ForwardBackwardLossBase", "CTCDecoderError", "DecoderResults", "NBestResults", "AlignmentResults",
+           "ErrorCounts",
            "GraphedStep", "GraphedCTCStep"]
 __version__ = "0.1.0"

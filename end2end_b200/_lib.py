@@ -35,9 +35,10 @@ EXPORTS = (
     "e2e_ctc_score_workspace_bytes", "e2e_ctc_score_device",
     "e2e_ctc_score_backward_workspace_bytes", "e2e_ctc_score_backward_device",
     "e2e_ctc_align_nbest_workspace_bytes", "e2e_ctc_align_nbest_device",
+    "e2e_ctc_edit_distance_workspace_bytes", "e2e_ctc_edit_distance_device",
 )
 KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score",
-                "score_backward", "score_backward_rows")
+                "score_backward", "score_backward_rows", "edit_distance")
 
 
 class Desc(ctypes.Structure):
@@ -50,6 +51,16 @@ class Desc(ctypes.Structure):
         ("logits_stride_b", ctypes.c_int64), ("logits_stride_t", ctypes.c_int64),
         ("grads_stride_b", ctypes.c_int64), ("grads_stride_t", ctypes.c_int64),
         ("targets_stride_b", ctypes.c_int64),
+    ]
+
+
+class EditDesc(ctypes.Structure):
+    """struct e2e_ctc_edit_desc"""
+    _fields_ = [
+        ("batch", ctypes.c_int32), ("n_hyp", ctypes.c_int32), ("hyp_width", ctypes.c_int32),
+        ("ref_width", ctypes.c_int32), ("tokens_itype", ctypes.c_int32), ("lengths_itype", ctypes.c_int32),
+        ("separator", ctypes.c_int32), ("reserved0", ctypes.c_int32),
+        ("hyp_stride_b", ctypes.c_int64), ("ref_stride_b", ctypes.c_int64),
     ]
 
 
@@ -142,6 +153,11 @@ def load():
     L.e2e_ctc_align_nbest_workspace_bytes.restype = sz
     L.e2e_ctc_align_nbest_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
     L.e2e_ctc_align_nbest_device.restype = ctypes.c_int
+    ep = ctypes.POINTER(EditDesc)
+    L.e2e_ctc_edit_distance_workspace_bytes.argtypes = [ep]
+    L.e2e_ctc_edit_distance_workspace_bytes.restype = sz
+    L.e2e_ctc_edit_distance_device.argtypes = [ep, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]
+    L.e2e_ctc_edit_distance_device.restype = ctypes.c_int
     L.e2e_ctc_host_alloc.argtypes = [sz, ctypes.POINTER(vp)]
     L.e2e_ctc_host_alloc.restype = ctypes.c_int
     L.e2e_ctc_host_free.argtypes = [vp]

@@ -19,7 +19,7 @@ LIB = os.path.join(LIBDIR, "libe2e_ctc.so")
 SOURCES = ["api.cu", "comm.cu", "ctc_rowstats.cu", "ctc_fused_a.cu", "ctc_fused_b.cu", "ctc_fused_c.cu",
            "ctc_wave_a.cu", "ctc_wave_b.cu", "ctc_sweep_a.cu", "ctc_sweep_b.cu", "ctc_sweep_c.cu", "ctc_sweep_d.cu",
            "ctc_grad.cu", "ctc_greedy.cu", "ctc_viterbi.cu", "ctc_noblank.cu", "ctc_beam.cu",
-           "ctc_score.cu"]
+           "ctc_score.cu", "edit_distance.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

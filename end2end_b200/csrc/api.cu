@@ -753,6 +753,57 @@ int e2e_ctc_score_backward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const
                                reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
+// ---- word / token errors of N hypotheses per utterance (K11) -----------------------------------------------------
+static int check_edit(const e2e_ctc_edit_desc* d) {
+  if (!d) { set_error("null descriptor"); return E2E_ERR_INVALID_ARGUMENT; }
+  if (d->batch < 1 || d->n_hyp < 1 || d->hyp_width < 0 || d->ref_width < 0) {
+    set_error("bad shape batch=%d n_hyp=%d hyp_width=%d ref_width=%d", d->batch, d->n_hyp, d->hyp_width, d->ref_width);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  if ((d->tokens_itype != E2E_I32 && d->tokens_itype != E2E_I64) || (d->lengths_itype != E2E_I32 && d->lengths_itype != E2E_I64)) {
+    set_error("bad index type");
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  if (d->separator < -1) { set_error("separator %d: -1 (token level) or a token id >= 0 (word level)", d->separator); return E2E_ERR_INVALID_ARGUMENT; }
+  if ((d->hyp_width > 0 && d->hyp_stride_b < d->hyp_width) || (d->ref_width > 0 && d->ref_stride_b < d->ref_width)) {
+    set_error("row stride below the width: hyps %lld < %d or refs %lld < %d", (long long)d->hyp_stride_b, d->hyp_width,
+              (long long)d->ref_stride_b, d->ref_width);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  if (d->ref_width > 4095 || d->hyp_width > 65535) {
+    set_error("edit distance: reference width %d (limit 4095) or hypothesis width %d (limit 65535) exceeds this build's limits",
+              d->ref_width, d->hyp_width);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  if ((long long)d->batch * ((d->n_hyp + 7) / 8) > 0x7fffffffLL) {
+    set_error("batch %d x n_hyp %d hypotheses exceed the grid (2^31 - 1 CTAs)", d->batch, d->n_hyp);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  return E2E_OK;
+}
+
+size_t e2e_ctc_edit_distance_workspace_bytes(const e2e_ctc_edit_desc* desc) {
+  if (check_edit(desc) != E2E_OK) return 0;
+  return 256;   // nothing is stashed; 0 stays the "unsupported" answer
+}
+
+int e2e_ctc_edit_distance_device(const e2e_ctc_edit_desc* desc, const void* hyps, const void* hyp_lengths,
+                                 const void* refs, const void* ref_lengths, int64_t* errors, int64_t* substitutions,
+                                 int64_t* insertions, int64_t* deletions, int64_t* reference_units,
+                                 void* workspace, size_t workspace_bytes, void* cuda_stream) {
+  int rc = check_edit(desc);
+  if (rc != E2E_OK) return rc;
+  if (!hyp_lengths || !ref_lengths || !errors || !substitutions || !insertions || !deletions || !reference_units ||
+      (!hyps && desc->hyp_width > 0) || (!refs && desc->ref_width > 0)) {
+    set_error("null pointer argument");
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  rc = check_ws(workspace, workspace_bytes, e2e_ctc_edit_distance_workspace_bytes(desc));
+  if (rc != E2E_OK) return rc;
+  return launch_edit_distance(*desc, hyps, hyp_lengths, refs, ref_lengths, errors, substitutions, insertions, deletions,
+                              reference_units, reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
 // ---- pinned host memory for result buffers -------------------------------------------------------
 // The host-buffer entry points write their results straight into PINNED caller buffers (see e2e_ctc_engine_loss_host);
 // a binding that has no pinned allocator of its own takes its result buffers from here.

@@ -115,7 +115,7 @@ constexpr int kFlagInfeasible = 1, kFlagInvalid = 2;
 void set_error(const char* fmt, ...);
 
 // Launch accounting + optional per-kernel device timing (CUDA events on the launching stream).
-enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kKernelScoreGrad, kKernelScoreRows, kNumKernels };
+enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kKernelScoreGrad, kKernelScoreRows, kKernelEdit, kNumKernels };
 // e2e_ctc_profile_read's smallest n_kinds: the kinds up to kKernelScore (kinds added later are dropped for such callers)
 constexpr int kMinProfileKinds = kKernelScore + 1;
 void launch_begin(int kind, cudaStream_t s);
@@ -277,6 +277,11 @@ bool score_backward_supported(const e2e_ctc_desc& d);
 size_t score_backward_workspace_bytes(const e2e_ctc_desc& d, int n_hyp);
 int launch_score_backward(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
                           const void* hyp_len, const double* grad_scores, void* grads, char* ws, cudaStream_t s);
+// edit distance of n_hyp hypotheses per utterance (K11): dynamic shared memory of a launch, and the launch
+size_t edit_distance_smem_bytes(int ref_width, int words);
+int launch_edit_distance(const e2e_ctc_edit_desc& d, const void* hyps, const void* hyp_lengths, const void* refs,
+                         const void* ref_lengths, int64_t* errors, int64_t* substitutions, int64_t* insertions,
+                         int64_t* deletions, int64_t* reference_units, cudaStream_t s);
 size_t noblank_workspace_bytes(const e2e_ctc_desc& d);
 bool noblank_supported(const e2e_ctc_desc& d);
 int launch_noblank(const e2e_ctc_desc& d, int space_idx, const void* lp, const void* targets, const void* in_len,

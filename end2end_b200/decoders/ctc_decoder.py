@@ -9,7 +9,9 @@
   host (N-best rescoring);
 * the exact CTC log-likelihood of given transcripts, N per utterance: ``score`` (``decode_nbest``'s list or any other);
 * timestamps of given transcripts, N per utterance: ``align`` -- the best path, each token's frame span, word spans and
-  the best path's log-probability.
+  the best path's log-probability;
+* word and token errors of N transcripts per utterance against a reference: ``errors`` -- the risk of N-best sequence
+  training and the counts behind WER / CER.
 
 KenLM decoding (``lm_path``) stays the reference's CPU code and is out of scope; asking for it here raises
 ``NotImplementedError`` instead of silently decoding without the model.
@@ -39,6 +41,12 @@ AlignmentResults = namedtuple("AlignmentResults", ["alignments",
                                                    "token_ends",
                                                    "path_scores",
                                                    "word_spans"])
+
+ErrorCounts = namedtuple("ErrorCounts", ["errors",
+                                         "substitutions",
+                                         "insertions",
+                                         "deletions",
+                                         "reference_units"])
 
 
 def word_spans(tokens, starts, ends, labels):
@@ -207,6 +215,37 @@ class CTCDecoder:
             spans = [[word_spans(hyps[b][n][:lens[b][n]], s0[b][n], s1[b][n], self._labels) for n in range(N)]
                      for b in range(B)]
         return AlignmentResults(aligned, starts, ends, path_scores, spans)
+
+    def errors(self, hypotheses, hypotheses_lengths, references, references_lengths, *, level="word"):
+        """Word or token errors of N transcripts per utterance against the utterance's reference, on the GPU: the risk
+        of minimum word error rate training and the counts behind WER and CER.  ``errors`` is the least number of unit
+        substitutions, insertions (a hypothesis unit with no reference counterpart) and deletions (a reference unit the
+        hypothesis misses) that turn the reference into the hypothesis, each costing 1.  The split is that of the
+        least-errors alignment with the most substitutions; tools with weighted costs (sclite) can split the same total
+        differently.
+
+        :param hypotheses: ``(B, N, max length)`` int32 / int64 labels (``decode_nbest``'s ``decoded_targets`` as they
+            come), or ``(B, max length)`` for one hypothesis per utterance (``decode`` / ``decode_greedy``'s
+            ``decoded_targets``)
+        :param hypotheses_lengths: ``(B, N)`` or ``(B,)`` to match; the single symbol ``-1`` with length 1 (``decode``'s
+            empty result) is the empty hypothesis, and so are the slots ``decode_nbest`` left unused (length 0): mask
+            them with ``nbest.scores == -inf``
+        :param references: ``(B, max length)`` int32 / int64 labels, e.g. ``CTCLoss``'s ``targets``
+        :param references_lengths: ``(B,)``, e.g. ``targets_lengths``
+        :param level: ``"word"``: units are words, maximal runs of labels other than ``" "`` (which ``labels`` must
+            hold), two words being equal iff they are the same labels; ``"token"``: every label is a unit (CER when the
+            labels are characters)
+        :return: ``ErrorCounts(errors, substitutions, insertions, deletions, reference_units)`` -- CPU int64 tensors,
+            ``(B, N)`` each (``N = 1`` for the two-dimensional form) and ``reference_units`` ``(B,)``, the number of
+            reference units.  WER is ``errors.sum() / reference_units.sum()`` over a corpus; ``errors / reference_units``
+            per utterance.  A length outside ``[0, width]`` raises ``ValueError`` (CPU lengths) or gives ``-1`` counts
+            for its pairs (CUDA lengths)
+        """
+        if level not in ("word", "token"):
+            raise ValueError("level must be \"word\" or \"token\", got %r" % (level,))
+        out = self._decoder.errors_device(hypotheses, hypotheses_lengths, references, references_lengths,
+                                          words=level == "word")
+        return ErrorCounts(*(t.cpu() for t in out))
 
     def decode_greedy(self, logits, logits_lengths=None):
         """

@@ -24,6 +24,7 @@ import os
 import torch
 
 from . import _lib
+from .utils.hypotheses import empty_marker_as_empty
 
 _DTYPES = {torch.float32: _lib.E2E_F32, torch.bfloat16: _lib.E2E_BF16,
            torch.float16: _lib.E2E_F16, torch.float64: _lib.E2E_F64}
@@ -74,6 +75,9 @@ def _as_index(t, device, name):
 _LIMITS = None
 #: longest hypothesis the Viterbi aligner takes (csrc/ctc_viterbi.cu: lattices of at most 2048 cells, 2 L + 1 for CTC)
 ALIGN_MAX_TARGETS = 1023
+#: widest reference and hypothesis rows the edit distance takes (csrc/edit_distance.cu: its key errors * 4096 -
+#: substitutions stays within int32)
+EDIT_MAX_REF_WIDTH, EDIT_MAX_HYP_WIDTH = 4095, 65535
 
 
 def _limits():
@@ -935,3 +939,80 @@ class CTCBeamEngine(CTCGreedyEngine):
                 ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(aligned),
                 _ptr(starts), _ptr(ends), _ptr(path_scores), _ptr(ws), ws.numel(), _stream(dev)))
         return aligned, starts, ends, path_scores
+
+    def errors_device(self, hyps, hyp_lengths, refs, ref_lengths, words=False):
+        """Edit distance of N hypotheses per utterance against the utterance's reference, on the GPU without
+        synchronising: ``(errors, substitutions, insertions, deletions)`` ``[B, N]`` int64 and ``reference_units`` ``[B]``
+        int64 (the WER / CER denominator).  ``hyps`` ``[B, N, W]`` with ``hyp_lengths`` ``[B, N]``, or ``[B, W]`` with
+        ``[B]`` (one hypothesis per utterance, counted as N = 1); ``refs`` ``[B, Wr]`` with ``ref_lengths`` ``[B]`` (the
+        loss's ``targets`` / ``targets_lengths``).  int32 and int64 may be mixed.  ``decode``'s empty result (the single
+        symbol ``-1`` with length 1) is the empty hypothesis.  ``words=False`` counts tokens (CER for character labels);
+        ``words=True`` counts words, maximal runs of tokens other than the label ``" "`` (WER).  Errors are the least
+        number of unit substitutions, insertions and deletions turning the reference into the hypothesis, split as the
+        least-errors alignment with the most substitutions.  Out-of-range lengths raise ``ValueError`` when they live on
+        the host and give ``-1`` counts for their pairs (a reference length: all N of its utterance and its
+        ``reference_units``) when they live on the device.  Input on the CPU is copied to the current CUDA device."""
+        _require_cuda()
+        if hyps.dim() == 2:                             # one hypothesis per utterance: decode's / decode_greedy's result
+            hyps, hyp_lengths = hyps[:, None], hyp_lengths.reshape(-1, 1)
+        if hyps.dim() != 3:
+            raise ValueError("hyps must be [batch, n_hyp, width] or [batch, width], got %s" % (tuple(hyps.shape),))
+        B, N, W = hyps.shape
+        if B < 1 or N < 1:
+            raise ValueError("hyps holds no hypothesis: %s" % (tuple(hyps.shape),))
+        if tuple(hyp_lengths.shape) != (B, N):
+            raise ValueError("hyp_lengths must have shape %s, got %s" % ((B, N), tuple(hyp_lengths.shape)))
+        if refs.dim() != 2 or refs.size(0) != B:
+            raise ValueError("refs must be [batch = %d, width], got %s" % (B, tuple(refs.shape)))
+        if tuple(ref_lengths.shape) != (B,):
+            raise ValueError("ref_lengths must have shape [batch = %d], got %s" % (B, tuple(ref_lengths.shape)))
+        Wr = refs.size(1)
+        if Wr > EDIT_MAX_REF_WIDTH or W > EDIT_MAX_HYP_WIDTH:
+            raise NotImplementedError("the edit distance supports reference width <= %d and hypothesis width <= %d, got %d and %d"
+                                      % (EDIT_MAX_REF_WIDTH, EDIT_MAX_HYP_WIDTH, Wr, W))
+        sep = -1
+        if words:
+            if self.space_idx < 0:
+                raise ValueError("word level needs a \" \" label to separate words; the labels have none")
+            sep = self.space_idx
+        hyp_lengths = empty_marker_as_empty(hyps, hyp_lengths)
+        # the loss's rule (_Problem): host-resident lengths are checked here, device-resident ones on the device
+        for name, lens, width in (("hyp_lengths", hyp_lengths, W), ("ref_lengths", ref_lengths, Wr)):
+            if not lens.is_cuda:
+                ll = lens.to(torch.int64)
+                if bool((ll < 0).any()) or bool((ll > width).any()):
+                    raise ValueError("%s must be in [0, %d]" % (name, width))
+        for name, t in (("hyps", hyps), ("refs", refs)):
+            if t.is_floating_point() or t.dtype == torch.bool:
+                raise TypeError("%s must be an integer tensor, got %s" % (name, t.dtype))
+        dev = next((t.device for t in (hyps, refs, hyp_lengths, ref_lengths) if t.is_cuda),
+                   torch.device("cuda", torch.cuda.current_device()))
+        with _on_device(dev):
+            hyps = _as_index(hyps, dev, "hyps").reshape(B * N, W)
+            refs = _as_index(refs, dev, "refs")
+            if hyps.dtype != refs.dtype:
+                hyps, refs = hyps.to(torch.int64), refs.to(torch.int64)
+            if W > 0 and (hyps.stride(1) != 1 or hyps.stride(0) < W):
+                hyps = hyps.contiguous()
+            if Wr > 0 and (refs.stride(1) != 1 or refs.stride(0) < Wr):
+                refs = refs.contiguous()
+            hyp_lengths = _as_index(hyp_lengths, dev, "hyp_lengths").reshape(B * N).contiguous()
+            ref_lengths = _as_index(ref_lengths, dev, "ref_lengths").contiguous()
+            if hyp_lengths.dtype != ref_lengths.dtype:
+                hyp_lengths, ref_lengths = hyp_lengths.to(torch.int64), ref_lengths.to(torch.int64)
+            d = _lib.EditDesc()
+            d.batch, d.n_hyp, d.hyp_width, d.ref_width = B, N, W, Wr
+            d.tokens_itype, d.lengths_itype = _ITYPES[hyps.dtype], _ITYPES[hyp_lengths.dtype]
+            d.separator = sep
+            d.hyp_stride_b = hyps.stride(0) if W > 0 else 0
+            d.ref_stride_b = refs.stride(0) if Wr > 0 else 0
+            need = self._L.e2e_ctc_edit_distance_workspace_bytes(ctypes.byref(d))
+            if need == 0:
+                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            counts = torch.empty(4, B, N, dtype=torch.int64, device=dev)
+            ref_units = torch.empty(B, dtype=torch.int64, device=dev)
+            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            _lib.check(self._L.e2e_ctc_edit_distance_device(
+                ctypes.byref(d), _ptr(hyps), _ptr(hyp_lengths), _ptr(refs), _ptr(ref_lengths), _ptr(counts[0]),
+                _ptr(counts[1]), _ptr(counts[2]), _ptr(counts[3]), _ptr(ref_units), _ptr(ws), ws.numel(), _stream(dev)))
+        return counts[0], counts[1], counts[2], counts[3], ref_units

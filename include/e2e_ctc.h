@@ -398,6 +398,42 @@ int e2e_ctc_engine_beam_nbest_host(e2e_ctc_engine* engine, const e2e_ctc_desc* d
                                    int64_t* decoded, int64_t* decoded_lengths, double* scores, double* log_probs,
                                    int64_t* ties);
 
+/* ------------------------------------------- N hypotheses per utterance: word / token errors ---- */
+
+/* Edit distance of n_hyp hypotheses per utterance against the utterance's reference transcript: the risk of N-best
+ * sequence training (minimum word error rate) and the counts behind WER / CER.  Row r = b * n_hyp + n of `hyps` is
+ * compared with row b of `refs`.  A token is any integer; the units compared are
+ *   separator < 0 (token level): every token row[0:length), so CER when tokens are characters;
+ *   separator >= 0 (word level): the words, maximal runs of tokens other than `separator`.  Separators are never units:
+ *       leading, trailing and repeated separators make no empty word.  Two words are equal iff they are the same token
+ *       sequence (a fingerprint filters, every match is confirmed token by token).
+ * errors is the least number of unit substitutions, insertions (a hypothesis unit with no reference counterpart) and
+ * deletions (a reference unit missing from the hypothesis), each costing 1, that turn the reference into the hypothesis.
+ * The split is that of the least-errors alignment with the most substitutions, so it is unique; tools with weighted
+ * costs (sclite) may split the same total differently.
+ *   hyps: [batch * n_hyp, hyp_width] (row stride hyp_stride_b), refs: [batch, ref_width] (row stride ref_stride_b), both
+ *       of tokens_itype; hyp_lengths [batch * n_hyp] and ref_lengths [batch] of lengths_itype;
+ *   errors, substitutions, insertions, deletions: [batch * n_hyp] int64; reference_units: [batch] int64, the number of
+ *       reference units (the WER / CER denominator).
+ * A length outside [0, width] gives -1 in every output of the pairs it belongs to (a reference length: all n_hyp pairs of
+ * the utterance and its reference_units); nothing out of range is read and the other pairs are unaffected.  Integer
+ * arithmetic without atomics: every run gives the same counts.  The call only enqueues work.  Limits: ref_width <= 4095
+ * and hyp_width <= 65535 (the DP key errors * 4096 - substitutions stays within int32); past them the workspace query
+ * returns 0 with the reason in e2e_last_error_string.  The workspace (256 bytes) is not used by the kernel. */
+typedef struct e2e_ctc_edit_desc {
+  int32_t batch, n_hyp, hyp_width, ref_width;
+  int32_t tokens_itype;              /* E2E_I32 / E2E_I64, both token matrices  */
+  int32_t lengths_itype;             /* E2E_I32 / E2E_I64, both length vectors  */
+  int32_t separator;                 /* -1: token level; else word level        */
+  int32_t reserved0;
+  int64_t hyp_stride_b, ref_stride_b;   /* elements between rows               */
+} e2e_ctc_edit_desc;
+size_t e2e_ctc_edit_distance_workspace_bytes(const e2e_ctc_edit_desc* desc);
+int e2e_ctc_edit_distance_device(const e2e_ctc_edit_desc* desc, const void* hyps, const void* hyp_lengths,
+                                 const void* refs, const void* ref_lengths, int64_t* errors, int64_t* substitutions,
+                                 int64_t* insertions, int64_t* deletions, int64_t* reference_units,
+                                 void* workspace, size_t workspace_bytes, void* cuda_stream);
+
 /* Pinned (page-locked, device-addressable) host memory for result buffers: when `losses` / `grads` of
  * e2e_ctc_engine_loss_host live in such memory the kernels store into them directly and no copy-out stage runs. */
 int e2e_ctc_host_alloc(size_t bytes, void** out);
@@ -416,7 +452,8 @@ uint64_t e2e_ctc_launch_count(void);
  * bracketed by CUDA events on its launching stream.  e2e_ctc_profile_read() waits for the pending
  * events, then fills ms[k] (summed device milliseconds) and launches[k] per kernel kind
  * k = 0 row_stats, 1 lattice, 2 gradient, 3 loss_reduce, 4 argmax, 5 collapse, 6 scale_rows, 7 viterbi,
- * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score, 12 score_backward, 13 score_backward_rows (n_kinds >= 12;
+ * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score, 12 score_backward, 13 score_backward_rows, 14 edit_distance
+ * (n_kinds >= 12;
  * the kinds past n_kinds are not reported), and clears the record.  All launches since the previous read must have been made on ONE device. */
 int e2e_ctc_profile_enable(int32_t on);
 int e2e_ctc_profile_read(double* ms, uint64_t* launches, int32_t n_kinds);
