@@ -9,8 +9,9 @@ from .engine import CTCGreedyEngine, CTCLossEngine, GraphedStep
 from .functions.forward_backward import ForwardBackwardLossFunction
 from .modules.ctc_loss import CTCLoss, ForwardBackwardLossBase, GraphedCTCStep
 from .modules.ctc_score import CTCScore
+from .modules.mwer_loss import MWERLoss
 
-__all__ = ["CTCLoss", "CTCScore", "CTCDecoder", "CTCEncoder", "CTCLossEngine", "CTCGreedyEngine",
+__all__ = ["CTCLoss", "CTCScore", "MWERLoss", "CTCDecoder", "CTCEncoder", "CTCLossEngine", "CTCGreedyEngine",
            "ForwardBackwardLossFunction", "ForwardBackwardLossBase", "CTCDecoderError", "DecoderResults", "NBestResults", "AlignmentResults",
            "ErrorCounts",
            "GraphedStep", "GraphedCTCStep"]

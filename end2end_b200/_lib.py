@@ -36,9 +36,11 @@ EXPORTS = (
     "e2e_ctc_score_backward_workspace_bytes", "e2e_ctc_score_backward_device",
     "e2e_ctc_align_nbest_workspace_bytes", "e2e_ctc_align_nbest_device",
     "e2e_ctc_edit_distance_workspace_bytes", "e2e_ctc_edit_distance_device",
+    "e2e_ctc_mwer_state_bytes", "e2e_ctc_mwer_backward_workspace_bytes", "e2e_ctc_mwer_forward_device",
+    "e2e_ctc_mwer_backward_device",
 )
 KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score",
-                "score_backward", "score_backward_rows", "edit_distance")
+                "score_backward", "score_backward_rows", "edit_distance", "mwer_forward", "mwer_weights", "mwer_backward")
 
 
 class Desc(ctypes.Structure):
@@ -149,6 +151,13 @@ def load():
     L.e2e_ctc_score_backward_workspace_bytes.restype = sz
     L.e2e_ctc_score_backward_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp]
     L.e2e_ctc_score_backward_device.restype = ctypes.c_int
+    for name in ("e2e_ctc_mwer_state_bytes", "e2e_ctc_mwer_backward_workspace_bytes"):
+        getattr(L, name).argtypes = [dp, i32]
+        getattr(L, name).restype = sz
+    L.e2e_ctc_mwer_forward_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, dbl, vp, vp, vp, sz, vp]
+    L.e2e_ctc_mwer_forward_device.restype = ctypes.c_int
+    L.e2e_ctc_mwer_backward_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, vp, sz, vp, sz, vp]
+    L.e2e_ctc_mwer_backward_device.restype = ctypes.c_int
     L.e2e_ctc_align_nbest_workspace_bytes.argtypes = [dp, i32]
     L.e2e_ctc_align_nbest_workspace_bytes.restype = sz
     L.e2e_ctc_align_nbest_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, sz, vp]

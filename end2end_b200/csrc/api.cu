@@ -1,6 +1,7 @@
 // C ABI of libe2e_ctc.so (include/e2e_ctc.h): argument checking, workspace planning, kernel
 // sequencing, and the host-buffer engine.  No torch / pybind11 types cross this boundary.
 #include <atomic>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -751,6 +752,59 @@ int e2e_ctc_score_backward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const
   if (rc != E2E_OK) return rc;
   return launch_score_backward(*desc, n_hyp, logits, hyps, logits_lengths, hyp_lengths, grad_scores, grads,
                                reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+// ---- MWER over the N-best list (K12a / K12b / K12c + the row kernel) ----------------------------------------------
+size_t e2e_ctc_mwer_state_bytes(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  if (check_score_backward(desc, n_hyp) != E2E_OK) return 0;
+  return mwer_state_bytes(*desc, n_hyp);   // 0 (message set) on overflow
+}
+
+size_t e2e_ctc_mwer_backward_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp) {
+  if (check_score_backward(desc, n_hyp) != E2E_OK) return 0;
+  return mwer_backward_workspace_bytes(*desc, n_hyp);
+}
+
+int e2e_ctc_mwer_forward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                                const void* logits_lengths, const void* hyp_lengths, const double* risk,
+                                const uint8_t* mask, double score_scale, double* losses, double* scores, void* state,
+                                size_t state_bytes, void* cuda_stream) {
+  int rc = check_score_backward(desc, n_hyp);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !hyp_lengths || !risk || !losses || (!hyps && desc->max_targets > 0)) {
+    set_error("null pointer argument");
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  if (!(score_scale > 0.0) || !std::isfinite(score_scale)) {
+    set_error("score_scale %g must be finite and > 0", score_scale);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  const size_t need = e2e_ctc_mwer_state_bytes(desc, n_hyp);
+  if (need == 0) return E2E_ERR_UNSUPPORTED;
+  rc = check_ws(state, state_bytes, need);
+  if (rc != E2E_OK) return rc;
+  return launch_mwer_forward(*desc, n_hyp, logits, hyps, logits_lengths, hyp_lengths, risk, mask, score_scale, losses,
+                             scores, reinterpret_cast<char*>(state), reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+int e2e_ctc_mwer_backward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                                 const void* logits_lengths, const void* hyp_lengths, const double* utt_scale,
+                                 void* grads, void* state, size_t state_bytes, void* workspace, size_t workspace_bytes,
+                                 void* cuda_stream) {
+  int rc = check_score_backward(desc, n_hyp);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !hyp_lengths || !utt_scale || !grads || (!hyps && desc->max_targets > 0)) {
+    set_error("null pointer argument");
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  const size_t need_state = e2e_ctc_mwer_state_bytes(desc, n_hyp);
+  const size_t need_ws = need_state ? e2e_ctc_mwer_backward_workspace_bytes(desc, n_hyp) : 0;
+  if (need_ws == 0) return E2E_ERR_UNSUPPORTED;
+  if ((rc = check_ws(state, state_bytes, need_state)) != E2E_OK) return rc;
+  if ((rc = check_ws(workspace, workspace_bytes, need_ws)) != E2E_OK) return rc;
+  return launch_mwer_backward(*desc, n_hyp, logits, hyps, logits_lengths, hyp_lengths, utt_scale, grads,
+                              reinterpret_cast<char*>(state), reinterpret_cast<char*>(workspace),
+                              reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
 // ---- word / token errors of N hypotheses per utterance (K11) -----------------------------------------------------

@@ -115,7 +115,7 @@ constexpr int kFlagInfeasible = 1, kFlagInvalid = 2;
 void set_error(const char* fmt, ...);
 
 // Launch accounting + optional per-kernel device timing (CUDA events on the launching stream).
-enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kKernelScoreGrad, kKernelScoreRows, kKernelEdit, kNumKernels };
+enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kKernelScoreGrad, kKernelScoreRows, kKernelEdit, kKernelMwerForward, kKernelMwerWeights, kKernelMwerBackward, kNumKernels };
 // e2e_ctc_profile_read's smallest n_kinds: the kinds up to kKernelScore (kinds added later are dropped for such callers)
 constexpr int kMinProfileKinds = kKernelScore + 1;
 void launch_begin(int kind, cudaStream_t s);
@@ -277,6 +277,16 @@ bool score_backward_supported(const e2e_ctc_desc& d);
 size_t score_backward_workspace_bytes(const e2e_ctc_desc& d, int n_hyp);
 int launch_score_backward(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
                           const void* hyp_len, const double* grad_scores, void* grads, char* ws, cudaStream_t s);
+// MWER over the N-best list (K12a/b/c, the scorer's passes split): the state kept from forward to backward and the
+// backward's scratch, each 0 with the message set on overflow; the forward writes losses [B] (scores [B * n_hyp] when not
+// null) and the state, the backward consumes the state (its checkpoints are overwritten: one forward, one backward)
+size_t mwer_state_bytes(const e2e_ctc_desc& d, int n_hyp);
+size_t mwer_backward_workspace_bytes(const e2e_ctc_desc& d, int n_hyp);
+int launch_mwer_forward(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
+                        const void* hyp_len, const double* risk, const unsigned char* mask, double score_scale,
+                        double* losses, double* scores, char* state, cudaStream_t s);
+int launch_mwer_backward(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
+                         const void* hyp_len, const double* utt_scale, void* grads, char* state, char* ws, cudaStream_t s);
 // edit distance of n_hyp hypotheses per utterance (K11): dynamic shared memory of a launch, and the launch
 size_t edit_distance_smem_bytes(int ref_width, int words);
 int launch_edit_distance(const e2e_ctc_edit_desc& d, const void* hyps, const void* hyp_lengths, const void* refs,

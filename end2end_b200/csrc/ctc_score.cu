@@ -228,9 +228,18 @@ __global__ void __launch_bounds__(kScoreWarps * 32) ctc_score_kernel(const Score
 // ------------------------------------------------------------------ K10: the scorer's backward ----------------------
 // d score[b, n] / d input: per group of kScoreWarps hypotheses, the occupancies gamma_bn(t, v) scaled by g[b, n] and summed
 // into one partial row per (utterance, group, frame); the row kernel below sums the groups and writes the dtype.
+//
+// One kernel body, three passes chosen at compile time.  K10 runs pass 1 (alpha, checkpoints, log p) and pass 2 (beta,
+// g * gamma) in one launch.  MWER splits them at that seam: K12a is pass 1 alone, for every in-list hypothesis, and keeps
+// the checkpoints and log p in the loss's state; K12c is pass 2 alone, from that state, with g = w_b * weight[b, n].
+enum : int { kPassBoth = 0, kPassAlpha = 1, kPassBeta = 2 };
+
 struct ScoreBwdParams {
   ScoreParams f;
-  const double* g;        // [B * N] upstream gradient of the scores
+  const double* g;        // [B * N] upstream gradient of the scores (K12c: the MWER weights of K12b)
+  const double* utt;      // K12c: [B] upstream gradient of each utterance's loss, w_b
+  const unsigned char* mask;   // K12a: [B * N] the slots in the list, or null (all)
+  double* logp;           // K12a writes, K12c reads: [B * N] log p of every slot (-inf: masked or infeasible; NaN: bad)
   double* ckpt;           // [B * N][nblk][Kc][32] alpha at the last frame of every staged block; then beta's carry
   double* scr;            // [B * N][FB][Kc][32] one block's alpha, overwritten by g * gamma
   double* part;           // [B][G][T][V] the group's partial rows (frames < T_b)
@@ -242,7 +251,7 @@ struct ScoreBwdParams {
 // K10's shared memory beyond K9's head: label chains [kScoreWarps][Lmax + 1] int | per warp {L, active, coefficient}
 size_t bwd_extra(const e2e_ctc_desc& d) { return a16((size_t)kScoreWarps * (d.max_targets + 1) * 4) + kScoreWarps * 16; }
 
-template <typename T, int K>
+template <typename T, int K, int PASS>
 __global__ void __launch_bounds__(kScoreWarps * 32, 1) ctc_score_bwd_kernel(const ScoreBwdParams q) {
   const ScoreParams& p = q.f;
   extern __shared__ __align__(16) unsigned char smem[];
@@ -270,7 +279,8 @@ __global__ void __launch_bounds__(kScoreWarps * 32, 1) ctc_score_bwd_kernel(cons
   const int Ti = p.in_len ? (int)max(-1LL, min((long long)INT_MAX, load_index(p.in_len, p.l_is64, b))) : p.T;
   const bool bad_utt = Ti < 1 || Ti > p.T;
   const int Tu = bad_utt ? 0 : Ti;
-  const double gv = live ? q.g[row] : 0.0;
+  const double gv = !live || PASS == kPassAlpha ? 0.0 : PASS == kPassBeta ? q.utt[b] * q.g[row] : q.g[row];
+  const bool in_list = live && (PASS != kPassAlpha || !q.mask || q.mask[row]);
   bool bad = false;
   int L = 0;
   if (live) {
@@ -288,8 +298,11 @@ __global__ void __launch_bounds__(kScoreWarps * 32, 1) ctc_score_bwd_kernel(cons
     if (bad) L = 0;
   }
   __syncwarp();
-  bool act = live && !bad && !bad_utt && gv != 0.0;   // a zero upstream gradient costs no sweep
-  if (act) {
+  // a zero upstream gradient costs no sweep, and so does a masked-out slot; K12c leaves a NaN weight (a bad utterance)
+  // to the coefficient below
+  bool act = live && !bad && !bad_utt &&
+             (PASS == kPassAlpha ? in_list : gv != 0.0 && (PASS == kPassBoth || gv == gv));
+  if (act && PASS != kPassAlpha) {
     // the labels grouped by symbol: chain[k] - 1 is the next position with label lab[k] (-1: none); bit 30 marks the
     // first position of every symbol other than the blank, whose lane sums the chain in position order
     for (int k = lane; k < L; k += 32) {
@@ -327,7 +340,7 @@ __global__ void __launch_bounds__(kScoreWarps * 32, 1) ctc_score_bwd_kernel(cons
 
   // ---- pass 1: alpha, a checkpoint at the end of every staged block but the last, log p ----
   double logp = -INFINITY;
-  if (__syncthreads_or(act)) {
+  if (PASS != kPassBeta && __syncthreads_or(act)) {
     for (int t0 = 0, blk = 0; t0 < Tu; t0 += p.FB, blk++) {
       const int nf = min(p.FB, Tu - t0);
       stage_block<T>(p, xb, E, stat, lab, L, Lp, t0, nf, warp, lane, act);
@@ -353,10 +366,21 @@ __global__ void __launch_bounds__(kScoreWarps * 32, 1) ctc_score_bwd_kernel(cons
       act = logp > -INFINITY;                         // an infeasible hypothesis contributes exactly 0
     }
   }
+  if (PASS == kPassAlpha) {                           // K12a: K9's score of every in-list slot, -inf for the others
+    if (live && lane == 0)
+      q.logp[row] = bad_utt ? (double)NAN : !in_list ? -INFINITY : bad ? (double)NAN : logp;
+    return;
+  }
+  if (PASS == kPassBeta) {                            // K12c: log p from K12a, through the state
+    logp = live ? q.logp[row] : -INFINITY;
+    act = act && logp > -INFINITY;
+  }
+  // K12c: a NaN weight marks a bad utterance; a bad slot with weight 0 is one K12a left out of the list
+  const bool nan_cf = PASS == kPassBeta ? gv != gv || (bad && gv != 0.0) : bad;
   if (lane == 0) {
     wL[warp] = L;
     wAct[warp] = act;
-    wCf[warp] = !live ? 0.0 : bad ? (double)NAN : act ? gv : 0.0;
+    wCf[warp] = !live ? 0.0 : nan_cf ? (double)NAN : act ? gv : 0.0;
   }
   const bool any = __syncthreads_or(act);
   if (threadIdx.x == 0) {
@@ -502,16 +526,86 @@ __global__ void __launch_bounds__(256) ctc_score_rows_kernel(const ScoreRowsPara
   }
 }
 
+// ------------------------------------------------------------------ K12b: MWER weights ------------------------------
+// One warp per utterance.  The list U_b: slots in the mask whose score is finite.  p = softmax(lambda s) over U_b (fp64,
+// max subtracted), loss_b = R_b = sum_U p r, weight = lambda p (r - R_b) in U_b and 0 elsewhere.  A NaN score or a
+// negative / NaN in-list risk: NaN loss and NaN weights for the utterance.  An empty list: loss 0.  Equal in-list risks
+// (one slot included): loss = that risk and weights exactly 0.  Lane-strided partial sums, then the butterfly: every
+// lane holds the same bits and every run gives them.
+struct MwerWeightsParams {
+  const double* s;           // [B * N] K12a's scores
+  const double* risk;        // [B * N]
+  const unsigned char* mask; // [B * N] or null
+  double* loss;              // [B]
+  double* w;                 // [B * N] lambda p (r - R)
+  double* scores;            // [B * N] copy of s for the caller, or null
+  double lam;
+  int B, N;
+};
+
+__global__ void __launch_bounds__(256) ctc_mwer_weights_kernel(const MwerWeightsParams k) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.x * 8 + warp;
+  if (b >= k.B) return;
+  const size_t r0 = (size_t)b * k.N;
+  bool bad = false;
+  double mx = -INFINITY, rlo = INFINITY, rhi = -INFINITY;
+  for (int n = lane; n < k.N; n += 32) {
+    const double s = k.s[r0 + n];
+    if (k.scores) k.scores[r0 + n] = s;
+    bad |= s != s;
+    if ((k.mask && !k.mask[r0 + n]) || !isfinite(s)) continue;
+    const double r = k.risk[r0 + n];
+    bad |= !(r >= 0.0);
+    mx = fmax(mx, __dmul_rn(k.lam, s));
+    rlo = fmin(rlo, r);
+    rhi = fmax(rhi, r);
+  }
+  bad = __any_sync(0xffffffffu, bad);
+  mx = warp_max(mx);
+  rlo = -warp_max(-rlo);
+  rhi = warp_max(rhi);
+  const bool spread = !bad && rlo < rhi;              // else every weight is 0 (or NaN) and no sum is needed
+  double z = 0.0;
+  if (spread) {
+    for (int n = lane; n < k.N; n += 32) {
+      const double s = k.s[r0 + n];
+      if ((k.mask && !k.mask[r0 + n]) || !isfinite(s)) continue;
+      z += exp(__dmul_rn(k.lam, s) - mx);
+    }
+    z = warp_sum(z);
+  }
+  double R = 0.0;
+  if (spread) {
+    for (int n = lane; n < k.N; n += 32) {
+      const double s = k.s[r0 + n];
+      if ((k.mask && !k.mask[r0 + n]) || !isfinite(s)) continue;
+      R += exp(__dmul_rn(k.lam, s) - mx) / z * k.risk[r0 + n];
+    }
+    R = warp_sum(R);
+  }
+  for (int n = lane; n < k.N; n += 32) {
+    double w = 0.0;
+    const double s = k.s[r0 + n];
+    if (bad) w = (double)NAN;
+    else if (spread && !(k.mask && !k.mask[r0 + n]) && isfinite(s)) w = k.lam * (exp(__dmul_rn(k.lam, s) - mx) / z) * (k.risk[r0 + n] - R);
+    k.w[r0 + n] = w;
+  }
+  if (lane == 0) k.loss[b] = bad ? (double)NAN : spread ? R : rlo < INFINITY ? rlo : 0.0;
+}
+
 struct ScoreBwdLayout {
   ScoreMode md;
   int G, Kc, nblk;
   size_t off_coef, off_used, off_ckpt, off_scr, off_part, total;
+  size_t off_logp, off_w, state;   // MWER: the state kept from forward to backward (logp | w | ckpt)
 };
 
 size_t align256s(size_t x) { return (x + 255) & ~(size_t)255; }
 
-// false (message set) when a size overflows size_t or a grid exceeds 2^31 - 1 CTAs
-bool bwd_layout(const e2e_ctc_desc& d, int n_hyp, ScoreBwdLayout* l) {
+// false (message set) when a size overflows size_t or a grid exceeds 2^31 - 1 CTAs.  K10: one workspace, coef | used |
+// ckpt | scr | part.  MWER: the checkpoints move to the state (logp | w | ckpt) and the workspace keeps the rest.
+bool bwd_layout(const e2e_ctc_desc& d, int n_hyp, ScoreBwdLayout* l, bool mwer = false) {
   l->md = score_mode(d, bwd_extra(d));
   l->G = (int)(((long long)n_hyp + kScoreWarps - 1) / kScoreWarps);
   l->Kc = (2 * d.max_targets + 1 + 31) / 32;
@@ -530,10 +624,22 @@ bool bwd_layout(const e2e_ctc_desc& d, int n_hyp, ScoreBwdLayout* l) {
   ovf |= __builtin_mul_overflow((size_t)groups, (size_t)d.max_frames, &a) || __builtin_mul_overflow(a, (size_t)d.alphabet, &a) ||
          __builtin_mul_overflow(a, sizeof(double), &part);
   size_t o = 0;
+  l->off_logp = l->off_w = l->state = 0;
+  if (mwer) {
+    const size_t row = align256s((size_t)d.batch * n_hyp * sizeof(double));
+    l->off_logp = o; o += row;
+    l->off_w = o; o += row;
+    l->off_ckpt = o;
+    ovf |= __builtin_add_overflow(o, align256s(ckpt), &o) || ckpt > ~(size_t)0 - 255;
+    l->state = o;
+    o = 0;
+  }
   l->off_coef = o; o += align256s(groups * sizeof(double));
   l->off_used = o; o += align256s(groups * sizeof(int));
-  l->off_ckpt = o;
-  ovf |= __builtin_add_overflow(o, align256s(ckpt), &o) || ckpt > ~(size_t)0 - 255;
+  if (!mwer) {
+    l->off_ckpt = o;
+    ovf |= __builtin_add_overflow(o, align256s(ckpt), &o) || ckpt > ~(size_t)0 - 255;
+  }
   l->off_scr = o;
   ovf |= __builtin_add_overflow(o, align256s(scr), &o) || scr > ~(size_t)0 - 255;
   l->off_part = o;
@@ -542,8 +648,87 @@ bool bwd_layout(const e2e_ctc_desc& d, int n_hyp, ScoreBwdLayout* l) {
   l->total = o;
   return true;
 }
-}  // namespace
 
+// the lattice kernel's arguments, shared by K10, K12a and K12c; ws / state carved as bwd_layout says
+void bwd_params(const e2e_ctc_desc& d, int n_hyp, const ScoreBwdLayout& l, const void* logits, const void* hyps,
+                const void* in_len, const void* hyp_len, char* ws, char* state, ScoreBwdParams* q) {
+  ScoreParams& p = q->f;
+  p.x = logits; p.hyps = hyps; p.in_len = in_len; p.hyp_len = hyp_len; p.out = nullptr;
+  p.sb = d.logits_stride_b; p.st = d.logits_stride_t; p.hs = d.targets_stride_b;
+  p.T = d.max_frames; p.V = d.alphabet; p.Lmax = d.max_targets; p.N = n_hyp; p.G = l.G;
+  p.blank = d.blank_idx; p.from_logits = d.from_logits;
+  p.t_is64 = d.targets_itype == E2E_I64; p.l_is64 = d.lengths_itype == E2E_I64;
+  p.dense = l.md.dense; p.FB = l.md.FB;
+  q->g = nullptr; q->utt = nullptr; q->mask = nullptr; q->logp = nullptr;
+  q->coef = ws ? reinterpret_cast<double*>(ws + l.off_coef) : nullptr;
+  q->used = ws ? reinterpret_cast<int*>(ws + l.off_used) : nullptr;
+  q->scr = ws ? reinterpret_cast<double*>(ws + l.off_scr) : nullptr;
+  q->part = ws ? reinterpret_cast<double*>(ws + l.off_part) : nullptr;
+  q->ckpt = reinterpret_cast<double*>((state ? state : ws) + l.off_ckpt);
+  if (state) {
+    q->logp = reinterpret_cast<double*>(state + l.off_logp);
+    q->g = reinterpret_cast<const double*>(state + l.off_w);
+  }
+  q->Kc = l.Kc; q->nblk = l.nblk;
+}
+
+// one lattice launch (K10, K12a or K12c), the K variant picked by the longest lattice
+template <typename T, int K, int PASS>
+int launch_lattice_k(const ScoreBwdLayout& l, const ScoreBwdParams& q, unsigned grid, int kind, cudaStream_t s) {
+  E2E_CUDA_TRY(cudaFuncSetAttribute(ctc_score_bwd_kernel<T, K, PASS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l.md.smem));
+  {
+    KernelTimer timer(kind, s);
+    ctc_score_bwd_kernel<T, K, PASS><<<grid, kScoreWarps * 32, l.md.smem, s>>>(q);
+  }
+  E2E_CUDA_TRY(cudaGetLastError());
+  return E2E_OK;
+}
+
+template <typename T, int PASS>
+int launch_lattice(const e2e_ctc_desc& d, const ScoreBwdLayout& l, const ScoreBwdParams& q, int kind, cudaStream_t s) {
+  const unsigned grid = (unsigned)((long long)d.batch * l.G);
+  const int cells = 2 * d.max_targets + 1;
+  if (cells <= 32 * 4) return launch_lattice_k<T, 4, PASS>(l, q, grid, kind, s);
+  if (cells <= 32 * 8) return launch_lattice_k<T, 8, PASS>(l, q, grid, kind, s);
+  if (cells <= 32 * 16) return launch_lattice_k<T, 16, PASS>(l, q, grid, kind, s);
+  return launch_lattice_k<T, 40, PASS>(l, q, grid, kind, s);
+}
+
+// the row kernel after K10 / K12c: the groups' partial rows in the input's dtype and layout
+template <typename T>
+int launch_rows(const e2e_ctc_desc& d, const ScoreBwdLayout& l, const ScoreBwdParams& q, void* grads, cudaStream_t s) {
+  ScoreRowsParams r;
+  r.x = q.f.x; r.in_len = q.f.in_len; r.part = q.part; r.coef = q.coef; r.used = q.used; r.grads = grads;
+  r.sb = d.logits_stride_b; r.st = d.logits_stride_t; r.gsb = d.grads_stride_b; r.gst = d.grads_stride_t;
+  r.B = d.batch; r.T = d.max_frames; r.V = d.alphabet; r.G = l.G; r.from_logits = d.from_logits; r.l_is64 = q.f.l_is64;
+  const unsigned grid_rows = (unsigned)(((long long)d.batch * d.max_frames + 7) / 8);
+  {
+    KernelTimer timer(kKernelScoreRows, s);
+    ctc_score_rows_kernel<T><<<grid_rows, 256, 0, s>>>(r);
+  }
+  E2E_CUDA_TRY(cudaGetLastError());
+  return E2E_OK;
+}
+
+// the lattice pass PASS and, for K10 / K12c, the row kernel, dispatched on the input dtype
+template <int PASS>
+int run_passes(const e2e_ctc_desc& d, const ScoreBwdLayout& l, const ScoreBwdParams& q, void* grads, int kind,
+               cudaStream_t s, const char* what) {
+  int rc;
+#define E2E_PASSES(TYPE)                                                      \
+  rc = launch_lattice<TYPE, PASS>(d, l, q, kind, s);                         \
+  if (rc == E2E_OK && PASS != kPassAlpha) rc = launch_rows<TYPE>(d, l, q, grads, s);
+  switch (d.dtype) {
+    case E2E_F32: E2E_PASSES(float); break;
+    case E2E_BF16: E2E_PASSES(__nv_bfloat16); break;
+    case E2E_F16: E2E_PASSES(__half); break;
+    case E2E_F64: E2E_PASSES(double); break;
+    default: set_error("%s: unsupported dtype %d", what, d.dtype); return E2E_ERR_INVALID_ARGUMENT;
+  }
+#undef E2E_PASSES
+  return rc;
+}
+}  // namespace
 bool score_supported(const e2e_ctc_desc& d) { return score_mode(d).FB >= 1; }
 
 int launch_score(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
@@ -598,54 +783,50 @@ int launch_score_backward(const e2e_ctc_desc& d, int n_hyp, const void* logits, 
   ScoreBwdLayout l;
   if (!bwd_layout(d, n_hyp, &l)) return E2E_ERR_UNSUPPORTED;
   ScoreBwdParams q;
-  ScoreParams& p = q.f;
-  p.x = logits; p.hyps = hyps; p.in_len = in_len; p.hyp_len = hyp_len; p.out = nullptr;
-  p.sb = d.logits_stride_b; p.st = d.logits_stride_t; p.hs = d.targets_stride_b;
-  p.T = d.max_frames; p.V = d.alphabet; p.Lmax = d.max_targets; p.N = n_hyp; p.G = l.G;
-  p.blank = d.blank_idx; p.from_logits = d.from_logits;
-  p.t_is64 = d.targets_itype == E2E_I64; p.l_is64 = d.lengths_itype == E2E_I64;
-  p.dense = l.md.dense; p.FB = l.md.FB;
+  bwd_params(d, n_hyp, l, logits, hyps, in_len, hyp_len, ws, nullptr, &q);
   q.g = grad_scores;
-  q.coef = reinterpret_cast<double*>(ws + l.off_coef);
-  q.used = reinterpret_cast<int*>(ws + l.off_used);
-  q.ckpt = reinterpret_cast<double*>(ws + l.off_ckpt);
-  q.scr = reinterpret_cast<double*>(ws + l.off_scr);
-  q.part = reinterpret_cast<double*>(ws + l.off_part);
-  q.Kc = l.Kc; q.nblk = l.nblk;
-  ScoreRowsParams r;
-  r.x = logits; r.in_len = in_len; r.part = q.part; r.coef = q.coef; r.used = q.used; r.grads = grads;
-  r.sb = d.logits_stride_b; r.st = d.logits_stride_t; r.gsb = d.grads_stride_b; r.gst = d.grads_stride_t;
-  r.B = d.batch; r.T = d.max_frames; r.V = d.alphabet; r.G = l.G; r.from_logits = d.from_logits; r.l_is64 = p.l_is64;
-  const unsigned grid = (unsigned)((long long)d.batch * l.G);
-  const unsigned grid_rows = (unsigned)(((long long)d.batch * d.max_frames + 7) / 8);
-  const int cells = 2 * d.max_targets + 1;
-#define E2E_K10_(TYPE, K_)                                                                                       \
-  do {                                                                                                          \
-    E2E_CUDA_TRY(cudaFuncSetAttribute(ctc_score_bwd_kernel<TYPE, K_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)l.md.smem)); \
-    KernelTimer timer(kKernelScoreGrad, s);                                                                     \
-    ctc_score_bwd_kernel<TYPE, K_><<<grid, kScoreWarps * 32, l.md.smem, s>>>(q);                                \
-  } while (0)
-#define E2E_K10(TYPE)                                                                                            \
-  do {                                                                                                          \
-    if (cells <= 32 * 4) E2E_K10_(TYPE, 4);                                                                     \
-    else if (cells <= 32 * 8) E2E_K10_(TYPE, 8);                                                                \
-    else if (cells <= 32 * 16) E2E_K10_(TYPE, 16);                                                              \
-    else E2E_K10_(TYPE, 40);                                                                                    \
-    E2E_CUDA_TRY(cudaGetLastError());                                                                           \
-    KernelTimer timer(kKernelScoreRows, s);                                                                     \
-    ctc_score_rows_kernel<TYPE><<<grid_rows, 256, 0, s>>>(r);                                                   \
-  } while (0)
-  switch (d.dtype) {
-    case E2E_F32: E2E_K10(float); break;
-    case E2E_BF16: E2E_K10(__nv_bfloat16); break;
-    case E2E_F16: E2E_K10(__half); break;
-    case E2E_F64: E2E_K10(double); break;
-    default: set_error("score backward: unsupported dtype %d", d.dtype); return E2E_ERR_INVALID_ARGUMENT;
+  return run_passes<kPassBoth>(d, l, q, grads, kKernelScoreGrad, s, "score backward");
+}
+
+size_t mwer_state_bytes(const e2e_ctc_desc& d, int n_hyp) {
+  ScoreBwdLayout l;
+  return bwd_layout(d, n_hyp, &l, true) ? l.state : 0;
+}
+
+size_t mwer_backward_workspace_bytes(const e2e_ctc_desc& d, int n_hyp) {
+  ScoreBwdLayout l;
+  return bwd_layout(d, n_hyp, &l, true) ? l.total : 0;
+}
+
+int launch_mwer_forward(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
+                        const void* hyp_len, const double* risk, const unsigned char* mask, double score_scale,
+                        double* losses, double* scores, char* state, cudaStream_t s) {
+  ScoreBwdLayout l;
+  if (!bwd_layout(d, n_hyp, &l, true)) return E2E_ERR_UNSUPPORTED;
+  ScoreBwdParams q;
+  bwd_params(d, n_hyp, l, logits, hyps, in_len, hyp_len, nullptr, state, &q);
+  q.mask = mask;
+  int rc = run_passes<kPassAlpha>(d, l, q, nullptr, kKernelMwerForward, s, "mwer forward");
+  if (rc != E2E_OK) return rc;
+  MwerWeightsParams k;
+  k.s = q.logp; k.risk = risk; k.mask = mask; k.loss = losses; k.w = const_cast<double*>(q.g); k.scores = scores;
+  k.lam = score_scale; k.B = d.batch; k.N = n_hyp;
+  {
+    KernelTimer timer(kKernelMwerWeights, s);
+    ctc_mwer_weights_kernel<<<(unsigned)((d.batch + 7) / 8), 256, 0, s>>>(k);
   }
-#undef E2E_K10
-#undef E2E_K10_
   E2E_CUDA_TRY(cudaGetLastError());
   return E2E_OK;
+}
+
+int launch_mwer_backward(const e2e_ctc_desc& d, int n_hyp, const void* logits, const void* hyps, const void* in_len,
+                         const void* hyp_len, const double* utt_scale, void* grads, char* state, char* ws, cudaStream_t s) {
+  ScoreBwdLayout l;
+  if (!bwd_layout(d, n_hyp, &l, true)) return E2E_ERR_UNSUPPORTED;
+  ScoreBwdParams q;
+  bwd_params(d, n_hyp, l, logits, hyps, in_len, hyp_len, ws, state, &q);
+  q.utt = utt_scale;
+  return run_passes<kPassBeta>(d, l, q, grads, kKernelMwerBackward, s, "mwer backward");
 }
 
 }  // namespace e2e

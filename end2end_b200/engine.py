@@ -19,6 +19,7 @@ PyTorch is used for device memory and streams only; every byte of arithmetic hap
 ``libe2e_ctc.so``.
 """
 import ctypes
+import math
 import os
 
 import torch
@@ -856,6 +857,74 @@ class CTCBeamEngine(CTCGreedyEngine):
             _lib.check(self._L.e2e_ctc_score_backward_device(
                 ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(g),
                 _ptr(grads), _ptr(ws), ws.numel(), _stream(dev)))
+        return grads
+
+    def mwer_workspace_bytes(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):
+        """``(state, backward scratch)`` bytes of ``mwer_forward_device`` / ``mwer_backward_device`` for these arguments."""
+        _require_cuda()
+        _, _, _, _, d, dev, N = self._score_args(logits, hyps, hyp_lengths, logits_lengths, from_logits)
+        with _on_device(dev):
+            return (int(self._L.e2e_ctc_mwer_state_bytes(ctypes.byref(d), N)),
+                    int(self._L.e2e_ctc_mwer_backward_workspace_bytes(ctypes.byref(d), N)))
+
+    def mwer_forward_device(self, logits, hyps, hyp_lengths, risk, mask=None, logits_lengths=None, from_logits=False,
+                            score_scale=1.0, state=None):
+        """Minimum word error rate over the list, forward (K12a scores + checkpoints, K12b weights), without
+        synchronising: ``(losses [B] float64, scores [B, N] float64, state)``.  ``risk`` ``[B, N]`` (any real dtype, e.g.
+        ``errors_device``'s word errors); ``mask`` ``[B, N]`` bool or ``None`` (every slot).  The list of utterance b is
+        its slots in the mask with a finite score; ``losses[b] = sum_n p_bn risk_bn`` with ``p`` the softmax of
+        ``score_scale * scores`` over the list.  ``scores`` are ``score_device``'s in the list and ``-inf`` outside it.
+        ``state`` (a uint8 device tensor, allocated when ``None``) is what ``mwer_backward_device`` consumes.  Argument
+        rules as for ``score_device``: host-resident lengths and labels are checked for every slot, masked or not
+        (``ValueError``); a bad device-resident length or label in the list, or a negative risk there, gives its
+        utterance a NaN loss, and one in a masked-out slot changes nothing.  ``score_scale`` must be finite and > 0."""
+        _require_cuda()
+        score_scale = float(score_scale)
+        if not math.isfinite(score_scale) or score_scale <= 0.0:
+            raise ValueError("score_scale must be finite and > 0, got %r" % score_scale)
+        logits, hyps, hyp_lengths, logits_lengths, d, dev, N = self._score_args(logits, hyps, hyp_lengths, logits_lengths,
+                                                                               from_logits)
+        B = d.batch
+        if tuple(risk.shape) != (B, N):
+            raise ValueError("risk must have shape [batch, n_hyp] = %s, got %s" % ((B, N), tuple(risk.shape)))
+        if mask is not None and tuple(mask.shape) != (B, N):
+            raise ValueError("mask must have shape [batch, n_hyp] = %s, got %s" % ((B, N), tuple(mask.shape)))
+        with _on_device(dev):
+            need = self._L.e2e_ctc_mwer_state_bytes(ctypes.byref(d), N)
+            if need == 0:
+                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            r = risk.detach().to(dev, torch.float64).contiguous()
+            m = None if mask is None else mask.detach().to(dev).ne(0).to(torch.uint8).contiguous()
+            if state is None:
+                state = torch.empty(need, dtype=torch.uint8, device=dev)
+            losses = torch.empty(B, dtype=torch.float64, device=dev)
+            scores = torch.empty(B, N, dtype=torch.float64, device=dev)
+            _lib.check(self._L.e2e_ctc_mwer_forward_device(
+                ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(r), _ptr(m),
+                score_scale, _ptr(losses), _ptr(scores), _ptr(state), state.numel(), _stream(dev)))
+        return losses, scores, state
+
+    def mwer_backward_device(self, logits, hyps, hyp_lengths, utt_scale, state, logits_lengths=None, from_logits=False):
+        """The gradient of ``sum_b utt_scale[b] * losses[b]`` of the ``mwer_forward_device`` call that filled ``state``
+        (same arguments), in ``score_backward_device``'s form and convention (K12c, then the row kernel).  ``utt_scale``
+        ``[B]``.  It overwrites the state's checkpoints: one forward's state serves one backward."""
+        _require_cuda()
+        logits, hyps, hyp_lengths, logits_lengths, d, dev, N = self._score_args(logits, hyps, hyp_lengths, logits_lengths,
+                                                                               from_logits)
+        B = d.batch
+        if tuple(utt_scale.shape) != (B,):
+            raise ValueError("utt_scale must have shape [batch] = (%d,), got %s" % (B, tuple(utt_scale.shape)))
+        with _on_device(dev):
+            need = self._L.e2e_ctc_mwer_backward_workspace_bytes(ctypes.byref(d), N)
+            if need == 0:
+                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            w = utt_scale.detach().to(dev, torch.float64).contiguous()
+            grads = torch.empty_like(logits)
+            d.grads_stride_b, d.grads_stride_t = grads.stride(0), grads.stride(1)
+            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            _lib.check(self._L.e2e_ctc_mwer_backward_device(
+                ctypes.byref(d), N, _ptr(logits), _ptr(hyps), _ptr(logits_lengths), _ptr(hyp_lengths), _ptr(w),
+                _ptr(grads), _ptr(state), state.numel(), _ptr(ws), ws.numel(), _stream(dev)))
         return grads
 
     def align_device(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):

@@ -365,6 +365,39 @@ int e2e_ctc_score_backward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const
                                   const void* logits_lengths, const void* hyp_lengths, const double* grad_scores,
                                   void* grads, void* workspace, size_t workspace_bytes, void* cuda_stream);
 
+/* Minimum word error rate (MWER) training over an N-best list (Prabhavalkar et al., 2018), forward and backward.  For
+ * utterance b the list U_b is the slots n with mask[b,n] != 0 (every slot when mask is NULL) whose score
+ * s_bn = log p(hyp_bn | x_b) (e2e_ctc_score_device's value, bit for bit) is finite;
+ *   p_bn = exp(lambda s_bn) / sum_{m in U_b} exp(lambda s_bm),   lambda = score_scale (finite, > 0);
+ *   losses[b] = R_b = sum_{n in U_b} p_bn risk[b,n];
+ *   d losses[b] / d s_bn = lambda p_bn (risk[b,n] - R_b), so the mean-risk baseline is part of the loss.
+ * The backward writes sum_b utt_scale[b] d losses[b] / d input, with e2e_ctc_score_backward_device's convention (the
+ * derivative of the score: sum_n g gamma on log-probabilities, sum_n g (gamma - softmax) on raw logits, 0 past T_b) and
+ * g_bn = utt_scale[b] lambda p_bn (risk[b,n] - R_b).  Rules: an empty list gives loss 0 and zero rows; equal risks over
+ * the list (a single slot included) give loss = that risk, exactly zero rows and no backward sweep; a NaN score (a bad
+ * device-resident length or label of an in-list slot, or a bad logits length) or a negative / NaN in-list risk gives
+ * that utterance a NaN loss and NaN rows t < T_b (all rows for a bad logits length).  Masked slots cost no sweep and their
+ * risks are not read; their lengths and labels only bound what is read, so an out-of-range one there changes nothing.
+ *   risk: [B * n_hyp] float64 on the device (e.g. word errors); mask: [B * n_hyp] uint8 or NULL;
+ *   losses: [B] float64; scores: [B * n_hyp] float64 or NULL (-inf for slots outside the list);
+ *   state: what the forward keeps for the backward (scores, weights, alpha checkpoints), e2e_ctc_mwer_state_bytes;
+ *   utt_scale: [B] float64 on the device, the upstream gradient of each loss;
+ *   workspace: the backward's scratch (as e2e_ctc_score_backward_device's, without the checkpoints),
+ *       e2e_ctc_mwer_backward_workspace_bytes.
+ * The backward overwrites the state's checkpoints: run the forward again before a second backward.  Both calls only
+ * enqueue work; fp64, fixed-order sums, no atomics: bitwise reproducible.  Limits as for the score; past them, with
+ * n_hyp < 1 or on overflow both size queries return 0 and set the message. */
+size_t e2e_ctc_mwer_state_bytes(const e2e_ctc_desc* desc, int32_t n_hyp);
+size_t e2e_ctc_mwer_backward_workspace_bytes(const e2e_ctc_desc* desc, int32_t n_hyp);
+int e2e_ctc_mwer_forward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                                const void* logits_lengths, const void* hyp_lengths, const double* risk,
+                                const uint8_t* mask, double score_scale, double* losses, double* scores, void* state,
+                                size_t state_bytes, void* cuda_stream);
+int e2e_ctc_mwer_backward_device(const e2e_ctc_desc* desc, int32_t n_hyp, const void* logits, const void* hyps,
+                                 const void* logits_lengths, const void* hyp_lengths, const double* utt_scale,
+                                 void* grads, void* state, size_t state_bytes, void* workspace, size_t workspace_bytes,
+                                 void* cuda_stream);
+
 /* -------------------------------------------------------------- engine, host pointers ------ */
 
 typedef struct e2e_ctc_engine e2e_ctc_engine;
@@ -452,7 +485,8 @@ uint64_t e2e_ctc_launch_count(void);
  * bracketed by CUDA events on its launching stream.  e2e_ctc_profile_read() waits for the pending
  * events, then fills ms[k] (summed device milliseconds) and launches[k] per kernel kind
  * k = 0 row_stats, 1 lattice, 2 gradient, 3 loss_reduce, 4 argmax, 5 collapse, 6 scale_rows, 7 viterbi,
- * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score, 12 score_backward, 13 score_backward_rows, 14 edit_distance
+ * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score, 12 score_backward, 13 score_backward_rows, 14 edit_distance,
+ * 15 mwer_forward, 16 mwer_weights, 17 mwer_backward (its row kernel counts as 13)
  * (n_kinds >= 12;
  * the kinds past n_kinds are not reported), and clears the record.  All launches since the previous read must have been made on ONE device. */
 int e2e_ctc_profile_enable(int32_t on);
