@@ -20,7 +20,6 @@ PyTorch is used for device memory and streams only; every byte of arithmetic hap
 """
 import ctypes
 import math
-import os
 
 import torch
 
@@ -96,19 +95,92 @@ def _dense3(x):
     return all(x.stride(i) > 0 or x.size(i) == 1 for i in (0, 1))
 
 
+def _host_layout(x):
+    """Host logits as the host engine copies them in: batch-major or time-major, dense either way."""
+    return x if x.is_contiguous() or x.permute(1, 0, 2).is_contiguous() else x.contiguous()
+
+
+def _check_logits(x, blank_idx, name):
+    """``(B, T, V)`` of a non-empty ``[batch, frames, alphabet]`` tensor of a supported dtype, with ``blank_idx`` inside
+    the alphabet unless it is ``None``."""
+    if x.dim() != 3:
+        raise ValueError("%s must be [batch, frames, alphabet], got %s" % (name, tuple(x.shape)))
+    if x.dtype not in _DTYPES:
+        raise TypeError("unsupported %s dtype %s" % (name, x.dtype))
+    B, T, V = x.shape
+    if B < 1 or T < 1 or V < 1:
+        raise ValueError("empty %s %s" % (name, tuple(x.shape)))
+    if blank_idx is not None and not 0 <= blank_idx < V:
+        raise ValueError("blank_idx %d outside the alphabet [0,%d)" % (blank_idx, V))
+    return B, T, V
+
+
+def _check_host_range(lengths, lo, hi, name):
+    """Host-resident lengths must lie in ``[lo, hi]``; device-resident ones are checked on the device."""
+    if not lengths.is_cuda:
+        t = lengths.to(torch.int64)
+        if bool((t < lo).any()) or bool((t > hi).any()):
+            raise ValueError("%s must be in [%d, %d]" % (name, lo, hi))
+
+
+def _check_host_labels(labels, lengths, V, name):
+    """Host-resident labels ``[..., L]`` must lie in ``[0, V)`` below their host-resident lengths ``[...]``."""
+    if not labels.is_cuda and not lengths.is_cuda and labels.size(-1) > 0:
+        valid = torch.arange(labels.size(-1)) < lengths.to(torch.int64).unsqueeze(-1)
+        t = labels.to(torch.int64)
+        if bool(((t < 0) | (t >= V))[valid].any()):
+            raise ValueError("%s must be in [0, %d)" % (name, V))
+
+
+def _index_args(targets, logits_lengths, targets_lengths, device):
+    """``targets [B, Lmax]`` with a unit label stride and the two length tensors, contiguous and of one dtype, as index
+    tensors on ``device``."""
+    targets = _as_index(targets, device, "targets")
+    if targets.size(1) > 0 and targets.stride(1) != 1:
+        targets = targets.contiguous()
+    logits_lengths = _as_index(logits_lengths, device, "logits_lengths")
+    targets_lengths = _as_index(targets_lengths, device, "targets_lengths")
+    if logits_lengths.dtype != targets_lengths.dtype:
+        logits_lengths, targets_lengths = logits_lengths.to(torch.int64), targets_lengths.to(torch.int64)
+    return targets, logits_lengths.contiguous(), targets_lengths.contiguous()
+
+
+def _desc(logits, blank_idx, targets, lengths, from_logits):
+    """The C descriptor of ``logits [B, T, V]`` with ``targets [B, Lmax]`` and ``lengths`` (each may be ``None``).  The
+    gradient strides stay 0: callers that write a gradient set them."""
+    d = _lib.Desc()
+    d.batch, d.max_frames, d.alphabet = logits.shape
+    d.max_targets = targets.size(1) if targets is not None else 0
+    d.blank_idx, d.dtype = int(blank_idx), _DTYPES[logits.dtype]
+    d.targets_itype = _ITYPES[targets.dtype] if targets is not None else _lib.E2E_I64
+    d.lengths_itype = _ITYPES[lengths.dtype] if lengths is not None else _lib.E2E_I64
+    d.from_logits = 1 if from_logits else 0
+    d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
+    d.targets_stride_b = targets.stride(0) if d.max_targets > 0 else 0
+    return d
+
+
+def _need(n):
+    """A workspace query's answer; 0 means the library cannot run these arguments, and its last error says why."""
+    if n == 0:
+        raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, _lib.load().e2e_last_error_string().decode("utf-8", "replace"))
+    return n
+
+
+def _host_engine(engines):
+    """The ``_HostEngine`` of the current CUDA device in an engine object's cache ``engines``, created on first use."""
+    dev = torch.cuda.current_device()
+    h = engines.get(dev)
+    if h is None:
+        h = engines[dev] = _HostEngine(dev)
+    return h
+
+
 class _Problem:
     """Validated, device-resident view of one batch plus the C descriptor."""
 
     def __init__(self, blank_idx, logits, targets, logits_lengths, targets_lengths, from_logits, device, validate=True):
-        if logits.dim() != 3:
-            raise ValueError("logits must be [batch, frames, alphabet], got %s" % (tuple(logits.shape),))
-        if logits.dtype not in _DTYPES:
-            raise TypeError("unsupported logits dtype %s" % logits.dtype)
-        B, T, V = logits.shape
-        if B < 1 or T < 1 or V < 1:
-            raise ValueError("empty logits %s" % (tuple(logits.shape),))
-        if not 0 <= blank_idx < V:
-            raise ValueError("blank_idx %d outside the alphabet [0,%d)" % (blank_idx, V))
+        B, T, V = _check_logits(logits, blank_idx, "logits")
         if targets.dim() != 2 or targets.size(0) != B:
             raise ValueError("targets must be [batch, max_target_length], got %s" % (tuple(targets.shape),))
         if logits_lengths.dim() != 1 or logits_lengths.numel() != B or \
@@ -121,39 +193,16 @@ class _Problem:
                                       % (lim.max_targets, lim.max_alphabet))
         # the reference has undefined behaviour on these; reject when it costs no device sync
         if validate and not logits_lengths.is_cuda and not targets_lengths.is_cuda:
-            ll, tl = logits_lengths.to(torch.int64), targets_lengths.to(torch.int64)
-            if bool((ll < 1).any()) or bool((ll > T).any()):
-                raise ValueError("logits_lengths must be in [1, %d]" % T)
-            if bool((tl < 0).any()) or bool((tl > Lmax).any()):
-                raise ValueError("targets_lengths must be in [0, %d]" % Lmax)
-            if not targets.is_cuda and Lmax > 0:
-                tg = targets.to(torch.int64)
-                valid = torch.arange(Lmax).unsqueeze(0) < tl.unsqueeze(1)
-                if bool(((tg < 0) | (tg >= V))[valid].any()):
-                    raise ValueError("target labels must be in [0, %d)" % V)
+            _check_host_range(logits_lengths, 1, T, "logits_lengths")
+            _check_host_range(targets_lengths, 0, Lmax, "targets_lengths")
+            _check_host_labels(targets, targets_lengths, V, "target labels")
         if not _dense3(logits):
             logits = logits.contiguous()
-        targets = _as_index(targets, device, "targets")
-        if Lmax > 0 and targets.stride(1) != 1:
-            targets = targets.contiguous()
-        logits_lengths = _as_index(logits_lengths, device, "logits_lengths")
-        targets_lengths = _as_index(targets_lengths, device, "targets_lengths")
-        if logits_lengths.dtype != targets_lengths.dtype:
-            logits_lengths, targets_lengths = logits_lengths.to(torch.int64), targets_lengths.to(torch.int64)
-        self.logits, self.targets = logits, targets
-        self.logits_lengths = logits_lengths.contiguous()
-        self.targets_lengths = targets_lengths.contiguous()
+        self.logits = logits
+        self.targets, self.logits_lengths, self.targets_lengths = _index_args(targets, logits_lengths, targets_lengths, device)
         self.B, self.T, self.V, self.Lmax = B, T, V, Lmax
-        d = _lib.Desc()
-        d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, Lmax
-        d.blank_idx, d.dtype = blank_idx, _DTYPES[logits.dtype]
-        d.targets_itype = _ITYPES[targets.dtype]
-        d.lengths_itype = _ITYPES[self.logits_lengths.dtype]
-        d.from_logits = 1 if from_logits else 0
-        d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
-        d.grads_stride_b, d.grads_stride_t = logits.stride(0), logits.stride(1)
-        d.targets_stride_b = targets.stride(0) if Lmax > 0 else 0
-        self.desc = d
+        self.desc = _desc(logits, blank_idx, self.targets, self.logits_lengths, from_logits)
+        self.desc.grads_stride_b, self.desc.grads_stride_t = logits.stride(0), logits.stride(1)
         self.workspace = None
 
     _FAST = {}
@@ -295,12 +344,8 @@ class CTCLossEngine:
         key = (grads.shape, grads.stride(), grads.dtype)
         d = self._scale_desc.get(key)
         if d is None:
-            d = _lib.Desc()
-            d.batch, d.max_frames, d.alphabet, d.max_targets = grads.size(0), grads.size(1), grads.size(2), 0
-            d.blank_idx, d.dtype = 0, _DTYPES[grads.dtype]
-            d.targets_itype = d.lengths_itype = _lib.E2E_I64
+            d = _desc(grads, 0, None, None, False)
             d.grads_stride_b, d.grads_stride_t = grads.stride(0), grads.stride(1)
-            d.logits_stride_b, d.logits_stride_t = grads.stride(0), grads.stride(1)
             if len(self._scale_desc) > 256:
                 self._scale_desc.clear()
             self._scale_desc[key] = d
@@ -370,14 +415,7 @@ class CTCLossEngine:
 
     # ------------------------------------------------------------------ internals --------------
     def _workspace(self, pb):
-        key = (pb.B, pb.T, pb.V, pb.Lmax, pb.desc.dtype, _lib.forced_kernel())
-        n = self._ws_bytes.get(key)
-        if n is None:
-            n = self._L.e2e_ctc_loss_workspace_bytes(ctypes.byref(pb.desc))
-            if n == 0:
-                raise _lib.E2EError(2, self._L.e2e_last_error_string().decode("utf-8", "replace"))
-            self._ws_bytes[key] = n
-        return torch.empty(n, dtype=torch.uint8, device=pb.logits.device)
+        return torch.empty(self._ws_need(pb), dtype=torch.uint8, device=pb.logits.device)
 
     def _scratch(self, pb):
         """Workspace of a call that is finished with it when the call's kernels are (the fused forward+backward
@@ -385,8 +423,6 @@ class CTCLossEngine:
         push a workspace-sized block through the caching allocator every step (interleaved with the live
         gradient blocks that fragments it into cudaMalloc/cudaFree cycles).  Kernels of successive calls on one
         stream are ordered, so the reuse is safe; other streams get their own buffer."""
-        if os.environ.get("E2E_CTC_NO_SCRATCH_CACHE"):
-            return self._workspace(pb)
         dev = pb.logits.device
         key = (dev.index, _raw_stream(dev.index if dev.index is not None else torch.cuda.current_device()))
         need = self._ws_need(pb)
@@ -400,24 +436,12 @@ class CTCLossEngine:
         key = (pb.B, pb.T, pb.V, pb.Lmax, pb.desc.dtype, _lib.forced_kernel())
         n = self._ws_bytes.get(key)
         if n is None:
-            n = self._L.e2e_ctc_loss_workspace_bytes(ctypes.byref(pb.desc))
-            if n == 0:
-                raise _lib.E2EError(2, self._L.e2e_last_error_string().decode("utf-8", "replace"))
-            self._ws_bytes[key] = n
+            n = self._ws_bytes[key] = _need(self._L.e2e_ctc_loss_workspace_bytes(ctypes.byref(pb.desc)))
         return n
 
-    def _host_engine(self, device):
-        h = self._host.get(device)
-        if h is None:
-            h = _HostEngine(device)
-            self._host[device] = h
-        return h
-
     def _compute_host(self, logits, targets, logits_lengths, targets_lengths, from_logits):
-        dev = torch.cuda.current_device()
         cpu = torch.device("cpu")
-        if not (logits.is_contiguous() or logits.permute(1, 0, 2).is_contiguous()):
-            logits = logits.contiguous()
+        logits = _host_layout(logits)
         # lengths and labels are range-checked by the library's host entry point (plain loops over the host
         # buffers) instead of a handful of small torch ops here
         pb = _Problem(self.blank_idx, logits, targets, logits_lengths, targets_lengths, from_logits, cpu, validate=False)
@@ -428,7 +452,7 @@ class CTCLossEngine:
         # recycles the blocks; an own pool (frombuffer over cudaHostAlloc blocks) measured 20 us SLOWER per call.
         losses = torch.empty(pb.B, dtype=logits.dtype, pin_memory=True)
         grads = pb.new_grads(pin=True)
-        h = self._host_engine(dev)
+        h = _host_engine(self._host)
         try:
             _lib.check(self._L.e2e_ctc_engine_loss_host(
                 h.handle, ctypes.byref(pb.desc), _ptr(pb.logits), _ptr(pb.targets), _ptr(pb.logits_lengths),
@@ -523,23 +547,15 @@ class CTCGreedyEngine:
         self._L = _lib.load()
         self._host = {}
 
-    def _desc(self, logits, lengths):
-        if logits.dim() != 3:
-            raise ValueError("logits must be [batch, frames, alphabet]")
-        if logits.dtype not in _DTYPES:
-            raise TypeError("unsupported logits dtype %s" % logits.dtype)
-        B, T, V = logits.shape
-        if B < 1 or T < 1 or V < 1:
-            raise ValueError("empty logits")
-        if not 0 <= self.blank_idx < V:
-            raise ValueError("blank_idx %d outside the alphabet [0,%d)" % (self.blank_idx, V))
-        d = _lib.Desc()
-        d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, 0
-        d.blank_idx, d.dtype = self.blank_idx, _DTYPES[logits.dtype]
-        d.targets_itype = _lib.E2E_I64
-        d.lengths_itype = _ITYPES[lengths.dtype] if lengths is not None else _lib.E2E_I64
-        d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
-        return d
+    def _greedy_args(self, logits, logits_lengths, **where):
+        """What both greedy variants prepare from ``logits`` in their layout: ``logits_lengths`` as an index tensor beside
+        them, the checked descriptor, and the outputs ``decoded [B, T]`` and ``lengths [B]`` allocated ``where`` (in pinned
+        host memory or on a device)."""
+        if logits_lengths is not None:
+            logits_lengths = _as_index(logits_lengths, logits.device, "logits_lengths").contiguous()
+        B, T, _ = _check_logits(logits, self.blank_idx, "logits")
+        d = _desc(logits, self.blank_idx, None, logits_lengths, False)
+        return logits_lengths, d, torch.empty(B, T, dtype=torch.int64, **where), torch.empty(B, dtype=torch.int64, **where)
 
     def decode_greedy_device(self, logits, logits_lengths=None):
         """Device tensors in, device tensors out (no synchronisation)."""
@@ -548,13 +564,8 @@ class CTCGreedyEngine:
         dev = logits.device
         if not _dense3(logits):
             logits = logits.contiguous()
-        if logits_lengths is not None:
-            logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
-        d = self._desc(logits, logits_lengths)
-        B, T = logits.size(0), logits.size(1)
+        logits_lengths, d, decoded, lengths = self._greedy_args(logits, logits_lengths, device=dev)
         with _on_device(dev):
-            decoded = torch.empty(B, T, dtype=torch.int64, device=dev)
-            lengths = torch.empty(B, dtype=torch.int64, device=dev)
             ws = torch.empty(self._L.e2e_ctc_greedy_workspace_bytes(ctypes.byref(d)), dtype=torch.uint8, device=dev)
             _lib.check(self._L.e2e_ctc_greedy_decode_device(
                 ctypes.byref(d), _ptr(logits), _ptr(logits_lengths), _ptr(decoded), _ptr(lengths),
@@ -567,21 +578,10 @@ class CTCGreedyEngine:
         if logits.is_cuda:
             decoded, lengths = self.decode_greedy_device(logits, logits_lengths_)
             return decoded.cpu(), lengths.cpu()
-        if not (logits.is_contiguous() or logits.permute(1, 0, 2).is_contiguous()):
-            logits = logits.contiguous()
-        lengths_in = None
-        if logits_lengths_ is not None:
-            lengths_in = _as_index(logits_lengths_, torch.device("cpu"), "logits_lengths").contiguous()
-        d = self._desc(logits, lengths_in)
-        B, T = logits.size(0), logits.size(1)
-        decoded = torch.empty(B, T, dtype=torch.int64, pin_memory=True)
-        lengths = torch.empty(B, dtype=torch.int64, pin_memory=True)
-        dev = torch.cuda.current_device()
-        h = self._host.get(dev)
-        if h is None:
-            h = self._host[dev] = _HostEngine(dev)
-        _lib.check(self._L.e2e_ctc_engine_greedy_host(h.handle, ctypes.byref(d), _ptr(logits), _ptr(lengths_in),
-                                                      _ptr(decoded), _ptr(lengths)))
+        logits = _host_layout(logits)
+        lengths_in, d, decoded, lengths = self._greedy_args(logits, logits_lengths_, pin_memory=True)
+        _lib.check(self._L.e2e_ctc_engine_greedy_host(_host_engine(self._host).handle, ctypes.byref(d), _ptr(logits),
+                                                      _ptr(lengths_in), _ptr(decoded), _ptr(lengths)))
         return decoded, lengths
 
 
@@ -606,11 +606,19 @@ class CTCBeamEngine(CTCGreedyEngine):
         self.last_ties = None
 
     def _beam_desc(self, logits, lengths, from_logits):
-        d = self._desc(logits, lengths)
-        d.from_logits = 1 if from_logits else 0
+        _check_logits(logits, self.blank_idx, "logits")
         if not -1 <= self.space_idx < logits.size(2):
             raise ValueError("the space label %d is outside the alphabet [0,%d)" % (self.space_idx, logits.size(2)))
-        return d
+        return _desc(logits, self.blank_idx, None, lengths, from_logits)
+
+    def _beam_args(self, logits, logits_lengths, from_logits, **where):
+        """``_greedy_args`` of both beam-search variants: the outputs are ``decoded [B, T]``, ``lengths [B]`` and
+        ``ties [B]``."""
+        if logits_lengths is not None:
+            logits_lengths = _as_index(logits_lengths, logits.device, "logits_lengths").contiguous()
+        d = self._beam_desc(logits, logits_lengths, from_logits)
+        B, T = d.batch, d.max_frames
+        return logits_lengths, d, tuple(torch.empty(*shape, dtype=torch.int64, **where) for shape in ((B, T), (B,), (B,)))
 
     def decode_device(self, logits, logits_lengths=None, from_logits=False):
         """Device tensors in, device tensors out (no synchronisation): ``(decoded [B,T] int64 zero padded, lengths [B],
@@ -620,47 +628,26 @@ class CTCBeamEngine(CTCGreedyEngine):
         dev = logits.device
         if not _dense3(logits):
             logits = logits.contiguous()
-        if logits_lengths is not None:
-            logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
-        d = self._beam_desc(logits, logits_lengths, from_logits)
-        B, T = logits.size(0), logits.size(1)
+        logits_lengths, d, out = self._beam_args(logits, logits_lengths, from_logits, device=dev)
         with _on_device(dev):
-            need = self._L.e2e_ctc_beam_workspace_bytes(ctypes.byref(d), self.beam_width)
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
-            decoded = torch.empty(B, T, dtype=torch.int64, device=dev)
-            lengths = torch.empty(B, dtype=torch.int64, device=dev)
-            ties = torch.empty(B, dtype=torch.int64, device=dev)
-            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            ws = torch.empty(_need(self._L.e2e_ctc_beam_workspace_bytes(ctypes.byref(d), self.beam_width)),
+                             dtype=torch.uint8, device=dev)
             _lib.check(self._L.e2e_ctc_beam_decode_device(
                 ctypes.byref(d), self.beam_width, self.space_idx, self.wip, _ptr(logits), _ptr(logits_lengths),
-                _ptr(decoded), _ptr(lengths), _ptr(ties), _ptr(ws), ws.numel(), _stream(dev)))
-        return decoded, lengths, ties
+                *map(_ptr, out), _ptr(ws), ws.numel(), _stream(dev)))
+        return out
 
     def decode(self, logits_, logits_lengths_=None, from_logits=False):
         _require_cuda()
         logits = logits_.detach()
         if logits.is_cuda:
-            decoded, lengths, ties = self.decode_device(logits, logits_lengths_, from_logits)
-            decoded, lengths, ties = decoded.cpu(), lengths.cpu(), ties.cpu()
+            decoded, lengths, ties = (t.cpu() for t in self.decode_device(logits, logits_lengths_, from_logits))
         else:
-            if not (logits.is_contiguous() or logits.permute(1, 0, 2).is_contiguous()):
-                logits = logits.contiguous()
-            lengths_in = None
-            if logits_lengths_ is not None:
-                lengths_in = _as_index(logits_lengths_, torch.device("cpu"), "logits_lengths").contiguous()
-            d = self._beam_desc(logits, lengths_in, from_logits)
-            B, T = logits.size(0), logits.size(1)
-            decoded = torch.empty(B, T, dtype=torch.int64, pin_memory=True)
-            lengths = torch.empty(B, dtype=torch.int64, pin_memory=True)
-            ties = torch.empty(B, dtype=torch.int64, pin_memory=True)
-            dev = torch.cuda.current_device()
-            h = self._host.get(dev)
-            if h is None:
-                h = self._host[dev] = _HostEngine(dev)
-            _lib.check(self._L.e2e_ctc_engine_beam_host(h.handle, ctypes.byref(d), self.beam_width, self.space_idx,
-                                                        self.wip, _ptr(logits), _ptr(lengths_in), _ptr(decoded),
-                                                        _ptr(lengths), _ptr(ties)))
+            logits = _host_layout(logits)
+            lengths_in, d, (decoded, lengths, ties) = self._beam_args(logits, logits_lengths_, from_logits, pin_memory=True)
+            _lib.check(self._L.e2e_ctc_engine_beam_host(_host_engine(self._host).handle, ctypes.byref(d), self.beam_width,
+                                                        self.space_idx, self.wip, _ptr(logits), _ptr(lengths_in),
+                                                        _ptr(decoded), _ptr(lengths), _ptr(ties)))
         self.last_ties = ties
         # ctc_decoder.cpp:186-196: the result matrix is as wide as the longest decoded sequence
         width = int(lengths.max()) if lengths.numel() else 0
@@ -671,6 +658,18 @@ class CTCBeamEngine(CTCGreedyEngine):
         if not 1 <= n_best <= self.beam_width:
             raise ValueError("n_best %d outside [1, beam_width = %d]" % (n_best, self.beam_width))
         return n_best
+
+    def _nbest_args(self, logits, logits_lengths, n_best, from_logits, **where):
+        """``_greedy_args`` of both N-best variants: the outputs are ``decoded [B, N, T]``, ``lengths [B, N]`` (int64),
+        ``scores [B, N]``, ``log_probs [B, N]`` (float64) and ``ties [B]`` (int64)."""
+        if logits_lengths is not None:
+            logits_lengths = _as_index(logits_lengths, logits.device, "logits_lengths").contiguous()
+        d = self._beam_desc(logits, logits_lengths, from_logits)
+        B, T = d.batch, d.max_frames
+        out = tuple(torch.empty(*shape, dtype=dt, **where) for shape, dt in (
+            ((B, n_best, T), torch.int64), ((B, n_best), torch.int64), ((B, n_best), torch.float64),
+            ((B, n_best), torch.float64), ((B,), torch.int64)))
+        return logits_lengths, d, out
 
     def decode_nbest_device(self, logits, logits_lengths=None, n_best=None, from_logits=False):
         """The ``n_best`` best prefixes of the same search (default: the whole final beam), device tensors in, device
@@ -684,25 +683,14 @@ class CTCBeamEngine(CTCGreedyEngine):
         dev = logits.device
         if not _dense3(logits):
             logits = logits.contiguous()
-        if logits_lengths is not None:
-            logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
-        d = self._beam_desc(logits, logits_lengths, from_logits)
-        B, T = logits.size(0), logits.size(1)
+        logits_lengths, d, out = self._nbest_args(logits, logits_lengths, n_best, from_logits, device=dev)
         with _on_device(dev):
-            need = self._L.e2e_ctc_beam_nbest_workspace_bytes(ctypes.byref(d), self.beam_width, n_best)
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
-            decoded = torch.empty(B, n_best, T, dtype=torch.int64, device=dev)
-            lengths = torch.empty(B, n_best, dtype=torch.int64, device=dev)
-            scores = torch.empty(B, n_best, dtype=torch.float64, device=dev)
-            log_probs = torch.empty(B, n_best, dtype=torch.float64, device=dev)
-            ties = torch.empty(B, dtype=torch.int64, device=dev)
-            ws = torch.empty(need, dtype=torch.uint8, device=dev)
+            ws = torch.empty(_need(self._L.e2e_ctc_beam_nbest_workspace_bytes(ctypes.byref(d), self.beam_width, n_best)),
+                             dtype=torch.uint8, device=dev)
             _lib.check(self._L.e2e_ctc_beam_nbest_device(
                 ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip, _ptr(logits), _ptr(logits_lengths),
-                _ptr(decoded), _ptr(lengths), _ptr(scores), _ptr(log_probs), _ptr(ties), _ptr(ws), ws.numel(),
-                _stream(dev)))
-        return decoded, lengths, scores, log_probs, ties
+                *map(_ptr, out), _ptr(ws), ws.numel(), _stream(dev)))
+        return out
 
     def decode_nbest(self, logits_, logits_lengths_=None, n_best=None, from_logits=False):
         """``decode_nbest_device`` for CPU or CUDA input, CPU results (CPU input goes through the host engine, as in
@@ -715,45 +703,25 @@ class CTCBeamEngine(CTCGreedyEngine):
             out = self.decode_nbest_device(logits, logits_lengths_, n_best, from_logits)
             decoded, lengths, scores, log_probs, ties = (t.cpu() for t in out)
         else:
-            if not (logits.is_contiguous() or logits.permute(1, 0, 2).is_contiguous()):
-                logits = logits.contiguous()
-            lengths_in = None
-            if logits_lengths_ is not None:
-                lengths_in = _as_index(logits_lengths_, torch.device("cpu"), "logits_lengths").contiguous()
-            d = self._beam_desc(logits, lengths_in, from_logits)
-            B, T = logits.size(0), logits.size(1)
-            decoded = torch.empty(B, n_best, T, dtype=torch.int64, pin_memory=True)
-            lengths = torch.empty(B, n_best, dtype=torch.int64, pin_memory=True)
-            scores = torch.empty(B, n_best, dtype=torch.float64, pin_memory=True)
-            log_probs = torch.empty(B, n_best, dtype=torch.float64, pin_memory=True)
-            ties = torch.empty(B, dtype=torch.int64, pin_memory=True)
-            dev = torch.cuda.current_device()
-            h = self._host.get(dev)
-            if h is None:
-                h = self._host[dev] = _HostEngine(dev)
+            logits = _host_layout(logits)
+            lengths_in, d, out = self._nbest_args(logits, logits_lengths_, n_best, from_logits, pin_memory=True)
             _lib.check(self._L.e2e_ctc_engine_beam_nbest_host(
-                h.handle, ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip, _ptr(logits),
-                _ptr(lengths_in), _ptr(decoded), _ptr(lengths), _ptr(scores), _ptr(log_probs), _ptr(ties)))
+                _host_engine(self._host).handle, ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip,
+                _ptr(logits), _ptr(lengths_in), *map(_ptr, out)))
+            decoded, lengths, scores, log_probs, ties = out
         self.last_ties = ties
         width = int(lengths.max()) if lengths.numel() else 0
         return decoded[:, :, :width].contiguous(), lengths, scores, log_probs
 
-    def _score_args(self, logits, hyps, hyp_lengths, logits_lengths, from_logits):
-        """The checks and the C descriptor shared by ``score_device`` and ``score_backward_device``: returns ``(logits,
-        hyps [B*N, Lmax], hyp_lengths [B*N], logits_lengths, desc, device, N)`` with every tensor on the device.  It
-        enters ``_on_device(device)`` itself for the copies and returns outside it: callers enter it again for their
-        allocations and the launch.  Host-resident lengths / labels are checked here, device-resident ones on the device
-        (the loss's rule, ``_Problem``)."""
+    def _score_args(self, logits, hyps, hyp_lengths, logits_lengths, from_logits, max_targets=None, noun="scorer"):
+        """The checks and the C descriptor shared by the scorer's entry points and ``align_device`` (whose kernel takes
+        hypotheses of up to ``max_targets`` labels instead of the build's limit, and which the error messages call the
+        ``noun``): returns ``(logits, hyps [B*N, Lmax], hyp_lengths [B*N], logits_lengths, desc, device, N)`` with every
+        tensor on the device.  It enters ``_on_device(device)`` itself for the copies and returns outside it: callers
+        enter it again for their allocations and the launch.  Host-resident lengths / labels are checked here,
+        device-resident ones on the device (the loss's rule, ``_Problem``)."""
         logits = logits.detach()
-        if logits.dim() != 3:
-            raise ValueError("logits must be [batch, frames, alphabet], got %s" % (tuple(logits.shape),))
-        if logits.dtype not in _DTYPES:
-            raise TypeError("unsupported logits dtype %s" % logits.dtype)
-        B, T, V = logits.shape
-        if B < 1 or T < 1 or V < 1:
-            raise ValueError("empty logits %s" % (tuple(logits.shape),))
-        if not 0 <= self.blank_idx < V:
-            raise ValueError("blank_idx %d outside the alphabet [0,%d)" % (self.blank_idx, V))
+        B, T, V = _check_logits(logits, self.blank_idx, "logits")
         if hyps.dim() != 3 or hyps.size(0) != B:
             raise ValueError("hyps must be [batch, n_hyp, max_length], got %s" % (tuple(hyps.shape),))
         N, Lmax = hyps.size(1), hyps.size(2)
@@ -764,22 +732,14 @@ class CTCBeamEngine(CTCGreedyEngine):
         if logits_lengths is not None and (logits_lengths.dim() != 1 or logits_lengths.numel() != B):
             raise ValueError("logits_lengths must have shape [batch]")
         lim = _limits()
-        if Lmax > lim.max_targets or V > lim.max_alphabet:
-            raise NotImplementedError("the scorer supports hypothesis length <= %d and alphabet <= %d"
-                                      % (lim.max_targets, lim.max_alphabet))
-        if logits_lengths is not None and not logits_lengths.is_cuda:
-            ll = logits_lengths.to(torch.int64)
-            if bool((ll < 1).any()) or bool((ll > T).any()):
-                raise ValueError("logits_lengths must be in [1, %d]" % T)
-        if not hyp_lengths.is_cuda:
-            hl = hyp_lengths.to(torch.int64)
-            if bool((hl < 0).any()) or bool((hl > Lmax).any()):
-                raise ValueError("hyp_lengths must be in [0, %d]" % Lmax)
-            if not hyps.is_cuda and Lmax > 0:
-                valid = torch.arange(Lmax) < hl.unsqueeze(-1)
-                hg = hyps.to(torch.int64)
-                if bool(((hg < 0) | (hg >= V))[valid].any()):
-                    raise ValueError("hypothesis labels must be in [0, %d)" % V)
+        max_targets = lim.max_targets if max_targets is None else max_targets
+        if Lmax > max_targets or V > lim.max_alphabet:
+            raise NotImplementedError("the %s supports hypothesis length <= %d and alphabet <= %d"
+                                      % (noun, max_targets, lim.max_alphabet))
+        if logits_lengths is not None:
+            _check_host_range(logits_lengths, 1, T, "logits_lengths")
+        _check_host_range(hyp_lengths, 0, Lmax, "hyp_lengths")
+        _check_host_labels(hyps, hyp_lengths, V, "hypothesis labels")
         dev = logits.device if logits.is_cuda else torch.device("cuda", torch.cuda.current_device())
         with _on_device(dev):
             if not logits.is_cuda:
@@ -794,14 +754,7 @@ class CTCBeamEngine(CTCGreedyEngine):
                 logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
                 if logits_lengths.dtype != hyp_lengths.dtype:
                     logits_lengths, hyp_lengths = logits_lengths.to(torch.int64), hyp_lengths.to(torch.int64)
-        d = _lib.Desc()
-        d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, Lmax
-        d.blank_idx, d.dtype = self.blank_idx, _DTYPES[logits.dtype]
-        d.targets_itype, d.lengths_itype = _ITYPES[hyps.dtype], _ITYPES[hyp_lengths.dtype]
-        d.from_logits = 1 if from_logits else 0
-        d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
-        d.targets_stride_b = hyps.stride(0) if Lmax > 0 else 0
-        return logits, hyps, hyp_lengths, logits_lengths, d, dev, N
+        return logits, hyps, hyp_lengths, logits_lengths, _desc(logits, self.blank_idx, hyps, hyp_lengths, from_logits), dev, N
 
     def score_device(self, logits, hyps, hyp_lengths, logits_lengths=None, from_logits=False):
         """CTC log-likelihood log p(hypothesis | x) of N hypotheses per utterance: ``[B, N]`` float64 on the logits' device,
@@ -814,9 +767,7 @@ class CTCBeamEngine(CTCGreedyEngine):
         logits, hyps, hyp_lengths, logits_lengths, d, dev, N = self._score_args(logits, hyps, hyp_lengths, logits_lengths,
                                                                                from_logits)
         with _on_device(dev):
-            need = self._L.e2e_ctc_score_workspace_bytes(ctypes.byref(d), N)
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            need = _need(self._L.e2e_ctc_score_workspace_bytes(ctypes.byref(d), N))
             scores = torch.empty(d.batch, N, dtype=torch.float64, device=dev)
             ws = torch.empty(need, dtype=torch.uint8, device=dev)
             _lib.check(self._L.e2e_ctc_score_device(
@@ -847,9 +798,7 @@ class CTCBeamEngine(CTCGreedyEngine):
         if tuple(grad_scores.shape) != (B, N):
             raise ValueError("grad_scores must have shape [batch, n_hyp] = %s, got %s" % ((B, N), tuple(grad_scores.shape)))
         with _on_device(dev):
-            need = self._L.e2e_ctc_score_backward_workspace_bytes(ctypes.byref(d), N)
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            need = _need(self._L.e2e_ctc_score_backward_workspace_bytes(ctypes.byref(d), N))
             g = grad_scores.detach().to(dev, torch.float64).contiguous()
             grads = torch.empty_like(logits)
             d.grads_stride_b, d.grads_stride_t = grads.stride(0), grads.stride(1)
@@ -890,9 +839,7 @@ class CTCBeamEngine(CTCGreedyEngine):
         if mask is not None and tuple(mask.shape) != (B, N):
             raise ValueError("mask must have shape [batch, n_hyp] = %s, got %s" % ((B, N), tuple(mask.shape)))
         with _on_device(dev):
-            need = self._L.e2e_ctc_mwer_state_bytes(ctypes.byref(d), N)
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            need = _need(self._L.e2e_ctc_mwer_state_bytes(ctypes.byref(d), N))
             r = risk.detach().to(dev, torch.float64).contiguous()
             m = None if mask is None else mask.detach().to(dev).ne(0).to(torch.uint8).contiguous()
             if state is None:
@@ -915,9 +862,7 @@ class CTCBeamEngine(CTCGreedyEngine):
         if tuple(utt_scale.shape) != (B,):
             raise ValueError("utt_scale must have shape [batch] = (%d,), got %s" % (B, tuple(utt_scale.shape)))
         with _on_device(dev):
-            need = self._L.e2e_ctc_mwer_backward_workspace_bytes(ctypes.byref(d), N)
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            need = _need(self._L.e2e_ctc_mwer_backward_workspace_bytes(ctypes.byref(d), N))
             w = utt_scale.detach().to(dev, torch.float64).contiguous()
             grads = torch.empty_like(logits)
             d.grads_stride_b, d.grads_stride_t = grads.stride(0), grads.stride(1)
@@ -938,67 +883,11 @@ class CTCBeamEngine(CTCGreedyEngine):
         they live on the host and give NaN scores and ``-1`` spans when they live on the device.  Input on the CPU is
         copied to the current CUDA device."""
         _require_cuda()
-        logits = logits.detach()
-        if logits.dim() != 3:
-            raise ValueError("logits must be [batch, frames, alphabet], got %s" % (tuple(logits.shape),))
-        if logits.dtype not in _DTYPES:
-            raise TypeError("unsupported logits dtype %s" % logits.dtype)
-        B, T, V = logits.shape
-        if B < 1 or T < 1 or V < 1:
-            raise ValueError("empty logits %s" % (tuple(logits.shape),))
-        if not 0 <= self.blank_idx < V:
-            raise ValueError("blank_idx %d outside the alphabet [0,%d)" % (self.blank_idx, V))
-        if hyps.dim() != 3 or hyps.size(0) != B:
-            raise ValueError("hyps must be [batch, n_hyp, max_length], got %s" % (tuple(hyps.shape),))
-        N, Lmax = hyps.size(1), hyps.size(2)
-        if N < 1:
-            raise ValueError("hyps holds no hypothesis")
-        if tuple(hyp_lengths.shape) != (B, N):
-            raise ValueError("hyp_lengths must have shape [batch, n_hyp] = %s, got %s" % ((B, N), tuple(hyp_lengths.shape)))
-        if logits_lengths is not None and (logits_lengths.dim() != 1 or logits_lengths.numel() != B):
-            raise ValueError("logits_lengths must have shape [batch]")
-        lim = _limits()
-        if Lmax > ALIGN_MAX_TARGETS or V > lim.max_alphabet:
-            raise NotImplementedError("the aligner supports hypothesis length <= %d and alphabet <= %d"
-                                      % (ALIGN_MAX_TARGETS, lim.max_alphabet))
-        # the loss's rule (_Problem): host-resident lengths / labels are checked here, device-resident ones on the device
-        if logits_lengths is not None and not logits_lengths.is_cuda:
-            ll = logits_lengths.to(torch.int64)
-            if bool((ll < 1).any()) or bool((ll > T).any()):
-                raise ValueError("logits_lengths must be in [1, %d]" % T)
-        if not hyp_lengths.is_cuda:
-            hl = hyp_lengths.to(torch.int64)
-            if bool((hl < 0).any()) or bool((hl > Lmax).any()):
-                raise ValueError("hyp_lengths must be in [0, %d]" % Lmax)
-            if not hyps.is_cuda and Lmax > 0:
-                valid = torch.arange(Lmax) < hl.unsqueeze(-1)
-                hg = hyps.to(torch.int64)
-                if bool(((hg < 0) | (hg >= V))[valid].any()):
-                    raise ValueError("hypothesis labels must be in [0, %d)" % V)
-        dev = logits.device if logits.is_cuda else torch.device("cuda", torch.cuda.current_device())
+        logits, hyps, hyp_lengths, logits_lengths, d, dev, N = self._score_args(
+            logits, hyps, hyp_lengths, logits_lengths, from_logits, ALIGN_MAX_TARGETS, "aligner")
+        B, T, Lmax = d.batch, d.max_frames, d.max_targets
         with _on_device(dev):
-            if not logits.is_cuda:
-                logits = logits.to(dev)
-            if not _dense3(logits):
-                logits = logits.contiguous()
-            hyps = _as_index(hyps, dev, "hyps").reshape(B * N, Lmax)
-            if Lmax > 0 and hyps.stride(1) != 1:
-                hyps = hyps.contiguous()
-            hyp_lengths = _as_index(hyp_lengths, dev, "hyp_lengths").reshape(B * N).contiguous()
-            if logits_lengths is not None:
-                logits_lengths = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
-                if logits_lengths.dtype != hyp_lengths.dtype:
-                    logits_lengths, hyp_lengths = logits_lengths.to(torch.int64), hyp_lengths.to(torch.int64)
-            d = _lib.Desc()
-            d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, Lmax
-            d.blank_idx, d.dtype = self.blank_idx, _DTYPES[logits.dtype]
-            d.targets_itype, d.lengths_itype = _ITYPES[hyps.dtype], _ITYPES[hyp_lengths.dtype]
-            d.from_logits = 1 if from_logits else 0
-            d.logits_stride_b, d.logits_stride_t = logits.stride(0), logits.stride(1)
-            d.targets_stride_b = hyps.stride(0) if Lmax > 0 else 0
-            need = self._L.e2e_ctc_align_nbest_workspace_bytes(ctypes.byref(d), N)
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            need = _need(self._L.e2e_ctc_align_nbest_workspace_bytes(ctypes.byref(d), N))
             aligned = torch.empty(B, N, T, dtype=torch.int64, device=dev)
             starts = torch.empty(B, N, Lmax, dtype=torch.int64, device=dev)
             ends = torch.empty(B, N, Lmax, dtype=torch.int64, device=dev)
@@ -1046,11 +935,8 @@ class CTCBeamEngine(CTCGreedyEngine):
             sep = self.space_idx
         hyp_lengths = empty_marker_as_empty(hyps, hyp_lengths)
         # the loss's rule (_Problem): host-resident lengths are checked here, device-resident ones on the device
-        for name, lens, width in (("hyp_lengths", hyp_lengths, W), ("ref_lengths", ref_lengths, Wr)):
-            if not lens.is_cuda:
-                ll = lens.to(torch.int64)
-                if bool((ll < 0).any()) or bool((ll > width).any()):
-                    raise ValueError("%s must be in [0, %d]" % (name, width))
+        _check_host_range(hyp_lengths, 0, W, "hyp_lengths")
+        _check_host_range(ref_lengths, 0, Wr, "ref_lengths")
         for name, t in (("hyps", hyps), ("refs", refs)):
             if t.is_floating_point() or t.dtype == torch.bool:
                 raise TypeError("%s must be an integer tensor, got %s" % (name, t.dtype))
@@ -1075,9 +961,7 @@ class CTCBeamEngine(CTCGreedyEngine):
             d.separator = sep
             d.hyp_stride_b = hyps.stride(0) if W > 0 else 0
             d.ref_stride_b = refs.stride(0) if Wr > 0 else 0
-            need = self._L.e2e_ctc_edit_distance_workspace_bytes(ctypes.byref(d))
-            if need == 0:
-                raise _lib.E2EError(_lib.E2E_ERR_UNSUPPORTED, self._L.e2e_last_error_string().decode("utf-8", "replace"))
+            need = _need(self._L.e2e_ctc_edit_distance_workspace_bytes(ctypes.byref(d)))
             counts = torch.empty(4, B, N, dtype=torch.int64, device=dev)
             ref_units = torch.empty(B, dtype=torch.int64, device=dev)
             ws = torch.empty(need, dtype=torch.uint8, device=dev)

@@ -11,7 +11,7 @@ import torch
 from torch.autograd import Function
 
 from .. import _lib
-from ..engine import _DTYPES, _ITYPES, _as_index, _dense3, _on_device, _ptr, _require_cuda, _stream
+from ..engine import _check_logits, _dense3, _desc, _index_args, _on_device, _ptr, _require_cuda, _stream
 
 
 def ctc_without_blank_3d_loss(log_probs, targets, logits_lengths, targets_lengths, space_idx=-1):
@@ -20,35 +20,18 @@ def ctc_without_blank_3d_loss(log_probs, targets, logits_lengths, targets_length
     _require_cuda()
     L = _lib.load()
     lp = log_probs.detach()
-    if lp.dim() != 3:
-        raise ValueError("logits must be [batch, frames, alphabet]")
-    if lp.dtype not in _DTYPES:
-        raise TypeError("unsupported dtype %s" % lp.dtype)
+    B, T, V = _check_logits(lp, None, "log_probs")
+    if targets.dim() != 2 or targets.size(0) != B:
+        raise ValueError("targets must be [batch, max_target_length]")
+    if not -1 <= space_idx < V:
+        raise ValueError("space_idx %d outside [-1,%d)" % (space_idx, V))
     if not lp.is_cuda:
         lp = lp.cuda()
     dev = lp.device
     if not _dense3(lp):
         lp = lp.contiguous()
-    B, T, V = lp.shape
-    if B < 1 or T < 1 or V < 1:
-        raise ValueError("empty logits %s" % (tuple(lp.shape),))
-    if targets.dim() != 2 or targets.size(0) != B:
-        raise ValueError("targets must be [batch, max_target_length]")
-    if not -1 <= space_idx < V:
-        raise ValueError("space_idx %d outside [-1,%d)" % (space_idx, V))
-    targets = _as_index(targets, dev, "targets")
-    if targets.size(1) > 0 and targets.stride(1) != 1:
-        targets = targets.contiguous()
-    ll = _as_index(logits_lengths, dev, "logits_lengths").contiguous()
-    tl = _as_index(targets_lengths, dev, "targets_lengths").contiguous()
-    if ll.dtype != tl.dtype:
-        ll, tl = ll.to(torch.int64), tl.to(torch.int64)
-    d = _lib.Desc()
-    d.batch, d.max_frames, d.alphabet, d.max_targets = B, T, V, targets.size(1)
-    d.blank_idx, d.dtype = 0, _DTYPES[lp.dtype]
-    d.targets_itype, d.lengths_itype = _ITYPES[targets.dtype], _ITYPES[ll.dtype]
-    d.logits_stride_b, d.logits_stride_t = lp.stride(0), lp.stride(1)
-    d.targets_stride_b = targets.stride(0) if targets.size(1) > 0 else 0
+    targets, ll, tl = _index_args(targets, logits_lengths, targets_lengths, dev)
+    d = _desc(lp, 0, targets, ll, False)
     with _on_device(dev):
         n = L.e2e_ctc_noblank_workspace_bytes(ctypes.byref(d))
         if n == 0:   # the shape is valid (checked above): the lattice or the alphabet is beyond the build's limits

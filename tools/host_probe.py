@@ -65,7 +65,7 @@ print("device step (graph replay): %.1f us" % timeit(lambda: g.launch(), n=200))
 # 5. where the Python wrapper's time goes (the pieces of CTCLossEngine._compute_host, timed separately)
 import ctypes
 from end2end_b200 import _lib
-from end2end_b200.engine import _Problem, _ptr
+from end2end_b200.engine import _Problem, _host_engine, _ptr
 cpu = torch.device("cpu")
 
 
@@ -85,7 +85,7 @@ print("  ... while the previous one is still alive: %.1f us" % t_us(lambda: (kee
 pb = _Problem(0, xp, tg, ll, tl, True, cpu, validate=False)
 losses = torch.empty(B, dtype=xp.dtype, pin_memory=True)
 grads = torch.empty_strided(xp.size(), xp.stride(), dtype=xp.dtype, pin_memory=True)
-h = eng._host_engine(torch.cuda.current_device())
+h = _host_engine(eng._host)
 L = _lib.load()
 for chunks in ("1", "2", "3", "4", "6", "8"):
     os.environ["E2E_CTC_HOST_CHUNKS"] = chunks
