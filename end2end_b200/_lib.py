@@ -38,9 +38,12 @@ EXPORTS = (
     "e2e_ctc_edit_distance_workspace_bytes", "e2e_ctc_edit_distance_device",
     "e2e_ctc_mwer_state_bytes", "e2e_ctc_mwer_backward_workspace_bytes", "e2e_ctc_mwer_forward_device",
     "e2e_ctc_mwer_backward_device",
+    "e2e_ctc_ngram_table_bytes", "e2e_ctc_ngram_build_device", "e2e_ctc_beam_lm_workspace_bytes",
+    "e2e_ctc_beam_lm_nbest_device",
 )
 KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score",
-                "score_backward", "score_backward_rows", "edit_distance", "mwer_forward", "mwer_weights", "mwer_backward")
+                "score_backward", "score_backward_rows", "edit_distance", "mwer_forward", "mwer_weights", "mwer_backward",
+                "beam_search_lm", "ngram_build")
 
 
 class Desc(ctypes.Structure):
@@ -63,6 +66,16 @@ class EditDesc(ctypes.Structure):
         ("ref_width", ctypes.c_int32), ("tokens_itype", ctypes.c_int32), ("lengths_itype", ctypes.c_int32),
         ("separator", ctypes.c_int32), ("reserved0", ctypes.c_int32),
         ("hyp_stride_b", ctypes.c_int64), ("ref_stride_b", ctypes.c_int64),
+    ]
+
+
+class NGramDesc(ctypes.Structure):
+    """struct e2e_ctc_ngram"""
+    _fields_ = [
+        ("table", ctypes.c_void_p), ("table_slots", ctypes.c_int64),
+        ("lex_child", ctypes.c_void_p), ("lex_word", ctypes.c_void_p), ("label_char", ctypes.c_void_p),
+        ("lex_nodes", ctypes.c_int32), ("n_chars", ctypes.c_int32), ("order", ctypes.c_int32),
+        ("bos_id", ctypes.c_int32), ("eos_id", ctypes.c_int32), ("unk_id", ctypes.c_int32),
     ]
 
 
@@ -143,6 +156,16 @@ def load():
     L.e2e_ctc_beam_nbest_device.restype = ctypes.c_int
     L.e2e_ctc_engine_beam_nbest_host.argtypes = [vp, dp, i32, i32, i32, dbl, vp, vp, vp, vp, vp, vp, vp]
     L.e2e_ctc_engine_beam_nbest_host.restype = ctypes.c_int
+    np_ = ctypes.POINTER(NGramDesc)
+    L.e2e_ctc_ngram_table_bytes.argtypes = [i64]
+    L.e2e_ctc_ngram_table_bytes.restype = sz
+    L.e2e_ctc_ngram_build_device.argtypes = [vp, i64, i64, vp, vp, vp, vp, vp]
+    L.e2e_ctc_ngram_build_device.restype = ctypes.c_int
+    L.e2e_ctc_beam_lm_workspace_bytes.argtypes = [dp, np_, i32, i32]
+    L.e2e_ctc_beam_lm_workspace_bytes.restype = sz
+    L.e2e_ctc_beam_lm_nbest_device.argtypes = [dp, i32, i32, i32, dbl, np_, dbl, dbl, vp, vp, vp, vp, vp, vp, vp, vp, vp,
+                                               vp, sz, vp]
+    L.e2e_ctc_beam_lm_nbest_device.restype = ctypes.c_int
     L.e2e_ctc_score_workspace_bytes.argtypes = [dp, i32]
     L.e2e_ctc_score_workspace_bytes.restype = sz
     L.e2e_ctc_score_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, sz, vp]

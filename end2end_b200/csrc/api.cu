@@ -679,6 +679,67 @@ int e2e_ctc_beam_decode_device(const e2e_ctc_desc* desc, int32_t beam_width, int
                      ties, reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
+// ---- the same search with a word n-gram LM fused in ---------------------------------------------------
+size_t e2e_ctc_ngram_table_bytes(int64_t slots) {
+  if (slots < 1 || (slots & (slots - 1))) { set_error("n-gram table slots %lld is no power of two", (long long)slots); return 0; }
+  return ngram_table_bytes(slots);
+}
+
+int e2e_ctc_ngram_build_device(void* table, int64_t slots, int64_t count, const int32_t* ids, const int32_t* orders,
+                               const double* probs, const double* bows, void* cuda_stream) {
+  if (!table || (count > 0 && (!ids || !orders || !probs || !bows))) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  if (slots < 1 || (slots & (slots - 1)) || count < 0 || count >= slots) {
+    set_error("n-gram table: %lld n-grams need a power-of-two number of slots above that, got %lld", (long long)count, (long long)slots);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  return launch_ngram_build(table, slots, count, ids, orders, probs, bows, reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+static int check_beam_lm(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, int32_t beam_width, int32_t n_best,
+                         int32_t space_idx, double wip, double lmwt, double oov_penalty, bool need_space) {
+  int rc = check_desc(desc, false);
+  if (rc != E2E_OK) return rc;
+  if (!lm || !lm->table || !lm->lex_child || !lm->lex_word || !lm->label_char) { set_error("null language model argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  if (lm->order < 1 || lm->order > 6) { set_error("language model order %d outside [1, 6]", lm->order); return E2E_ERR_INVALID_ARGUMENT; }
+  if (lm->table_slots < 1 || (lm->table_slots & (lm->table_slots - 1)) || lm->lex_nodes < 1 || lm->n_chars < 0) {
+    set_error("malformed language model descriptor"); return E2E_ERR_INVALID_ARGUMENT;
+  }
+  if (need_space && (space_idx < 0 || space_idx >= desc->alphabet)) {
+    set_error("a language model needs the space label: space_idx %d outside [0,%d)", space_idx, desc->alphabet);
+    return E2E_ERR_INVALID_ARGUMENT;
+  }
+  auto finite = [](double x) { return x == x && x != INFINITY && x != -INFINITY; };
+  if (!finite(lmwt) || !finite(oov_penalty)) { set_error("lmwt and oov_penalty must be finite"); return E2E_ERR_INVALID_ARGUMENT; }
+  rc = check_beam(desc, beam_width, n_best, need_space ? space_idx : -1, wip);
+  if (rc != E2E_OK) return rc;
+  if (!beam_supported(*desc, beam_width, true)) {
+    set_error("beam search with a language model: beam_width %d with alphabet %d exceeds this build's limits (beam, bitmap and LM state <= 200 KB of shared memory)",
+              beam_width, desc->alphabet);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  return E2E_OK;
+}
+
+size_t e2e_ctc_beam_lm_workspace_bytes(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, int32_t beam_width, int32_t n_best) {
+  if (check_beam_lm(desc, lm, beam_width, n_best, -1, 0.0, 0.0, 0.0, false) != E2E_OK) return 0;
+  return align256(beam_workspace_bytes(*desc, beam_width));
+}
+
+int e2e_ctc_beam_lm_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx,
+                                 double wip, const e2e_ctc_ngram* lm, double lmwt, double oov_penalty, const void* logits,
+                                 const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths, double* scores,
+                                 double* log_probs, double* lm_scores, int64_t* oov_words, int64_t* ties, void* workspace,
+                                 size_t workspace_bytes, void* cuda_stream) {
+  int rc = check_beam_lm(desc, lm, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, true);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !decoded || !decoded_lengths || !scores || !lm_scores || !oov_words) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  rc = check_ws(workspace, workspace_bytes, e2e_ctc_beam_lm_workspace_bytes(desc, lm, beam_width, n_best));
+  if (rc != E2E_OK) return rc;
+  return launch_beam_lm(*desc, *lm, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, logits, logits_lengths, decoded,
+                        decoded_lengths, scores, log_probs, lm_scores, oov_words, ties, reinterpret_cast<char*>(workspace),
+                        reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
 // ---- CTC log-likelihood of N hypotheses per utterance (K9) -------------------------------------------
 static int check_score(const e2e_ctc_desc* desc, int32_t n_hyp) {
   int rc = check_desc(desc, true);

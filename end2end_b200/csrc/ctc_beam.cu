@@ -39,6 +39,11 @@
 //
 // Arithmetic: fp64 log-space with the reference's two-argument log_sum_exp (src/utils/math_utils.h:8-16) and the score
 // expression of :311-315 evaluated in its order without fused multiply-adds.
+//
+// The LM template parameter fuses a word n-gram language model into the same search (include/e2e_ctc.h, e2e_ctc_ngram).
+// Only a member's space extension completes a word, so only that extension's score changes (BeamExt): the symbol filter,
+// the select and the trie are as above.  Each new member looks up what completing its current word would add once,
+// right after the write phase; LM = false compiles to the LM-free kernel unchanged.
 #include <cstdio>
 #include <cstdlib>
 
@@ -66,6 +71,89 @@ struct BeamParams {
   int kc_cap;                // keys the shared-memory cache holds (0: none)
   double wip;
 };
+
+// ---- word n-gram language model (the LM variant, e2e_ctc_beam_lm_nbest_device) ----------------------------------------
+struct __align__(16) NGramEntry {   // 48 bytes: one n-gram of the open-addressing table (n == 0: empty slot)
+  int n, w[6], pad;
+  double prob, bow;                 // log10 probability and backoff weight, as the ARPA file gives them
+};
+struct BeamLMParams {
+  const NGramEntry* table; unsigned long long mask;   // slots - 1 (a power of two)
+  const int* lex_child;      // [lex_nodes][n_chars]: child of a lexicon node for a character, -1: no word spelled so
+  const int* lex_word;       // [lex_nodes]: the word a node spells, -1: none
+  const int* label_char;     // [V]: character id of a label, -1 for the blank and the space
+  int n_chars, order, bos, eos, unk;
+  double lmwt, oov_penalty;
+  double* lm_scores;         // [B, n_best]: lm of the returned prefixes, end-of-utterance terms included
+  long long* oov_words;      // [B, n_best]
+};
+constexpr int kLMMaxOrder = 6, kLMCtx = kLMMaxOrder - 1;
+
+__device__ __forceinline__ unsigned long long ngram_hash(const int* w, int n) {   // n is a compile-time constant at the call sites
+  unsigned long long h = 0x9e3779b97f4a7c15ull * (unsigned long long)(n + 1);
+#pragma unroll
+  for (int i = 0; i < kLMMaxOrder; i++) {
+    if (i < n) { h ^= (unsigned)w[i]; h *= 0xff51afd7ed558ccdull; h ^= h >> 33; }
+  }
+  return h;
+}
+
+// the table entry of the n-gram w[0..n) or null
+__device__ __forceinline__ const NGramEntry* ngram_find(const NGramEntry* table, unsigned long long mask, const int* w, int n) {
+  unsigned long long slot = ngram_hash(w, n) & mask;
+  while (true) {
+    const NGramEntry* e = table + slot;
+    const int en = __ldg(&e->n);
+    if (en == 0) return nullptr;
+    if (en == n) {
+      bool eq = true;
+#pragma unroll
+      for (int i = 0; i < kLMMaxOrder; i++) if (i < n) eq = eq && __ldg(&e->w[i]) == w[i];
+      if (eq) return e;
+    }
+    slot = (slot + 1) & mask;
+  }
+}
+
+// ln10 * log10 P(w | history) with ARPA backoff: from the longest context down, either (context, w) is an n-gram (add its
+// probability, stop) or it is not (add the context's backoff weight, 0 if it is no n-gram, and drop its oldest word).
+// h4 is the most recent word of the history, h0 the oldest; -1 marks its start.  The context is at most order - 1 words.
+// (out of line: it is called once per new member and once per final prefix, and the frame loop must fit the instruction
+// cache)
+__device__ __noinline__ double lm_term(const NGramEntry* table, unsigned long long mask, int order, int h0, int h1, int h2,
+                                       int h3, int h4, int w) {
+  const int h[kLMCtx] = {h0, h1, h2, h3, h4};
+  int nctx = 0;
+#pragma unroll
+  for (int i = kLMCtx - 1; i >= 0; i--) if (h[i] >= 0 && nctx == kLMCtx - 1 - i && nctx < order - 1) nctx++;
+  double t = 0.0;
+#pragma unroll
+  for (int j = kLMCtx; j >= 0; j--) {   // context length j
+    if (j > nctx) continue;
+    int key[kLMMaxOrder];
+#pragma unroll
+    for (int i = 0; i < kLMMaxOrder; i++) key[i] = i < j ? h[kLMCtx - j + i] : (i == j ? w : -1);
+    const NGramEntry* e = ngram_find(table, mask, key, j + 1);
+    if (e) { t = __dadd_rn(t, __ldg(&e->prob)); break; }
+    if (j > 0) { const NGramEntry* c = ngram_find(table, mask, key, j); if (c) t = __dadd_rn(t, __ldg(&c->bow)); }
+  }
+  return __dmul_rn(t, 2.302585092994045684);   // M_LN10
+}
+
+__global__ void ngram_build_kernel(NGramEntry* table, unsigned long long mask, long long count, const int* ids,
+                                   const int* orders, const double* probs, const double* bows) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  int w[kLMMaxOrder];
+#pragma unroll
+  for (int k = 0; k < kLMMaxOrder; k++) w[k] = ids[i * kLMMaxOrder + k];
+  const int n = orders[i];
+  unsigned long long slot = ngram_hash(w, n) & mask;
+  while (atomicCAS(&table[slot].n, 0, n) != 0) slot = (slot + 1) & mask;   // the n-grams are distinct: no key to compare
+#pragma unroll
+  for (int k = 0; k < kLMMaxOrder; k++) table[slot].w[k] = k < n ? w[k] : -1;
+  table[slot].prob = probs[i]; table[slot].bow = bows[i];
+}
 
 #ifndef E2E_BEAM_DIGIT
 #define E2E_BEAM_DIGIT 8
@@ -107,6 +195,11 @@ struct BeamBuf {          // one copy of the beam (+ the pruned prefixes that st
   double *pb, *pnb;
   int *node, *par, *last, *nw, *dep, *pslot;   // trie node, parent node, last symbol, words, length, parent's slot or -1
   int *zn, *zp, *zc;                           // blocked extensions: node, parent's slot, symbol
+  // LM variant: lexicon node of the current word (-1: no word is spelled so), the word its completion scores (-1: the
+  // current word is empty; the <unk> id when out of vocabulary), OOV words so far, the last words (h[kLMCtx - 1] the most
+  // recent, -1 before the start), the LM sum and what completing the current word adds to it
+  int *lex, *cw, *oov, *h[kLMCtx];
+  double *lm, *sd;
 };
 struct BeamSmem {
   double* lp;            // [Vp]
@@ -120,6 +213,26 @@ struct BeamSmem {
   unsigned long long* kc;   // [W][nR] keys of the extensions (0: none) when they fit
   int* rc;               // [nR] the symbols a member is extended with this frame, ascending (never the blank)
   unsigned* rmask;       // [VW] the same set as a bit mask
+  double *lmx, *lms, *oox, *oos;   // LM variant: lmwt * lm and oov * oov_penalty of an extension other than space / with the space
+};
+
+// get_prev_full_prob_with_lmwt (:311-315) with a language model: ((log p + lmwt * lm) - words * wip) + oov * oov_penalty
+__device__ __forceinline__ double beam_score_lm(double full, double lmw, int num_words, double wip, double oovw) {
+  return __dadd_rn(__dsub_rn(__dadd_rn(full, lmw), __dmul_rn((double)num_words, wip)), oovw);
+}
+
+// What an extension of one member adds to its value besides the frame's log-probability; one key expression for every
+// site that builds an extension key.  Only the space extension completes a word, so the LM changes only that one.
+template <bool LM>
+struct BeamExt {
+  double penx, pens, lmx, lms, oox, oos;
+  __device__ __forceinline__ BeamExt(const BeamSmem& S, int s)
+      : penx(S.penx[s]), pens(S.pens[s]), lmx(LM ? S.lmx[s] : 0.0), lms(LM ? S.lms[s] : 0.0), oox(LM ? S.oox[s] : 0.0),
+        oos(LM ? S.oos[s] : 0.0) {}
+  __device__ __forceinline__ unsigned long long key(double v, bool space) const {
+    if (!LM) return beam_key(__dsub_rn(__dadd_rn(v, 0.0), space ? pens : penx));
+    return beam_key(__dadd_rn(__dsub_rn(__dadd_rn(v, space ? lms : lmx), space ? pens : penx), space ? oos : oox));
+  }
 };
 
 // :381-390: a repeated character extends from the blank-ending mass only
@@ -133,8 +246,8 @@ __device__ long long g_beam_prof[16];
 #else
 #define BEAM_T(k) do { } while (0)
 #endif
-template <typename T, bool CACHE, int NT>
-__global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
+template <typename T, bool CACHE, int NT, bool LM>
+__global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, const BeamLMParams q) {
 #ifdef BEAM_PROF
   long long prof_t = clock64();
 #endif
@@ -173,6 +286,20 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
     S.rc = reinterpret_cast<int*>(take(4 * (size_t)V));
     S.rmask = reinterpret_cast<unsigned*>(take(4 * (size_t)VW));
     S.kc = reinterpret_cast<unsigned long long*>(take(CACHE ? (size_t)8 * p.kc_cap : 0));
+    if (LM) {
+      BeamBuf* bufs[2] = {&C, &N};
+#pragma unroll
+      for (int k = 0; k < 2; k++) {
+        BeamBuf& u = *bufs[k];
+        u.lm = reinterpret_cast<double*>(take(8 * WB)); u.sd = reinterpret_cast<double*>(take(8 * WB));
+        u.lex = reinterpret_cast<int*>(take(4 * WB)); u.cw = reinterpret_cast<int*>(take(4 * WB));
+        u.oov = reinterpret_cast<int*>(take(4 * WB));
+#pragma unroll
+        for (int i = 0; i < kLMCtx; i++) u.h[i] = reinterpret_cast<int*>(take(4 * WB));
+      }
+      S.lmx = reinterpret_cast<double*>(take(8 * WB)); S.lms = reinterpret_cast<double*>(take(8 * WB));
+      S.oox = reinterpret_cast<double*>(take(8 * WB)); S.oos = reinterpret_cast<double*>(take(8 * WB));
+    }
   }
 
   long long Ti_ll = p.in_len ? load_index(p.in_len, p.len_is64, b) : (long long)p.T;
@@ -186,6 +313,11 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
     nodes[0] = r;
     C.node[0] = 0; C.par[0] = -1; C.last[0] = -1; C.nw[0] = 0; C.dep[0] = 0; C.pslot[0] = -1; C.pb[0] = 0.0; C.pnb[0] = -INFINITY;
     s_ties = 0; s_ovf = 0; s_nz2 = 0; s_tie_now = 0;
+    if (LM) {   // the empty prefix: no word yet, the history is <s>
+      C.lex[0] = 0; C.cw[0] = -1; C.oov[0] = 0; C.lm[0] = 0.0; C.sd[0] = 0.0;
+#pragma unroll
+      for (int i = 0; i < kLMCtx; i++) C.h[i][0] = i == kLMCtx - 1 ? q.bos : -1;
+    }
   }
   // The first kFront threads (8 warps) run the head of a frame -- staging the row, the log-softmax, the members' own
   // updates -- synchronising among themselves on a named barrier.  With 512 threads the other half spends that time
@@ -339,6 +471,14 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
       const int nwx = nws + ((nws == 0 || last == p.space) ? 1 : 0); // :252-257 for a symbol other than space
       S.nwx[s] = nwx;
       S.penx[s] = __dmul_rn((double)nwx, p.wip); S.pens[s] = __dmul_rn((double)nws, p.wip);
+      if (LM) {   // a space extension completes the current word (if any): its LM term and OOV count join the score
+        const double lm = C.lm[s];
+        const int oov = C.oov[s], cw = C.cw[s];
+        const double lmx = __dmul_rn(q.lmwt, lm), oox = __dmul_rn((double)oov, q.oov_penalty);
+        S.lmx[s] = lmx; S.oox[s] = oox;
+        S.lms[s] = cw >= 0 ? __dmul_rn(q.lmwt, __dadd_rn(lm, C.sd[s])) : lmx;
+        S.oos[s] = cw >= 0 ? __dmul_rn((double)(oov + (cw == q.unk ? 1 : 0)), q.oov_penalty) : oox;
+      }
     }
     }   // front threads
     __syncthreads();   // the members' updates are done; so are last frame's releases
@@ -381,7 +521,10 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
     __syncthreads();
     BEAM_T(2);
     // ---- phase C: scores of the members and of the fresh extensions; how many prefixes are there now (:392-399) ------
-    if (tid < W) S.mkey[tid] = beam_key(beam_score(beam_lse(S.npnb[tid], S.npb[tid]), C.nw[tid], p.wip));
+    if (tid < W) {
+      if (LM) S.mkey[tid] = beam_key(beam_score_lm(beam_lse(S.npnb[tid], S.npb[tid]), S.lmx[tid], C.nw[tid], p.wip, S.oox[tid]));
+      else S.mkey[tid] = beam_key(beam_score(beam_lse(S.npnb[tid], S.npb[tid]), C.nw[tid], p.wip));
+    }
     {
       int excl = 0;
       for (int i = tid; i < W * VW; i += kBeamThreads) excl += __popc(S.bitmap[i] & S.rmask[i % VW]);
@@ -400,7 +543,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
             for (int s = warp - mw; s < W && s >= 0; s += kBeamWarps - mw) {
         const int last = C.last[s];
         const double base = S.full[s], baseb = C.pb[s];
-        const double penx = S.penx[s], pens = S.pens[s];
+        const BeamExt<LM> ex(S, s);
                       for (int j0 = 0; j0 < nR; j0 += 32) {
           const int j = j0 + lane;
           if (j < nR) {
@@ -408,7 +551,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
             unsigned long long k = 0ull;
             if (!((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
               const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-              k = beam_key(__dsub_rn(__dadd_rn(v, 0.0), c == p.space ? pens : penx));
+              k = ex.key(v, c == p.space);
               kmax = k > kmax ? k : kmax; kmin = k < kmin ? k : kmin;
             }
             S.kc[s * nR + j] = k;
@@ -551,7 +694,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
                         for (int s = warp; s < W; s += kBeamWarps) {
             const int last = C.last[s];
             const double base = S.full[s], baseb = C.pb[s];
-            const double penx = S.penx[s], pens = S.pens[s];
+            const BeamExt<LM> ex(S, s);
                           for (int j0 = 0; j0 < nR; j0 += 32) {
               const int j = j0 + lane;
               const int c = j < nR ? sym(j) : 0;
@@ -559,7 +702,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
               unsigned long long k = 0ull;
               if (valid) {
                 const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-                k = beam_key(__dsub_rn(__dadd_rn(v, 0.0), c == p.space ? pens : penx));
+                k = ex.key(v, c == p.space);
                 valid = (k & pm) == (prefix & pm);
               }
               const unsigned d = (unsigned)(k >> sh) & (kBeamBins - 1);
@@ -617,7 +760,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
         for (int s = warp; s < W; s += kBeamWarps) {
       const int last = C.last[s];
       const double base = S.full[s], baseb = C.pb[s];
-      const double penx = S.penx[s], pens = S.pens[s];
+      const BeamExt<LM> ex(S, s);
       int ngt = 0, neq = 0;
             for (int j0 = 0; j0 < nR; j0 += 32) {
         const int j = j0 + lane;
@@ -626,7 +769,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
         if (use_cache) { if (j < nR) k = S.kc[s * nR + j]; }
         else if (j < nR && !((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
           const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-          k = beam_key(__dsub_rn(__dadd_rn(v, 0.0), c == p.space ? pens : penx));
+          k = ex.key(v, c == p.space);
         }
         const unsigned long long kq = k >> sh;
         ngt += __popc(__ballot_sync(0xffffffffu, k != 0ull && kq > tcls));
@@ -669,12 +812,17 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
         N.pb[ns] = S.npb[s]; N.pnb[ns] = S.npnb[s];
         const int sp = C.pslot[s];
         N.pslot[ns] = sp >= 0 ? new_slot(sp) : -1;
+        if (LM) {
+          N.lex[ns] = C.lex[s]; N.cw[ns] = C.cw[s]; N.oov[ns] = C.oov[s]; N.lm[ns] = C.lm[s]; N.sd[ns] = C.sd[s];
+#pragma unroll
+          for (int i = 0; i < kLMCtx; i++) N.h[i][ns] = C.h[i][s];
+        }
       }
     }
         for (int s = warp; s < W; s += kBeamWarps) {
       const int last = C.last[s];
       const double base = S.full[s], baseb = C.pb[s];
-      const double penx = S.penx[s], pens = S.pens[s];
+      const BeamExt<LM> ex(S, s);
       int gb = S.cgt[W + s], eb = S.ceq[W + s];
       const int pn = C.node[s], pd = C.dep[s];
       const int psl = new_slot(s);
@@ -685,7 +833,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
         if (use_cache) { if (j < nR) k = S.kc[s * nR + j]; }
         else if (j < nR && !((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
           const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-          k = beam_key(__dsub_rn(__dadd_rn(v, 0.0), c == p.space ? pens : penx));
+          k = ex.key(v, c == p.space);
         }
         const unsigned long long kq = k >> sh;
         const bool isgt = k != 0ull && kq > tcls, iseq = k != 0ull && kq == tcls;
@@ -701,11 +849,39 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
           BeamNode r; r.parent = pn; r.chr = c; r.refs = 1; r.depth = pd + 1;
           nodes[id] = r;
           atomicAdd(&nodes[pn].refs, 1);
+          if (LM) {
+            const int cw = C.cw[s];
+            if (c == p.space) {   // completes the current word, if there is one; the next word starts at the lexicon's root
+              const bool done = cw >= 0;
+              N.lm[ns] = done ? __dadd_rn(C.lm[s], C.sd[s]) : C.lm[s];
+              N.oov[ns] = C.oov[s] + (done && cw == q.unk ? 1 : 0);
+#pragma unroll
+              for (int i = 0; i < kLMCtx; i++) N.h[i][ns] = done ? (i == kLMCtx - 1 ? cw : C.h[i + 1][s]) : C.h[i][s];
+              N.lex[ns] = 0; N.cw[ns] = -1; N.sd[ns] = 0.0;
+            } else {              // the word grows; what completing it adds is looked up below, once per new member
+              const int lx = C.lex[s];
+              N.lex[ns] = lx >= 0 ? __ldg(&q.lex_child[(long long)lx * q.n_chars + __ldg(&q.label_char[c])]) : -1;
+              N.lm[ns] = C.lm[s]; N.oov[ns] = C.oov[s];
+#pragma unroll
+              for (int i = 0; i < kLMCtx; i++) N.h[i][ns] = C.h[i][s];
+            }
+          }
         }
         gb += __popc(mg); eb += __popc(me);
       }
     }
     __syncthreads();
+    if (LM) {   // the new members whose word grew: the word a space would complete, and its LM term
+      for (int ns = keepm + tid; ns < keepall; ns += kBeamThreads) {
+        if (N.last[ns] == p.space) continue;
+        const int lx = N.lex[ns];
+        int w = lx >= 0 ? __ldg(&q.lex_word[lx]) : -1;
+        if (w < 0) w = q.unk;
+        N.cw[ns] = w;
+        N.sd[ns] = lm_term(q.table, q.mask, q.order, N.h[0][ns], N.h[1][ns], N.h[2][ns], N.h[3][ns], N.h[4][ns], w);
+      }
+      __syncthreads();
+    }
     BEAM_T(7);
     // ---- carried into the next frame: the nodes to release, this frame's cut (slot of a member after the prune) ------
     {
@@ -722,7 +898,23 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
   //      Every member ranks itself by counting over the keys: rank = keys above + equal keys at lower positions, so rank 0
   //      is the member the reference's prefixes[0] is when no two scores are equal. ----------------------------------------
   __syncthreads();   // the last frame's tail still reads the member keys
-  if (tid < W) S.mkey[tid] = beam_key(beam_score(beam_lse(C.pnb[tid], C.pb[tid]), C.nw[tid], p.wip));
+  if (tid < W) {
+    if (LM) {   // end of the utterance: a trailing word is completed, then </s> is scored
+      const int cw = C.cw[tid];
+      const bool done = cw >= 0;
+      int h[kLMCtx];
+#pragma unroll
+      for (int i = 0; i < kLMCtx; i++) h[i] = done ? (i == kLMCtx - 1 ? cw : C.h[i + 1][tid]) : C.h[i][tid];
+      double lm = done ? __dadd_rn(C.lm[tid], C.sd[tid]) : C.lm[tid];
+      const int oov = C.oov[tid] + (done && cw == q.unk ? 1 : 0);
+      lm = __dadd_rn(lm, lm_term(q.table, q.mask, q.order, h[0], h[1], h[2], h[3], h[4], q.eos));
+      S.lms[tid] = lm; S.nwx[tid] = oov;
+      S.mkey[tid] = beam_key(beam_score_lm(beam_lse(C.pnb[tid], C.pb[tid]), __dmul_rn(q.lmwt, lm), C.nw[tid], p.wip,
+                                           __dmul_rn((double)oov, q.oov_penalty)));
+    } else {
+      S.mkey[tid] = beam_key(beam_score(beam_lse(C.pnb[tid], C.pb[tid]), C.nw[tid], p.wip));
+    }
+  }
   if (tid == 0) s_tie_now = 0;
   __syncthreads();
   const int NB = p.n_best;
@@ -746,7 +938,14 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
       p.decoded_len[o] = len;
       if (p.scores) {
         const double lp = beam_lse(C.pnb[tid], C.pb[tid]);
-        p.scores[o] = beam_score(lp, C.nw[tid], p.wip);
+        if (LM) {
+          const double lm = S.lms[tid];
+          const int oov = S.nwx[tid];
+          p.scores[o] = beam_score_lm(lp, __dmul_rn(q.lmwt, lm), C.nw[tid], p.wip, __dmul_rn((double)oov, q.oov_penalty));
+          q.lm_scores[o] = lm; q.oov_words[o] = oov;
+        } else {
+          p.scores[o] = beam_score(lp, C.nw[tid], p.wip);
+        }
         if (p.log_probs) p.log_probs[o] = lp;
       }
       S.cgt[rank] = len;
@@ -755,6 +954,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
     const long long o = (long long)b * NB + tid;
     p.decoded_len[o] = 0;
     if (p.scores) { p.scores[o] = -INFINITY; if (p.log_probs) p.log_probs[o] = -INFINITY; }
+    if (LM) { q.lm_scores[o] = -INFINITY; q.oov_words[o] = 0; }
     S.cgt[tid] = 0;
   }
   __syncthreads();
@@ -765,7 +965,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p) {
   }
 }
 
-size_t beam_smem_bytes(int V, int WB, size_t kc_cap) {
+size_t beam_smem_bytes(int V, int WB, size_t kc_cap, bool lm) {
   auto a16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
   const int VW = (V + 31) >> 5, Vp = (V + 1) & ~1;
   size_t n = 2 * a16(sizeof(double) * Vp);   // lp, raw
@@ -778,6 +978,7 @@ size_t beam_smem_bytes(int V, int WB, size_t kc_cap) {
   n += a16(4 * (size_t)kBeamBins) + 2 * a16(8 * (size_t)WB);   // hist, penx, pens
   n += a16(4 * (size_t)V) + a16(4 * (size_t)VW);               // rc, rmask
   n += a16(8 * kc_cap);
+  if (lm) n += 8 * a16(8 * (size_t)WB) + (2 * (3 + kLMCtx)) * a16(4 * (size_t)WB);   // lm, sd x 2, lmx, lms, oox, oos; lex, cw, oov, h x 2
   return n;
 }
 
@@ -785,13 +986,13 @@ constexpr size_t kBeamSmemLimit = 200 * 1024;
 // How a shape runs: the symbols extended per frame (all, or the beam_width + 2 most probable + the space for large alphabets)
 // and how many extension keys are cached in shared memory (0: recomputed in every pass).
 struct BeamMode { int prefilter; int kc_cap; size_t smem; bool ok; };
-BeamMode beam_mode(int V, int WB) {
+BeamMode beam_mode(int V, int WB, bool lm) {
   BeamMode m{0, 0, 0, false};
   const long long all = (long long)V * WB;
   if (all <= kBeamKeyCache) { m.kc_cap = (int)all; }
   else if (V - 1 >= WB + 3) { m.prefilter = 1; m.kc_cap = kBeamKeyCache; }
-  m.smem = beam_smem_bytes(V, WB, (size_t)m.kc_cap);
-  if (m.smem > kBeamSmemLimit && m.kc_cap) { m.kc_cap = 0; m.smem = beam_smem_bytes(V, WB, 0); }   // no room for the cache
+  m.smem = beam_smem_bytes(V, WB, (size_t)m.kc_cap, lm);
+  if (m.smem > kBeamSmemLimit && m.kc_cap) { m.kc_cap = 0; m.smem = beam_smem_bytes(V, WB, 0, lm); }   // no room for the cache
   m.ok = m.smem <= kBeamSmemLimit;
   return m;
 }
@@ -803,13 +1004,28 @@ size_t beam_workspace_bytes(const e2e_ctc_desc& d, int beam_width) {
   return (size_t)d.batch * cap * sizeof(BeamNode);
 }
 
-bool beam_supported(const e2e_ctc_desc& d, int beam_width) {
-  return beam_width >= 1 && beam_width <= kBeamMaxWidth && beam_mode(d.alphabet, beam_width).ok;
+bool beam_supported(const e2e_ctc_desc& d, int beam_width, bool lm) {
+  return beam_width >= 1 && beam_width <= kBeamMaxWidth && beam_mode(d.alphabet, beam_width, lm).ok;
 }
 
-int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
-                const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
-                char* ws, cudaStream_t s) {
+size_t ngram_table_bytes(long long slots) { return (size_t)slots * sizeof(NGramEntry); }
+
+int launch_ngram_build(void* table, long long slots, long long count, const int* ids, const int* orders, const double* probs,
+                       const double* bows, cudaStream_t s) {
+  E2E_CUDA_TRY(cudaMemsetAsync(table, 0, ngram_table_bytes(slots), s));
+  if (count > 0) {
+    KernelTimer timer(kKernelNGramBuild, s);
+    ngram_build_kernel<<<(unsigned)((count + 255) / 256), 256, 0, s>>>(reinterpret_cast<NGramEntry*>(table),
+                                                                         (unsigned long long)slots - 1ull, count, ids, orders,
+                                                                         probs, bows);
+  }
+  E2E_CUDA_TRY(cudaGetLastError());
+  return E2E_OK;
+}
+
+static int launch_beam_impl(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
+                            const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs,
+                            int64_t* ties, char* ws, cudaStream_t s, const BeamLMParams* lmp) {
   BeamParams p;
   p.logits = logits; p.dtype = d.dtype; p.sb = d.logits_stride_b; p.st = d.logits_stride_t;
   p.in_len = in_len; p.len_is64 = d.lengths_itype == E2E_I64;
@@ -820,27 +1036,34 @@ int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx
   p.node_cap = (long long)d.max_frames * beam_width + 1;
   p.B = d.batch; p.T = d.max_frames; p.V = d.alphabet; p.blank = d.blank_idx; p.beam = beam_width; p.space = space_idx;
   p.from_logits = d.from_logits; p.wip = wip;
-  const BeamMode md = beam_mode(d.alphabet, beam_width);
+  const bool lm = lmp != nullptr;
+  BeamLMParams q{};
+  if (lm) q = *lmp;
+  const BeamMode md = beam_mode(d.alphabet, beam_width, lm);
   static const int no_pref = []() { const char* v = getenv("E2E_CTC_BEAM_NOPREFILTER"); return (v && *v) ? atoi(v) : 0; }();   // tests / experiments
   p.prefilter = no_pref ? 0 : md.prefilter;
   p.kc_cap = (no_pref && md.prefilter) ? 0 : md.kc_cap;
   const bool cache = p.kc_cap > 0;
-  const size_t smem = beam_smem_bytes(d.alphabet, beam_width, (size_t)p.kc_cap);
+  const size_t smem = beam_smem_bytes(d.alphabet, beam_width, (size_t)p.kc_cap, lm);
   int dev = 0, sms = 148;
   E2E_CUDA_TRY(cudaGetDevice(&dev));
   E2E_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   static const int force_wide = []() { const char* v = getenv("E2E_CTC_BEAM_WIDE"); return (v && *v) ? atoi(v) : -1; }();   // experiments only
   const bool wide = force_wide >= 0 ? force_wide != 0 : d.batch <= sms;
-  KernelTimer timer(kKernelBeam, s);
-#define E2E_K8_(TYPE, CACHE_, NT_)                                                                            \
+  KernelTimer timer(lm ? kKernelBeamLM : kKernelBeam, s);
+#define E2E_K8_(TYPE, CACHE_, NT_, LM_)                                                                       \
   do {                                                                                                       \
-    E2E_CUDA_TRY(cudaFuncSetAttribute(ctc_beam_kernel<TYPE, CACHE_, NT_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    ctc_beam_kernel<TYPE, CACHE_, NT_><<<(unsigned)d.batch, NT_, smem, s>>>(p);                              \
+    E2E_CUDA_TRY(cudaFuncSetAttribute(ctc_beam_kernel<TYPE, CACHE_, NT_, LM_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    ctc_beam_kernel<TYPE, CACHE_, NT_, LM_><<<(unsigned)d.batch, NT_, smem, s>>>(p, q);                      \
+  } while (0)
+#define E2E_K8L(TYPE, LM_)                                                                                   \
+  do {                                                                                                       \
+    if (cache) { if (wide) E2E_K8_(TYPE, true, 512, LM_); else E2E_K8_(TYPE, true, 256, LM_); }              \
+    else { if (wide) E2E_K8_(TYPE, false, 512, LM_); else E2E_K8_(TYPE, false, 256, LM_); }                  \
   } while (0)
 #define E2E_K8(TYPE)                                                                                         \
   do {                                                                                                       \
-    if (cache) { if (wide) E2E_K8_(TYPE, true, 512); else E2E_K8_(TYPE, true, 256); }                        \
-    else { if (wide) E2E_K8_(TYPE, false, 512); else E2E_K8_(TYPE, false, 256); }                            \
+    if (lm) E2E_K8L(TYPE, true); else E2E_K8L(TYPE, false);                                                  \
   } while (0)
   switch (d.dtype) {
     case E2E_F32: E2E_K8(float); break;
@@ -850,6 +1073,7 @@ int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx
     default: set_error("beam: unsupported dtype %d", d.dtype); return E2E_ERR_INVALID_ARGUMENT;
   }
 #undef E2E_K8
+#undef E2E_K8L
 #undef E2E_K8_
 #ifdef BEAM_PROF
   {
@@ -863,6 +1087,27 @@ int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx
 #endif
   E2E_CUDA_TRY(cudaGetLastError());
   return E2E_OK;
+}
+
+int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
+                const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
+                char* ws, cudaStream_t s) {
+  return launch_beam_impl(d, beam_width, n_best, space_idx, wip, logits, in_len, decoded, decoded_len, scores, log_probs,
+                          ties, ws, s, nullptr);
+}
+
+int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, int beam_width, int n_best, int space_idx, double wip,
+                   double lmwt, double oov_penalty, const void* logits, const void* in_len, int64_t* decoded,
+                   int64_t* decoded_len, double* scores, double* log_probs, double* lm_scores, int64_t* oov_words,
+                   int64_t* ties, char* ws, cudaStream_t s) {
+  BeamLMParams q;
+  q.table = reinterpret_cast<const NGramEntry*>(lm.table); q.mask = (unsigned long long)lm.table_slots - 1ull;
+  q.lex_child = lm.lex_child; q.lex_word = lm.lex_word; q.label_char = lm.label_char;
+  q.n_chars = lm.n_chars; q.order = lm.order; q.bos = lm.bos_id; q.eos = lm.eos_id; q.unk = lm.unk_id;
+  q.lmwt = lmwt; q.oov_penalty = oov_penalty;
+  q.lm_scores = lm_scores; q.oov_words = reinterpret_cast<long long*>(oov_words);
+  return launch_beam_impl(d, beam_width, n_best, space_idx, wip, logits, in_len, decoded, decoded_len, scores, log_probs,
+                          ties, ws, s, &q);
 }
 
 }  // namespace e2e

@@ -7,14 +7,30 @@
   (decoders/ctc_decoder.py:76-115; src/decoders/ctc_decoder.cpp:153-198, 353-441) -- SURVEY.md 8(f3);
 * the N best prefixes of that search with their scores: ``decode_nbest``, for rescoring with any language model on the
   host (N-best rescoring);
+* the same search with a word n-gram language model fused in (shallow fusion): ``decode`` / ``decode_nbest`` with
+  ``lm=NGramLM.from_arpa(path)``, weighted by the constructor's ``lmwt``, ``wip``, ``oov_penalty`` and
+  ``case_sensitive``;
 * the exact CTC log-likelihood of given transcripts, N per utterance: ``score`` (``decode_nbest``'s list or any other);
 * timestamps of given transcripts, N per utterance: ``align`` -- the best path, each token's frame span, word spans and
   the best path's log-probability;
 * word and token errors of N transcripts per utterance against a reference: ``errors`` -- the risk of N-best sequence
   training and the counts behind WER / CER.
 
-KenLM decoding (``lm_path``) stays the reference's CPU code and is out of scope; asking for it here raises
-``NotImplementedError`` instead of silently decoding without the model.
+KenLM decoding through ``lm_path`` (binary models) stays the reference's CPU code and is out of scope; asking for it here
+raises ``NotImplementedError`` instead of silently decoding without the model.  Text ARPA models are read by
+``NGramLM.from_arpa`` and passed as ``lm=``.
+
+Language-model fusion (include/e2e_ctc.h, e2e_ctc_ngram, has the full definition):
+
+* a word is a maximal run of labels other than the blank and ``" "``; its spelling is the concatenation of its labels
+  (every label but the blank must be one character, and ``" "`` must be a label).  With ``case_sensitive=False`` the
+  labels are lowercased before a spelling is looked up; the model's vocabulary is used as written;
+* a completed word whose spelling is no unigram of the model is out of vocabulary (OOV) and scored as ``<unk>``;
+* the history starts as ``<s>``; extending a prefix with ``" "`` completes its current word ``w`` (if non-empty):
+  ``lm += ln(10) * log10 P(w | history)`` with ARPA backoff and ``oov += 1`` for an OOV word.  Partial words are never
+  scored; for the final ranking a trailing word is completed and ``</s>`` is scored;
+* ``score = ((log p(prefix) + lmwt * lm) - words * wip) + oov * oov_penalty`` ranks and prunes the beam.
+
 """
 from collections import namedtuple
 
@@ -35,6 +51,14 @@ NBestResults = namedtuple("NBestResults", ["decoded_targets",
                                            "decoded_sentences",
                                            "scores",
                                            "log_probs"])
+
+NBestLMResults = namedtuple("NBestLMResults", ["decoded_targets",
+                                               "decoded_targets_lengths",
+                                               "decoded_sentences",
+                                               "scores",
+                                               "log_probs",
+                                               "lm_scores",
+                                               "oov_words"])
 
 AlignmentResults = namedtuple("AlignmentResults", ["alignments",
                                                    "token_starts",
@@ -77,8 +101,10 @@ class CTCDecoder:
     :param labels: list of strings with labels (including the blank symbol), e.g. ``["_", "a", "b"]``
     :param wip: word insertion penalty of the beam search (score = log p - number of words * wip; words are
         separated by the label ``" "``)
-    :param lm_path, lmwt, oov_penalty, case_sensitive: language-model options of the reference's beam search;
-        accepted for signature compatibility.  A non-empty ``lm_path`` is refused by ``decode``
+    :param lm_path: refused by ``decode`` (KenLM's binary models are not read); pass ``lm=NGramLM.from_arpa(path)``
+        to ``decode`` / ``decode_nbest`` instead
+    :param lmwt, oov_penalty, case_sensitive: language-model weight, score added per OOV word, and whether labels are
+        matched to the model's words as written (``False``: labels are lowercased first); used with ``lm=``
     """
 
     def __init__(self, beam_width=100, after_logsoftmax=False, blank_idx=0, time_major=False, labels=None,
@@ -95,9 +121,9 @@ class CTCDecoder:
         self._case_sensitive = case_sensitive
         self._decoder = CTCBeamEngine(self._blank_idx, max(int(self._beam_width), 1), self._labels, self._wip)
 
-    def decode(self, logits, logits_lengths=None):
-        """Prefix beam search (`<https://arxiv.org/abs/1408.2873>`_) without a language model; greedy decoding when
-        ``beam_width == 1`` (decoders/ctc_decoder.py:76-115).
+    def decode(self, logits, logits_lengths=None, *, lm=None):
+        """Prefix beam search (`<https://arxiv.org/abs/1408.2873>`_), with the word n-gram model ``lm`` fused in if
+        given; greedy decoding when ``beam_width == 1`` (decoders/ctc_decoder.py:76-115), where ``lm`` is refused.
 
         :param logits: ``(T, B, V)`` if ``time_major`` else ``(B, T, V)``; CPU or CUDA tensor; log-probabilities if
             ``after_logsoftmax`` else raw network outputs
@@ -106,13 +132,20 @@ class CTCDecoder:
             int64, decoded_sentences list[str])`` -- CPU tensors, as in the reference.  An utterance whose best
             prefix is empty comes back as the single symbol ``-1`` with length 1 (the reference's behaviour); its
             sentence is ``""``
+        :param lm: ``NGramLM`` or ``None``; CPU logits are copied to its device
         """
+        if lm is not None:
+            if self._beam_width == 1:
+                raise ValueError("decode with beam_width == 1 is greedy and takes no language model")
+            nb = self.decode_nbest(logits, logits_lengths, n_best=1, lm=lm)
+            return DecoderResults(nb.decoded_targets[:, 0], nb.decoded_targets_lengths[:, 0],
+                                  [s[0] for s in nb.decoded_sentences])
         if self._beam_width == 1:
             return self.decode_greedy(logits, logits_lengths)
         if self._lm_path:
             raise NotImplementedError(
-                "decoding with a KenLM language model stays the reference's CPU code and is outside this engine's "
-                "scope; construct CTCDecoder without lm_path")
+                "decoding with a KenLM model through lm_path stays the reference's CPU code; construct CTCDecoder "
+                "without lm_path and pass lm=NGramLM.from_arpa(path) to decode")
         if self._time_major:
             logits = logits.transpose(1, 0)
         decoded_targets, decoded_targets_lengths = self._decoder.decode(
@@ -120,7 +153,7 @@ class CTCDecoder:
         decoded_sentences = self._sentences(decoded_targets, decoded_targets_lengths)
         return DecoderResults(decoded_targets, decoded_targets_lengths, decoded_sentences)
 
-    def decode_nbest(self, logits, logits_lengths=None, *, n_best):
+    def decode_nbest(self, logits, logits_lengths=None, *, n_best, lm=None):
         """The ``n_best`` best prefixes of the LM-free prefix beam search and their scores, for rescoring with a
         language model of the caller's choice.  Always the prefix beam search: with ``beam_width == 1`` that is a
         beam of width 1, not the greedy path ``decode`` takes.
@@ -135,21 +168,46 @@ class CTCDecoder:
             ``log_probs`` is the prefix's acoustic log-probability without the word penalty.  The empty prefix is the
             single symbol ``-1`` with length 1, as in ``decode``; slots past the number of prefixes the final beam
             holds (short utterances, tiny alphabets) have length 0, sentence ``""`` and ``-inf`` scores
+        :param lm: ``NGramLM`` or ``None``.  With a model the search itself is scored with it (module docstring) and the
+            result is ``NBestLMResults(decoded_targets, decoded_targets_lengths, decoded_sentences, scores, log_probs,
+            lm_scores, oov_words)``: ``scores = ((log_probs + lmwt * lm_scores) - words * wip) + oov_words *
+            oov_penalty`` ranks the list, ``log_probs`` is acoustic only, ``lm_scores`` [B, N] float64 is the unweighted
+            natural-log LM score with the end-of-utterance terms and ``oov_words`` [B, N] int64 counts OOV words.  CPU
+            logits are copied to the model's device; logits on another CUDA device raise ``ValueError``
         """
         if self._lm_path:
             raise NotImplementedError(
-                "decoding with a KenLM language model stays the reference's CPU code and is outside this engine's "
-                "scope; construct CTCDecoder without lm_path and rescore the decode_nbest list with the model")
+                "decoding with a KenLM model through lm_path stays the reference's CPU code; construct CTCDecoder "
+                "without lm_path and pass lm=NGramLM.from_arpa(path), or rescore the decode_nbest list with the model")
         if not 1 <= int(n_best) <= self._decoder.beam_width:
             raise ValueError("n_best %d outside [1, beam_width = %d]" % (int(n_best), self._decoder.beam_width))
         if self._time_major:
             logits = logits.transpose(1, 0)
+        if lm is not None:
+            return self._decode_nbest_lm(logits, logits_lengths, int(n_best), lm)
         decoded_targets, decoded_targets_lengths, scores, log_probs = self._decoder.decode_nbest(
             logits, logits_lengths, n_best=int(n_best), from_logits=not self._after_logsoftmax)
         B, N = decoded_targets_lengths.shape
         flat = self._sentences(decoded_targets.reshape(B * N, -1), decoded_targets_lengths.reshape(-1))
         decoded_sentences = [flat[b * N:(b + 1) * N] for b in range(B)]
         return NBestResults(decoded_targets, decoded_targets_lengths, decoded_sentences, scores, log_probs)
+
+    def _decode_nbest_lm(self, logits, logits_lengths, n_best, lm):
+        if not logits.is_cuda:
+            logits = logits.to(lm.device)
+        elif logits.device != lm.device:
+            raise ValueError("logits on %s, the language model on %s" % (logits.device, lm.device))
+        out = self._decoder.decode_nbest_lm_device(logits, lm, logits_lengths, n_best, not self._after_logsoftmax,
+                                                   lmwt=self._lmwt, oov_penalty=self._oov_penalty,
+                                                   case_sensitive=self._case_sensitive)
+        decoded, lengths, scores, log_probs, lm_scores, oov_words, ties = (t.cpu() for t in out)
+        self._decoder.last_ties = ties
+        width = int(lengths.max()) if lengths.numel() else 0
+        decoded = decoded[:, :, :width].contiguous()
+        B, N = lengths.shape
+        flat = self._sentences(decoded.reshape(B * N, -1), lengths.reshape(-1))
+        sentences = [flat[b * N:(b + 1) * N] for b in range(B)]
+        return NBestLMResults(decoded, lengths, sentences, scores, log_probs, lm_scores, oov_words)
 
     def score(self, logits, hypotheses, hypotheses_lengths, logits_lengths=None):
         """The CTC log-likelihood ``log p(hypothesis | logits)`` of N transcripts per utterance: minus the CTC loss of each

@@ -315,6 +315,68 @@ int e2e_ctc_beam_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int3
                               double* scores, double* log_probs, int64_t* ties, void* workspace, size_t workspace_bytes,
                               void* cuda_stream);
 
+/* ------------------------------------------------------- prefix beam search with a word n-gram LM ---- */
+
+/* A word n-gram language model fused into the prefix beam search (shallow fusion).
+ *   words: a word is a maximal run of labels other than the blank and the space (space_idx, which is required); its
+ *       spelling is the concatenation of its labels' characters (every label but the blank is one character; with
+ *       case folding the caller lowercases the labels before building the lexicon).  The special tokens <s>, </s> and
+ *       <unk> are never spelled;
+ *   vocabulary: a completed word whose spelling is no unigram of the model is out of vocabulary (OOV) and is scored as
+ *       <unk> (a model without <unk> gets it with log10 probability -100 and backoff 0);
+ *   when the LM scores: the history starts as <s>.  A space extension of a prefix whose current word is non-empty
+ *       completes that word w: lm += ln10 * log10 P(w | history) with ARPA backoff, oov += 1 if w is OOV, and w joins the
+ *       history (of which the last order - 1 words are the context).  Partial words are never scored.  For the final
+ *       ranking only, a non-empty trailing word is completed the same way and then </s> is scored;
+ *   backoff: from the longest context to the shortest, either the n-gram (context, w) exists -- add its log10
+ *       probability and stop -- or it does not -- add the context's backoff weight (0 if the context is no n-gram) and
+ *       drop the context's oldest word.  A word's term is t * M_LN10, t being that fp64 sum in that order; lm adds the
+ *       terms in word order;
+ *   score = ((log p(prefix) + lmwt * lm) - words * wip) + oov * oov_penalty in fp64, in that order, without fused
+ *       multiply-adds.  Extensions are ranked and pruned with it; the final list is ranked with it including the
+ *       end-of-utterance terms.
+ * Since the LM changes only a member's space extension, the member's other extensions still rank by the symbol's
+ * log-probability alone: the large-alphabet symbol filter stays exact. */
+typedef struct e2e_ctc_ngram {
+  const void* table;          /* e2e_ctc_ngram_table_bytes(table_slots) device bytes filled by e2e_ctc_ngram_build_device */
+  int64_t table_slots;        /* a power of two larger than the number of n-grams */
+  const int32_t* lex_child;   /* [lex_nodes][n_chars] device: the lexicon trie's child of a node for a character, -1: none;
+                                 node 0 is the root (the empty spelling) */
+  const int32_t* lex_word;    /* [lex_nodes] device: the word id a node spells, -1: none */
+  const int32_t* label_char;  /* [alphabet] device: the character id of every label other than the blank and the space */
+  int32_t lex_nodes, n_chars;
+  int32_t order;              /* 1..6 */
+  int32_t bos_id, eos_id, unk_id;   /* word ids of <s>, </s>, <unk> */
+} e2e_ctc_ngram;
+
+/* Bytes of an n-gram table of `slots` entries (48 each). */
+size_t e2e_ctc_ngram_table_bytes(int64_t slots);
+/* Fills `table` (e2e_ctc_ngram_table_bytes(slots) device bytes; cleared first) with `count` distinct n-grams: open
+ * addressing keyed by the full n-gram, so that lookups do not depend on the insertion order.
+ *   ids: [count][6] int32 word ids, the n-gram's words oldest first (entries past its order are ignored);
+ *   orders: [count] int32 in [1, 6]; probs, bows: [count] float64 log10 probability and backoff weight.
+ * slots must be a power of two and larger than count.  Enqueues only. */
+int e2e_ctc_ngram_build_device(void* table, int64_t slots, int64_t count, const int32_t* ids, const int32_t* orders,
+                               const double* probs, const double* bows, void* cuda_stream);
+
+/* The N best prefixes of the prefix beam search with the language model above fused in.  Arguments as for
+ * e2e_ctc_beam_nbest_device, plus:
+ *   space_idx: required (>= 0);
+ *   lm: the model and the lexicon of these labels; lmwt, oov_penalty: finite;
+ *   scores: [B,N] float64, the score above with the end-of-utterance terms;
+ *   log_probs (optional): the acoustic log p(prefix) alone;
+ *   lm_scores: [B,N] float64, lm unweighted, natural log, end-of-utterance terms included;
+ *   oov_words: [B,N] int64;
+ *   slots past the final beam: length 0, scores = log_probs = lm_scores = -inf, oov_words 0.
+ * The workspace query returns 0 (E2E_ERR_UNSUPPORTED) when the beam's state with the LM's does not fit shared memory. */
+size_t e2e_ctc_beam_lm_workspace_bytes(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, int32_t beam_width,
+                                       int32_t n_best);
+int e2e_ctc_beam_lm_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx,
+                                 double wip, const e2e_ctc_ngram* lm, double lmwt, double oov_penalty, const void* logits,
+                                 const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths, double* scores,
+                                 double* log_probs, double* lm_scores, int64_t* oov_words, int64_t* ties, void* workspace,
+                                 size_t workspace_bytes, void* cuda_stream);
+
 /* ------------------------------------------------------- N hypotheses per utterance: score ---- */
 
 /* The CTC log-likelihood log p(y | x) of n_hyp hypotheses per utterance, forward only (no gradient, nothing kept for a
@@ -486,7 +548,7 @@ uint64_t e2e_ctc_launch_count(void);
  * events, then fills ms[k] (summed device milliseconds) and launches[k] per kernel kind
  * k = 0 row_stats, 1 lattice, 2 gradient, 3 loss_reduce, 4 argmax, 5 collapse, 6 scale_rows, 7 viterbi,
  * 8 ctc_without_blank, 9 beam_search, 10 order, 11 score, 12 score_backward, 13 score_backward_rows, 14 edit_distance,
- * 15 mwer_forward, 16 mwer_weights, 17 mwer_backward (its row kernel counts as 13)
+ * 15 mwer_forward, 16 mwer_weights, 17 mwer_backward (its row kernel counts as 13), 18 beam_search_lm, 19 ngram_build
  * (n_kinds >= 12;
  * the kinds past n_kinds are not reported), and clears the record.  All launches since the previous read must have been made on ONE device. */
 int e2e_ctc_profile_enable(int32_t on);
