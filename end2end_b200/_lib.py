@@ -39,7 +39,7 @@ EXPORTS = (
     "e2e_ctc_mwer_state_bytes", "e2e_ctc_mwer_backward_workspace_bytes", "e2e_ctc_mwer_forward_device",
     "e2e_ctc_mwer_backward_device",
     "e2e_ctc_ngram_table_bytes", "e2e_ctc_ngram_build_device", "e2e_ctc_beam_lm_workspace_bytes",
-    "e2e_ctc_beam_lm_nbest_device",
+    "e2e_ctc_beam_lm_nbest_device", "e2e_ctc_beam_lm_tokens_workspace_bytes", "e2e_ctc_beam_lm_tokens_nbest_device",
 )
 KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score",
                 "score_backward", "score_backward_rows", "edit_distance", "mwer_forward", "mwer_weights", "mwer_backward",
@@ -77,6 +77,11 @@ class NGramDesc(ctypes.Structure):
         ("lex_nodes", ctypes.c_int32), ("n_chars", ctypes.c_int32), ("order", ctypes.c_int32),
         ("bos_id", ctypes.c_int32), ("eos_id", ctypes.c_int32), ("unk_id", ctypes.c_int32),
     ]
+
+
+class NGramTokensDesc(ctypes.Structure):
+    """struct e2e_ctc_ngram_tokens"""
+    _fields_ = [("label_kind", ctypes.c_void_p), ("label_off", ctypes.c_void_p), ("label_chars", ctypes.c_void_p)]
 
 
 class Limits(ctypes.Structure):
@@ -166,6 +171,12 @@ def load():
     L.e2e_ctc_beam_lm_nbest_device.argtypes = [dp, i32, i32, i32, dbl, np_, dbl, dbl, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                                vp, sz, vp]
     L.e2e_ctc_beam_lm_nbest_device.restype = ctypes.c_int
+    tp_ = ctypes.POINTER(NGramTokensDesc)
+    L.e2e_ctc_beam_lm_tokens_workspace_bytes.argtypes = [dp, np_, tp_, i32, i32]
+    L.e2e_ctc_beam_lm_tokens_workspace_bytes.restype = sz
+    L.e2e_ctc_beam_lm_tokens_nbest_device.argtypes = [dp, i32, i32, dbl, np_, tp_, dbl, dbl, vp, vp, vp, vp, vp, vp, vp, vp,
+                                                      vp, vp, sz, vp]
+    L.e2e_ctc_beam_lm_tokens_nbest_device.restype = ctypes.c_int
     L.e2e_ctc_score_workspace_bytes.argtypes = [dp, i32]
     L.e2e_ctc_score_workspace_bytes.restype = sz
     L.e2e_ctc_score_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, sz, vp]

@@ -695,11 +695,14 @@ int e2e_ctc_ngram_build_device(void* table, int64_t slots, int64_t count, const 
   return launch_ngram_build(table, slots, count, ids, orders, probs, bows, reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
-static int check_beam_lm(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, int32_t beam_width, int32_t n_best,
-                         int32_t space_idx, double wip, double lmwt, double oov_penalty, bool need_space) {
+// tokens: null for a character alphabet (lm->label_char), the sub-word labels' text otherwise
+static int check_beam_lm(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens,
+                         int32_t beam_width, int32_t n_best, int32_t space_idx, double wip, double lmwt, double oov_penalty,
+                         bool need_space) {
   int rc = check_desc(desc, false);
   if (rc != E2E_OK) return rc;
-  if (!lm || !lm->table || !lm->lex_child || !lm->lex_word || !lm->label_char) { set_error("null language model argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  if (!lm || !lm->table || !lm->lex_child || !lm->lex_word || !(tokens || lm->label_char)) { set_error("null language model argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  if (tokens && (!tokens->label_kind || !tokens->label_off || !tokens->label_chars)) { set_error("null label text argument"); return E2E_ERR_INVALID_ARGUMENT; }
   if (lm->order < 1 || lm->order > 6) { set_error("language model order %d outside [1, 6]", lm->order); return E2E_ERR_INVALID_ARGUMENT; }
   if (lm->table_slots < 1 || (lm->table_slots & (lm->table_slots - 1)) || lm->lex_nodes < 1 || lm->n_chars < 0) {
     set_error("malformed language model descriptor"); return E2E_ERR_INVALID_ARGUMENT;
@@ -721,7 +724,7 @@ static int check_beam_lm(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, int3
 }
 
 size_t e2e_ctc_beam_lm_workspace_bytes(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, int32_t beam_width, int32_t n_best) {
-  if (check_beam_lm(desc, lm, beam_width, n_best, -1, 0.0, 0.0, 0.0, false) != E2E_OK) return 0;
+  if (check_beam_lm(desc, lm, nullptr, beam_width, n_best, -1, 0.0, 0.0, 0.0, false) != E2E_OK) return 0;
   return align256(beam_workspace_bytes(*desc, beam_width));
 }
 
@@ -730,12 +733,37 @@ int e2e_ctc_beam_lm_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, i
                                  const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths, double* scores,
                                  double* log_probs, double* lm_scores, int64_t* oov_words, int64_t* ties, void* workspace,
                                  size_t workspace_bytes, void* cuda_stream) {
-  int rc = check_beam_lm(desc, lm, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, true);
+  int rc = check_beam_lm(desc, lm, nullptr, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, true);
   if (rc != E2E_OK) return rc;
   if (!logits || !decoded || !decoded_lengths || !scores || !lm_scores || !oov_words) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
   rc = check_ws(workspace, workspace_bytes, e2e_ctc_beam_lm_workspace_bytes(desc, lm, beam_width, n_best));
   if (rc != E2E_OK) return rc;
-  return launch_beam_lm(*desc, *lm, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, logits, logits_lengths, decoded,
+  return launch_beam_lm(*desc, *lm, nullptr, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, logits, logits_lengths,
+                        decoded, decoded_lengths, scores, log_probs, lm_scores, oov_words, ties,
+                        reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
+// ---- the same over sub-word labels (word starts, continuations, boundaries) ---------------------------
+size_t e2e_ctc_beam_lm_tokens_workspace_bytes(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm,
+                                              const e2e_ctc_ngram_tokens* tokens, int32_t beam_width, int32_t n_best) {
+  if (!tokens) { set_error("null label text argument"); return 0; }
+  if (check_beam_lm(desc, lm, tokens, beam_width, n_best, -1, 0.0, 0.0, 0.0, false) != E2E_OK) return 0;
+  return align256(beam_workspace_bytes(*desc, beam_width));
+}
+
+int e2e_ctc_beam_lm_tokens_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, double wip,
+                                        const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens, double lmwt,
+                                        double oov_penalty, const void* logits, const void* logits_lengths,
+                                        int64_t* decoded, int64_t* decoded_lengths, double* scores, double* log_probs,
+                                        double* lm_scores, int64_t* oov_words, int64_t* ties, void* workspace,
+                                        size_t workspace_bytes, void* cuda_stream) {
+  if (!tokens) { set_error("null label text argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  int rc = check_beam_lm(desc, lm, tokens, beam_width, n_best, -1, wip, lmwt, oov_penalty, false);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !decoded || !decoded_lengths || !scores || !lm_scores || !oov_words) { set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  rc = check_ws(workspace, workspace_bytes, e2e_ctc_beam_lm_tokens_workspace_bytes(desc, lm, tokens, beam_width, n_best));
+  if (rc != E2E_OK) return rc;
+  return launch_beam_lm(*desc, *lm, tokens, beam_width, n_best, -1, wip, lmwt, oov_penalty, logits, logits_lengths, decoded,
                         decoded_lengths, scores, log_probs, lm_scores, oov_words, ties, reinterpret_cast<char*>(workspace),
                         reinterpret_cast<cudaStream_t>(cuda_stream));
 }

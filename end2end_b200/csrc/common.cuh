@@ -268,10 +268,11 @@ int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx
                 const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
                 char* ws, cudaStream_t s);
 // the same search with a word n-gram LM fused (e2e_ctc_beam_lm_nbest_device): scores, lm_scores, oov_words required
-int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, int beam_width, int n_best, int space_idx, double wip,
-                   double lmwt, double oov_penalty, const void* logits, const void* in_len, int64_t* decoded,
-                   int64_t* decoded_len, double* scores, double* log_probs, double* lm_scores, int64_t* oov_words,
-                   int64_t* ties, char* ws, cudaStream_t s);
+// tokens: null for a character alphabet (the space is the boundary, lm.label_char every other label's character)
+int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, const e2e_ctc_ngram_tokens* tokens, int beam_width,
+                   int n_best, int space_idx, double wip, double lmwt, double oov_penalty, const void* logits,
+                   const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs,
+                   double* lm_scores, int64_t* oov_words, int64_t* ties, char* ws, cudaStream_t s);
 size_t ngram_table_bytes(long long slots);
 int launch_ngram_build(void* table, long long slots, long long count, const int* ids, const int* orders, const double* probs,
                        const double* bows, cudaStream_t s);

@@ -40,10 +40,13 @@
 // Arithmetic: fp64 log-space with the reference's two-argument log_sum_exp (src/utils/math_utils.h:8-16) and the score
 // expression of :311-315 evaluated in its order without fused multiply-adds.
 //
-// The LM template parameter fuses a word n-gram language model into the same search (include/e2e_ctc.h, e2e_ctc_ngram).
-// Only a member's space extension completes a word, so only that extension's score changes (BeamExt): the symbol filter,
-// the select and the trie are as above.  Each new member looks up what completing its current word would add once,
-// right after the write phase; LM = false compiles to the LM-free kernel unchanged.
+// The LM template parameter fuses a word n-gram language model into the same search (include/e2e_ctc.h, e2e_ctc_ngram and
+// e2e_ctc_ngram_tokens).  Every label has a kind: a continuation grows the current word, a word start or a boundary
+// completes it (characters: the space is the boundary, every other label a continuation).  For one member the
+// extensions of one kind differ only by the label's log-probability (BeamExt), so the symbol filter ranks each kind on
+// its own, and the select and the trie are as above.  Each new member walks the lexicon through its label's characters
+// and looks up what completing its current word would add once, right after the write phase; LM = false compiles to the
+// LM-free kernel unchanged.
 #include <cstdio>
 #include <cstdlib>
 
@@ -81,7 +84,13 @@ struct BeamLMParams {
   const NGramEntry* table; unsigned long long mask;   // slots - 1 (a power of two)
   const int* lex_child;      // [lex_nodes][n_chars]: child of a lexicon node for a character, -1: no word spelled so
   const int* lex_word;       // [lex_nodes]: the word a node spells, -1: none
-  const int* label_char;     // [V]: character id of a label, -1 for the blank and the space
+  // the labels' text: label c spells label_chars[label_off[c] .. label_off[c + 1]) (character ids; a word start's marker
+  // stripped) and is of kind label_kind[c] (0 continuation, 1 word start, 2 boundary).  Character alphabets pass null
+  // label_kind and label_off: label_chars[c] is the one character of label c, the space is the boundary, every other
+  // label a continuation.
+  const signed char* label_kind;
+  const int* label_off;
+  const int* label_chars;
   int n_chars, order, bos, eos, unk;
   double lmwt, oov_penalty;
   double* lm_scores;         // [B, n_best]: lm of the returned prefixes, end-of-utterance terms included
@@ -213,7 +222,11 @@ struct BeamSmem {
   unsigned long long* kc;   // [W][nR] keys of the extensions (0: none) when they fit
   int* rc;               // [nR] the symbols a member is extended with this frame, ascending (never the blank)
   unsigned* rmask;       // [VW] the same set as a bit mask
-  double *lmx, *lms, *oox, *oos;   // LM variant: lmwt * lm and oov * oov_penalty of an extension other than space / with the space
+  double *lmx, *lms, *oox, *oos;   // LM variant: lmwt * lm and oov * oov_penalty of a continuation / of an extension that
+                                   // completes the current word (word start or boundary)
+  // LM variant, at the start of the dynamic shared memory (no register holds the table's address across the frame loop):
+  unsigned char* kind;   // [V] kind of every label (0 continuation, 1 word start, 2 boundary)
+  double* pen1;          // word penalty of a word-start extension
 };
 
 // get_prev_full_prob_with_lmwt (:311-315) with a language model: ((log p + lmwt * lm) - words * wip) + oov * oov_penalty
@@ -222,16 +235,20 @@ __device__ __forceinline__ double beam_score_lm(double full, double lmw, int num
 }
 
 // What an extension of one member adds to its value besides the frame's log-probability; one key expression for every
-// site that builds an extension key.  Only the space extension completes a word, so the LM changes only that one.
+// site that builds an extension key.  Without the LM only the space scores differently (it adds no word).  With the LM
+// the label's kind decides: a word start or a boundary completes the current word (lms, oos), a word start adds a word.
+// So for one member the extensions of one kind rank by the label's log-probability alone.
 template <bool LM>
 struct BeamExt {
-  double penx, pens, lmx, lms, oox, oos;
+  double penx, pens, pen1, lmx, lms, oox, oos;
   __device__ __forceinline__ BeamExt(const BeamSmem& S, int s)
-      : penx(S.penx[s]), pens(S.pens[s]), lmx(LM ? S.lmx[s] : 0.0), lms(LM ? S.lms[s] : 0.0), oox(LM ? S.oox[s] : 0.0),
-        oos(LM ? S.oos[s] : 0.0) {}
-  __device__ __forceinline__ unsigned long long key(double v, bool space) const {
-    if (!LM) return beam_key(__dsub_rn(__dadd_rn(v, 0.0), space ? pens : penx));
-    return beam_key(__dadd_rn(__dsub_rn(__dadd_rn(v, space ? lms : lmx), space ? pens : penx), space ? oos : oox));
+      : penx(S.penx[s]), pens(S.pens[s]), pen1(LM ? S.pen1[s] : 0.0), lmx(LM ? S.lmx[s] : 0.0), lms(LM ? S.lms[s] : 0.0),
+        oox(LM ? S.oox[s] : 0.0), oos(LM ? S.oos[s] : 0.0) {}
+  __device__ __forceinline__ unsigned long long key(double v, int c, const BeamSmem& S, int space) const {
+    if (!LM) return beam_key(__dsub_rn(__dadd_rn(v, 0.0), c == space ? pens : penx));
+    const int k = S.kind[c];
+    if (k == 0) return beam_key(__dadd_rn(__dsub_rn(__dadd_rn(v, lmx), penx), oox));
+    return beam_key(__dadd_rn(__dsub_rn(__dadd_rn(v, lms), k == 1 ? pen1 : pens), oos));
   }
 };
 
@@ -265,6 +282,10 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
   {
     unsigned char* q = smem_raw;
     auto take = [&](size_t bytes) { unsigned char* r = q; q += (bytes + 15) & ~(size_t)15; return r; };
+    if (LM) {   // padded to 128 bytes: every array after it is aligned as in the LM-free layout
+      S.kind = take((size_t)V); S.pen1 = reinterpret_cast<double*>(take(8 * WB));
+      q = smem_raw + ((q - smem_raw + 127) & ~(ptrdiff_t)127);
+    }
     S.lp = reinterpret_cast<double*>(take(sizeof(double) * Vp));
     raw = reinterpret_cast<raw_t*>(take(sizeof(double) * Vp));
     C.pb = reinterpret_cast<double*>(take(8 * WB)); C.pnb = reinterpret_cast<double*>(take(8 * WB));
@@ -326,6 +347,19 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
   constexpr int kFront = 256;
   constexpr int kCascOff = kBeamThreads >= 2 * kBeamMaxWidth ? kBeamMaxWidth : 0;   // thread kCascOff + u releases member u
   auto front_sync = [&]() { asm volatile("bar.sync 1, %0;" ::"n"(kFront) : "memory"); };
+  __shared__ int s_ncls[2];   // LM variant: labels of kind 0 / kind 1 (the blank aside)
+  if (LM) {
+    if (tid < 2) s_ncls[tid] = 0;
+    __syncthreads();
+    int n0 = 0, n1 = 0;
+    for (int c = tid; c < V; c += kBeamThreads) {
+      const int k = q.label_kind ? (int)__ldg(&q.label_kind[c]) : (c == p.space ? 2 : 0);
+      S.kind[c] = (unsigned char)k;
+      if (c != p.blank) { n0 += k == 0; n1 += k == 1; }
+    }
+    n0 = warp_sum(n0); n1 = warp_sum(n1);
+    if (lane == 0) { if (n0) atomicAdd(&s_ncls[0], n0); if (n1) atomicAdd(&s_ncls[1], n1); }
+  }
   if (!p.prefilter) {   // every symbol but the blank, in order
     for (int i = tid; i < VW; i += kBeamThreads) {
       unsigned m = (32 * i + 32 <= V) ? 0xffffffffu : ((1u << (V - 32 * i)) - 1u);
@@ -402,49 +436,66 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
     if (p.prefilter) {
       // ---- large alphabets: for a given member the extensions with an ordinary symbol rank by the symbol's log-probability,
       //      so only the beam_width + 2 most probable symbols (the member's own last symbol and the space score differently)
-      //      plus the space can be among the beam_width best prefixes.  Their threshold by radix select over the row. --------
-      const int kR = min(WB + 2, V - 1);
-      unsigned long long rprefix = 0ull;
-      int rremaining = kR, shr = 56;
+      //      plus the space can be among the beam_width best prefixes.  Their threshold by radix select over the row.
+      //      With the LM the same holds within each kind of label (BeamExt): the beam_width + 2 most probable continuations,
+      //      the beam_width + 2 most probable word starts, each class by its own select, and every boundary. ------------------
+      constexpr int kCls = LM ? 2 : 1;
+      unsigned long long rcls0 = ~0ull, rcls1 = ~0ull;
+      int shr0 = 56, shr1 = 56;
       for (int i = tid; i < VW; i += kFront) S.rmask[i] = 0u;
-      for (; shr >= 0; shr -= 8) {
-        for (int i = tid; i < kBeamBins; i += kFront) S.hist[i] = 0u;
-        front_sync();
-        const unsigned long long pm = shr == 56 ? 0ull : (~0ull << (shr + 8));
-        for (int c = tid; c < V; c += kFront) {
-          if (c == p.blank) continue;
-          const unsigned long long k = beam_key(S.lp[c]);
-          if ((k & pm) == (rprefix & pm)) atomicAdd(&S.hist[(unsigned)(k >> shr) & 255u], 1u);
+#pragma unroll
+      for (int cl = 0; cl < kCls; cl++) {
+        const int kR = LM ? min(WB + 2, s_ncls[cl]) : min(WB + 2, V - 1);
+        unsigned long long rprefix = 0ull;
+        int rremaining = kR, shr = 56;
+        for (; (!LM || kR > 0) && shr >= 0; shr -= 8) {
+          for (int i = tid; i < kBeamBins; i += kFront) S.hist[i] = 0u;
+          front_sync();
+          const unsigned long long pm = shr == 56 ? 0ull : (~0ull << (shr + 8));
+          for (int c = tid; c < V; c += kFront) {
+            if (c == p.blank || (LM && S.kind[c] != cl)) continue;
+            const unsigned long long k = beam_key(S.lp[c]);
+            if ((k & pm) == (rprefix & pm)) atomicAdd(&S.hist[(unsigned)(k >> shr) & 255u], 1u);
+          }
+          front_sync();
+          // every warp finds the bin on its own: the same registers everywhere, nothing to broadcast through shared memory
+          unsigned h[8], mine = 0;
+#pragma unroll
+          for (int j = 0; j < 8; j++) { h[j] = S.hist[lane * 8 + j]; mine += h[j]; }
+          unsigned above = mine;
+#pragma unroll
+          for (int o = 1; o < 32; o <<= 1) { const unsigned u = __shfl_down_sync(0xffffffffu, above, o); if (lane + o < 32) above += u; }
+          above -= mine;
+          const bool here = above < (unsigned)rremaining && above + mine >= (unsigned)rremaining;
+          unsigned acc = above, hd = h[0]; int d = 0;
+#pragma unroll
+          for (int j = 7; j > 0; j--) {
+            if (d == 0) { if (acc + h[j] >= (unsigned)rremaining) { d = j; hd = h[j]; } else acc += h[j]; }
+          }
+          const int src = __ffs(__ballot_sync(0xffffffffu, here)) - 1;
+          const int bin = __shfl_sync(0xffffffffu, lane * 8 + d, src);
+          const int need_r = __shfl_sync(0xffffffffu, rremaining - (int)acc, src);
+          const int cnt_r = __shfl_sync(0xffffffffu, (int)hd, src);
+          rprefix |= (unsigned long long)bin << shr;
+          rremaining = need_r;
+          front_sync();                       // the histogram is cleared again at the top
+          if (cnt_r == need_r || shr == 0) break;
         }
-        front_sync();
-        // every warp finds the bin on its own: the same registers everywhere, nothing to broadcast through shared memory
-        unsigned h[8], mine = 0;
-#pragma unroll
-        for (int j = 0; j < 8; j++) { h[j] = S.hist[lane * 8 + j]; mine += h[j]; }
-        unsigned above = mine;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const unsigned u = __shfl_down_sync(0xffffffffu, above, o); if (lane + o < 32) above += u; }
-        above -= mine;
-        const bool here = above < (unsigned)rremaining && above + mine >= (unsigned)rremaining;
-        unsigned acc = above, hd = h[0]; int d = 0;
-#pragma unroll
-        for (int j = 7; j > 0; j--) {
-          if (d == 0) { if (acc + h[j] >= (unsigned)rremaining) { d = j; hd = h[j]; } else acc += h[j]; }
-        }
-        const int src = __ffs(__ballot_sync(0xffffffffu, here)) - 1;
-        const int bin = __shfl_sync(0xffffffffu, lane * 8 + d, src);
-        const int need_r = __shfl_sync(0xffffffffu, rremaining - (int)acc, src);
-        const int cnt_r = __shfl_sync(0xffffffffu, (int)hd, src);
-        rprefix |= (unsigned long long)bin << shr;
-        rremaining = need_r;
-        front_sync();                       // the histogram is cleared again at the top
-        if (cnt_r == need_r || shr == 0) break;
+        if (!LM || kR > 0) { if (cl == 0) { rcls0 = rprefix >> shr; shr0 = shr; } else { rcls1 = rprefix >> shr; shr1 = shr; } }
       }
-      const unsigned long long rcls = rprefix >> shr;
       int nlist = 0;
       for (int c0 = 0; c0 < V; c0 += kFront) {   // the list, in symbol order
         const int c = c0 + tid;
-        const bool in = c < V && c != p.blank && ((beam_key(S.lp[c]) >> shr) >= rcls || c == p.space);
+        bool in = c < V && c != p.blank;
+        if (LM) {
+          if (in) {
+            const int kd = S.kind[c];
+            const unsigned long long k = beam_key(S.lp[c]);
+            in = kd == 2 || (kd == 0 ? (k >> shr0) >= rcls0 : (k >> shr1) >= rcls1);
+          }
+        } else {
+          in = in && ((beam_key(S.lp[c]) >> shr0) >= rcls0 || c == p.space);
+        }
         const unsigned m = __ballot_sync(0xffffffffu, in);
         if (lane == 0) s_wcnt[warp] = __popc(m);
         front_sync();
@@ -468,10 +519,12 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
       const int last = C.last[s];
       S.npnb[s] = last >= 0 ? __dadd_rn(S.lp[last], pnbv) : -INFINITY;
       const int nws = C.nw[s];
-      const int nwx = nws + ((nws == 0 || last == p.space) ? 1 : 0); // :252-257 for a symbol other than space
+      // :252-257 for a symbol other than space; with the LM, for a continuation (the current word is empty after a boundary)
+      const int nwx = nws + ((nws == 0 || (LM ? S.kind[last] == 2 : last == p.space)) ? 1 : 0);
       S.nwx[s] = nwx;
       S.penx[s] = __dmul_rn((double)nwx, p.wip); S.pens[s] = __dmul_rn((double)nws, p.wip);
-      if (LM) {   // a space extension completes the current word (if any): its LM term and OOV count join the score
+      if (LM) {   // a word start or a boundary completes the current word (if any): its LM term and OOV count join the score
+        S.pen1[s] = __dmul_rn((double)(nws + 1), p.wip);
         const double lm = C.lm[s];
         const int oov = C.oov[s], cw = C.cw[s];
         const double lmx = __dmul_rn(q.lmwt, lm), oox = __dmul_rn((double)oov, q.oov_penalty);
@@ -551,7 +604,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
             unsigned long long k = 0ull;
             if (!((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
               const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-              k = ex.key(v, c == p.space);
+              k = ex.key(v, c, S, p.space);
               kmax = k > kmax ? k : kmax; kmin = k < kmin ? k : kmin;
             }
             S.kc[s * nR + j] = k;
@@ -702,7 +755,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
               unsigned long long k = 0ull;
               if (valid) {
                 const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-                k = ex.key(v, c == p.space);
+                k = ex.key(v, c, S, p.space);
                 valid = (k & pm) == (prefix & pm);
               }
               const unsigned d = (unsigned)(k >> sh) & (kBeamBins - 1);
@@ -769,7 +822,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         if (use_cache) { if (j < nR) k = S.kc[s * nR + j]; }
         else if (j < nR && !((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
           const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-          k = ex.key(v, c == p.space);
+          k = ex.key(v, c, S, p.space);
         }
         const unsigned long long kq = k >> sh;
         ngt += __popc(__ballot_sync(0xffffffffu, k != 0ull && kq > tcls));
@@ -833,7 +886,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         if (use_cache) { if (j < nR) k = S.kc[s * nR + j]; }
         else if (j < nR && !((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
           const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-          k = ex.key(v, c == p.space);
+          k = ex.key(v, c, S, p.space);
         }
         const unsigned long long kq = k >> sh;
         const bool isgt = k != 0ull && kq > tcls, iseq = k != 0ull && kq == tcls;
@@ -844,23 +897,23 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
           const int ns = g + min(e, need);
           const int id = node0 + (ns - keepm);
           N.node[ns] = id; N.par[ns] = pn; N.last[ns] = c; N.dep[ns] = pd + 1; N.pslot[ns] = psl;
-          N.nw[ns] = c == p.space ? C.nw[s] : S.nwx[s];
+          if (LM) { const int kd = S.kind[c]; N.nw[ns] = kd == 0 ? S.nwx[s] : C.nw[s] + (kd == 1 ? 1 : 0); }
+          else N.nw[ns] = c == p.space ? C.nw[s] : S.nwx[s];
           N.pb[ns] = -INFINITY; N.pnb[ns] = BEAM_EXT_VALUE(c, last, baseb, base);
           BeamNode r; r.parent = pn; r.chr = c; r.refs = 1; r.depth = pd + 1;
           nodes[id] = r;
           atomicAdd(&nodes[pn].refs, 1);
           if (LM) {
             const int cw = C.cw[s];
-            if (c == p.space) {   // completes the current word, if there is one; the next word starts at the lexicon's root
+            if (S.kind[c] != 0) {   // completes the current word, if there is one; the next word starts at the lexicon's root
               const bool done = cw >= 0;
               N.lm[ns] = done ? __dadd_rn(C.lm[s], C.sd[s]) : C.lm[s];
               N.oov[ns] = C.oov[s] + (done && cw == q.unk ? 1 : 0);
 #pragma unroll
               for (int i = 0; i < kLMCtx; i++) N.h[i][ns] = done ? (i == kLMCtx - 1 ? cw : C.h[i + 1][s]) : C.h[i][s];
               N.lex[ns] = 0; N.cw[ns] = -1; N.sd[ns] = 0.0;
-            } else {              // the word grows; what completing it adds is looked up below, once per new member
-              const int lx = C.lex[s];
-              N.lex[ns] = lx >= 0 ? __ldg(&q.lex_child[(long long)lx * q.n_chars + __ldg(&q.label_char[c])]) : -1;
+            } else {                // the word grows; its spelling is walked below, once per new member
+              N.lex[ns] = C.lex[s];
               N.lm[ns] = C.lm[s]; N.oov[ns] = C.oov[s];
 #pragma unroll
               for (int i = 0; i < kLMCtx; i++) N.h[i][ns] = C.h[i][s];
@@ -871,10 +924,15 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
       }
     }
     __syncthreads();
-    if (LM) {   // the new members whose word grew: the word a space would complete, and its LM term
+    if (LM) {   // the new members whose label spells characters: walk the lexicon through them (it stops as soon as no word
+                //  is spelled so), then the word a completion would score and its LM term
       for (int ns = keepm + tid; ns < keepall; ns += kBeamThreads) {
-        if (N.last[ns] == p.space) continue;
-        const int lx = N.lex[ns];
+        const int c = N.last[ns];
+        if (S.kind[c] == 2) continue;
+        int lx = N.lex[ns];
+        const int i0 = q.label_off ? __ldg(&q.label_off[c]) : c, i1 = q.label_off ? __ldg(&q.label_off[c + 1]) : c + 1;
+        for (int i = i0; i < i1 && lx >= 0; i++) lx = __ldg(&q.lex_child[(long long)lx * q.n_chars + __ldg(&q.label_chars[i])]);
+        N.lex[ns] = lx;
         int w = lx >= 0 ? __ldg(&q.lex_word[lx]) : -1;
         if (w < 0) w = q.unk;
         N.cw[ns] = w;
@@ -978,7 +1036,10 @@ size_t beam_smem_bytes(int V, int WB, size_t kc_cap, bool lm) {
   n += a16(4 * (size_t)kBeamBins) + 2 * a16(8 * (size_t)WB);   // hist, penx, pens
   n += a16(4 * (size_t)V) + a16(4 * (size_t)VW);               // rc, rmask
   n += a16(8 * kc_cap);
-  if (lm) n += 8 * a16(8 * (size_t)WB) + (2 * (3 + kLMCtx)) * a16(4 * (size_t)WB);   // lm, sd x 2, lmx, lms, oox, oos; lex, cw, oov, h x 2
+  if (lm) {   // kind, pen1 (padded to 128 bytes); lm, sd x 2, lmx, lms, oox, oos; lex, cw, oov, h x 2
+    n += (a16((size_t)V) + a16(8 * (size_t)WB) + 127) & ~(size_t)127;
+    n += 8 * a16(8 * (size_t)WB) + (2 * (3 + kLMCtx)) * a16(4 * (size_t)WB);
+  }
   return n;
 }
 
@@ -1096,13 +1157,16 @@ int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx
                           ties, ws, s, nullptr);
 }
 
-int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, int beam_width, int n_best, int space_idx, double wip,
-                   double lmwt, double oov_penalty, const void* logits, const void* in_len, int64_t* decoded,
-                   int64_t* decoded_len, double* scores, double* log_probs, double* lm_scores, int64_t* oov_words,
-                   int64_t* ties, char* ws, cudaStream_t s) {
+int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, const e2e_ctc_ngram_tokens* tokens, int beam_width,
+                   int n_best, int space_idx, double wip, double lmwt, double oov_penalty, const void* logits,
+                   const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs,
+                   double* lm_scores, int64_t* oov_words, int64_t* ties, char* ws, cudaStream_t s) {
   BeamLMParams q;
   q.table = reinterpret_cast<const NGramEntry*>(lm.table); q.mask = (unsigned long long)lm.table_slots - 1ull;
-  q.lex_child = lm.lex_child; q.lex_word = lm.lex_word; q.label_char = lm.label_char;
+  q.lex_child = lm.lex_child; q.lex_word = lm.lex_word;
+  q.label_kind = tokens ? reinterpret_cast<const signed char*>(tokens->label_kind) : nullptr;
+  q.label_off = tokens ? tokens->label_off : nullptr;
+  q.label_chars = tokens ? tokens->label_chars : lm.label_char;
   q.n_chars = lm.n_chars; q.order = lm.order; q.bos = lm.bos_id; q.eos = lm.eos_id; q.unk = lm.unk_id;
   q.lmwt = lmwt; q.oov_penalty = oov_penalty;
   q.lm_scores = lm_scores; q.oov_words = reinterpret_cast<long long*>(oov_words);

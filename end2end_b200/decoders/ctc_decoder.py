@@ -31,6 +31,22 @@ Language-model fusion (include/e2e_ctc.h, e2e_ctc_ngram, has the full definition
   scored; for the final ranking a trailing word is completed and ``</s>`` is scored;
 * ``score = ((log p(prefix) + lmwt * lm) - words * wip) + oov * oov_penalty`` ranks and prunes the beam.
 
+Sub-word alphabets (word pieces) set ``decoder.word_marker = "\u2581"`` (SentencePiece's marker, or any non-empty
+string; the constructor keeps the reference's signature): with a model the words are then made by the labels' kinds
+instead of ``" "``
+(include/e2e_ctc.h, e2e_ctc_ngram_tokens; ``NGramLM.lexicon`` / ``lm.ngram.label_kinds``):
+
+* a label that does not start with the marker continues the current word (a new word if it was empty);
+* the marker followed by characters completes the current word (if non-empty) and starts a new one with those
+  characters;
+* the marker alone completes the current word (if non-empty) and starts an empty one;
+* a word's spelling is its labels' text with the marker stripped, so ``"\u2581th" "e"`` and ``"\u2581the"`` both score
+  ``the``.  No label may be empty, contain ``" "`` or contain the marker other than at its start (``ValueError``).
+
+With ``word_marker`` set, ``decoded_sentences`` of every decode method render each marker as a space and drop leading
+and trailing spaces: ``["\u2581the", "\u2581c", "at"]`` is ``"the cat"``.  The LM-free search's ``wip`` count, ``errors(
+level="word")`` and ``word_spans`` keep the ``" "`` rule.
+
 """
 from collections import namedtuple
 
@@ -105,6 +121,10 @@ class CTCDecoder:
         to ``decode`` / ``decode_nbest`` instead
     :param lmwt, oov_penalty, case_sensitive: language-model weight, score added per OOV word, and whether labels are
         matched to the model's words as written (``False``: labels are lowercased first); used with ``lm=``
+
+    ``word_marker`` (attribute, default ``None``: labels are characters and ``" "`` separates words) is the string that
+    starts a word in sub-word ``labels``, e.g. ``"\u2581"``; it is used by ``lm=`` fusion and the rendering of
+    ``decoded_sentences`` (module docstring)
     """
 
     def __init__(self, beam_width=100, after_logsoftmax=False, blank_idx=0, time_major=False, labels=None,
@@ -119,7 +139,19 @@ class CTCDecoder:
         self._oov_penalty = oov_penalty
         self._time_major = time_major
         self._case_sensitive = case_sensitive
+        self._word_marker = None
         self._decoder = CTCBeamEngine(self._blank_idx, max(int(self._beam_width), 1), self._labels, self._wip)
+
+    @property
+    def word_marker(self):
+        """``None`` or the string that starts a word in sub-word labels (module docstring)."""
+        return self._word_marker
+
+    @word_marker.setter
+    def word_marker(self, marker):
+        if marker is not None and (not isinstance(marker, str) or not marker):
+            raise ValueError("the word marker must be None or a non-empty string, got %r" % (marker,))
+        self._word_marker = marker
 
     def decode(self, logits, logits_lengths=None, *, lm=None):
         """Prefix beam search (`<https://arxiv.org/abs/1408.2873>`_), with the word n-gram model ``lm`` fused in if
@@ -199,7 +231,8 @@ class CTCDecoder:
             raise ValueError("logits on %s, the language model on %s" % (logits.device, lm.device))
         out = self._decoder.decode_nbest_lm_device(logits, lm, logits_lengths, n_best, not self._after_logsoftmax,
                                                    lmwt=self._lmwt, oov_penalty=self._oov_penalty,
-                                                   case_sensitive=self._case_sensitive)
+                                                   case_sensitive=self._case_sensitive,
+                                                   word_marker=self._word_marker)
         decoded, lengths, scores, log_probs, lm_scores, oov_words, ties = (t.cpu() for t in out)
         self._decoder.last_ties = ties
         width = int(lengths.max()) if lengths.numel() else 0
@@ -324,4 +357,7 @@ class CTCDecoder:
         if not self._labels:
             return [""] * targets.size(0)
         rows, lens = targets.tolist(), lengths.tolist()
-        return ["".join(self._labels[i] for i in row[:n] if i >= 0) for row, n in zip(rows, lens)]
+        out = ["".join(self._labels[i] for i in row[:n] if i >= 0) for row, n in zip(rows, lens)]
+        if self._word_marker is not None:   # sub-word labels: every marker is a space, none at either end
+            out = [s.replace(self._word_marker, " ").strip(" ") for s in out]
+        return out

@@ -715,24 +715,28 @@ class CTCBeamEngine(CTCGreedyEngine):
         return decoded[:, :, :width].contiguous(), lengths, scores, log_probs
 
     def decode_nbest_lm_device(self, logits, lm, logits_lengths=None, n_best=None, from_logits=False, lmwt=1.0,
-                               oov_penalty=0.0, case_sensitive=True):
+                               oov_penalty=0.0, case_sensitive=True, word_marker=None):
         """The ``n_best`` best prefixes of the prefix beam search with the word n-gram model ``lm`` (an ``NGramLM``)
         fused in, device tensors in (on ``lm``'s device), device tensors out (no synchronisation): ``(decoded [B,N,T]
         int64 zero padded, lengths [B,N], scores [B,N] float64, log_probs [B,N] float64, lm_scores [B,N] float64,
         oov_words [B,N] int64, ties [B])``.  Ranked by ``scores = ((log_probs + lmwt * lm_scores) - words * wip) +
         oov_words * oov_penalty``, highest first (include/e2e_ctc.h, e2e_ctc_beam_lm_nbest_device).  Raises
-        ``NotImplementedError`` when the beam's state with the model's does not fit the kernel."""
+        ``NotImplementedError`` when the beam's state with the model's does not fit the kernel.  With ``word_marker``
+        the labels are sub-word units (``NGramLM.lexicon``; e2e_ctc_beam_lm_tokens_nbest_device) and need no ``" "``."""
         _require_cuda()
         n_best = self._n_best(n_best)
         logits = logits.detach()
         dev = logits.device
         if dev != lm.device:
             raise ValueError("logits on %s, the language model on %s" % (dev, lm.device))
-        if self.space_idx < 0:
+        if word_marker is None and self.space_idx < 0:
             raise ValueError("a language model needs the label \" \" between words")
         if not _dense3(logits):
             logits = logits.contiguous()
-        desc = lm.lexicon(self.labels, self.blank_idx, case_sensitive)
+        desc = lm.lexicon(self.labels, self.blank_idx, case_sensitive, word_marker)
+        tokens = None
+        if word_marker is not None:
+            desc, tokens = desc
         if len(self.labels) != logits.size(2):
             raise ValueError("%d labels for an alphabet of %d" % (len(self.labels), logits.size(2)))
         logits_lengths, d, out = self._nbest_args(logits, logits_lengths, n_best, from_logits, device=dev)
@@ -740,17 +744,27 @@ class CTCBeamEngine(CTCGreedyEngine):
         lm_scores = torch.empty(d.batch, n_best, dtype=torch.float64, device=dev)
         oov_words = torch.empty(d.batch, n_best, dtype=torch.int64, device=dev)
         with _on_device(dev):
-            n = self._L.e2e_ctc_beam_lm_workspace_bytes(ctypes.byref(d), ctypes.byref(desc), self.beam_width, n_best)
+            if tokens is None:
+                n = self._L.e2e_ctc_beam_lm_workspace_bytes(ctypes.byref(d), ctypes.byref(desc), self.beam_width, n_best)
+            else:
+                n = self._L.e2e_ctc_beam_lm_tokens_workspace_bytes(ctypes.byref(d), ctypes.byref(desc), ctypes.byref(tokens),
+                                                                   self.beam_width, n_best)
             if n == 0:
                 msg = self._L.e2e_last_error_string().decode("utf-8", "replace")
                 if "limits" in msg:
                     raise NotImplementedError(msg)
                 raise ValueError(msg)
             ws = torch.empty(n, dtype=torch.uint8, device=dev)
-            _lib.check(self._L.e2e_ctc_beam_lm_nbest_device(
-                ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip, ctypes.byref(desc), float(lmwt),
-                float(oov_penalty), _ptr(logits), _ptr(logits_lengths), _ptr(decoded), _ptr(lengths), _ptr(scores),
-                _ptr(log_probs), _ptr(lm_scores), _ptr(oov_words), _ptr(ties), _ptr(ws), ws.numel(), _stream(dev)))
+            outs = (_ptr(logits), _ptr(logits_lengths), _ptr(decoded), _ptr(lengths), _ptr(scores), _ptr(log_probs),
+                    _ptr(lm_scores), _ptr(oov_words), _ptr(ties), _ptr(ws), ws.numel(), _stream(dev))
+            if tokens is None:
+                _lib.check(self._L.e2e_ctc_beam_lm_nbest_device(
+                    ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip, ctypes.byref(desc), float(lmwt),
+                    float(oov_penalty), *outs))
+            else:
+                _lib.check(self._L.e2e_ctc_beam_lm_tokens_nbest_device(
+                    ctypes.byref(d), self.beam_width, n_best, self.wip, ctypes.byref(desc), ctypes.byref(tokens),
+                    float(lmwt), float(oov_penalty), *outs))
         return decoded, lengths, scores, log_probs, lm_scores, oov_words, ties
 
     def _score_args(self, logits, hyps, hyp_lengths, logits_lengths, from_logits, max_targets=None, noun="scorer"):

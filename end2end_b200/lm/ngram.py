@@ -4,7 +4,11 @@
 The n-grams go into one open-addressing table on the device, keyed by the whole n-gram and built by the library's insert
 kernel, so a lookup costs a few probes of a table that stays in L2 for small models and its result does not depend on
 the order the n-grams were inserted in.  The lexicon (a trie over the characters of the vocabulary's spellings) depends on
-the decoder's labels and case folding; it is built on first use for each and kept with the model.
+the decoder's labels, case folding and word marker; it is built on first use for each and kept with the model.
+
+Labels are either characters (``" "`` separates words) or sub-word units with a word marker (SentencePiece's ``"\u2581"``):
+:func:`label_kinds` sorts the latter into continuations, word starts and boundaries (include/e2e_ctc.h,
+e2e_ctc_ngram_tokens).
 """
 import ctypes
 import math
@@ -126,6 +130,42 @@ def parse_arpa(path):
     return vocab, ngrams
 
 
+#: the kinds of sub-word labels (include/e2e_ctc.h, e2e_ctc_ngram_tokens)
+CONTINUATION, WORD_START, BOUNDARY = 0, 1, 2
+
+
+def label_kinds(labels, blank_idx, word_marker, case_sensitive=True):
+    """``(kinds, texts)`` of sub-word ``labels`` with the word marker ``word_marker``: for every label its kind
+    (``CONTINUATION``: does not start with the marker; ``WORD_START``: the marker and at least one character;
+    ``BOUNDARY``: exactly the marker) and the characters it adds to a word's spelling (the marker stripped, lowercased
+    when ``case_sensitive`` is false).  The blank is ``(CONTINUATION, "")`` and never read.  Raises ``ValueError`` for an
+    empty marker, an empty label, a label containing ``" "`` and a label containing the marker anywhere but at its
+    start."""
+    if not isinstance(word_marker, str) or not word_marker:
+        raise ValueError("the word marker must be a non-empty string, got %r" % (word_marker,))
+    m = word_marker
+    kinds, texts = [], []
+    for i, lab in enumerate(labels):
+        if i == blank_idx:
+            kinds.append(CONTINUATION)
+            texts.append("")
+            continue
+        if not isinstance(lab, str) or not lab:
+            raise ValueError("label %d is empty or no string: %r" % (i, lab))
+        if " " in lab:
+            raise ValueError("label %d %r contains \" \"; words are separated by the marker %r" % (i, lab, m))
+        if lab.find(m, 1) >= 0:
+            raise ValueError("label %d %r contains the marker %r other than at its start" % (i, lab, m))
+        if lab.startswith(m):
+            rest = lab[len(m):]
+            kinds.append(WORD_START if rest else BOUNDARY)
+        else:
+            rest = lab
+            kinds.append(CONTINUATION)
+        texts.append(rest if case_sensitive else rest.lower())
+    return kinds, texts
+
+
 class NGramLM:
     """A word n-gram model on one CUDA device.  Build it with :meth:`from_arpa`; pass it to ``CTCDecoder.decode`` /
     ``decode_nbest`` as ``lm=``.  ``order``, ``vocab`` (word id -> word) and ``n_ngrams`` describe it."""
@@ -180,15 +220,19 @@ class NGramLM:
         vocab, ngrams = parse_arpa(path)
         return cls(vocab, ngrams, device)
 
-    def lexicon(self, labels, blank_idx, case_sensitive=True):
+    def lexicon(self, labels, blank_idx, case_sensitive=True, word_marker=None):
         """The ``e2e_ctc_ngram`` descriptor of this model for the decoder's ``labels`` (built on first use and kept).
-        Every label except the blank must be one character and ``" "`` must be a label; labels are lowercased when
-        ``case_sensitive`` is false.  Words with a character no label spells are unreachable and left out."""
+        Without ``word_marker`` every label except the blank must be one character and ``" "`` must be a label; with it
+        the labels are sub-word units classified by :func:`label_kinds`, and the result is the pair ``(e2e_ctc_ngram,
+        e2e_ctc_ngram_tokens)``.  Labels are lowercased when ``case_sensitive`` is false.  Words with a character no
+        label spells are unreachable and left out."""
         labels = list(labels)
-        key = (tuple(labels), int(blank_idx), bool(case_sensitive))
+        key = (tuple(labels), int(blank_idx), bool(case_sensitive), word_marker)
         hit = self._lexicons.get(key)
         if hit is not None:
             return hit[0]
+        if word_marker is not None:
+            return self._token_lexicon(key, labels, blank_idx, case_sensitive, word_marker)
         if " " not in labels:
             raise ValueError("a language model needs the label \" \" between words")
         char_id, label_char = {}, []
@@ -203,6 +247,31 @@ class NGramLM:
                 continue
             ch = lab if case_sensitive else lab.lower()
             label_char.append(char_id.setdefault(ch, len(char_id)))
+        d, kept = self._trie(char_id)
+        lc_t = torch.tensor(label_char, dtype=torch.int32).to(self.device)
+        d.label_char = lc_t.data_ptr()
+        self._lexicons[key] = (d, kept, lc_t)
+        return d
+
+    def _token_lexicon(self, key, labels, blank_idx, case_sensitive, word_marker):
+        kinds, texts = label_kinds(labels, blank_idx, word_marker, case_sensitive)
+        char_id, off, chars = {}, [0], []
+        for t in texts:
+            chars.extend(char_id.setdefault(ch, len(char_id)) for ch in t)
+            off.append(len(chars))
+        d, kept = self._trie(char_id)
+        dev = self.device
+        kind_t = torch.tensor(kinds, dtype=torch.int8).to(dev)
+        off_t = torch.tensor(off, dtype=torch.int32).to(dev)
+        chars_t = torch.tensor(chars or [0], dtype=torch.int32).to(dev)
+        tok = _lib.NGramTokensDesc()
+        tok.label_kind, tok.label_off, tok.label_chars = kind_t.data_ptr(), off_t.data_ptr(), chars_t.data_ptr()
+        self._lexicons[key] = ((d, tok), kept, kind_t, off_t, chars_t)
+        return d, tok
+
+    def _trie(self, char_id):
+        """The e2e_ctc_ngram descriptor (without label_char) of the lexicon over the characters ``char_id`` and the
+        device tensors it points into."""
         n_chars = len(char_id)
         child, word = [[-1] * n_chars], [-1]        # node 0: the empty spelling
         for wid, w in enumerate(self.vocab):
@@ -220,12 +289,11 @@ class NGramLM:
             word[node] = wid
         dev = self.device
         tensors = (torch.tensor(child, dtype=torch.int32).reshape(-1) if n_chars else torch.full((1,), -1, dtype=torch.int32),
-                   torch.tensor(word, dtype=torch.int32), torch.tensor(label_char, dtype=torch.int32))
-        child_t, word_t, lc_t = (t.to(dev) for t in tensors)
+                   torch.tensor(word, dtype=torch.int32))
+        child_t, word_t = (t.to(dev) for t in tensors)
         d = _lib.NGramDesc()
         d.table, d.table_slots = self.table.data_ptr(), self.table_slots
-        d.lex_child, d.lex_word, d.label_char = child_t.data_ptr(), word_t.data_ptr(), lc_t.data_ptr()
+        d.lex_child, d.lex_word = child_t.data_ptr(), word_t.data_ptr()
         d.lex_nodes, d.n_chars, d.order = len(word), n_chars, self.order
         d.bos_id, d.eos_id, d.unk_id = self.bos_id, self.eos_id, self.unk_id
-        self._lexicons[key] = (d, child_t, word_t, lc_t)
-        return d
+        return d, (child_t, word_t)

@@ -377,6 +377,39 @@ int e2e_ctc_beam_lm_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, i
                                  double* log_probs, double* lm_scores, int64_t* oov_words, int64_t* ties, void* workspace,
                                  size_t workspace_bytes, void* cuda_stream);
 
+/* The same search over a sub-word (word-piece) alphabet.  A word marker (SentencePiece's U+2581, say) starts a new word,
+ * and every label other than the blank is of one of three kinds:
+ *   0, continuation: the label does not start with the marker.  It appends its characters to the prefix's current word;
+ *       the prefix's word count grows by 1 if the current word was empty;
+ *   1, word start: the marker followed by at least one character.  It completes the current word (if non-empty), then
+ *       starts a new word holding the characters after the marker; the word count grows by 1;
+ *   2, boundary: exactly the marker.  It completes the current word (if non-empty) and starts an empty word; the word
+ *       count does not change.
+ * Completing a word, the end-of-utterance terms, OOV handling, the backoff arithmetic and the score are those of
+ * e2e_ctc_beam_lm_nbest_device.  A word's spelling is the concatenation of its labels' characters, the marker stripped,
+ * so (marker M) "Mth" "e" and "Mthe" spell the same word; they remain different prefixes (prefixes are label sequences).  The
+ * character search is the special case in which every label is one character, the space is the only boundary and no
+ * label is a word start.  No label may be empty or contain the marker anywhere but at its start (the caller checks).
+ * For one member the extensions with labels of one kind rank by the label's log-probability alone, so the
+ * large-alphabet symbol filter takes the beam_width + 2 most probable labels of kind 0 and of kind 1 (ties included)
+ * and every label of kind 2. */
+typedef struct e2e_ctc_ngram_tokens {
+  const int8_t* label_kind;    /* [alphabet] device: 0, 1 or 2 as above (the blank's entry is ignored) */
+  const int32_t* label_off;    /* [alphabet + 1] device: label c spells label_chars[label_off[c] .. label_off[c + 1]) */
+  const int32_t* label_chars;  /* device: character ids of e2e_ctc_ngram's lexicon (lex_child's columns), the marker
+                                  stripped and, with case folding, lowercased by the caller */
+} e2e_ctc_ngram_tokens;
+
+/* Arguments and results as for e2e_ctc_beam_lm_nbest_device, without space_idx; lm->label_char is not read. */
+size_t e2e_ctc_beam_lm_tokens_workspace_bytes(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm,
+                                              const e2e_ctc_ngram_tokens* tokens, int32_t beam_width, int32_t n_best);
+int e2e_ctc_beam_lm_tokens_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, double wip,
+                                        const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens, double lmwt,
+                                        double oov_penalty, const void* logits, const void* logits_lengths,
+                                        int64_t* decoded, int64_t* decoded_lengths, double* scores, double* log_probs,
+                                        double* lm_scores, int64_t* oov_words, int64_t* ties, void* workspace,
+                                        size_t workspace_bytes, void* cuda_stream);
+
 /* ------------------------------------------------------- N hypotheses per utterance: score ---- */
 
 /* The CTC log-likelihood log p(y | x) of n_hyp hypotheses per utterance, forward only (no gradient, nothing kept for a
