@@ -40,10 +40,11 @@ EXPORTS = (
     "e2e_ctc_mwer_backward_device",
     "e2e_ctc_ngram_table_bytes", "e2e_ctc_ngram_build_device", "e2e_ctc_beam_lm_workspace_bytes",
     "e2e_ctc_beam_lm_nbest_device", "e2e_ctc_beam_lm_tokens_workspace_bytes", "e2e_ctc_beam_lm_tokens_nbest_device",
+    "e2e_ctc_beam_bias_workspace_bytes", "e2e_ctc_beam_bias_nbest_device",
 )
 KERNEL_KINDS = ("row_stats", "lattice", "gradient", "loss_reduce", "argmax", "collapse", "scale_rows", "viterbi", "ctc_without_blank", "beam_search", "order", "score",
                 "score_backward", "score_backward_rows", "edit_distance", "mwer_forward", "mwer_weights", "mwer_backward",
-                "beam_search_lm", "ngram_build")
+                "beam_search_lm", "ngram_build", "beam_search_bias")
 
 
 class Desc(ctypes.Structure):
@@ -82,6 +83,12 @@ class NGramDesc(ctypes.Structure):
 class NGramTokensDesc(ctypes.Structure):
     """struct e2e_ctc_ngram_tokens"""
     _fields_ = [("label_kind", ctypes.c_void_p), ("label_off", ctypes.c_void_p), ("label_chars", ctypes.c_void_p)]
+
+
+class BiasDesc(ctypes.Structure):
+    """struct e2e_ctc_bias"""
+    _fields_ = [("label_col", ctypes.c_void_p), ("next", ctypes.c_void_p), ("partial", ctypes.c_void_p),
+                ("complete", ctypes.c_void_p), ("nodes", ctypes.c_int32), ("n_cols", ctypes.c_int32)]
 
 
 class Limits(ctypes.Structure):
@@ -177,6 +184,12 @@ def load():
     L.e2e_ctc_beam_lm_tokens_nbest_device.argtypes = [dp, i32, i32, dbl, np_, tp_, dbl, dbl, vp, vp, vp, vp, vp, vp, vp, vp,
                                                       vp, vp, sz, vp]
     L.e2e_ctc_beam_lm_tokens_nbest_device.restype = ctypes.c_int
+    bp_ = ctypes.POINTER(BiasDesc)
+    L.e2e_ctc_beam_bias_workspace_bytes.argtypes = [dp, np_, tp_, bp_, i32, i32]
+    L.e2e_ctc_beam_bias_workspace_bytes.restype = sz
+    L.e2e_ctc_beam_bias_nbest_device.argtypes = [dp, i32, i32, i32, dbl, np_, tp_, dbl, dbl, bp_, vp, vp, vp, vp, vp, vp,
+                                                 vp, vp, vp, vp, vp, sz, vp]
+    L.e2e_ctc_beam_bias_nbest_device.restype = ctypes.c_int
     L.e2e_ctc_score_workspace_bytes.argtypes = [dp, i32]
     L.e2e_ctc_score_workspace_bytes.restype = sz
     L.e2e_ctc_score_device.argtypes = [dp, i32, vp, vp, vp, vp, vp, vp, sz, vp]

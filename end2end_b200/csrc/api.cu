@@ -768,6 +768,49 @@ int e2e_ctc_beam_lm_tokens_nbest_device(const e2e_ctc_desc* desc, int32_t beam_w
                         reinterpret_cast<cudaStream_t>(cuda_stream));
 }
 
+// ---- the same searches with phrase biasing -----------------------------------------------------------
+static int check_beam_bias(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens,
+                           const e2e_ctc_bias* bias, int32_t beam_width, int32_t n_best, int32_t space_idx, double wip,
+                           double lmwt, double oov_penalty, bool launch) {
+  if (!bias || !bias->label_col || !bias->next || !bias->partial || !bias->complete) { set_error("null bias argument"); return E2E_ERR_INVALID_ARGUMENT; }
+  if (bias->nodes < 1 || bias->n_cols < 0) { set_error("malformed bias descriptor: nodes %d, n_cols %d", bias->nodes, bias->n_cols); return E2E_ERR_INVALID_ARGUMENT; }
+  if (!lm && tokens) { set_error("label text without a language model"); return E2E_ERR_INVALID_ARGUMENT; }
+  int rc = lm ? check_beam_lm(desc, lm, tokens, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, launch && !tokens)
+              : check_beam(desc, beam_width, n_best, launch ? space_idx : -1, wip);
+  if (rc != E2E_OK) return rc;
+  if (!beam_supported(*desc, beam_width, lm != nullptr, true)) {
+    set_error("beam search with phrase biasing: beam_width %d with alphabet %d exceeds this build's limits (beam, bitmap, LM and bias state <= 200 KB of shared memory)",
+              beam_width, desc->alphabet);
+    return E2E_ERR_UNSUPPORTED;
+  }
+  return E2E_OK;
+}
+
+size_t e2e_ctc_beam_bias_workspace_bytes(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm,
+                                         const e2e_ctc_ngram_tokens* tokens, const e2e_ctc_bias* bias,
+                                         int32_t beam_width, int32_t n_best) {
+  if (check_beam_bias(desc, lm, tokens, bias, beam_width, n_best, -1, 0.0, 0.0, 0.0, false) != E2E_OK) return 0;
+  return align256(beam_workspace_bytes(*desc, beam_width));
+}
+
+int e2e_ctc_beam_bias_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx,
+                                   double wip, const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens, double lmwt,
+                                   double oov_penalty, const e2e_ctc_bias* bias, const void* logits,
+                                   const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths, double* scores,
+                                   double* log_probs, double* lm_scores, int64_t* oov_words, double* bias_scores,
+                                   int64_t* ties, void* workspace, size_t workspace_bytes, void* cuda_stream) {
+  int rc = check_beam_bias(desc, lm, tokens, bias, beam_width, n_best, space_idx, wip, lmwt, oov_penalty, true);
+  if (rc != E2E_OK) return rc;
+  if (!logits || !decoded || !decoded_lengths || !scores || !bias_scores || (lm && (!lm_scores || !oov_words))) {
+    set_error("null pointer argument"); return E2E_ERR_INVALID_ARGUMENT;
+  }
+  rc = check_ws(workspace, workspace_bytes, e2e_ctc_beam_bias_workspace_bytes(desc, lm, tokens, bias, beam_width, n_best));
+  if (rc != E2E_OK) return rc;
+  return launch_beam_bias(*desc, lm, tokens, *bias, beam_width, n_best, tokens ? -1 : space_idx, wip, lmwt, oov_penalty,
+                          logits, logits_lengths, decoded, decoded_lengths, scores, log_probs, lm_scores, oov_words,
+                          bias_scores, ties, reinterpret_cast<char*>(workspace), reinterpret_cast<cudaStream_t>(cuda_stream));
+}
+
 // ---- CTC log-likelihood of N hypotheses per utterance (K9) -------------------------------------------
 static int check_score(const e2e_ctc_desc* desc, int32_t n_hyp) {
   int rc = check_desc(desc, true);

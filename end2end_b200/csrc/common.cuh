@@ -115,7 +115,7 @@ constexpr int kFlagInfeasible = 1, kFlagInvalid = 2;
 void set_error(const char* fmt, ...);
 
 // Launch accounting + optional per-kernel device timing (CUDA events on the launching stream).
-enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kKernelScoreGrad, kKernelScoreRows, kKernelEdit, kKernelMwerForward, kKernelMwerWeights, kKernelMwerBackward, kKernelBeamLM, kKernelNGramBuild, kNumKernels };
+enum { kKernelRowStats = 0, kKernelLattice, kKernelGrad, kKernelReduce, kKernelArgmax, kKernelCollapse, kKernelScale, kKernelViterbi, kKernelNoBlank, kKernelBeam, kKernelOrder, kKernelScore, kKernelScoreGrad, kKernelScoreRows, kKernelEdit, kKernelMwerForward, kKernelMwerWeights, kKernelMwerBackward, kKernelBeamLM, kKernelNGramBuild, kKernelBeamBias, kNumKernels };
 // e2e_ctc_profile_read's smallest n_kinds: the kinds up to kKernelScore (kinds added later are dropped for such callers)
 constexpr int kMinProfileKinds = kKernelScore + 1;
 void launch_begin(int kind, cudaStream_t s);
@@ -262,7 +262,7 @@ int launch_reduce(const void* losses, int dtype, int B, double scale, void* out,
 int launch_greedy(const e2e_ctc_desc& d, const void* logits, const void* in_len, int64_t* decoded,
                   int64_t* decoded_len, char* ws, cudaStream_t s);
 size_t beam_workspace_bytes(const e2e_ctc_desc& d, int beam_width);
-bool beam_supported(const e2e_ctc_desc& d, int beam_width, bool lm = false);
+bool beam_supported(const e2e_ctc_desc& d, int beam_width, bool lm = false, bool bias = false);
 // decoded [B, n_best, T], decoded_len [B, n_best]; scores / log_probs [B, n_best] or null (log_probs is ignored without scores)
 int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
                 const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
@@ -273,6 +273,13 @@ int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, const e2e_ctc
                    int n_best, int space_idx, double wip, double lmwt, double oov_penalty, const void* logits,
                    const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs,
                    double* lm_scores, int64_t* oov_words, int64_t* ties, char* ws, cudaStream_t s);
+// the same search with phrase biasing (e2e_ctc_beam_bias_nbest_device): lm null for none, tokens null for characters;
+// scores and bias_scores required, lm_scores and oov_words with a model
+int launch_beam_bias(const e2e_ctc_desc& d, const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens,
+                     const e2e_ctc_bias& bias, int beam_width, int n_best, int space_idx, double wip, double lmwt,
+                     double oov_penalty, const void* logits, const void* in_len, int64_t* decoded, int64_t* decoded_len,
+                     double* scores, double* log_probs, double* lm_scores, int64_t* oov_words, double* bias_scores,
+                     int64_t* ties, char* ws, cudaStream_t s);
 size_t ngram_table_bytes(long long slots);
 int launch_ngram_build(void* table, long long slots, long long count, const int* ids, const int* orders, const double* probs,
                        const double* bows, cudaStream_t s);

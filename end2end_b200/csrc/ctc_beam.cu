@@ -47,6 +47,12 @@
 // its own, and the select and the trie are as above.  Each new member walks the lexicon through its label's characters
 // and looks up what completing its current word would add once, right after the write phase; LM = false compiles to the
 // LM-free kernel unchanged.
+//
+// The BIAS template parameter boosts caller-given phrases (include/e2e_ctc.h, e2e_ctc_bias), with or without the LM: every
+// member carries its node of an Aho-Corasick automaton over labels and its committed bonus, and every key adds committed
+// + partial credit of the extended prefix.  A label in no phrase moves to the root and adds the member's committed
+// bonus alone, so the symbol filter ranks those labels as before and extends every member with every phrase label as
+// well; BIAS = false compiles to the kernel without it unchanged.
 #include <cstdio>
 #include <cstdlib>
 
@@ -97,6 +103,16 @@ struct BeamLMParams {
   long long* oov_words;      // [B, n_best]
 };
 constexpr int kLMMaxOrder = 6, kLMCtx = kLMMaxOrder - 1;
+
+// ---- phrase biasing (the BIAS variant, e2e_ctc_beam_bias_nbest_device): an Aho-Corasick automaton over labels ----------
+struct BeamBiasParams {
+  const int* label_col;      // [V]: column of a phrase label in next, -1 for every other label (those go to the root)
+  const int* next;           // [nodes][n_cols]: the full transition function over the phrase labels
+  const double* partial;     // [nodes]: phi of the node's label string (withdrawn at the end)
+  const double* complete;    // [nodes]: what reaching the node adds to committed (the phrases that end there)
+  int n_cols;
+  double* bias_scores;       // [B, n_best]: committed of the returned prefixes
+};
 
 __device__ __forceinline__ unsigned long long ngram_hash(const int* w, int n) {   // n is a compile-time constant at the call sites
   unsigned long long h = 0x9e3779b97f4a7c15ull * (unsigned long long)(n + 1);
@@ -209,6 +225,8 @@ struct BeamBuf {          // one copy of the beam (+ the pruned prefixes that st
   // recent, -1 before the start), the LM sum and what completing the current word adds to it
   int *lex, *cw, *oov, *h[kLMCtx];
   double *lm, *sd;
+  int* bn;                 // BIAS variant: automaton node of the prefix
+  double* bc;              //   and its committed bias
 };
 struct BeamSmem {
   double* lp;            // [Vp]
@@ -227,6 +245,9 @@ struct BeamSmem {
   // LM variant, at the start of the dynamic shared memory (no register holds the table's address across the frame loop):
   unsigned char* kind;   // [V] kind of every label (0 continuation, 1 word start, 2 boundary)
   double* pen1;          // word penalty of a word-start extension
+  int* col;              // BIAS variant, there as well: [V] column of every label in the automaton, -1: no phrase label
+  double* bcom;          // BIAS variant: a member's committed bias this frame (what a non-phrase label extends it with)
+  int* bnode;            //   and its automaton node
 };
 
 // get_prev_full_prob_with_lmwt (:311-315) with a language model: ((log p + lmwt * lm) - words * wip) + oov * oov_penalty
@@ -237,14 +258,38 @@ __device__ __forceinline__ double beam_score_lm(double full, double lmw, int num
 // What an extension of one member adds to its value besides the frame's log-probability; one key expression for every
 // site that builds an extension key.  Without the LM only the space scores differently (it adds no word).  With the LM
 // the label's kind decides: a word start or a boundary completes the current word (lms, oos), a word start adds a word.
-// So for one member the extensions of one kind rank by the label's log-probability alone.
-template <bool LM>
+// So for one member the extensions of one kind rank by the label's log-probability alone.  With BIAS the bias of the
+// extended prefix is added last; every label that is not a phrase label gives the member's committed bias, so the
+// extensions of one kind by non-phrase labels still rank by the label's log-probability alone.
+template <bool LM, bool BIAS>
 struct BeamExt {
-  double penx, pens, pen1, lmx, lms, oox, oos;
-  __device__ __forceinline__ BeamExt(const BeamSmem& S, int s)
+  double penx, pens, pen1, lmx, lms, oox, oos, com;
+  const int* row;   // BIAS: the member's row of the automaton's transitions
+  __device__ __forceinline__ BeamExt(const BeamSmem& S, int s, const BeamBiasParams& z)
       : penx(S.penx[s]), pens(S.pens[s]), pen1(LM ? S.pen1[s] : 0.0), lmx(LM ? S.lmx[s] : 0.0), lms(LM ? S.lms[s] : 0.0),
-        oox(LM ? S.oox[s] : 0.0), oos(LM ? S.oos[s] : 0.0) {}
-  __device__ __forceinline__ unsigned long long key(double v, int c, const BeamSmem& S, int space) const {
+        oox(LM ? S.oox[s] : 0.0), oos(LM ? S.oos[s] : 0.0), com(BIAS ? S.bcom[s] : 0.0),
+        row(BIAS ? z.next + (long long)S.bnode[s] * z.n_cols : nullptr) {}
+  // the automaton node the label moves the member to (the root for a label in no phrase)
+  __device__ __forceinline__ int bias_node(int c, const BeamSmem& S) const {
+    const int col = S.col[c];
+    return col < 0 ? 0 : __ldg(&row[col]);
+  }
+  // committed + phi of the extended prefix, (committed + complete) + partial
+  __device__ __forceinline__ double bias(int c, const BeamSmem& S, const BeamBiasParams& z) const {
+    const int col = S.col[c];
+    if (col < 0) return com;
+    const int n = __ldg(&row[col]);
+    return __dadd_rn(__dadd_rn(com, __ldg(&z.complete[n])), __ldg(&z.partial[n]));
+  }
+  __device__ __forceinline__ unsigned long long key(double v, int c, const BeamSmem& S, int space,
+                                                    const BeamBiasParams& z) const {
+    if (BIAS) {
+      double e;
+      if (!LM) e = __dsub_rn(__dadd_rn(v, 0.0), c == space ? pens : penx);
+      else if (S.kind[c] == 0) e = __dadd_rn(__dsub_rn(__dadd_rn(v, lmx), penx), oox);
+      else e = __dadd_rn(__dsub_rn(__dadd_rn(v, lms), S.kind[c] == 1 ? pen1 : pens), oos);
+      return beam_key(__dadd_rn(e, bias(c, S, z)));
+    }
     if (!LM) return beam_key(__dsub_rn(__dadd_rn(v, 0.0), c == space ? pens : penx));
     const int k = S.kind[c];
     if (k == 0) return beam_key(__dadd_rn(__dsub_rn(__dadd_rn(v, lmx), penx), oox));
@@ -263,8 +308,8 @@ __device__ long long g_beam_prof[16];
 #else
 #define BEAM_T(k) do { } while (0)
 #endif
-template <typename T, bool CACHE, int NT, bool LM>
-__global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, const BeamLMParams q) {
+template <typename T, bool CACHE, int NT, bool LM, bool BIAS>
+__global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, const BeamLMParams q, const BeamBiasParams z) {
 #ifdef BEAM_PROF
   long long prof_t = clock64();
 #endif
@@ -282,8 +327,9 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
   {
     unsigned char* q = smem_raw;
     auto take = [&](size_t bytes) { unsigned char* r = q; q += (bytes + 15) & ~(size_t)15; return r; };
-    if (LM) {   // padded to 128 bytes: every array after it is aligned as in the LM-free layout
-      S.kind = take((size_t)V); S.pen1 = reinterpret_cast<double*>(take(8 * WB));
+    if (LM || BIAS) {   // padded to 128 bytes: every array after it is aligned as in the LM-free layout
+      if (LM) { S.kind = take((size_t)V); S.pen1 = reinterpret_cast<double*>(take(8 * WB)); }
+      if (BIAS) S.col = reinterpret_cast<int*>(take(4 * (size_t)V));
       q = smem_raw + ((q - smem_raw + 127) & ~(ptrdiff_t)127);
     }
     S.lp = reinterpret_cast<double*>(take(sizeof(double) * Vp));
@@ -321,6 +367,12 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
       S.lmx = reinterpret_cast<double*>(take(8 * WB)); S.lms = reinterpret_cast<double*>(take(8 * WB));
       S.oox = reinterpret_cast<double*>(take(8 * WB)); S.oos = reinterpret_cast<double*>(take(8 * WB));
     }
+    if (BIAS) {
+      C.bc = reinterpret_cast<double*>(take(8 * WB)); N.bc = reinterpret_cast<double*>(take(8 * WB));
+      S.bcom = reinterpret_cast<double*>(take(8 * WB));
+      C.bn = reinterpret_cast<int*>(take(4 * WB)); N.bn = reinterpret_cast<int*>(take(4 * WB));
+      S.bnode = reinterpret_cast<int*>(take(4 * WB));
+    }
   }
 
   long long Ti_ll = p.in_len ? load_index(p.in_len, p.len_is64, b) : (long long)p.T;
@@ -339,6 +391,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
 #pragma unroll
       for (int i = 0; i < kLMCtx; i++) C.h[i][0] = i == kLMCtx - 1 ? q.bos : -1;
     }
+    if (BIAS) { C.bn[0] = 0; C.bc[0] = 0.0; }   // the automaton's root, nothing committed
   }
   // The first kFront threads (8 warps) run the head of a frame -- staging the row, the log-softmax, the members' own
   // updates -- synchronising among themselves on a named barrier.  With 512 threads the other half spends that time
@@ -347,15 +400,17 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
   constexpr int kFront = 256;
   constexpr int kCascOff = kBeamThreads >= 2 * kBeamMaxWidth ? kBeamMaxWidth : 0;   // thread kCascOff + u releases member u
   auto front_sync = [&]() { asm volatile("bar.sync 1, %0;" ::"n"(kFront) : "memory"); };
-  __shared__ int s_ncls[2];   // LM variant: labels of kind 0 / kind 1 (the blank aside)
-  if (LM) {
+  __shared__ int s_ncls[2];   // LM / BIAS variants: labels of kind 0 / kind 1 (the blank and the phrase labels aside)
+  if (LM || BIAS) {
     if (tid < 2) s_ncls[tid] = 0;
     __syncthreads();
     int n0 = 0, n1 = 0;
     for (int c = tid; c < V; c += kBeamThreads) {
-      const int k = q.label_kind ? (int)__ldg(&q.label_kind[c]) : (c == p.space ? 2 : 0);
-      S.kind[c] = (unsigned char)k;
-      if (c != p.blank) { n0 += k == 0; n1 += k == 1; }
+      const int k = !LM ? 0 : q.label_kind ? (int)__ldg(&q.label_kind[c]) : (c == p.space ? 2 : 0);
+      if (LM) S.kind[c] = (unsigned char)k;
+      bool ranked = c != p.blank;
+      if (BIAS) { const int col = __ldg(&z.label_col[c]); S.col[c] = col; ranked = ranked && col < 0; }
+      if (ranked) { n0 += k == 0; n1 += k == 1; }
     }
     n0 = warp_sum(n0); n1 = warp_sum(n1);
     if (lane == 0) { if (n0) atomicAdd(&s_ncls[0], n0); if (n1) atomicAdd(&s_ncls[1], n1); }
@@ -438,22 +493,23 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
       //      so only the beam_width + 2 most probable symbols (the member's own last symbol and the space score differently)
       //      plus the space can be among the beam_width best prefixes.  Their threshold by radix select over the row.
       //      With the LM the same holds within each kind of label (BeamExt): the beam_width + 2 most probable continuations,
-      //      the beam_width + 2 most probable word starts, each class by its own select, and every boundary. ------------------
+      //      the beam_width + 2 most probable word starts, each class by its own select, and every boundary.
+      //      With BIAS the selects rank the labels of no phrase only, and every phrase label is extended. ------------------
       constexpr int kCls = LM ? 2 : 1;
       unsigned long long rcls0 = ~0ull, rcls1 = ~0ull;
       int shr0 = 56, shr1 = 56;
       for (int i = tid; i < VW; i += kFront) S.rmask[i] = 0u;
 #pragma unroll
       for (int cl = 0; cl < kCls; cl++) {
-        const int kR = LM ? min(WB + 2, s_ncls[cl]) : min(WB + 2, V - 1);
+        const int kR = (LM || BIAS) ? min(WB + 2, s_ncls[cl]) : min(WB + 2, V - 1);
         unsigned long long rprefix = 0ull;
         int rremaining = kR, shr = 56;
-        for (; (!LM || kR > 0) && shr >= 0; shr -= 8) {
+        for (; (!(LM || BIAS) || kR > 0) && shr >= 0; shr -= 8) {
           for (int i = tid; i < kBeamBins; i += kFront) S.hist[i] = 0u;
           front_sync();
           const unsigned long long pm = shr == 56 ? 0ull : (~0ull << (shr + 8));
           for (int c = tid; c < V; c += kFront) {
-            if (c == p.blank || (LM && S.kind[c] != cl)) continue;
+            if (c == p.blank || (LM && S.kind[c] != cl) || (BIAS && S.col[c] >= 0)) continue;
             const unsigned long long k = beam_key(S.lp[c]);
             if ((k & pm) == (rprefix & pm)) atomicAdd(&S.hist[(unsigned)(k >> shr) & 255u], 1u);
           }
@@ -481,7 +537,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
           front_sync();                       // the histogram is cleared again at the top
           if (cnt_r == need_r || shr == 0) break;
         }
-        if (!LM || kR > 0) { if (cl == 0) { rcls0 = rprefix >> shr; shr0 = shr; } else { rcls1 = rprefix >> shr; shr1 = shr; } }
+        if (!(LM || BIAS) || kR > 0) { if (cl == 0) { rcls0 = rprefix >> shr; shr0 = shr; } else { rcls1 = rprefix >> shr; shr1 = shr; } }
       }
       int nlist = 0;
       for (int c0 = 0; c0 < V; c0 += kFront) {   // the list, in symbol order
@@ -496,6 +552,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         } else {
           in = in && ((beam_key(S.lp[c]) >> shr0) >= rcls0 || c == p.space);
         }
+        if (BIAS) in = in || (c < V && c != p.blank && S.col[c] >= 0);
         const unsigned m = __ballot_sync(0xffffffffu, in);
         if (lane == 0) s_wcnt[warp] = __popc(m);
         front_sync();
@@ -532,6 +589,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         S.lms[s] = cw >= 0 ? __dmul_rn(q.lmwt, __dadd_rn(lm, C.sd[s])) : lmx;
         S.oos[s] = cw >= 0 ? __dmul_rn((double)(oov + (cw == q.unk ? 1 : 0)), q.oov_penalty) : oox;
       }
+      if (BIAS) { S.bcom[s] = C.bc[s]; S.bnode[s] = C.bn[s]; }   // a label in no phrase extends it with this bias
     }
     }   // front threads
     __syncthreads();   // the members' updates are done; so are last frame's releases
@@ -575,7 +633,12 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
     BEAM_T(2);
     // ---- phase C: scores of the members and of the fresh extensions; how many prefixes are there now (:392-399) ------
     if (tid < W) {
-      if (LM) S.mkey[tid] = beam_key(beam_score_lm(beam_lse(S.npnb[tid], S.npb[tid]), S.lmx[tid], C.nw[tid], p.wip, S.oox[tid]));
+      if (BIAS) {   // the member's bias: committed + phi of its automaton node
+        const double e = LM ? beam_score_lm(beam_lse(S.npnb[tid], S.npb[tid]), S.lmx[tid], C.nw[tid], p.wip, S.oox[tid])
+                            : beam_score(beam_lse(S.npnb[tid], S.npb[tid]), C.nw[tid], p.wip);
+        S.mkey[tid] = beam_key(__dadd_rn(e, __dadd_rn(C.bc[tid], __ldg(&z.partial[C.bn[tid]]))));
+      }
+      else if (LM) S.mkey[tid] = beam_key(beam_score_lm(beam_lse(S.npnb[tid], S.npb[tid]), S.lmx[tid], C.nw[tid], p.wip, S.oox[tid]));
       else S.mkey[tid] = beam_key(beam_score(beam_lse(S.npnb[tid], S.npb[tid]), C.nw[tid], p.wip));
     }
     {
@@ -596,7 +659,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
             for (int s = warp - mw; s < W && s >= 0; s += kBeamWarps - mw) {
         const int last = C.last[s];
         const double base = S.full[s], baseb = C.pb[s];
-        const BeamExt<LM> ex(S, s);
+        const BeamExt<LM, BIAS> ex(S, s, z);
                       for (int j0 = 0; j0 < nR; j0 += 32) {
           const int j = j0 + lane;
           if (j < nR) {
@@ -604,7 +667,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
             unsigned long long k = 0ull;
             if (!((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
               const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-              k = ex.key(v, c, S, p.space);
+              k = ex.key(v, c, S, p.space, z);
               kmax = k > kmax ? k : kmax; kmin = k < kmin ? k : kmin;
             }
             S.kc[s * nR + j] = k;
@@ -747,7 +810,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
                         for (int s = warp; s < W; s += kBeamWarps) {
             const int last = C.last[s];
             const double base = S.full[s], baseb = C.pb[s];
-            const BeamExt<LM> ex(S, s);
+            const BeamExt<LM, BIAS> ex(S, s, z);
                           for (int j0 = 0; j0 < nR; j0 += 32) {
               const int j = j0 + lane;
               const int c = j < nR ? sym(j) : 0;
@@ -755,7 +818,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
               unsigned long long k = 0ull;
               if (valid) {
                 const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-                k = ex.key(v, c, S, p.space);
+                k = ex.key(v, c, S, p.space, z);
                 valid = (k & pm) == (prefix & pm);
               }
               const unsigned d = (unsigned)(k >> sh) & (kBeamBins - 1);
@@ -813,7 +876,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         for (int s = warp; s < W; s += kBeamWarps) {
       const int last = C.last[s];
       const double base = S.full[s], baseb = C.pb[s];
-      const BeamExt<LM> ex(S, s);
+      const BeamExt<LM, BIAS> ex(S, s, z);
       int ngt = 0, neq = 0;
             for (int j0 = 0; j0 < nR; j0 += 32) {
         const int j = j0 + lane;
@@ -822,7 +885,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         if (use_cache) { if (j < nR) k = S.kc[s * nR + j]; }
         else if (j < nR && !((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
           const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-          k = ex.key(v, c, S, p.space);
+          k = ex.key(v, c, S, p.space, z);
         }
         const unsigned long long kq = k >> sh;
         ngt += __popc(__ballot_sync(0xffffffffu, k != 0ull && kq > tcls));
@@ -870,12 +933,13 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
 #pragma unroll
           for (int i = 0; i < kLMCtx; i++) N.h[i][ns] = C.h[i][s];
         }
+        if (BIAS) { N.bn[ns] = C.bn[s]; N.bc[ns] = C.bc[s]; }
       }
     }
         for (int s = warp; s < W; s += kBeamWarps) {
       const int last = C.last[s];
       const double base = S.full[s], baseb = C.pb[s];
-      const BeamExt<LM> ex(S, s);
+      const BeamExt<LM, BIAS> ex(S, s, z);
       int gb = S.cgt[W + s], eb = S.ceq[W + s];
       const int pn = C.node[s], pd = C.dep[s];
       const int psl = new_slot(s);
@@ -886,7 +950,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         if (use_cache) { if (j < nR) k = S.kc[s * nR + j]; }
         else if (j < nR && !((S.bitmap[s * VW + (c >> 5)] >> (c & 31)) & 1u)) {
           const double v = BEAM_EXT_VALUE(c, last, baseb, base);
-          k = ex.key(v, c, S, p.space);
+          k = ex.key(v, c, S, p.space, z);
         }
         const unsigned long long kq = k >> sh;
         const bool isgt = k != 0ull && kq > tcls, iseq = k != 0ull && kq == tcls;
@@ -903,6 +967,10 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
           BeamNode r; r.parent = pn; r.chr = c; r.refs = 1; r.depth = pd + 1;
           nodes[id] = r;
           atomicAdd(&nodes[pn].refs, 1);
+          if (BIAS) {   // the automaton moves by the label; committed takes what the phrases ending there add
+            const int bn = ex.bias_node(c, S);
+            N.bn[ns] = bn; N.bc[ns] = S.col[c] < 0 ? ex.com : __dadd_rn(ex.com, __ldg(&z.complete[bn]));
+          }
           if (LM) {
             const int cw = C.cw[s];
             if (S.kind[c] != 0) {   // completes the current word, if there is one; the next word starts at the lexicon's root
@@ -967,10 +1035,12 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
       const int oov = C.oov[tid] + (done && cw == q.unk ? 1 : 0);
       lm = __dadd_rn(lm, lm_term(q.table, q.mask, q.order, h[0], h[1], h[2], h[3], h[4], q.eos));
       S.lms[tid] = lm; S.nwx[tid] = oov;
-      S.mkey[tid] = beam_key(beam_score_lm(beam_lse(C.pnb[tid], C.pb[tid]), __dmul_rn(q.lmwt, lm), C.nw[tid], p.wip,
-                                           __dmul_rn((double)oov, q.oov_penalty)));
+      const double e = beam_score_lm(beam_lse(C.pnb[tid], C.pb[tid]), __dmul_rn(q.lmwt, lm), C.nw[tid], p.wip,
+                                     __dmul_rn((double)oov, q.oov_penalty));
+      S.mkey[tid] = beam_key(BIAS ? __dadd_rn(e, C.bc[tid]) : e);   // partial credit is withdrawn: committed only
     } else {
-      S.mkey[tid] = beam_key(beam_score(beam_lse(C.pnb[tid], C.pb[tid]), C.nw[tid], p.wip));
+      const double e = beam_score(beam_lse(C.pnb[tid], C.pb[tid]), C.nw[tid], p.wip);
+      S.mkey[tid] = beam_key(BIAS ? __dadd_rn(e, C.bc[tid]) : e);
     }
   }
   if (tid == 0) s_tie_now = 0;
@@ -1004,6 +1074,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
         } else {
           p.scores[o] = beam_score(lp, C.nw[tid], p.wip);
         }
+        if (BIAS) { p.scores[o] = __dadd_rn(p.scores[o], C.bc[tid]); z.bias_scores[o] = C.bc[tid]; }
         if (p.log_probs) p.log_probs[o] = lp;
       }
       S.cgt[rank] = len;
@@ -1013,6 +1084,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
     p.decoded_len[o] = 0;
     if (p.scores) { p.scores[o] = -INFINITY; if (p.log_probs) p.log_probs[o] = -INFINITY; }
     if (LM) { q.lm_scores[o] = -INFINITY; q.oov_words[o] = 0; }
+    if (BIAS) z.bias_scores[o] = -INFINITY;
     S.cgt[tid] = 0;
   }
   __syncthreads();
@@ -1023,7 +1095,7 @@ __global__ void __launch_bounds__(NT, 1) ctc_beam_kernel(const BeamParams p, con
   }
 }
 
-size_t beam_smem_bytes(int V, int WB, size_t kc_cap, bool lm) {
+size_t beam_smem_bytes(int V, int WB, size_t kc_cap, bool lm, bool bias) {
   auto a16 = [](size_t x) { return (x + 15) & ~(size_t)15; };
   const int VW = (V + 31) >> 5, Vp = (V + 1) & ~1;
   size_t n = 2 * a16(sizeof(double) * Vp);   // lp, raw
@@ -1036,10 +1108,10 @@ size_t beam_smem_bytes(int V, int WB, size_t kc_cap, bool lm) {
   n += a16(4 * (size_t)kBeamBins) + 2 * a16(8 * (size_t)WB);   // hist, penx, pens
   n += a16(4 * (size_t)V) + a16(4 * (size_t)VW);               // rc, rmask
   n += a16(8 * kc_cap);
-  if (lm) {   // kind, pen1 (padded to 128 bytes); lm, sd x 2, lmx, lms, oox, oos; lex, cw, oov, h x 2
-    n += (a16((size_t)V) + a16(8 * (size_t)WB) + 127) & ~(size_t)127;
-    n += 8 * a16(8 * (size_t)WB) + (2 * (3 + kLMCtx)) * a16(4 * (size_t)WB);
-  }
+  // kind, pen1 (LM), col (BIAS), padded to 128 bytes
+  if (lm || bias) n += ((lm ? a16((size_t)V) + a16(8 * (size_t)WB) : 0) + (bias ? a16(4 * (size_t)V) : 0) + 127) & ~(size_t)127;
+  if (lm) n += 8 * a16(8 * (size_t)WB) + (2 * (3 + kLMCtx)) * a16(4 * (size_t)WB);   // lm, sd x 2, lmx, lms, oox, oos; lex, cw, oov, h x 2
+  if (bias) n += 3 * a16(8 * (size_t)WB) + 3 * a16(4 * (size_t)WB);                   // bc x 2, bcom; bn x 2, bnode
   return n;
 }
 
@@ -1047,13 +1119,13 @@ constexpr size_t kBeamSmemLimit = 200 * 1024;
 // How a shape runs: the symbols extended per frame (all, or the beam_width + 2 most probable + the space for large alphabets)
 // and how many extension keys are cached in shared memory (0: recomputed in every pass).
 struct BeamMode { int prefilter; int kc_cap; size_t smem; bool ok; };
-BeamMode beam_mode(int V, int WB, bool lm) {
+BeamMode beam_mode(int V, int WB, bool lm, bool bias) {
   BeamMode m{0, 0, 0, false};
   const long long all = (long long)V * WB;
   if (all <= kBeamKeyCache) { m.kc_cap = (int)all; }
   else if (V - 1 >= WB + 3) { m.prefilter = 1; m.kc_cap = kBeamKeyCache; }
-  m.smem = beam_smem_bytes(V, WB, (size_t)m.kc_cap, lm);
-  if (m.smem > kBeamSmemLimit && m.kc_cap) { m.kc_cap = 0; m.smem = beam_smem_bytes(V, WB, 0, lm); }   // no room for the cache
+  m.smem = beam_smem_bytes(V, WB, (size_t)m.kc_cap, lm, bias);
+  if (m.smem > kBeamSmemLimit && m.kc_cap) { m.kc_cap = 0; m.smem = beam_smem_bytes(V, WB, 0, lm, bias); }   // no room for the cache
   m.ok = m.smem <= kBeamSmemLimit;
   return m;
 }
@@ -1065,8 +1137,8 @@ size_t beam_workspace_bytes(const e2e_ctc_desc& d, int beam_width) {
   return (size_t)d.batch * cap * sizeof(BeamNode);
 }
 
-bool beam_supported(const e2e_ctc_desc& d, int beam_width, bool lm) {
-  return beam_width >= 1 && beam_width <= kBeamMaxWidth && beam_mode(d.alphabet, beam_width, lm).ok;
+bool beam_supported(const e2e_ctc_desc& d, int beam_width, bool lm, bool bias) {
+  return beam_width >= 1 && beam_width <= kBeamMaxWidth && beam_mode(d.alphabet, beam_width, lm, bias).ok;
 }
 
 size_t ngram_table_bytes(long long slots) { return (size_t)slots * sizeof(NGramEntry); }
@@ -1086,7 +1158,8 @@ int launch_ngram_build(void* table, long long slots, long long count, const int*
 
 static int launch_beam_impl(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx, double wip, const void* logits,
                             const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs,
-                            int64_t* ties, char* ws, cudaStream_t s, const BeamLMParams* lmp) {
+                            int64_t* ties, char* ws, cudaStream_t s, const BeamLMParams* lmp,
+                            const BeamBiasParams* zp) {
   BeamParams p;
   p.logits = logits; p.dtype = d.dtype; p.sb = d.logits_stride_b; p.st = d.logits_stride_t;
   p.in_len = in_len; p.len_is64 = d.lengths_itype == E2E_I64;
@@ -1100,31 +1173,35 @@ static int launch_beam_impl(const e2e_ctc_desc& d, int beam_width, int n_best, i
   const bool lm = lmp != nullptr;
   BeamLMParams q{};
   if (lm) q = *lmp;
-  const BeamMode md = beam_mode(d.alphabet, beam_width, lm);
+  const bool bias = zp != nullptr;
+  BeamBiasParams z{};
+  if (bias) z = *zp;
+  const BeamMode md = beam_mode(d.alphabet, beam_width, lm, bias);
   static const int no_pref = []() { const char* v = getenv("E2E_CTC_BEAM_NOPREFILTER"); return (v && *v) ? atoi(v) : 0; }();   // tests / experiments
   p.prefilter = no_pref ? 0 : md.prefilter;
   p.kc_cap = (no_pref && md.prefilter) ? 0 : md.kc_cap;
   const bool cache = p.kc_cap > 0;
-  const size_t smem = beam_smem_bytes(d.alphabet, beam_width, (size_t)p.kc_cap, lm);
+  const size_t smem = beam_smem_bytes(d.alphabet, beam_width, (size_t)p.kc_cap, lm, bias);
   int dev = 0, sms = 148;
   E2E_CUDA_TRY(cudaGetDevice(&dev));
   E2E_CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   static const int force_wide = []() { const char* v = getenv("E2E_CTC_BEAM_WIDE"); return (v && *v) ? atoi(v) : -1; }();   // experiments only
   const bool wide = force_wide >= 0 ? force_wide != 0 : d.batch <= sms;
-  KernelTimer timer(lm ? kKernelBeamLM : kKernelBeam, s);
-#define E2E_K8_(TYPE, CACHE_, NT_, LM_)                                                                       \
+  KernelTimer timer(bias ? kKernelBeamBias : lm ? kKernelBeamLM : kKernelBeam, s);
+#define E2E_K8_(TYPE, CACHE_, NT_, LM_, BIAS_)                                                               \
   do {                                                                                                       \
-    E2E_CUDA_TRY(cudaFuncSetAttribute(ctc_beam_kernel<TYPE, CACHE_, NT_, LM_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
-    ctc_beam_kernel<TYPE, CACHE_, NT_, LM_><<<(unsigned)d.batch, NT_, smem, s>>>(p, q);                      \
+    E2E_CUDA_TRY(cudaFuncSetAttribute(ctc_beam_kernel<TYPE, CACHE_, NT_, LM_, BIAS_>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
+    ctc_beam_kernel<TYPE, CACHE_, NT_, LM_, BIAS_><<<(unsigned)d.batch, NT_, smem, s>>>(p, q, z);            \
   } while (0)
-#define E2E_K8L(TYPE, LM_)                                                                                   \
+#define E2E_K8L(TYPE, LM_, BIAS_)                                                                            \
   do {                                                                                                       \
-    if (cache) { if (wide) E2E_K8_(TYPE, true, 512, LM_); else E2E_K8_(TYPE, true, 256, LM_); }              \
-    else { if (wide) E2E_K8_(TYPE, false, 512, LM_); else E2E_K8_(TYPE, false, 256, LM_); }                  \
+    if (cache) { if (wide) E2E_K8_(TYPE, true, 512, LM_, BIAS_); else E2E_K8_(TYPE, true, 256, LM_, BIAS_); } \
+    else { if (wide) E2E_K8_(TYPE, false, 512, LM_, BIAS_); else E2E_K8_(TYPE, false, 256, LM_, BIAS_); }     \
   } while (0)
 #define E2E_K8(TYPE)                                                                                         \
   do {                                                                                                       \
-    if (lm) E2E_K8L(TYPE, true); else E2E_K8L(TYPE, false);                                                  \
+    if (bias) { if (lm) E2E_K8L(TYPE, true, true); else E2E_K8L(TYPE, false, true); }                        \
+    else { if (lm) E2E_K8L(TYPE, true, false); else E2E_K8L(TYPE, false, false); }                           \
   } while (0)
   switch (d.dtype) {
     case E2E_F32: E2E_K8(float); break;
@@ -1154,13 +1231,11 @@ int launch_beam(const e2e_ctc_desc& d, int beam_width, int n_best, int space_idx
                 const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs, int64_t* ties,
                 char* ws, cudaStream_t s) {
   return launch_beam_impl(d, beam_width, n_best, space_idx, wip, logits, in_len, decoded, decoded_len, scores, log_probs,
-                          ties, ws, s, nullptr);
+                          ties, ws, s, nullptr, nullptr);
 }
 
-int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, const e2e_ctc_ngram_tokens* tokens, int beam_width,
-                   int n_best, int space_idx, double wip, double lmwt, double oov_penalty, const void* logits,
-                   const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs,
-                   double* lm_scores, int64_t* oov_words, int64_t* ties, char* ws, cudaStream_t s) {
+static BeamLMParams beam_lm_params(const e2e_ctc_ngram& lm, const e2e_ctc_ngram_tokens* tokens, double lmwt,
+                                   double oov_penalty, double* lm_scores, int64_t* oov_words) {
   BeamLMParams q;
   q.table = reinterpret_cast<const NGramEntry*>(lm.table); q.mask = (unsigned long long)lm.table_slots - 1ull;
   q.lex_child = lm.lex_child; q.lex_word = lm.lex_word;
@@ -1170,8 +1245,30 @@ int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, const e2e_ctc
   q.n_chars = lm.n_chars; q.order = lm.order; q.bos = lm.bos_id; q.eos = lm.eos_id; q.unk = lm.unk_id;
   q.lmwt = lmwt; q.oov_penalty = oov_penalty;
   q.lm_scores = lm_scores; q.oov_words = reinterpret_cast<long long*>(oov_words);
+  return q;
+}
+
+int launch_beam_lm(const e2e_ctc_desc& d, const e2e_ctc_ngram& lm, const e2e_ctc_ngram_tokens* tokens, int beam_width,
+                   int n_best, int space_idx, double wip, double lmwt, double oov_penalty, const void* logits,
+                   const void* in_len, int64_t* decoded, int64_t* decoded_len, double* scores, double* log_probs,
+                   double* lm_scores, int64_t* oov_words, int64_t* ties, char* ws, cudaStream_t s) {
+  const BeamLMParams q = beam_lm_params(lm, tokens, lmwt, oov_penalty, lm_scores, oov_words);
   return launch_beam_impl(d, beam_width, n_best, space_idx, wip, logits, in_len, decoded, decoded_len, scores, log_probs,
-                          ties, ws, s, &q);
+                          ties, ws, s, &q, nullptr);
+}
+
+int launch_beam_bias(const e2e_ctc_desc& d, const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens,
+                     const e2e_ctc_bias& bias, int beam_width, int n_best, int space_idx, double wip, double lmwt,
+                     double oov_penalty, const void* logits, const void* in_len, int64_t* decoded, int64_t* decoded_len,
+                     double* scores, double* log_probs, double* lm_scores, int64_t* oov_words, double* bias_scores,
+                     int64_t* ties, char* ws, cudaStream_t s) {
+  BeamBiasParams z;
+  z.label_col = bias.label_col; z.next = bias.next; z.partial = bias.partial; z.complete = bias.complete;
+  z.n_cols = bias.n_cols; z.bias_scores = bias_scores;
+  BeamLMParams q{};
+  if (lm) q = beam_lm_params(*lm, tokens, lmwt, oov_penalty, lm_scores, oov_words);
+  return launch_beam_impl(d, beam_width, n_best, space_idx, wip, logits, in_len, decoded, decoded_len, scores, log_probs,
+                          ties, ws, s, lm ? &q : nullptr, &z);
 }
 
 }  // namespace e2e

@@ -76,6 +76,8 @@ NBestLMResults = namedtuple("NBestLMResults", ["decoded_targets",
                                                "lm_scores",
                                                "oov_words"])
 
+NBestBiasResults = namedtuple("NBestBiasResults", NBestLMResults._fields + ("bias_scores",))
+
 AlignmentResults = namedtuple("AlignmentResults", ["alignments",
                                                    "token_starts",
                                                    "token_ends",
@@ -153,7 +155,7 @@ class CTCDecoder:
             raise ValueError("the word marker must be None or a non-empty string, got %r" % (marker,))
         self._word_marker = marker
 
-    def decode(self, logits, logits_lengths=None, *, lm=None):
+    def decode(self, logits, logits_lengths=None, *, lm=None, bias=None):
         """Prefix beam search (`<https://arxiv.org/abs/1408.2873>`_), with the word n-gram model ``lm`` fused in if
         given; greedy decoding when ``beam_width == 1`` (decoders/ctc_decoder.py:76-115), where ``lm`` is refused.
 
@@ -165,11 +167,12 @@ class CTCDecoder:
             prefix is empty comes back as the single symbol ``-1`` with length 1 (the reference's behaviour); its
             sentence is ``""``
         :param lm: ``NGramLM`` or ``None``; CPU logits are copied to its device
+        :param bias: ``PhraseBias`` or ``None``: phrases boosted inside the search (``decode_nbest``)
         """
-        if lm is not None:
+        if lm is not None or bias is not None:
             if self._beam_width == 1:
-                raise ValueError("decode with beam_width == 1 is greedy and takes no language model")
-            nb = self.decode_nbest(logits, logits_lengths, n_best=1, lm=lm)
+                raise ValueError("decode with beam_width == 1 is greedy and takes no language model or phrase bias")
+            nb = self.decode_nbest(logits, logits_lengths, n_best=1, lm=lm, bias=bias)
             return DecoderResults(nb.decoded_targets[:, 0], nb.decoded_targets_lengths[:, 0],
                                   [s[0] for s in nb.decoded_sentences])
         if self._beam_width == 1:
@@ -185,7 +188,7 @@ class CTCDecoder:
         decoded_sentences = self._sentences(decoded_targets, decoded_targets_lengths)
         return DecoderResults(decoded_targets, decoded_targets_lengths, decoded_sentences)
 
-    def decode_nbest(self, logits, logits_lengths=None, *, n_best, lm=None):
+    def decode_nbest(self, logits, logits_lengths=None, *, n_best, lm=None, bias=None):
         """The ``n_best`` best prefixes of the LM-free prefix beam search and their scores, for rescoring with a
         language model of the caller's choice.  Always the prefix beam search: with ``beam_width == 1`` that is a
         beam of width 1, not the greedy path ``decode`` takes.
@@ -206,6 +209,13 @@ class CTCDecoder:
             oov_penalty`` ranks the list, ``log_probs`` is acoustic only, ``lm_scores`` [B, N] float64 is the unweighted
             natural-log LM score with the end-of-utterance terms and ``oov_words`` [B, N] int64 counts OOV words.  CPU
             logits are copied to the model's device; logits on another CUDA device raise ``ValueError``
+        :param bias: ``PhraseBias`` or ``None``, with or without ``lm``.  With it the phrases are boosted inside the
+            search (include/e2e_ctc.h, e2e_ctc_bias: completed phrases and partial credit while one is spelled; the
+            partial credit is withdrawn for the final ranking) and the result is ``NBestBiasResults``: the fields of
+            ``NBestLMResults`` plus ``bias_scores`` [B, N] float64, the bonus of the phrases each hypothesis completed,
+            so that ``scores`` is the expression above plus ``bias_scores``.  ``lm_scores`` and ``oov_words`` are 0
+            without ``lm``.  CPU logits are copied to the bias's device; logits, ``lm`` and ``bias`` on different
+            devices raise ``ValueError``
         """
         if self._lm_path:
             raise NotImplementedError(
@@ -215,6 +225,8 @@ class CTCDecoder:
             raise ValueError("n_best %d outside [1, beam_width = %d]" % (int(n_best), self._decoder.beam_width))
         if self._time_major:
             logits = logits.transpose(1, 0)
+        if bias is not None:
+            return self._decode_nbest_bias(logits, logits_lengths, int(n_best), lm, bias)
         if lm is not None:
             return self._decode_nbest_lm(logits, logits_lengths, int(n_best), lm)
         decoded_targets, decoded_targets_lengths, scores, log_probs = self._decoder.decode_nbest(
@@ -233,14 +245,30 @@ class CTCDecoder:
                                                    lmwt=self._lmwt, oov_penalty=self._oov_penalty,
                                                    case_sensitive=self._case_sensitive,
                                                    word_marker=self._word_marker)
-        decoded, lengths, scores, log_probs, lm_scores, oov_words, ties = (t.cpu() for t in out)
-        self._decoder.last_ties = ties
+        return NBestLMResults(*self._nbest_host(*out))
+
+    def _decode_nbest_bias(self, logits, logits_lengths, n_best, lm, bias):
+        if lm is not None and lm.device != bias.device:
+            raise ValueError("the language model on %s, the phrase bias on %s" % (lm.device, bias.device))
+        if not logits.is_cuda:
+            logits = logits.to(bias.device)
+        out = self._decoder.decode_nbest_bias_device(logits, bias, lm, logits_lengths, n_best, not self._after_logsoftmax,
+                                                     lmwt=self._lmwt, oov_penalty=self._oov_penalty,
+                                                     case_sensitive=self._case_sensitive,
+                                                     word_marker=self._word_marker)
+        return NBestBiasResults(*self._nbest_host(*out))
+
+    def _nbest_host(self, decoded, lengths, *fields):
+        """The device results of an N-best search on the host: targets cut to the longest hypothesis, the sentences,
+        the remaining fields; the last one (the tie counters) goes to ``last_ties``."""
+        decoded, lengths, *fields = (t.cpu() for t in (decoded, lengths) + fields)
+        self._decoder.last_ties = fields.pop()
         width = int(lengths.max()) if lengths.numel() else 0
         decoded = decoded[:, :, :width].contiguous()
         B, N = lengths.shape
         flat = self._sentences(decoded.reshape(B * N, -1), lengths.reshape(-1))
         sentences = [flat[b * N:(b + 1) * N] for b in range(B)]
-        return NBestLMResults(decoded, lengths, sentences, scores, log_probs, lm_scores, oov_words)
+        return (decoded, lengths, sentences, *fields)
 
     def score(self, logits, hypotheses, hypotheses_lengths, logits_lengths=None):
         """The CTC log-likelihood ``log p(hypothesis | logits)`` of N transcripts per utterance: minus the CTC loss of each

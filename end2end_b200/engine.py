@@ -767,6 +767,56 @@ class CTCBeamEngine(CTCGreedyEngine):
                     float(lmwt), float(oov_penalty), *outs))
         return decoded, lengths, scores, log_probs, lm_scores, oov_words, ties
 
+    def decode_nbest_bias_device(self, logits, bias, lm=None, logits_lengths=None, n_best=None, from_logits=False,
+                                 lmwt=1.0, oov_penalty=0.0, case_sensitive=True, word_marker=None):
+        """``decode_nbest_device`` (``lm=None``) or ``decode_nbest_lm_device`` with the phrases of ``bias`` (a
+        ``PhraseBias``) boosted inside the search (include/e2e_ctc.h, e2e_ctc_bias), device tensors in (on the bias's
+        device, and the model's), device tensors out (no synchronisation): ``(decoded, lengths, scores, log_probs,
+        lm_scores, oov_words, bias_scores, ties)``.  ``scores`` is the unbiased expression plus ``bias_scores`` [B,N]
+        float64, the bonus of the phrases each hypothesis completed; ``lm_scores`` and ``oov_words`` are 0 without a
+        model.  Raises ``NotImplementedError`` when the beam's state with the bias's does not fit the kernel."""
+        _require_cuda()
+        n_best = self._n_best(n_best)
+        logits = logits.detach()
+        dev = logits.device
+        if dev != bias.device:
+            raise ValueError("logits on %s, the phrase bias on %s" % (dev, bias.device))
+        if lm is not None and dev != lm.device:
+            raise ValueError("logits on %s, the language model on %s" % (dev, lm.device))
+        if not _dense3(logits):
+            logits = logits.contiguous()
+        desc = tokens = None
+        if lm is not None:
+            if word_marker is None and self.space_idx < 0:
+                raise ValueError("a language model needs the label \" \" between words")
+            desc = lm.lexicon(self.labels, self.blank_idx, case_sensitive, word_marker)
+            if word_marker is not None:
+                desc, tokens = desc
+            if len(self.labels) != logits.size(2):
+                raise ValueError("%d labels for an alphabet of %d" % (len(self.labels), logits.size(2)))
+        bd = bias.descriptor(logits.size(2))
+        logits_lengths, d, out = self._nbest_args(logits, logits_lengths, n_best, from_logits, device=dev)
+        decoded, lengths, scores, log_probs, ties = out
+        lm_scores = torch.zeros(d.batch, n_best, dtype=torch.float64, device=dev)
+        oov_words = torch.zeros(d.batch, n_best, dtype=torch.int64, device=dev)
+        bias_scores = torch.empty(d.batch, n_best, dtype=torch.float64, device=dev)
+        ref = lambda x: None if x is None else ctypes.byref(x)   # noqa: E731
+        with _on_device(dev):
+            n = self._L.e2e_ctc_beam_bias_workspace_bytes(ctypes.byref(d), ref(desc), ref(tokens), ctypes.byref(bd),
+                                                          self.beam_width, n_best)
+            if n == 0:
+                msg = self._L.e2e_last_error_string().decode("utf-8", "replace")
+                if "limits" in msg:
+                    raise NotImplementedError(msg)
+                raise ValueError(msg)
+            ws = torch.empty(n, dtype=torch.uint8, device=dev)
+            _lib.check(self._L.e2e_ctc_beam_bias_nbest_device(
+                ctypes.byref(d), self.beam_width, n_best, self.space_idx, self.wip, ref(desc), ref(tokens), float(lmwt),
+                float(oov_penalty), ctypes.byref(bd), _ptr(logits), _ptr(logits_lengths), _ptr(decoded), _ptr(lengths),
+                _ptr(scores), _ptr(log_probs), _ptr(lm_scores), _ptr(oov_words), _ptr(bias_scores), _ptr(ties), _ptr(ws),
+                ws.numel(), _stream(dev)))
+        return decoded, lengths, scores, log_probs, lm_scores, oov_words, bias_scores, ties
+
     def _score_args(self, logits, hyps, hyp_lengths, logits_lengths, from_logits, max_targets=None, noun="scorer"):
         """The checks and the C descriptor shared by the scorer's entry points and ``align_device`` (whose kernel takes
         hypotheses of up to ``max_targets`` labels instead of the build's limit, and which the error messages call the

@@ -1,4 +1,5 @@
-"""Word language models for the GPU prefix beam search."""
+"""Word language models and phrase biasing for the GPU prefix beam search."""
+from .bias import PhraseBias
 from .ngram import NGramLM
 
-__all__ = ["NGramLM"]
+__all__ = ["NGramLM", "PhraseBias"]

@@ -410,6 +410,62 @@ int e2e_ctc_beam_lm_tokens_nbest_device(const e2e_ctc_desc* desc, int32_t beam_w
                                         double* lm_scores, int64_t* oov_words, int64_t* ties, void* workspace,
                                         size_t workspace_bytes, void* cuda_stream);
 
+/* Phrase biasing (contextual biasing, hot words) inside the prefix beam search, with or without a language model.
+ *   phrases: p = (p_1 .. p_k), k >= 1 labels other than the blank, each with a per-token weight w_p > 0 (finite,
+ *       natural-log units); no two phrases are equal.  Phrases match on a prefix's label sequence (its collapsed labels,
+ *       the sequence the trie stores), at label level: a word-piece model's caller passes its tokenizer's segmentation,
+ *       and other segmentations as further phrases;
+ *   committed(y): a left fold over the positions i = 1 .. |y| of out_i, where out_i is the sum, over the phrases that
+ *       are a suffix of y_1 .. y_i taken in ascending phrase index, of w_p * k_p.  Every occurrence counts, overlapping
+ *       ones included;
+ *   phi(y) = d * max{ w_p : y's suffix of length d is a proper prefix of p }, d the length of the longest suffix of y
+ *       that is a proper prefix of some phrase; phi = 0 when d = 0.  A phrase that has just completed earns no partial
+ *       credit of its own, so no bonus is counted twice;
+ *   score during the search: the expression of the search without the bias plus (committed + phi), added last, in
+ *       fp64, without fused multiply-adds: beam_score + (committed + phi) without a model, score_lm + (committed + phi)
+ *       with one.  The bias is a function of the label sequence, so a merge into a living prefix changes nothing;
+ *   final ranking and the returned scores: committed only (partial credit is withdrawn at the end, as the model adds
+ *       </s>); bias_scores = committed, so scores = expression without the bias + bias_scores exactly.
+ * With no phrase ever matched committed + phi = 0: every key and score is that of the unbiased search, bit for bit.
+ *
+ * The caller builds an Aho-Corasick automaton over labels.  Node 0 is the root; a node is a prefix of some phrase.
+ * The labels that occur in some phrase (phrase labels) get columns label_col[c] in [0, n_cols); every other label has
+ * label_col = -1 and moves any node to the root.  For each node:
+ *   next[node][col]: the full transition function (the longest suffix of the node's string extended by the label that
+ *       is a node);
+ *   partial[node]: phi of the node's label string (it depends on that string only);
+ *   complete[node]: out of the node's string: the node's own phrase and those along its dictionary-suffix chain,
+ *       w_p * k_p summed in ascending phrase index.
+ * An extension by label c moves a prefix in node s to n' = next[s][label_col[c]] (or the root) and its bias is
+ * (committed + complete[n']) + partial[n'].  For one member every label in no phrase gives the same bias (its
+ * committed), so within each class the large-alphabet symbol filter ranks only labels in no phrase and extends every
+ * member with every phrase label in addition: the filter stays exact, and its cost grows with the number of distinct
+ * phrase labels. */
+typedef struct e2e_ctc_bias {
+  const int32_t* label_col;   /* [alphabet] device: column of a phrase label, -1 for every other label (and the blank) */
+  const int32_t* next;        /* [nodes][n_cols] device: values in [0, nodes) */
+  const double* partial;      /* [nodes] device */
+  const double* complete;     /* [nodes] device */
+  int32_t nodes, n_cols;      /* nodes >= 1, n_cols >= 0 */
+} e2e_ctc_bias;
+
+/* The N best prefixes of the prefix beam search with phrase biasing.  One entry point for the three searches:
+ *   lm == NULL: the LM-free search of e2e_ctc_beam_nbest_device (space_idx as there; tokens must be NULL; lmwt and
+ *       oov_penalty are ignored; lm_scores and oov_words may be NULL and are not written);
+ *   lm != NULL, tokens == NULL: the character search of e2e_ctc_beam_lm_nbest_device (space_idx required);
+ *   lm != NULL, tokens != NULL: the sub-word search of e2e_ctc_beam_lm_tokens_nbest_device (space_idx ignored).
+ * Results as there, plus bias_scores: [B,N] float64, committed of each returned prefix (slots past the final beam: -inf).
+ * The workspace query returns 0 (E2E_ERR_UNSUPPORTED) when the beam's state with the bias's does not fit shared memory. */
+size_t e2e_ctc_beam_bias_workspace_bytes(const e2e_ctc_desc* desc, const e2e_ctc_ngram* lm,
+                                         const e2e_ctc_ngram_tokens* tokens, const e2e_ctc_bias* bias,
+                                         int32_t beam_width, int32_t n_best);
+int e2e_ctc_beam_bias_nbest_device(const e2e_ctc_desc* desc, int32_t beam_width, int32_t n_best, int32_t space_idx,
+                                   double wip, const e2e_ctc_ngram* lm, const e2e_ctc_ngram_tokens* tokens, double lmwt,
+                                   double oov_penalty, const e2e_ctc_bias* bias, const void* logits,
+                                   const void* logits_lengths, int64_t* decoded, int64_t* decoded_lengths, double* scores,
+                                   double* log_probs, double* lm_scores, int64_t* oov_words, double* bias_scores,
+                                   int64_t* ties, void* workspace, size_t workspace_bytes, void* cuda_stream);
+
 /* ------------------------------------------------------- N hypotheses per utterance: score ---- */
 
 /* The CTC log-likelihood log p(y | x) of n_hyp hypotheses per utterance, forward only (no gradient, nothing kept for a
